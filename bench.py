@@ -10,6 +10,10 @@ batched, on 1/2/4/8 B200 (weak scaling: every GPU convolves its own rows, no col
 One step = one pass of `convolve_signal` (1023-tap raised cosine, SURVEY.md section 8 config C2a-B)
 over ROWS = 64 independent 2^20-point complex f32 vectors per GPU (512 MiB in, 512 MiB out: larger than
 the 126 MB L2, so no L2 flush is needed between iterations).  Rank 0 prints ONE JSON line.
+
+--dump-outputs DIR writes rank 0's results of the last device-resident step and of the last end-to-end step
+as a fixed sample (see output_sample) to DIR/*.npy, float32 (re, im) pairs, 48 MiB in all.  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -55,6 +59,16 @@ def make_rows(rows, seed):
         out[r].real = rng.uniform(-10, 10, N_POINTS).astype(np.float32)
         out[r].imag = rng.uniform(-10, 10, N_POINTS).astype(np.float32)
     return out
+
+
+def output_sample(y):
+    """Fixed sample of a (ROWS, N_POINTS) complex64 result: two whole rows (their edges included) and 2^20 points
+    drawn over all rows, as float32 arrays of (re, im) pairs (16 MiB + 8 MiB)."""
+    rng = np.random.default_rng(20261020)
+    rows = np.sort(rng.choice(ROWS, 2, replace=False))
+    flat = np.sort(rng.integers(0, ROWS * N_POINTS, 1 << 20))
+    return {"rows": y[rows].view(np.float32).reshape(len(rows), N_POINTS, 2),
+            "points": y.reshape(-1)[flat].view(np.float32).reshape(-1, 2)}
 
 
 def peaks():
@@ -195,6 +209,8 @@ def run_gpu(args):
     if not host_in or not host_out:
         raise SystemExit("pinned host allocation failed")
     hin = np.ctypeslib.as_array((ctypes.c_float * (2 * ROWS * N_POINTS)).from_address(host_in))
+    hout = np.ctypeslib.as_array((ctypes.c_float * (2 * ROWS * N_POINTS)).from_address(host_out))
+    dumps = {}
     from basic_dsp_b200.sharding import row_shard
     row0, row1 = row_shard(world * ROWS, world, rank)     # weak scaling: ROWS rows per GPU, contiguous blocks
     assert row1 - row0 == ROWS
@@ -244,6 +260,11 @@ def run_gpu(args):
     total_ms_max = float(t.item())
     samples = world * ROWS * N_POINTS * args.steps
     value = samples / (total_ms_max * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:
+        L.bdsp_memcpy_d2h(host_out, d_out, nbytes)
+        L.bdsp_sync()
+        for k_, a in output_sample(hout.view(np.complex64).reshape(ROWS, N_POINTS)).items():
+            dumps["device_" + k_] = a
 
     # ---- end to end through the C ABI with HOST buffers: upload -> convolve_signal32 -> download, every step --------
     # Rows are pipelined over DEPTH (stream, vector handle) pairs so that the upload of row r+1, the kernel
@@ -287,6 +308,9 @@ def run_gpu(args):
         e2e_step()
     barrier()
     e2e_s = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:
+        for k_, a in output_sample(hout.view(np.complex64).reshape(ROWS, N_POINTS)).items():
+            dumps["e2e_" + k_] = a
     t = torch.tensor([e2e_s], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -321,7 +345,6 @@ def run_gpu(args):
     copy_ceiling_gbs = world * 2.0 * nbytes * 3 / float(t.item()) / 1e9          # aggregate, both directions
     e2e_gbs = e2e_value * 1e6 * 16.0 / 1e9                                       # 8 B up + 8 B down per sample
     # the e2e result of the last row must equal the device-resident result (same kernel, same input)
-    hout = np.ctypeslib.as_array((ctypes.c_float * (2 * ROWS * N_POINTS)).from_address(host_out))
     chk = np.empty(row_floats, dtype=np.float32)
     L.bdsp_memcpy_d2h(chk.ctypes.data, d_out + (ROWS - 1) * row_floats * 4, row_floats * 4)
     L.bdsp_sync()
@@ -380,6 +403,10 @@ def run_gpu(args):
                                               "C port of the reference's overlap_discard incl. scalar head/tail (oracle/ref_port.c)" % (cores, sec)}
         print(json.dumps(line))
         sampler.stop()
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumps.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     barrier()
     L.bdsp_conv_plan_destroy(plan)
     for p in (d_in, d_out, d_h):
@@ -399,7 +426,12 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config measurements (C1 ... C5b) on the N=1 line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last step's results to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":

@@ -1,13 +1,15 @@
 """ctypes loader for oracle/ref_port.c (C port of the reference's CPU convolve_signal path).
 TEST / BASELINE INFRASTRUCTURE ONLY - never imported by basic_dsp_b200."""
 import ctypes
+import hashlib
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_SO = os.path.join(_HERE, "_build", "libref_port.so")
+_BUILD = os.path.join(_HERE, "_build")
 _lib = None
 
 
@@ -16,30 +18,42 @@ def _host_tag():
         with open("/proc/cpuinfo") as fh:
             for line in fh:
                 if line.startswith("flags"):
-                    return str(hash(line) & 0xFFFFFFFF)
+                    return hashlib.sha256(line.encode()).hexdigest()[:16]
     except OSError:
         pass
     return "unknown"
 
 
-def build(force=False):
-    """(Re)builds the port with -march=native; a tag file makes a box with another CPU rebuild it."""
-    src = os.path.join(_HERE, "ref_port.c")
-    tag_file = os.path.join(_HERE, "_build", "host_tag")
-    tag = _host_tag()
-    stale = (not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src)
-             or not os.path.exists(tag_file) or open(tag_file).read() != tag)
-    if force or stale:
-        subprocess.check_call(["make", "-C", _HERE, "-B"], stdout=subprocess.DEVNULL)
-        with open(tag_file, "w") as fh:
-            fh.write(tag)
-    return _SO
+def _current(out):
+    """True when `out` holds a port built from the current source for this host's CPU."""
+    so, tag_file = os.path.join(out, "libref_port.so"), os.path.join(out, "host_tag")
+    if not os.path.exists(so) or not os.path.exists(tag_file):
+        return False
+    if os.path.getmtime(so) < os.path.getmtime(os.path.join(_HERE, "ref_port.c")):
+        return False
+    with open(tag_file) as fh:
+        return fh.read() == _host_tag()
+
+
+def build(force=False, out=_BUILD):
+    """(Re)builds the port with -march=native into `out`; a tag file makes a box with another CPU rebuild it."""
+    if force or not _current(out):
+        subprocess.check_call(["make", "-C", _HERE, "-B", "OUT=" + out], stdout=subprocess.DEVNULL)
+        with open(os.path.join(out, "host_tag"), "w") as fh:
+            fh.write(_host_tag())
+    return os.path.join(out, "libref_port.so")
 
 
 def lib():
+    """Loads the port built in oracle/_build, or, when that build is missing or stale, one built in a temporary
+    directory: the source tree may be read-only."""
     global _lib
     if _lib is None:
-        _lib = ctypes.CDLL(build())
+        if _current(_BUILD):
+            _lib = ctypes.CDLL(os.path.join(_BUILD, "libref_port.so"))
+        else:
+            with tempfile.TemporaryDirectory(prefix="ref_port-") as tmp:
+                _lib = ctypes.CDLL(build(out=tmp))
         P = ctypes.c_void_p
         _lib.ref_convolve_signal_c32.restype = ctypes.c_int
         _lib.ref_convolve_signal_c32.argtypes = [P, ctypes.c_size_t, P, ctypes.c_size_t, P]
