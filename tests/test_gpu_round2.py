@@ -56,10 +56,15 @@ def test_convolve_signal_rows_8192_point_blocks(n, rows, l):
 
 
 @pytest.mark.parametrize("dtype,n,rows,l", [(np.float32, 1 << 16, 3, 4095), (np.float32, 1 << 16, 2, 8191), (np.float32, 1 << 16, 2, 8192),
-                                            (np.float32, 20000, 2, 4096), (np.float64, 1 << 15, 2, 4095), (np.float64, 1 << 15, 2, 4096)])
+                                            (np.float32, 20000, 2, 4096), (np.float64, 1 << 15, 2, 4095), (np.float64, 1 << 15, 2, 4096),
+                                            (np.float32, 20000, 3, 24), (np.float64, 20000, 2, 24), (np.float64, 20000, 3, 1023),
+                                            (np.float64, 20000, 2, 2048), (np.float32, 3000, 4, 1000), (np.float64, 1500, 3, 700),
+                                            (np.float32, 20001, 3, 1023)])
 def test_convolve_signal_rows_tap_counts_at_the_block_limits(dtype, n, rows, l):
     """Impulse responses one short of / exactly at the longest block transform (regression: the 8192-point block step is 0
-    for 8191 taps and must not be divided by)."""
+    for 8191 taps and must not be divided by), and at the other limits of the rows dispatch: <= 24 taps (direct FIR),
+    c64 <= 2048 taps (fused 4096-point blocks), fewer than 4096 points (generic blocks whose loads wrap around the row)
+    and odd row lengths (the unaligned fused 4096-point kernel)."""
     L = bd.lib()
     sfx = "c32" if dtype == np.float32 else "c64"
     rng = np.random.default_rng(n + l + rows)
