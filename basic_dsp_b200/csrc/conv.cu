@@ -101,10 +101,10 @@ template <typename T> size_t ols_max_taps() { return fft_block_max_n<T>() / 2; }
 
 bool ols4096_applicable(size_t N, size_t L, size_t M);
 int ols4096_prepare(const void* Hs, void* Hpos, size_t L, cudaStream_t st);
-int ols4096_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, const void* Hpos, cudaTextureObject_t htex, cudaStream_t st);
+int ols4096_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, cudaTextureObject_t htex, cudaStream_t st);
 bool ols8192_applicable(size_t N, size_t L);
 int ols8192_prepare(const void* Hs, void* Hpos, size_t L, cudaStream_t st);
-int ols8192_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, const void* Hpos, cudaTextureObject_t htex, cudaStream_t st);
+int ols8192_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, cudaTextureObject_t htex, cudaStream_t st);
 long long ols8192_blocks(size_t N, size_t L);
 bool ols64_applicable(size_t N, size_t L, size_t M);
 int ols64_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, const void* Hs, cudaStream_t st);
@@ -186,16 +186,8 @@ void ols_plan_destroy(OlsPlan* p) {
 // Choice between the two fused block lengths where both apply (2 <= L <= 2046).  Measured on B200, 64 x 2^20 points
 // (profiles/r2_ols_block_choice.txt): per POINT the 4096-point kernel is ~20 % faster (four independently phased CTAs per
 // SM against two), so the 8192-point kernel only wins once its better block efficiency (M - L)/M outweighs that.
-#ifndef BDSP_OLS8192_MIN_TAPS
 #define BDSP_OLS8192_MIN_TAPS 1450
-#endif
-#ifndef BDSP_OLS8192_MIN_BLOCKS
 #define BDSP_OLS8192_MIN_BLOCKS 592
-#endif
-static int ols_forced_block() {   // BDSP_OLS_FORCE=4096|8192: measurement override
-    static const int v = [] { const char* e = getenv("BDSP_OLS_FORCE"); return e ? atoi(e) : 0; }();
-    return v;
-}
 
 template <typename T>
 int ols_plan_convolve(const OlsPlan* p, const void* x, void* y, size_t N, size_t batch, int is_real, cudaStream_t st) {
@@ -209,17 +201,15 @@ int ols_plan_convolve(const OlsPlan* p, const void* x, void* y, size_t N, size_t
     if (sizeof(T) == 4 && !is_real && L > 4094 && is_pow2(N) && N >= (1u << 15) && N <= (1u << 24) && p->taps_dev)
         return fft_convolve_full<T>(x, y, p->taps_dev, N, batch, L, 0, p->h_is_real, st);
     if (sizeof(T) == 4 && !is_real) {
-        const int force = ols_forced_block();
         // (ols8192_blocks divides by the block step, which is only positive for applicable lengths)
-        const bool can8 = ols8192_applicable(N, L);
-        const bool want8 = can8 && (force ? force == 8192
-                                          : (L >= BDSP_OLS8192_MIN_TAPS && ols8192_blocks(N, L) * (long long)batch >= BDSP_OLS8192_MIN_BLOCKS));
+        const bool want8 = ols8192_applicable(N, L) && L >= BDSP_OLS8192_MIN_TAPS &&
+                           ols8192_blocks(N, L) * (long long)batch >= BDSP_OLS8192_MIN_BLOCKS;
         if (p->htex2 && want8)
-            return ols8192_convolve(x, y, N, batch, L, reinterpret_cast<const C*>(p->Hs2) + p->M2, p->htex2, st);
+            return ols8192_convolve(x, y, N, batch, L, p->htex2, st);
         if (p->htex && M == 4096 && ols4096_applicable(N, L, M))
-            return ols4096_convolve(x, y, N, batch, L, reinterpret_cast<const C*>(p->Hs) + M, p->htex, st);
+            return ols4096_convolve(x, y, N, batch, L, p->htex, st);
         if (p->htex && M == 8192 && ols8192_applicable(N, L))
-            return ols8192_convolve(x, y, N, batch, L, reinterpret_cast<const C*>(p->Hs) + M, p->htex, st);
+            return ols8192_convolve(x, y, N, batch, L, p->htex, st);
     }
     if (sizeof(T) == 8 && !is_real && ols64_applicable(N, L, M)) return ols64_convolve(x, y, N, batch, L, p->Hs, st);   // fused 4096-point c64 blocks
     const size_t step = M - L + 1;

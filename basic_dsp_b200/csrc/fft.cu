@@ -176,14 +176,9 @@ __device__ __forceinline__ int spad_host_dev(int n) { return n + (n >> 4) + 1; }
 // ------------------------------------------------------------------------------------------
 // single-CTA kernel: nfft sequences of n = 2^log2n points per CTA
 // ------------------------------------------------------------------------------------------
-#ifndef BDSP_TILE_F64_RADIX8
-#define BDSP_TILE_F64_RADIX8 1
-#endif
-#ifndef BDSP_BLOCK_POINTS
 #define BDSP_BLOCK_POINTS 1024
-#endif
 template <typename T, bool INV, bool REAL_IN, bool MAG>
-__global__ void __launch_bounds__(sizeof(T) == 4 ? 1024 : 1024, 1) fft_block_kernel(const void* __restrict__ in_, void* __restrict__ out_, int log2n, int nfft,
+__global__ void __launch_bounds__(1024, 1) fft_block_kernel(const void* __restrict__ in_, void* __restrict__ out_, int log2n, int nfft,
                                  long long batch, long long in_rot, T scale, OutMap om,
                                  const typename CpxOf<T>::type* __restrict__ tw, InMul im) {
     typedef typename CpxOf<T>::type C;
@@ -222,7 +217,7 @@ __global__ void __launch_bounds__(sizeof(T) == 4 ? 1024 : 1024, 1) fft_block_ker
         }
     }
     __syncthreads();
-    if constexpr (sizeof(T) == 8 && BDSP_TILE_F64_RADIX8) {
+    if constexpr (sizeof(T) == 8) {
         // f64: radix-8 stages, 8 points per thread (see fft_tile_kernel)
         int Ns = 1, rem = log2n;
         while (rem >= 3) { stockham_stage_strided<T, 8, INV, 1>(s, n, nfft, n, Ns, tw); Ns <<= 3; rem -= 3; }
@@ -268,7 +263,7 @@ struct TileParams {
 };
 
 template <typename T, bool INV>
-__global__ void __launch_bounds__(sizeof(T) == 4 ? 1024 : 512, (sizeof(T) == 8 && BDSP_TILE_F64_RADIX8) ? 2 : 1) fft_tile_kernel(TileParams p, T scale, const typename CpxOf<T>::type* __restrict__ tw) {
+__global__ void __launch_bounds__(sizeof(T) == 4 ? 1024 : 512, sizeof(T) == 8 ? 2 : 1) fft_tile_kernel(TileParams p, T scale, const typename CpxOf<T>::type* __restrict__ tw) {
     typedef typename CpxOf<T>::type C;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     C* s = reinterpret_cast<C*>(smem_raw);
@@ -367,7 +362,7 @@ __global__ void __launch_bounds__(sizeof(T) == 4 ? 1024 : 512, (sizeof(T) == 8 &
         const int n = m;
         int Ns = 1, rem = p.log2m;
         // same stage sequence as block_fft, but with the padded sequence stride
-        if constexpr (sizeof(T) == 8 && BDSP_TILE_F64_RADIX8) {
+        if constexpr (sizeof(T) == 8) {
             // f64: radix-8 stages, 8 points per thread (half the registers of radix 16 -> twice the resident warps;
             // 2^9 = 8*8*8 needs the same three stages as 16*16*2)
             while (rem >= 3) { stockham_stage_strided<T, 8, INV, 1>(s, n, ct * Q, sstride, Ns, tw); Ns <<= 3; rem -= 3; }
@@ -429,9 +424,6 @@ __global__ void __launch_bounds__(sizeof(T) == 4 ? 1024 : 512, (sizeof(T) == 8 &
     }
 }
 
-#ifndef BDSP_F64_TILE_KERNELS
-#define BDSP_F64_TILE_KERNELS 1
-#endif
 #include "fft64t.cuh"   // namespace bdsp::f64t
 
 // ------------------------------------------------------------------------------------------
@@ -588,7 +580,7 @@ template <typename T, bool INV>
 int launch_block(const void* in, void* out, size_t n, size_t batch, bool real_in, bool mag, long long in_rot,
                  T scale, const OutMap& om, cudaStream_t st, const InMul& im = InMul()) {
     typedef typename CpxOf<T>::type C;
-    if constexpr (sizeof(T) == 8 && BDSP_F64_TILE_KERNELS) {
+    if constexpr (sizeof(T) == 8) {
         // c64 rows of 1024 / 2048 / 4096 points: the 8-points-per-thread row kernel of fft64t.cuh
         // (in place only with the plain row layout: a row's loads all precede its stores, rows do not overlap)
         if (n >= 1024 && n <= 4096 && (in != out || (om.seq_group == 1 && om.oes == 1 && om.group_stride == (long long)n && !real_in && !mag))) {
@@ -604,7 +596,7 @@ int launch_block(const void* in, void* out, size_t n, size_t batch, bool real_in
     if (nfft < 1) nfft = 1;
     if ((size_t)nfft > batch) nfft = (int)batch;
     int threads = block_fft_threads((int)n, nfft);
-    if (sizeof(T) == 8 && BDSP_TILE_F64_RADIX8) { threads = ((int)n * nfft / 8 + 31) / 32 * 32; if (threads < 32) threads = 32; }
+    if (sizeof(T) == 8) { threads = ((int)n * nfft / 8 + 31) / 32 * 32; if (threads < 32) threads = 32; }
     const size_t smem = spad_host(n * nfft) * sizeof(C);
     const long long grid = ((long long)batch + nfft - 1) / nfft;
     const C* tw = twiddle_table<T>();
@@ -628,7 +620,7 @@ int launch_block(const void* in, void* out, size_t n, size_t batch, bool real_in
 template <typename T, bool INV>
 int launch_tile(const TileParams& p, long long batch, T scale, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
-    if constexpr (sizeof(T) == 8 && BDSP_F64_TILE_KERNELS) {
+    if constexpr (sizeof(T) == 8) {
         // c64: compile-time specialised passes for m = 64 .. 512 (fft64t.cuh); anything else runs the generic tile kernel
         const double2* twt = twiddle_table<double>();
         if (!twt) return -1001;
@@ -638,7 +630,7 @@ int launch_tile(const TileParams& p, long long batch, T scale, cudaStream_t st) 
     const int m = 1 << p.log2m;
     const size_t smem = (spad_host((size_t)(m + 16) * p.ct * p.q) + (size_t)p.ct * (33 + (((p.q * m + 31) >> 5) | 1)) + (p.q > 1 ? 32 : 0)) * sizeof(C);
     int threads = block_fft_threads(m, p.ct * p.q);
-    if (sizeof(T) == 8 && BDSP_TILE_F64_RADIX8) { threads = (m * p.ct * p.q / 8 + 31) / 32 * 32; if (threads < 32) threads = 32; }
+    if (sizeof(T) == 8) { threads = (m * p.ct * p.q / 8 + 31) / 32 * 32; if (threads < 32) threads = 32; }
     if (threads > (sizeof(T) == 4 ? 1024 : 512)) { set_last_error("fft tile: %d threads", threads); return -2; }
     const long long grid = batch * p.o1_count * (p.lanes / p.ct);
     int rc = set_smem(fft_tile_kernel<T, INV>, smem);
@@ -654,9 +646,7 @@ template <typename T> int tile_log2m_max() { return sizeof(T) == 4 ? 10 : 9; }
 // lanes per tile: 128 contiguous bytes per row segment (f32: 16, f64: 8) -> 72 KB tiles, 3 CTAs per SM
 // lanes per f64 tile: 4 (64-byte row segments, twice the CTAs) measured mixed on B200: C5a 8.83 -> 8.51 ms, 2^18 0.80 -> 0.73 ms,
 // but 2^14 0.82 -> 0.88 and 2^20 1.20 -> 1.31 ms per 2^25 points; 8 stays the default
-#ifndef BDSP_TILE_LANES_F64
 #define BDSP_TILE_LANES_F64 8
-#endif
 template <typename T> long long tile_lanes() { return sizeof(T) == 8 ? BDSP_TILE_LANES_F64 : 8; }
 
 // power-of-two transform of `batch` sequences; handles any supported size

@@ -15,18 +15,10 @@
 //     m-point transforms, results K = ka + 3 kb (time_freq/mod.rs:32-63: rustfft plans any length; BASELINE C5a).
 #pragma once
 
-#ifndef F64T_MIN_CTAS
 #define F64T_MIN_CTAS 4
-#endif
-#ifndef F64T_Q3_LCT
 #define F64T_Q3_LCT 2   // lanes (log2) per tile of the radix-3 first pass: 3 x 256 x 4 points, 384 threads
-#endif
-#ifndef F64T_Q3_MIN_CTAS
 #define F64T_Q3_MIN_CTAS 2
-#endif
-#ifndef F64T_POINTS_LOG2
 #define F64T_POINTS_LOG2 11
-#endif
 namespace f64t {
 
 __device__ __forceinline__ double2 conj_if(double2 w, bool c) { return c ? make_double2(w.x, -w.y) : w; }

@@ -110,8 +110,6 @@ int fftc_try(const void* in, void* out, size_t n, size_t rows, bool inverse, siz
     if (n != 65536 || rows == 0 || rows > 8 || in == out) return 1;
     if ((in_rot != 0 && in_rot != n / 2) || (out_rot != 0 && out_rot != n / 2)) return 1;
     if ((reinterpret_cast<uintptr_t>(in) & 7) || (reinterpret_cast<uintptr_t>(out) & 7)) return 1;
-    static const bool off = [] { const char* e = getenv("BDSP_FFTC"); return e && e[0] == '0'; }();
-    if (off) return 1;
     auto kf = fftc65536_kernel<false>;
     auto ki = fftc65536_kernel<true>;
     // per-device configuration; a device / driver that cannot place a 16-CTA cluster takes the two-pass path

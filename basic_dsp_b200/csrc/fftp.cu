@@ -11,28 +11,22 @@
 //   ROWS      last pass of a multi-pass transform: four adjacent 4096-point rows per CTA, transposing store
 //   TQ = Q    last pass with 16/Q adjacent rows of 256*Q points per CTA (128 threads), transposing store
 //   RIN       the input holds real scalars
-//   CL = 2    (measured, not default) two CTAs per sequence, as a thread-block cluster with distributed shared memory or,
-//             with FP_DUP, as two independent CTAs that each repeat F0
 // fftp_col16_kernel / fftp_col256_kernel: first pass(es) of the multi-pass transforms: 16- / 256-point (NH = 2: 32- / 512-point)
 //   columns of 16 adjacent columns per CTA, inter-pass twiddle evaluated with sincospif on exact arguments.
 // Dispatchers: fftp_try (single pass), fftp_try_real, fftp_two_pass_try (2^15..2^20), fftp_three_pass_try (2^21..2^24),
 //   fftp_rows1k_try (packed last pass behind a generic column pass).
 // Replaces rustfft for these lengths (vector/src/vector_types/time_freq/mod.rs:45-58) incl. the fused
 // fft_shift (time_to_freq.rs:163), ifft's scale + ifft_shift (freq_to_time.rs:165-167) and magnitude.
-#include <cooperative_groups.h>
-
 #include <map>
 #include <mutex>
 #include <vector>
 
 #include "fftp.cuh"
 
-namespace cg = cooperative_groups;
-
 namespace bdsp {
 using namespace ols16;
 
-// ROWS = true (R0 = 4, CL = 1): the CTA transforms FOUR independent, adjacent 4096-point rows (no F0) and
+// ROWS = true (R0 = 4): the CTA transforms FOUR independent, adjacent 4096-point rows (no F0) and
 // writes result k of row r to out[(r0 + r) + n1 * k]: the transposing last pass of a two-pass transform of
 // n1 * 4096 points, with the four rows providing the contiguous 32 bytes of every store sector.
 // TQ = Q in {2, 4} (with ROWS, R0 = 1): the CTA's 4096 points are 16/Q adjacent rows of 256*Q points (k0 = (16/Q)*q + row):
@@ -46,30 +40,11 @@ using namespace ols16;
 // NATQ = Q in {1, 2, 4, 8} (R0 = 1, no ROWS): the CTA's 4096 contiguous points are 16/Q independent rows of 256*Q points
 // (k0 = q + Q*row); the first stage is a radix-Q butterfly inside every row, results are stored in natural order.
 // Batched 512 / 1024 / 2048-point transforms with the structure of the 4096-point kernel.
-template <int R0, int CL, bool INV, bool SHIFT_IN, bool SHIFT_OUT, bool MAG, bool ROWS, int TQ = 0, int NATQ = 0, bool RIN = false, int SQ = 0>
-// FP_PREFETCH=1: persistent CTAs + register prefetch of the next row.  Measured on B200 (C3): 0.336 ms vs
-// 0.275 ms without (register pressure -> spills; the extra barrier), so it is off by default.
-#ifndef FP_PREFETCH
-#define FP_PREFETCH 0
-#endif
-#ifndef FP_MINB256
-#define FP_MINB256 2
-#endif
-#ifndef FP_DUP
-#define FP_DUP 1
-#endif
-// result stores: FP_STREAM_STORES=1 uses st.global.cs (evict-first) for the write-once output (measured: no difference)
-#ifndef FP_STREAM_STORES
-#define FP_STREAM_STORES 0
-#endif
-#if FP_STREAM_STORES
-#define FP_ST(p, v) __stcs((p), (v))
-#else
-#define FP_ST(p, v) (*(p) = (v))
-#endif
-__global__ void __launch_bounds__(128 * (R0 / CL), (R0 / CL) == 2 ? FP_MINB256 : 4 / (R0 / CL))
+#define FP_MINB256 2   // CTAs per SM for the 256-thread 8192-point kernel
+template <int R0, bool INV, bool SHIFT_IN, bool SHIFT_OUT, bool MAG, bool ROWS, int TQ = 0, int NATQ = 0, bool RIN = false, int SQ = 0>
+__global__ void __launch_bounds__(128 * R0, R0 == 2 ? FP_MINB256 : 4 / R0)
 fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long rows, float scale, const float* __restrict__ tw, int n1, int n2c) {
-    constexpr int NSB = R0 / CL;          // sub-blocks (4096-point transforms) owned by this CTA
+    constexpr int NSB = R0;               // sub-blocks (4096-point transforms) owned by this CTA
     constexpr int NT = 128 * NSB;         // threads
     constexpr int N = 4096 * R0;
     constexpr int FP_B = FP_B_OF(NSB);
@@ -77,32 +52,9 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
     float* sre = smem;
     float* sim = smem + NSB * FP_B;
     const int t = threadIdx.x;
-    const int rank = CL > 1 ? (int)(blockIdx.x % CL) : 0;
-    // CL == 1: persistent CTAs walk the rows and prefetch the next row's inputs (registers) while the
-    // last stage of the current row runs, so that the HBM latency of the load phase is hidden even with
-    // one CTA per SM.  CL == 2: one cluster per row.
-    constexpr bool PREFETCH = FP_PREFETCH && (CL == 1 && R0 > 1);
-    // CL > 1 without a cluster (FP_DUP): the CL CTAs of a row each run the first stage over ALL columns (the second
-    // reader is served by L2) and keep only their own NSB sub-blocks: no distributed shared memory, no cluster barrier,
-    // and CL smaller CTAs per row that overlap their phases on the SM.  Measured on B200 (C3): one CTA 0.278 ms, two CTAs
-    // 0.293 ms, four CTAs (four reads of the row through L2) 0.461 ms.
-    constexpr bool DUP = FP_DUP && CL > 1;
-    constexpr int NU = R0 > 1 ? (2048 / (DUP ? 1 : CL)) / NT : 1;   // column pairs per thread in F0
-    float4 raw[PREFETCH ? NU * R0 : 1];
-    const long long row_step = gridDim.x / CL;
-    long long row = blockIdx.x / CL;
-    if constexpr (PREFETCH) {
-        if (row < rows) {
-            const float2* xr0 = x + (size_t)row * (size_t)N;
-#pragma unroll
-            for (int u = 0; u < NU; u++)
-#pragma unroll
-                for (int n3 = 0; n3 < R0; n3++) {
-                    const int src = SHIFT_IN ? ((n3 + R0 / 2) % R0) : n3;
-                    raw[u * R0 + n3] = __ldg(reinterpret_cast<const float4*>(xr0 + 2 * (t + NT * u) + 4096 * src));
-                }
-        }
-    }
+    constexpr int NU = R0 > 1 ? 2048 / NT : 1;   // column pairs per thread in F0
+    const long long row_step = gridDim.x;
+    long long row = blockIdx.x;
     for (; row < rows; row += row_step) {
     // ROWS: `row` counts groups of NSB rows; groups_per_seq = n1 / NSB
     constexpr bool R1K = TQ > 0;
@@ -132,33 +84,16 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
     cp v[16];
     // ------------------------------------------------------------------ F0: radix-R0 over stride 4096
     if constexpr (R0 > 1 && !ROWS) {
-        float* rre[CL];
-        float* rim[CL];
-        if constexpr (CL > 1 && !DUP) {
-            cg::cluster_group cluster = cg::this_cluster();
-#pragma unroll
-            for (int o = 0; o < CL; o++) {
-                rre[o] = cluster.map_shared_rank(sre, o);
-                rim[o] = cluster.map_shared_rank(sim, o);
-            }
-            cluster.sync();   // the partner CTA is resident (and done with its previous row) before anyone writes into its shared memory
-        } else {
-            rre[0] = sre; rim[0] = sim;
-        }
         const float* tw0 = tw + 1024 + (R0 == 4 ? 8192 : 0);
 #pragma unroll
         for (int u = 0; u < NU; u++) {
-            const int pi = (DUP ? 0 : rank * (2048 / CL)) + t + NT * u;     // column pair index, c = 2*pi
+            const int pi = t + NT * u;     // column pair index, c = 2*pi
             const int c = 2 * pi;
             cp a[R0];
 #pragma unroll
             for (int n3 = 0; n3 < R0; n3++) {
-                float4 ab;
-                if constexpr (PREFETCH) ab = raw[u * R0 + n3];
-                else {
-                    const int src = SHIFT_IN ? ((n3 + R0 / 2) % R0) : n3;
-                    ab = ldpair(xr + c + 4096 * src);
-                }
+                const int src = SHIFT_IN ? ((n3 + R0 / 2) % R0) : n3;
+                const float4 ab = ldpair(xr + c + 4096 * src);
                 a[n3].re = make_float2(ab.x, ab.z);
                 a[n3].im = make_float2(ab.y, ab.w);
             }
@@ -178,20 +113,11 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
             const int off = 272 * prow + 16 * g + ((j + 4 * fp_rot(prow, g)) & 15);
 #pragma unroll
             for (int k = 0; k < R0; k++) {
-                const int owner = k / NSB, lsb = k % NSB;
-                if (DUP) {
-                    if (owner == rank) {
-                        *reinterpret_cast<float2*>(sre + lsb * FP_B + off) = a[k].re;
-                        *reinterpret_cast<float2*>(sim + lsb * FP_B + off) = a[k].im;
-                    }
-                } else {
-                    *reinterpret_cast<float2*>(rre[owner] + lsb * FP_B + off) = a[k].re;
-                    *reinterpret_cast<float2*>(rim[owner] + lsb * FP_B + off) = a[k].im;
-                }
+                *reinterpret_cast<float2*>(sre + k * FP_B + off) = a[k].re;
+                *reinterpret_cast<float2*>(sim + k * FP_B + off) = a[k].im;
             }
         }
-        if constexpr (CL > 1 && !DUP) cg::this_cluster().sync();
-        else __syncthreads();
+        __syncthreads();
     }
     // ------------------------------------------------------------------ F1: stride 256 inside every sub-block
     const int sb = t >> 7, tt = t & 127;
@@ -390,19 +316,6 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
         }
     }
     __syncthreads();
-    if constexpr (PREFETCH) {
-        const long long nrow = row + row_step;
-        if (nrow < rows) {
-            const float2* xn = x + (size_t)nrow * (size_t)N;
-#pragma unroll
-            for (int u = 0; u < NU; u++)
-#pragma unroll
-                for (int n3 = 0; n3 < R0; n3++) {
-                    const int src = SHIFT_IN ? ((n3 + R0 / 2) % R0) : n3;
-                    raw[u * R0 + n3] = __ldg(reinterpret_cast<const float4*>(xn + 2 * (t + NT * u) + 4096 * src));
-                }
-        }
-    }
     // ------------------------------------------------------------------ F3: 16 contiguous points -> global
 #pragma unroll 1
     for (int half = 0; half < 2; half++) {
@@ -429,7 +342,7 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
             P[2 * q].im = make_float2(fi.x, fi.y); P[2 * q + 1].im = make_float2(fi.z, fi.w);
         }
         fft16_dif<INV>(P);
-        // slot j holds k2 = bitrev4(j); k = (rank*NSB + lsb) + R0*(k0 + 16*k1 + 256*k2)
+        // slot j holds k2 = bitrev4(j); k = lsb + R0*(k0 + 16*k1 + 256*k2)
         // (ROWS: k = (NSB*grp + lsb) + n1*(k0 + 16*k1 + 256*k2))
         // (TQ: row = k0 % RPC, k = (RPC*grp + row) + n1*((k0 / RPC) + Q*(k1 + 16*k2)))
         const size_t kst = ROWS ? (size_t)n1 * (size_t)n2c : (size_t)R0;
@@ -439,7 +352,7 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
         const size_t klow = SQ ? (size_t)((k0 * (16 / (SQ ? SQ : 1)) + k1 / (SQ ? SQ : 1)) * (16 * SQ) + (k1 % (SQ ? SQ : 1)))
                             : NATQ ? (size_t)((k0 / (NATQ ? NATQ : 1)) * (256 * NATQ) + (k0 % (NATQ ? NATQ : 1)) + NATQ * k1)
                             : R1K ? kbase + (size_t)(RPC * grp + (k0 % RPC)) + kst * (size_t)((k0 / RPC) + TQ * k1)
-                                : kbase + (ROWS ? (size_t)(NSB * grp + lsb) : (size_t)(rank * NSB + lsb)) + kst * (size_t)(k0 + 16 * k1);
+                                : kbase + (ROWS ? (size_t)(NSB * grp + lsb) : (size_t)lsb) + kst * (size_t)(k0 + 16 * k1);
         const size_t k2s = SQ ? (size_t)SQ : NATQ ? (size_t)(16 * NATQ) : R1K ? (size_t)(16 * TQ) * kst : (size_t)256 * kst;
         if constexpr (MAG) {
             float* o = reinterpret_cast<float*>(out_) + seq * seq_len + klow;
@@ -447,16 +360,16 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
             for (int m = 0; m < 8; m++) {
                 pk m2 = pfma(P[m].re, P[m].re, pmul(P[m].im, P[m].im));
                 const int ka = bitrev4(2 * m) ^ (SHIFT_OUT ? 8 : 0), kb = bitrev4(2 * m + 1) ^ (SHIFT_OUT ? 8 : 0);
-                FP_ST(o + k2s * ka, sqrtf(m2.x) * scale);
-                FP_ST(o + k2s * kb, sqrtf(m2.y) * scale);
+                o[k2s * ka] = sqrtf(m2.x) * scale;
+                o[k2s * kb] = sqrtf(m2.y) * scale;
             }
         } else {
             float2* o = reinterpret_cast<float2*>(out_) + seq * seq_len + klow;
 #pragma unroll
             for (int m = 0; m < 8; m++) {
                 const int ka = bitrev4(2 * m) ^ (SHIFT_OUT ? 8 : 0), kb = bitrev4(2 * m + 1) ^ (SHIFT_OUT ? 8 : 0);
-                FP_ST(o + k2s * ka, make_float2(P[m].re.x * scale, P[m].im.x * scale));
-                FP_ST(o + k2s * kb, make_float2(P[m].re.y * scale, P[m].im.y * scale));
+                o[k2s * ka] = make_float2(P[m].re.x * scale, P[m].im.x * scale);
+                o[k2s * kb] = make_float2(P[m].re.y * scale, P[m].im.y * scale);
             }
         }
     }
@@ -735,11 +648,10 @@ const float* fftp_twiddles() {
 
 namespace {
 
-template <int R0, int CL, bool INV, bool SI, bool SO, bool MAG, bool ROWS = false, int TQ = 0, int NATQ = 0, bool RIN = false, int SQ = 0>
+template <int R0, bool INV, bool SI, bool SO, bool MAG, bool ROWS = false, int TQ = 0, int NATQ = 0, bool RIN = false, int SQ = 0>
 int fftp_launch(const void* in, void* out, size_t rows, float scale, cudaStream_t st, int n1 = 1, int n2c = 1) {
-    constexpr int NSB = R0 / CL;
-    const size_t smem = (size_t)2 * NSB * FP_B_OF(NSB) * sizeof(float);
-    auto kern = fftp_kernel<R0, CL, INV, SI, SO, MAG, ROWS, TQ, NATQ, RIN, SQ>;
+    const size_t smem = (size_t)2 * R0 * FP_B_OF(R0) * sizeof(float);
+    auto kern = fftp_kernel<R0, INV, SI, SO, MAG, ROWS, TQ, NATQ, RIN, SQ>;
     static PerDeviceOnce configured;   // per instantiation and device
     if (configured.need()) {
         BDSP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -747,26 +659,8 @@ int fftp_launch(const void* in, void* out, size_t rows, float scale, cudaStream_
     }
     const float* tw = fftp_twiddles();
     if (!tw) return -1001;
-    cudaLaunchConfig_t cfg = {};
-    // CL == 1 and n >= 8192: persistent CTAs (one per SM, 139/70 KB of shared memory each)
-    size_t ctas = rows * CL;
-    if (FP_PREFETCH && CL == 1 && R0 > 1) {
-        const size_t per_sm = R0 == 4 ? 1 : 2;
-        const size_t cap = (size_t)sm_count() * per_sm;
-        if (ctas > cap) ctas = cap;
-    }
-    cfg.gridDim = dim3((unsigned)ctas);
-    cfg.blockDim = dim3(128 * NSB);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CL;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = (CL > 1 && !FP_DUP) ? 1 : 0;
-    BDSP_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, reinterpret_cast<const float2*>(in), out, (long long)rows, scale, tw, n1, n2c));
+    kern<<<(unsigned)rows, 128 * R0, smem, st>>>(reinterpret_cast<const float2*>(in), out, (long long)rows, scale, tw, n1, n2c);
+    BDSP_CUDA_OK(cudaGetLastError());
     BDSP_LAUNCHED();
     return 0;
 }
@@ -774,55 +668,52 @@ int fftp_launch(const void* in, void* out, size_t rows, float scale, cudaStream_
 template <int Q>
 int fftp_dispatch_nat(const void* in, void* out, size_t groups, bool inv, bool shift_in, bool shift_out, bool mag, float scale, cudaStream_t st) {
     if (!inv) {
-        if (mag) return shift_out ? fftp_launch<1, 1, false, false, true, true, false, 0, Q>(in, out, groups, scale, st)
-                                  : fftp_launch<1, 1, false, false, false, true, false, 0, Q>(in, out, groups, scale, st);
-        return shift_out ? fftp_launch<1, 1, false, false, true, false, false, 0, Q>(in, out, groups, scale, st)
-                         : fftp_launch<1, 1, false, false, false, false, false, 0, Q>(in, out, groups, scale, st);
+        if (mag) return shift_out ? fftp_launch<1, false, false, true, true, false, 0, Q>(in, out, groups, scale, st)
+                                  : fftp_launch<1, false, false, false, true, false, 0, Q>(in, out, groups, scale, st);
+        return shift_out ? fftp_launch<1, false, false, true, false, false, 0, Q>(in, out, groups, scale, st)
+                         : fftp_launch<1, false, false, false, false, false, 0, Q>(in, out, groups, scale, st);
     }
     if (mag || shift_out) return 1;
-    return shift_in ? fftp_launch<1, 1, true, true, false, false, false, 0, Q>(in, out, groups, scale, st)
-                    : fftp_launch<1, 1, true, false, false, false, false, 0, Q>(in, out, groups, scale, st);
+    return shift_in ? fftp_launch<1, true, true, false, false, false, 0, Q>(in, out, groups, scale, st)
+                    : fftp_launch<1, true, false, false, false, false, 0, Q>(in, out, groups, scale, st);
 }
 
 // rows of 64 / 128 points (fftp_kernel<SQ>): whole groups of 4096 points
 template <int P>
 int fftp_dispatch_short(const void* in, void* out, size_t groups, bool inv, bool shift_in, bool shift_out, bool mag, float scale, cudaStream_t st) {
     if (!inv) {
-        if (mag) return shift_out ? fftp_launch<1, 1, false, false, true, true, false, 0, 1, false, P>(in, out, groups, scale, st)
-                                  : fftp_launch<1, 1, false, false, false, true, false, 0, 1, false, P>(in, out, groups, scale, st);
-        return shift_out ? fftp_launch<1, 1, false, false, true, false, false, 0, 1, false, P>(in, out, groups, scale, st)
-                         : fftp_launch<1, 1, false, false, false, false, false, 0, 1, false, P>(in, out, groups, scale, st);
+        if (mag) return shift_out ? fftp_launch<1, false, false, true, true, false, 0, 1, false, P>(in, out, groups, scale, st)
+                                  : fftp_launch<1, false, false, false, true, false, 0, 1, false, P>(in, out, groups, scale, st);
+        return shift_out ? fftp_launch<1, false, false, true, false, false, 0, 1, false, P>(in, out, groups, scale, st)
+                         : fftp_launch<1, false, false, false, false, false, 0, 1, false, P>(in, out, groups, scale, st);
     }
     if (mag || shift_out) return 1;
-    return shift_in ? fftp_launch<1, 1, true, true, false, false, false, 0, 1, false, P>(in, out, groups, scale, st)
-                    : fftp_launch<1, 1, true, false, false, false, false, 0, 1, false, P>(in, out, groups, scale, st);
+    return shift_in ? fftp_launch<1, true, true, false, false, false, 0, 1, false, P>(in, out, groups, scale, st)
+                    : fftp_launch<1, true, false, false, false, false, 0, 1, false, P>(in, out, groups, scale, st);
 }
 
-template <int R0, int CL>
+template <int R0>
 int fftp_dispatch(const void* in, void* out, size_t rows, bool inv, bool shift_in, bool shift_out, bool mag, float scale,
                   cudaStream_t st) {
     if (!inv) {
-        if (mag) return shift_out ? fftp_launch<R0, CL, false, false, true, true>(in, out, rows, scale, st)
-                                  : fftp_launch<R0, CL, false, false, false, true>(in, out, rows, scale, st);
-        return shift_out ? fftp_launch<R0, CL, false, false, true, false>(in, out, rows, scale, st)
-                         : fftp_launch<R0, CL, false, false, false, false>(in, out, rows, scale, st);
+        if (mag) return shift_out ? fftp_launch<R0, false, false, true, true>(in, out, rows, scale, st)
+                                  : fftp_launch<R0, false, false, false, true>(in, out, rows, scale, st);
+        return shift_out ? fftp_launch<R0, false, false, true, false>(in, out, rows, scale, st)
+                         : fftp_launch<R0, false, false, false, false>(in, out, rows, scale, st);
     }
     if (mag || shift_out) return 1;   // not instantiated: caller falls back to the generic kernel
-    return shift_in ? fftp_launch<R0, CL, true, true, false, false>(in, out, rows, scale, st)
-                    : fftp_launch<R0, CL, true, false, false, false>(in, out, rows, scale, st);
+    return shift_in ? fftp_launch<R0, true, true, false, false>(in, out, rows, scale, st)
+                    : fftp_launch<R0, true, false, false, false>(in, out, rows, scale, st);
 }
 
 
-#ifndef FP_ROWS_DEFAULT
-#define FP_ROWS_DEFAULT 4
-#endif
-template <int NR>
+// last pass over 4096-point rows, four adjacent rows per 512-thread CTA
 int fftp_rows_pass(const void* tmp, void* out, size_t groups, bool inverse, bool so, bool magnitude, float sc, cudaStream_t st, int n1) {
-    if (inverse) return fftp_launch<NR, 1, true, false, false, false, true>(tmp, out, groups, sc, st, n1);
-    if (magnitude) return so ? fftp_launch<NR, 1, false, false, true, true, true>(tmp, out, groups, sc, st, n1)
-                             : fftp_launch<NR, 1, false, false, false, true, true>(tmp, out, groups, sc, st, n1);
-    return so ? fftp_launch<NR, 1, false, false, true, false, true>(tmp, out, groups, sc, st, n1)
-              : fftp_launch<NR, 1, false, false, false, false, true>(tmp, out, groups, sc, st, n1);
+    if (inverse) return fftp_launch<4, true, false, false, false, true>(tmp, out, groups, sc, st, n1);
+    if (magnitude) return so ? fftp_launch<4, false, false, true, true, true>(tmp, out, groups, sc, st, n1)
+                             : fftp_launch<4, false, false, false, true, true>(tmp, out, groups, sc, st, n1);
+    return so ? fftp_launch<4, false, false, true, false, true>(tmp, out, groups, sc, st, n1)
+              : fftp_launch<4, false, false, false, false, true>(tmp, out, groups, sc, st, n1);
 }
 
 template <bool INV, bool SI, bool RIN = false>
@@ -856,11 +747,11 @@ int fftp_colpass(const void* in, void* tmp, int n1, int log2n2, size_t rows, cud
 template <int Q>
 int fftp_rowsq_pass(const void* tmp, void* out, size_t groups, bool inverse, bool so, bool magnitude, float sc, cudaStream_t st, int n1,
                     int n2c = 1) {
-    if (inverse) return fftp_launch<1, 1, true, false, false, false, true, Q>(tmp, out, groups, sc, st, n1, n2c);
-    if (magnitude) return so ? fftp_launch<1, 1, false, false, true, true, true, Q>(tmp, out, groups, sc, st, n1, n2c)
-                             : fftp_launch<1, 1, false, false, false, true, true, Q>(tmp, out, groups, sc, st, n1, n2c);
-    return so ? fftp_launch<1, 1, false, false, true, false, true, Q>(tmp, out, groups, sc, st, n1, n2c)
-              : fftp_launch<1, 1, false, false, false, false, true, Q>(tmp, out, groups, sc, st, n1, n2c);
+    if (inverse) return fftp_launch<1, true, false, false, false, true, Q>(tmp, out, groups, sc, st, n1, n2c);
+    if (magnitude) return so ? fftp_launch<1, false, false, true, true, true, Q>(tmp, out, groups, sc, st, n1, n2c)
+                             : fftp_launch<1, false, false, false, true, true, Q>(tmp, out, groups, sc, st, n1, n2c);
+    return so ? fftp_launch<1, false, false, true, false, true, Q>(tmp, out, groups, sc, st, n1, n2c)
+              : fftp_launch<1, false, false, false, false, true, Q>(tmp, out, groups, sc, st, n1, n2c);
 }
 }  // namespace
 
@@ -872,7 +763,7 @@ int fftp_two_pass_try(const void* in, void* out, void* tmp, size_t n, size_t row
     // n = n1 * N2:  2^15 = 32 x 1024, 2^16 = 256 x 256, 2^17 = 256 x 512, 2^18 = 256 x 1024, 2^19 = 512 x 1024, 2^20 = 256 x 4096.
     // (two adjacent 2048-point rows give only 16-byte store runs: 16 x 2048 took 0.46 ms and 256 x 2048 0.48 ms per 2^26 points)
     // Last pass: 16/Q adjacent rows of N2 = 256*Q points per 128-thread CTA (Q = N2/256 <= 8), or four 4096-point rows per
-    // 512-thread CTA.  BDSP_FFTP_2_16=16 selects the 16 x 4096 split for 2^16 (A/B runs).
+    // 512-thread CTA.
     int n1, log2n2;
     switch (n) {
     case 1u << 15: n1 = 32; log2n2 = 10; break;
@@ -883,56 +774,31 @@ int fftp_two_pass_try(const void* in, void* out, void* tmp, size_t n, size_t row
     case 1u << 20: n1 = 256; log2n2 = 12; break;
     default: return 1;
     }
-    static const bool split16 = [] { const char* e = getenv("BDSP_FFTP_2_16"); return e && e[0] == '1'; }();
-    if (n == (1u << 16) && split16) { n1 = 16; log2n2 = 12; }
     if ((in_rot != 0 && in_rot != n / 2) || (out_rot != 0 && out_rot != n / 2)) return 1;
     if (inverse && (magnitude || out_rot != 0)) return 1;
     if ((reinterpret_cast<uintptr_t>(in) & (real_in ? 7 : 15)) || (reinterpret_cast<uintptr_t>(out) & 7) || (reinterpret_cast<uintptr_t>(tmp) & 15)) return 1;
     if (tmp == in || tmp == out) return 1;
     const int tq = log2n2 < 12 ? 1 << (log2n2 - 8) : 0;
-    // rows per CTA in the 4096-point last pass: 4 (one 512-thread CTA per SM, full 32-byte store sectors) or 2 (two 256-thread
-    // CTAs per SM whose phases overlap; 16-byte half sectors that pair up in L2).  Measured on B200 (64 x 2^20):
-    // 0.453 ms with 4 rows, 0.494 ms with 2, so 4 is the default; BDSP_FFTP_ROWS selects for A/B runs.
-    static const int rows_per_cta = [] {
-        const char* e = getenv("BDSP_FFTP_ROWS");
-        return (e && e[0] == '4') ? 4 : (e && e[0] == '2') ? 2 : FP_ROWS_DEFAULT;
-    }();
-    const int rpc = tq ? 16 / tq : rows_per_cta;
+    // The 4096-point last pass takes four rows per 512-thread CTA (one CTA per SM, full 32-byte store sectors).  Measured on
+    // B200 (64 x 2^20): 0.453 ms, against 0.494 ms with two rows per 256-thread CTA (16-byte half sectors, two CTAs per SM).
+    const int rpc = tq ? 16 / tq : 4;
     const size_t groups = rows * (size_t)(n1 / rpc);
     if (groups > 0x7fffffffull || rows * 4096 > 0x7fffffffull) return 1;
     const bool si = in_rot != 0, so = out_rot != 0;
     const float sc = (float)scale;
-    // BDSP_FFTP_CHUNK_MB=<m> processes the sequences in chunks whose intermediate (8 bytes per point) is <= m MB so
-    // that it can stay in the 126 MB L2 between the passes.  Measured on B200 (64 x 2^20): one launch pair over the
-    // whole batch 0.448 ms; 64 MB chunks 0.571 ms; 32 MB 0.596 ms; 8 MB 1.18 ms (launch rate and wave tails cost more
-    // than the saved DRAM traffic), so chunking is off unless requested.
-    static const size_t chunk_bytes = [] {
-        const char* e = getenv("BDSP_FFTP_CHUNK_MB");
-        const long mb = e ? atol(e) : 0;
-        return mb > 0 ? (size_t)mb << 20 : ~(size_t)0;
-    }();
-    size_t chunk = chunk_bytes / (n * sizeof(float2));
-    if (chunk < 1) chunk = 1;
-    const size_t out_elem = magnitude ? sizeof(float) : sizeof(float2);
-    for (size_t r0 = 0; r0 < rows; r0 += chunk) {
-        const size_t nr = rows - r0 < chunk ? rows - r0 : chunk;
-        const void* cin = reinterpret_cast<const char*>(in) + r0 * n * (real_in ? sizeof(float) : sizeof(float2));
-        void* cout = reinterpret_cast<char*>(out) + r0 * n * out_elem;
-        const size_t groups_c = nr * (size_t)(n1 / rpc);
-        int rc;
-        if (real_in) rc = fftp_colpass<false, false, true>(cin, tmp, n1, log2n2, nr, st, im);
-        else if (inverse) rc = si ? fftp_colpass<true, true>(cin, tmp, n1, log2n2, nr, st, im) : fftp_colpass<true, false>(cin, tmp, n1, log2n2, nr, st, im);
-        else rc = si ? fftp_colpass<false, true>(cin, tmp, n1, log2n2, nr, st, im) : fftp_colpass<false, false>(cin, tmp, n1, log2n2, nr, st, im);
-        if (rc) return rc;
-        if (tq == 8) rc = fftp_rowsq_pass<8>(tmp, cout, groups_c, inverse, so, magnitude, sc, st, n1);
-        else if (tq == 4) rc = fftp_rowsq_pass<4>(tmp, cout, groups_c, inverse, so, magnitude, sc, st, n1);
-        else if (tq == 2) rc = fftp_rowsq_pass<2>(tmp, cout, groups_c, inverse, so, magnitude, sc, st, n1);
-        else if (tq == 1) rc = fftp_rowsq_pass<1>(tmp, cout, groups_c, inverse, so, magnitude, sc, st, n1);
-        else if (rows_per_cta == 4) rc = fftp_rows_pass<4>(tmp, cout, groups_c, inverse, so, magnitude, sc, st, n1);
-        else rc = fftp_rows_pass<2>(tmp, cout, groups_c, inverse, so, magnitude, sc, st, n1);
-        if (rc) return rc;
-    }
-    return 0;
+    // One launch pair over the whole batch.  Measured on B200 (64 x 2^20): 0.448 ms, against 0.571 / 0.596 / 1.18 ms for
+    // chunks of sequences whose intermediate (8 bytes per point) is 64 / 32 / 8 MB and could stay in the 126 MB L2 between
+    // the passes: launch rate and wave tails cost more than the saved DRAM traffic.
+    int rc;
+    if (real_in) rc = fftp_colpass<false, false, true>(in, tmp, n1, log2n2, rows, st, im);
+    else if (inverse) rc = si ? fftp_colpass<true, true>(in, tmp, n1, log2n2, rows, st, im) : fftp_colpass<true, false>(in, tmp, n1, log2n2, rows, st, im);
+    else rc = si ? fftp_colpass<false, true>(in, tmp, n1, log2n2, rows, st, im) : fftp_colpass<false, false>(in, tmp, n1, log2n2, rows, st, im);
+    if (rc) return rc;
+    if (tq == 8) return fftp_rowsq_pass<8>(tmp, out, groups, inverse, so, magnitude, sc, st, n1);
+    if (tq == 4) return fftp_rowsq_pass<4>(tmp, out, groups, inverse, so, magnitude, sc, st, n1);
+    if (tq == 2) return fftp_rowsq_pass<2>(tmp, out, groups, inverse, so, magnitude, sc, st, n1);
+    if (tq == 1) return fftp_rowsq_pass<1>(tmp, out, groups, inverse, so, magnitude, sc, st, n1);
+    return fftp_rows_pass(tmp, out, groups, inverse, so, magnitude, sc, st, n1);
 }
 
 
@@ -990,27 +856,8 @@ int fftp_rows1k_try(const void* tmp, void* out, size_t n, size_t rows, bool inve
     return fftp_rowsq_pass<4>(tmp, out, groups, inverse, out_rot != 0, magnitude, (float)scale, st, n1);
 }
 
-// CTAs per sequence for n >= 8192: 1 = one persistent CTA per SM with register prefetch (default,
-// measured faster on B200), 2 = thread-block cluster of two CTAs exchanging the first stage through
-// distributed shared memory.  BDSP_FFTP_CLUSTER=2 selects the latter (for A/B measurements).
-static int fftp_cluster_mode() {
-    static int mode = [] {
-        const char* e = getenv("BDSP_FFTP_CLUSTER");
-        return (e && e[0] == '2') ? 2 : 1;
-    }();
-    return mode;
-}
-
 int fftp16k_try(const void* in, void* out, size_t rows, bool inverse, bool shift_in, bool shift_out, bool magnitude, float scale,
                 cudaStream_t st);
-// BDSP_FFTP16K=0 selects round 1's one-CTA-per-row kernel for 16384-point rows (A/B measurements)
-static int fftp16k_mode() {
-    static int mode = [] {
-        const char* e = getenv("BDSP_FFTP16K");
-        return (e && e[0] == '0') ? 0 : 1;
-    }();
-    return mode;
-}
 
 // returns 0 on success, 1 when this configuration is not covered (caller uses the generic kernel)
 int fftp_try(const void* in, void* out, size_t n, size_t rows, bool inverse, size_t in_rot, size_t out_rot, double scale,
@@ -1037,25 +884,23 @@ int fftp_try(const void* in, void* out, size_t n, size_t rows, bool inverse, siz
     if (rows * 2 > 0x7fffffffull) return 1;
     const bool si = in_rot != 0, so = out_rot != 0;
     const float sc = (float)scale;
-    if (n == 4096) return fftp_dispatch<1, 1>(in, out, rows, inverse, si, so, magnitude, sc, st);
-    if (n == 16384 && fftp16k_mode() && rows >= 2) {
+    if (n == 4096) return fftp_dispatch<1>(in, out, rows, inverse, si, so, magnitude, sc, st);
+    if (n == 16384 && rows >= 2) {
         // persistent CTAs with the rolling F3 || F0 pipeline (fftp16k.cu)
         const int rc = fftp16k_try(in, out, rows, inverse, si, so, magnitude, sc, st);
         if (rc <= 0) return rc;
     }
-    if (n == 8192) return fftp_cluster_mode() == 2 ? fftp_dispatch<2, 2>(in, out, rows, inverse, si, so, magnitude, sc, st)
-                                              : fftp_dispatch<2, 1>(in, out, rows, inverse, si, so, magnitude, sc, st);
-    return fftp_cluster_mode() == 2 ? fftp_dispatch<4, 2>(in, out, rows, inverse, si, so, magnitude, sc, st)
-                               : fftp_dispatch<4, 1>(in, out, rows, inverse, si, so, magnitude, sc, st);
+    if (n == 8192) return fftp_dispatch<2>(in, out, rows, inverse, si, so, magnitude, sc, st);
+    return fftp_dispatch<4>(in, out, rows, inverse, si, so, magnitude, sc, st);
 }
 
 // real-input forward transforms (fftp_kernel<RIN>): rows of `n` real scalars, n in {512 ... 16384}
 template <int R0, int Q, int SQ = 0>
 int fftp_dispatch_real(const void* in, void* out, size_t groups, bool shift_out, bool mag, float scale, cudaStream_t st) {
-    if (mag) return shift_out ? fftp_launch<R0, 1, false, false, true, true, false, 0, Q, true, SQ>(in, out, groups, scale, st)
-                              : fftp_launch<R0, 1, false, false, false, true, false, 0, Q, true, SQ>(in, out, groups, scale, st);
-    return shift_out ? fftp_launch<R0, 1, false, false, true, false, false, 0, Q, true, SQ>(in, out, groups, scale, st)
-                     : fftp_launch<R0, 1, false, false, false, false, false, 0, Q, true, SQ>(in, out, groups, scale, st);
+    if (mag) return shift_out ? fftp_launch<R0, false, false, true, true, false, 0, Q, true, SQ>(in, out, groups, scale, st)
+                              : fftp_launch<R0, false, false, false, true, false, 0, Q, true, SQ>(in, out, groups, scale, st);
+    return shift_out ? fftp_launch<R0, false, false, true, false, false, 0, Q, true, SQ>(in, out, groups, scale, st)
+                     : fftp_launch<R0, false, false, false, false, false, 0, Q, true, SQ>(in, out, groups, scale, st);
 }
 
 int fftp_try_real(const void* in, void* out, size_t n, size_t rows, size_t out_rot, double scale, bool magnitude, cudaStream_t st) {

@@ -20,34 +20,6 @@ using namespace ols16;
 
 #define F16_NT 512
 #define F16_B FP_B_OF(4)
-#ifndef F16_GROUP_BARRIER
-#define F16_GROUP_BARRIER 1  // the F1 -> F2 exchange stays inside a sub-block: named barrier over its 128 threads
-#endif
-#ifndef F16_X_NOALLOC
-#define F16_X_NOALLOC 0
-#endif
-#ifndef F16_FAST_SQRT
-#define F16_FAST_SQRT 1
-#endif
-#if F16_FAST_SQRT
-#define F16_SQRT(v) sqrt_fast(v)
-#else
-#define F16_SQRT(v) sqrtf(v)
-#endif
-// F0 inputs of the NEXT row for the thread groups of the first half of the last section (half of the row, 64 KB) arrive by
-// bulk asynchronous copies (cp.async.bulk + mbarrier, issued at the top of the iteration) in a staging buffer next to the
-// row buffer; the second half's register loads are issued at the start of the section instead of in its middle.  The
-// section waits for global loads issued only ~300 instructions earlier (ncu: long_scoreboard the top stall,
-// profiles/r2_fftp16k_ncu.txt).  Measured on B200 (C3): 0.2686 ms with the staging against 0.2657 ms without (same box,
-// alternating runs) - the exposed load latency is not what bounds the row time, so the option is off.
-#ifndef F16_TMA_STAGE
-#define F16_TMA_STAGE 0
-#endif
-#define F16_STG_CHUNK 130                       // float2 per staged chunk: 128 columns + 2 (the 16 chunks of a quarter shift by 4 banks)
-#define F16_STG_BYTES (64 * F16_STG_CHUNK * 8)
-#ifndef F16_L2_PREFETCH
-#define F16_L2_PREFETCH 1   // one thread asks L2 for the row after the next while the current one is computed
-#endif
 
 // the two adjacent column pairs (2*lsb, 2*lsb + 1) of group (k0, k1): F0 inputs of one row, 8 x 128-bit loads
 struct F16Raw { float4 v[2][4]; };
@@ -59,14 +31,7 @@ __device__ __forceinline__ void f16_load(F16Raw& r, const float2* __restrict__ x
 #pragma unroll
         for (int n3 = 0; n3 < 4; n3++) {
             const int src = SHIFT_IN ? ((n3 + 2) & 3) : n3;
-#if F16_X_NOALLOC
-            float4 q;
-            asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(q.x), "=f"(q.y), "=f"(q.z), "=f"(q.w)
-                         : "l"(xr + c0 + 2 * u + 4096 * src));
-            r.v[u][n3] = q;
-#else
             r.v[u][n3] = __ldg(reinterpret_cast<const float4*>(xr + c0 + 2 * u + 4096 * src));
-#endif
         }
 }
 
@@ -82,16 +47,6 @@ fftp16k_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long 
     const long long row_step = gridDim.x;
     long long row = blockIdx.x;
     if (row >= rows) return;
-#if F16_TMA_STAGE
-    float2* stg = reinterpret_cast<float2*>(smem + 2 * 4 * F16_B);
-    const unsigned stg_addr = (unsigned)__cvta_generic_to_shared(stg);
-    const unsigned mbar = stg_addr + F16_STG_BYTES;
-    if (t == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(mbar));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    unsigned stg_phase = 0;
-#endif
 
     // F3 / F0 geometry of this thread's two groups: gl = t + 512*half = lsb + 4*(k0 + 16*k1)
     int g_k0[2], g_k1[2];
@@ -155,23 +110,11 @@ fftp16k_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long 
         const long long nrow = row + row_step;
         const bool has_next = nrow < rows;
         const float2* xn = x + (size_t)(has_next ? nrow : row) * (size_t)N;
-#if F16_TMA_STAGE
-        if (has_next && t < 64) {
-            // chunk t: quarter n3 = t >> 4, columns 256 k0 .. 256 k0 + 127 (k0 = t & 15) of the next row
-            if (t == 0) asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mbar), "r"(64 * 1024) : "memory");
-            const int n3 = t >> 4, k0c = t & 15;
-            const int src = SHIFT_IN ? ((n3 + 2) & 3) : n3;
-            const float2* g = xn + 4096 * src + 256 * k0c;
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(stg_addr + (unsigned)(t * F16_STG_CHUNK * 8)), "l"(g), "r"(1024), "r"(mbar) : "memory");
-        }
-#endif
-#if F16_L2_PREFETCH
+        // one thread asks L2 for the row after the next while the current one is computed
         if (t == 0 && nrow + row_step < rows) {
             const float2* pf = x + (size_t)(nrow + row_step) * (size_t)N;
             asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(pf), "r"(N * 8) : "memory");
         }
-#endif
         cp v[16];
         // ------------------------------------------------------------------ F1: stride 256 inside sub-block sb
         {
@@ -198,11 +141,8 @@ fftp16k_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long 
                 *reinterpret_cast<float2*>(bim + 272 * k0 + off[(k0 >> 1) & 3]) = v[s].im;
             }
         }
-#if F16_GROUP_BARRIER
+        // the F1 -> F2 exchange stays inside a sub-block: named barrier over its 128 threads
         asm volatile("bar.sync %0, 128;" ::"r"(sb + 1) : "memory");
-#else
-        __syncthreads();
-#endif
         // ------------------------------------------------------------------ F2: stride 16
         {
             const int k0 = tt >> 3, n0 = 2 * (tt & 7);
@@ -236,16 +176,10 @@ fftp16k_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long 
         }
         __syncthreads();
         // ------------------------------------------------------------------ F3 of this row  ||  F0 of the next row
-#if F16_TMA_STAGE
-        F16Raw raw1;
-        if (has_next) f16_load<SHIFT_IN>(raw1, xn, c0_of(1));
-#endif
 #pragma unroll
         for (int half = 0; half < 2; half++) {
-#if !F16_TMA_STAGE
             F16Raw raw;
             if (has_next) f16_load<SHIFT_IN>(raw, xn, c0_of(half));
-#endif
             const int k0 = g_k0[half], k1 = g_k1[half];
             const int r = fp_rot(k0, k1);
             const int base = lsb * F16_B + 272 * k0 + 16 * k1;
@@ -268,8 +202,8 @@ fftp16k_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long 
                 for (int m = 0; m < 8; m++) {
                     pk m2 = pfma(P[m].re, P[m].re, pmul(P[m].im, P[m].im));
                     const int ka = bitrev4(2 * m) ^ (SHIFT_OUT ? 8 : 0), kb = bitrev4(2 * m + 1) ^ (SHIFT_OUT ? 8 : 0);
-                    o[1024 * ka] = F16_SQRT(m2.x) * scale;
-                    o[1024 * kb] = F16_SQRT(m2.y) * scale;
+                    o[1024 * ka] = sqrt_fast(m2.x) * scale;
+                    o[1024 * kb] = sqrt_fast(m2.y) * scale;
                 }
             } else {
                 float2* o = reinterpret_cast<float2*>(out_) + (size_t)row * N + klow;
@@ -280,31 +214,8 @@ fftp16k_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long 
                     o[1024 * kb] = make_float2(P[m].re.y * scale, P[m].im.y * scale);
                 }
             }
-#if F16_TMA_STAGE
-            if (has_next) {
-                if (half == 0) {
-                    // staged chunk (n3, k0): columns 2 (8 k1 + 2 lsb + u) .. + 1 of its 128
-                    asm volatile("{\n.reg .pred p;\nF16_WAIT:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n@p bra F16_DONE;\nbra F16_WAIT;\nF16_DONE:\n}"
-                                 ::"r"(mbar), "r"(stg_phase) : "memory");
-                    F16Raw raw0;
-                    const float2* sp = stg + k0 * F16_STG_CHUNK + 2 * (8 * k1 + 2 * lsb);
-#pragma unroll
-                    for (int u = 0; u < 2; u++)
-#pragma unroll
-                        for (int n3 = 0; n3 < 4; n3++)
-                            raw0.v[u][n3] = *reinterpret_cast<const float4*>(sp + n3 * 16 * F16_STG_CHUNK + 2 * u);
-                    f0_store(raw0, 0);
-                } else {
-                    f0_store(raw1, 1);
-                }
-            }
-#else
             if (has_next) f0_store(raw, half);
-#endif
         }
-#if F16_TMA_STAGE
-        if (has_next) stg_phase ^= 1;
-#endif
         __syncthreads();
     }
 }
@@ -312,7 +223,7 @@ fftp16k_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long 
 namespace {
 template <bool INV, bool SI, bool SO, bool MAG>
 int f16_launch(const void* in, void* out, size_t rows, float scale, cudaStream_t st) {
-    const size_t smem = (size_t)2 * 4 * F16_B * sizeof(float) + (F16_TMA_STAGE ? F16_STG_BYTES + 16 : 0);
+    const size_t smem = (size_t)2 * 4 * F16_B * sizeof(float);
     auto kern = fftp16k_kernel<INV, SI, SO, MAG>;
     static PerDeviceOnce configured;   // per instantiation and device
     if (configured.need()) {

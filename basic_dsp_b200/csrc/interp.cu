@@ -165,29 +165,17 @@ interp_poly_tiled_kernel(const void* __restrict__ x_, void* __restrict__ y_, con
 // threads per CTA: small CTAs keep the barrier-separated load / compute / store phases of different CTAs overlapping on
 // the SM.  Measured on B200 (C4a, 2^24 samples x4): 256 threads 0.160 ms, 128: 0.142, 64: 0.133, 32: 0.136 while the vector's last
 // tile was the kernel's tail (+ ~25 us on every variant); with the end tiles first: 256: 0.117, 128: 0.109, 64: 0.111, 32: 0.118.
-#ifndef IPF_THREADS
 #define IPF_THREADS 64
-#endif
-// persistent double-buffered variant (interp_poly_f32p_kernel): measured on B200 (C4a) 0.1335-0.1364 ms against 0.1330-0.1368 ms
-// for the one-tile-per-CTA kernel, with or without a start-up skew of the resident CTAs - off
-#ifndef IPF_PERSISTENT
-#define IPF_PERSISTENT 0
-#endif
-#ifndef IPF_STAGGER_NS
-#define IPF_STAGGER_NS 220
-#endif
 // positions per thread (IPF_LRP = log2): 8 -> 64 registers, 1024 threads per SM; 16 -> half the shared loads and loop overhead
 // per FFMA2, but 127 registers and 512 threads per SM.  Measured on B200 (C4a): 8 positions 0.131 ms; 16 positions 0.162 ms
 // (64-thread CTAs), 0.160 (32), 0.185 (128): the FMA pipe needs the resident warps more than it needs fewer instructions
-#ifndef IPF_LRP
 #define IPF_LRP 3
-#endif
 #define IPF_RP (1 << IPF_LRP)
 #define IPF_POS (IPF_THREADS * IPF_RP)
 #define IPF_ROW (4 * IPF_RP + 2)   // staging row stride in floats (odd number of 8-byte words: conflict-free 64-bit stores)
 __device__ __forceinline__ int ipf_skew(int i) { return i + (i >> IPF_LRP); }
 
-__global__ void __launch_bounds__(IPF_THREADS, (IPF_LRP == 3 ? 1024 : 512) / IPF_THREADS)
+__global__ void __launch_bounds__(IPF_THREADS, 1024 / IPF_THREADS)
 interp_poly_f32_kernel(const float* __restrict__ x, float* __restrict__ y, const float* __restrict__ tab, long long N,
                        long long new_points, int F, int L, long long scalar_len) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -334,148 +322,6 @@ interp_poly_f32_kernel(const float* __restrict__ x, float* __restrict__ y, const
     }
 }
 
-#if IPF_PERSISTENT
-// ------------------------------------------------------------------------------------------
-// Persistent, double-buffered form of interp_poly_f32_kernel for F = 4 (BASELINE C4a): a CTA walks tiles of IPF_POS
-// positions; the window of the NEXT tile arrives through cp.async (two 4-byte copies per sample: the duplicated {x, x}
-// layout) while the current tile is in its FFMA2 loop, so no tile waits for global memory and the tap table is loaded once
-// per CTA.  Results leave through the tile's own window buffer, one warp's 1024 outputs at a time.
-// ------------------------------------------------------------------------------------------
-__device__ __forceinline__ void ipf_cp4(void* smem_dst, const void* gsrc) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
-}
-
-__global__ void __launch_bounds__(IPF_THREADS, 1024 / IPF_THREADS)
-interp_poly_f32p_kernel(const float* __restrict__ x, float* __restrict__ y, const float* __restrict__ tab, long long N,
-                        long long new_points, int L, long long scalar_len, long long ntiles, int buf_f2, int nsm) {
-    static_assert(IPF_LRP == 3 && IPF_THREADS == 64, "persistent interpolation kernel: 64 threads x 8 positions");
-    constexpr int F = 4;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int J = 2 * L + 3;
-    const int JI = 2 * L + 2;
-    float4* stab = reinterpret_cast<float4*>(smem_raw);
-    float2* bufs = reinterpret_cast<float2*>(stab + J);        // two window buffers of buf_f2 float2 each
-    const int W = IPF_POS + JI - 1 + IPF_RP;
-    const int t = threadIdx.x;
-    // work item -> tile: the vector's last tile (slow per-output path) is item 0, so that it does not end up as the tail
-    auto tile_of = [&](long long item) { return item == 0 ? ntiles - 1 : item - 1; };
-    auto interior_of = [&](long long item) {
-        const long long r0 = tile_of(item) * IPF_POS;
-        return (r0 * F >= scalar_len) && ((r0 + IPF_POS) * F <= new_points - scalar_len);
-    };
-    auto prefetch = [&](long long item, float2* dst) {
-        const long long tile = tile_of(item);
-        const float* xs = x + (tile * IPF_POS - L - 1);
-        const long long wmax = N - 1 - (tile * IPF_POS - L - 1);   // read-ahead slots stay inside the vector
-        for (int w = t; w < W; w += IPF_THREADS) {
-            float2* d = dst + ipf_skew(w);
-            const float* g = xs + (w <= wmax ? w : (int)wmax);
-            ipf_cp4(&d->x, g);
-            ipf_cp4(&d->y, g);
-        }
-    };
-    for (int j = t; j < J; j += IPF_THREADS) stab[j] = make_float4(tab[j], tab[J + j], tab[2 * J + j], tab[3 * J + j]);
-    long long tile = blockIdx.x;
-    int b = 0;
-#if IPF_STAGGER_NS > 0
-    // The CTAs of an SM start together and every tile costs the same, so they would stay in lockstep: all in the FFMA2 loop
-    // (one pipe) at the same time, then all in the load / store phases.  A start-up skew per resident slot keeps their phases apart.
-    {
-        const unsigned slot = blockIdx.x / (unsigned)nsm;
-        if (slot) __nanosleep(slot * IPF_STAGGER_NS);
-    }
-#endif
-    if (tile < ntiles && interior_of(tile)) prefetch(tile, bufs);
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    for (; tile < ntiles; tile += gridDim.x, b ^= 1) {
-        float2* sxx = bufs + b * buf_f2;
-        const long long nxt = tile + gridDim.x;
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-        __syncthreads();                                       // this tile's window (and the tap table) is in shared memory;
-                                                               // everybody is done with the other buffer
-        if (nxt < ntiles && interior_of(nxt)) prefetch(nxt, bufs + (b ^ 1) * buf_f2);
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        const long long r0 = tile_of(tile) * IPF_POS;
-        if (!interior_of(tile)) {                              // first / last tiles of the vector: per-output taps with wrap-around
-            for (long long i = r0 * F + t; i < (r0 + IPF_POS) * F && i < new_points; i += IPF_THREADS) {
-                const long long r = i / F; const int s = (int)(i - r * F);
-                const bool in = (i >= scalar_len) && (i < new_points - scalar_len);
-                const float* tp = tab + (in ? 0 : F * J) + s * J;
-                long long g = (r - L - 1) % N; if (g < 0) g += N;
-                float acc = 0.f;
-                for (int j = 0; j < J; j++) {
-                    acc += x[g] * tp[j];
-                    g++; if (g >= N) g -= N;
-                }
-                y[i] = acc;
-            }
-            continue;
-        }
-        float2 acc[IPF_RP][2];
-#pragma unroll
-        for (int p = 0; p < IPF_RP; p++) { acc[p][0] = make_float2(0.f, 0.f); acc[p][1] = make_float2(0.f, 0.f); }
-        const float2* wbase = sxx + t * (IPF_RP + 1);
-        float2 win[IPF_RP];
-#pragma unroll
-        for (int p = 0; p < IPF_RP; p++) win[p] = wbase[p];
-        const int full = JI & ~(IPF_RP - 1);
-        const float2* wp = wbase + (IPF_RP + 1);
-        const float4* tp = stab;
-        for (int jb = 0; jb < full; jb += IPF_RP, wp += IPF_RP + 1, tp += IPF_RP) {
-#pragma unroll
-            for (int jj = 0; jj < IPF_RP; jj++) {
-                const float4 t4 = tp[jj];
-                const float2 ta = make_float2(t4.x, t4.y), tb = make_float2(t4.z, t4.w);
-#pragma unroll
-                for (int p = 0; p < IPF_RP; p++) {
-                    const float2 xx = win[(jj + p) % IPF_RP];
-                    acc[p][0] = __ffma2_rn(xx, ta, acc[p][0]);
-                    acc[p][1] = __ffma2_rn(xx, tb, acc[p][1]);
-                }
-                win[jj] = wp[jj];
-            }
-        }
-#pragma unroll
-        for (int jj = 0; jj < IPF_RP; jj++) {
-            if (full + jj < JI) {
-                const float4 t4 = tp[jj];
-                const float2 ta = make_float2(t4.x, t4.y), tb = make_float2(t4.z, t4.w);
-#pragma unroll
-                for (int p = 0; p < IPF_RP; p++) {
-                    const float2 xx = win[(jj + p) % IPF_RP];
-                    acc[p][0] = __ffma2_rn(xx, ta, acc[p][0]);
-                    acc[p][1] = __ffma2_rn(xx, tb, acc[p][1]);
-                }
-                win[jj] = wp[jj];
-            }
-        }
-        // results: warp by warp through this tile's window buffer (32 threads x 32 outputs = 1024 contiguous floats)
-        float* so = reinterpret_cast<float*>(sxx);
-        float* yo = y + r0 * F;
-#pragma unroll 1
-        for (int wsel = 0; wsel < IPF_THREADS / 32; wsel++) {
-            __syncthreads();                                   // window reads / the previous warp's copy-out are complete
-            if ((t >> 5) == wsel) {
-#pragma unroll
-                for (int p = 0; p < IPF_RP; p++) {
-                    *reinterpret_cast<float2*>(so + (t & 31) * IPF_ROW + 4 * p) = acc[p][0];
-                    *reinterpret_cast<float2*>(so + (t & 31) * IPF_ROW + 4 * p + 2) = acc[p][1];
-                }
-            }
-            __syncthreads();
-#pragma unroll
-            for (int it = 0; it < 4; it++) {
-                const int o = 4 * (t + IPF_THREADS * it);      // 0 .. 1023
-                const float* sp = so + (o >> 5) * IPF_ROW + (o & 31);
-                const float2 a = *reinterpret_cast<const float2*>(sp), c = *reinterpret_cast<const float2*>(sp + 2);
-                *reinterpret_cast<float4*>(yo + wsel * 1024 + o) = make_float4(a.x, a.y, c.x, c.y);
-            }
-        }
-    }
-}
-
-#endif
-
 template <typename T>
 int interp_poly(const void* x, void* y, const T* tab_dev, size_t N, size_t new_points, int F, int L, int is_complex,
                 cudaStream_t st) {
@@ -497,29 +343,6 @@ int interp_poly(const void* x, void* y, const T* tab_dev, size_t N, size_t new_p
         interp_poly_tiled_kernel<T, CP, FM, RPV><<<(unsigned)grid, IP2_THREADS, smem, st>>>(x, y, tab_dev, (long long)N, (long long)new_points, F, L, scalar_len); \
     } while (0)
         if (is_complex) { if (F <= 4) BDSP_IP2(true, 4, 2); else BDSP_IP2(true, 8, 1); }
-#if IPF_PERSISTENT
-        else if (F == 4 && sizeof(T) == 4 && rows >= 64 * IPF_POS) {
-            // long real f32 vectors, factor 4: persistent CTAs with the next tile's window in flight during the FFMA2 loop
-            const size_t wlen = (size_t)IPF_POS + J + 2 * IPF_RP;
-            size_t buf_f2 = wlen + wlen / IPF_RP + 2;
-            const size_t stage_f2 = (size_t)32 * IPF_ROW / 2 + 1;
-            if (buf_f2 < stage_f2) buf_f2 = stage_f2;
-            buf_f2 = (buf_f2 + 1) & ~(size_t)1;
-            const size_t smem = (size_t)J * 16 + 2 * buf_f2 * 8;
-            const long long ntiles = (rows + IPF_POS - 1) / IPF_POS;
-            long long grid = (long long)sm_count() * (1024 / IPF_THREADS);
-            if (grid > ntiles) grid = ntiles;
-            static PerDeviceOnce configured;
-            if (configured.need()) {
-                BDSP_CUDA_OK(cudaFuncSetAttribute(interp_poly_f32p_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem > 48 * 1024 ? smem : 48 * 1024)));
-                BDSP_CUDA_OK(cudaFuncSetAttribute(interp_poly_f32p_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                configured.mark();
-            }
-            interp_poly_f32p_kernel<<<(unsigned)grid, IPF_THREADS, smem, st>>>(reinterpret_cast<const float*>(x), reinterpret_cast<float*>(y),
-                                                                               reinterpret_cast<const float*>(tab_dev), (long long)N,
-                                                                               (long long)new_points, L, scalar_len, ntiles, (int)buf_f2, sm_count());
-        }
-#endif
         else if (F <= 4 && sizeof(T) == 4) {
             const size_t wlen = (size_t)IPF_POS + J + 2 * IPF_RP;
             size_t smem = (size_t)J * 16 + (wlen + wlen / IPF_RP + 2) * 8;

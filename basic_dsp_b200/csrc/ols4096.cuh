@@ -1,20 +1,9 @@
-// Fused overlap-save block for the fast convolution hot path: 4096-point forward FFT, spectrum
-// multiply and 4096-point inverse FFT in ONE kernel with the block resident in shared memory.
+// Planar packed-FP32x2 building blocks of the fftp* kernels (fftp.cu, fftp16k.cu).
 // Written for sm_100a: all butterfly arithmetic uses the packed FP32x2 instructions of Blackwell
 // (FADD2 / FMUL2 / FFMA2 via __fadd2_rn / __fmul2_rn / __ffma2_rn), which halve the issue slots per
-// flop; shared memory is planar (re plane, im plane) so that one 64-bit register pair holds the same
+// flop; data are planar (re plane, im plane) so that one 64-bit register pair holds the same
 // component of two adjacent points ("two columns per thread").
-//
-// Structure (N = 4096 = 16^3, 128 threads, 32 points per thread):
-//   F1  radix-16 DIF over stride 256, inputs straight from global memory      -> smem
-//   F2  radix-16 DIF over stride 16                                            -> smem
-//   F3  radix-16 DIF over stride 1  |  * H (position order)  |  radix-16 DIT over stride 1   (registers) -> smem
-//   I2  radix-16 DIT over stride 16                                            -> smem
-//   I1  radix-16 DIT over stride 256, valid outputs straight to global memory
-// The forward transform leaves the spectrum in digit-reversed order, the impulse-response spectrum
-// is stored in the same order by the plan (ols4096_prepare), and the inverse transform consumes that
-// order, so no reordering pass exists.  One swizzled layout (phys()) serves all three access
-// patterns without bank conflicts, every exchange is in place per thread -> 4 __syncthreads per block.
+// (The file is named after round 1's planar 4096-point overlap-save kernel, for which these pieces were written.)
 #pragma once
 #include "common.cuh"
 
@@ -23,10 +12,6 @@ namespace ols16 {
 
 typedef float2 pk;
 struct cp { pk re, im; };
-
-#define OLS_M 4096
-#define OLS_THREADS 128
-#define OLS_PLANE (16 * 272)
 
 __device__ __forceinline__ pk padd(pk a, pk b) { return __fadd2_rn(a, b); }
 __device__ __forceinline__ pk pneg(pk a) { return make_float2(-a.x, -a.y); }
@@ -39,20 +24,12 @@ __device__ __forceinline__ pk splat(float v) { return make_float2(v, v); }
 __device__ __forceinline__ float sqrt_fast(float v) { float r; asm("sqrt.approx.f32 %0, %1;" : "=f"(r) : "f"(v)); return r; }
 // {re0, im0, re1, im1} (two adjacent interleaved points) -> planar pairs {re0, re1}, {im0, im1}; the explicit 64-bit packs
 // keep the compiler from materialising each pair twice (once per consumer)
-#ifndef OLS_PACK_ASM
-#define OLS_PACK_ASM 1
-#endif
 __device__ __forceinline__ void planar_of(const float4& ab, pk& re, pk& im) {
-#if OLS_PACK_ASM
     unsigned long long r, i;
     asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(ab.x), "f"(ab.z));
     asm("mov.b64 %0, {%1, %2};" : "=l"(i) : "f"(ab.y), "f"(ab.w));
     re = *reinterpret_cast<pk*>(&r);
     im = *reinterpret_cast<pk*>(&i);
-#else
-    re = make_float2(ab.x, ab.z);
-    im = make_float2(ab.y, ab.w);
-#endif
 }
 
 __device__ __forceinline__ cp cadd(cp a, cp b) { cp r; r.re = padd(a.re, b.re); r.im = padd(a.im, b.im); return r; }
@@ -150,24 +127,9 @@ template <bool SLOTMAP> __device__ __forceinline__ void apply_twiddles(cp (&v)[1
     }
 }
 
-// 128-bit read-only global load that does not allocate in L1 (the block inputs are used once; a load that allocates
-// passes the L1 data RAM twice: fill + read)
-#ifndef OLS_X_NOALLOC
-#define OLS_X_NOALLOC 0
-#endif
-__device__ __forceinline__ float4 ldg_x4(const float4* p) {
-#if OLS_X_NOALLOC
-    float4 r;
-    asm("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    return r;
-#else
-    return __ldg(p);
-#endif
-}
-
-// swizzled shared-memory layout, see header comment.  p = 256*k0 + 16*g + j
+// swizzled shared-memory layout of a 16 x 256-point tile: point 16*g + j of row k0 lives at
+// 272*k0 + 16*g + ((j + 4*rot_of(g)) & 15), which keeps the row- and column-wise accesses free of bank conflicts
 __device__ __forceinline__ int rot_of(int g) { return (g >> 1) & 3; }
-__device__ __forceinline__ int phys(int k0, int g, int j) { return 272 * k0 + 16 * g + ((j + 4 * rot_of(g)) & 15); }
 
 // ---- in-register 16-point transforms over 16 CONTIGUOUS points, packed over adjacent points ------
 // P[m] = {a[2m], a[2m+1]}.  DIF, natural in -> bit-reversed out; INV selects exp(+i...).
@@ -215,54 +177,9 @@ template <bool INV> __device__ __forceinline__ void fft16_dif(cp (&P)[8]) {
         P[b + 1] = o;
     }
 }
-__device__ __forceinline__ void fft16_dif_fwd(cp (&P)[8]) { fft16_dif<false>(P); }
-
-// Inverse: DIT, bit-reversed in -> natural out.
-__device__ __forceinline__ void fft16_dit_inv(cp (&P)[8]) {
-    // level 1', span 1 (with the {1, +i} twiddle of level 2' folded into the odd slots) + level 2', span 2
-#pragma unroll
-    for (int b = 0; b < 8; b += 2) {
-        cp e, o;
-        e.re = make_float2(P[b].re.x + P[b].re.y, P[b].re.x - P[b].re.y);
-        e.im = make_float2(P[b].im.x + P[b].im.y, P[b].im.x - P[b].im.y);
-        // second operand: {x + y, i * (x - y)} = {(x.re + y.re, x.im + y.im), (y.im - x.im, x.re - y.re)}
-        o.re = make_float2(P[b + 1].re.x + P[b + 1].re.y, P[b + 1].im.y - P[b + 1].im.x);
-        o.im = make_float2(P[b + 1].im.x + P[b + 1].im.y, P[b + 1].re.x - P[b + 1].re.y);
-        P[b] = cadd(e, o);
-        P[b + 1] = csub(e, o);
-    }
-    // level 3', span 4: conj(W8^{j})
-    const pk t2r[2] = {make_float2(1.f, OLS_H), make_float2(0.f, -OLS_H)};
-    const pk t2i[2] = {make_float2(0.f, OLS_H), make_float2(1.f, OLS_H)};
-#pragma unroll
-    for (int b = 0; b < 8; b += 4) {
-#pragma unroll
-        for (int m = 0; m < 2; m++) {
-            cp t = cmulc(P[b + m + 2], t2r[m], t2i[m]);
-            cp u = P[b + m];
-            P[b + m] = cadd(u, t);
-            P[b + m + 2] = csub(u, t);
-        }
-    }
-    // level 4', span 8: conj(W16^{j})
-    const pk t1r[4] = {make_float2(1.f, OLS_C1), make_float2(OLS_H, OLS_S1), make_float2(0.f, -OLS_S1), make_float2(-OLS_H, -OLS_C1)};
-    const pk t1i[4] = {make_float2(0.f, OLS_S1), make_float2(OLS_H, OLS_C1), make_float2(1.f, OLS_C1), make_float2(OLS_H, OLS_S1)};
-#pragma unroll
-    for (int m = 0; m < 4; m++) {
-        cp t = cmulc(P[m + 4], t1r[m], t1i[m]);
-        cp u = P[m];
-        P[m] = cadd(u, t);
-        P[m + 4] = csub(u, t);
-    }
-}
 
 // bit reversal of a 4-bit index (host + device)
 __host__ __device__ __forceinline__ int bitrev4(int j) { return ((j & 1) << 3) | ((j & 2) << 1) | ((j & 4) >> 1) | ((j & 8) >> 3); }
-// frequency index held at block position p after F1, F2, F3
-__host__ __device__ __forceinline__ int freq_of_pos(int p) {
-    const int k0 = p >> 8, k1 = (p >> 4) & 15, jj = p & 15;
-    return k0 + 16 * k1 + 256 * bitrev4(jj);
-}
 
 }  // namespace ols16
 }  // namespace bdsp

@@ -30,20 +30,7 @@ using namespace cx;
 
 #define OI_M 4096
 #define OI_T 128
-// spectrum H through the texture path (0) or as plain 128-bit global loads (1)
-#ifndef OI_H_LDG
-#define OI_H_LDG 0
-#endif
-// 1: request the spectrum values of a half before its shared loads and transform (32 more live registers)
-#ifndef OI_H_EARLY
-#define OI_H_EARLY 0
-#endif
-#ifndef OLS_L2_AHEAD
-#define OLS_L2_AHEAD 0   // blocks ahead (740 = resident CTAs): measured 0.3194 vs 0.3183 ms without - off
-#endif
-#ifndef OI_MIN_CTAS
 #define OI_MIN_CTAS 5
-#endif
 
 // twiddle table (float2): [0,256) W4096^col; [256 + 16 k + c] W256^{k c}, k, c in [0,16)
 #define OI_TW_C2 (256 + 256)
@@ -55,7 +42,7 @@ using namespace cx;
 template <bool ALIGNED>
 __global__ void __launch_bounds__(OI_T, OI_MIN_CTAS)
 ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int m_first, int step, int shift,
-                int blocks_per_vec, const float2* __restrict__ tw, cudaTextureObject_t htex, const float4* __restrict__ hpos) {
+                int blocks_per_vec, const float2* __restrict__ tw, cudaTextureObject_t htex) {
     __shared__ __align__(16) float2 sm[OI_M];
     const int t = threadIdx.x;
     const int vec = blockIdx.x / blocks_per_vec;
@@ -73,22 +60,6 @@ ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
         const int col = 2 * t;
         // block position p holds x[(p0 + p) mod N], p0 = i0 + shift - m_first  (p0 > -4096, even)
         const int p0 = i0 + shift - m_first;
-#if OLS_L2_AHEAD > 0
-        // one thread asks L2 for the NEW inputs (step points) of the block that takes this CTA's slot next: blocks are
-        // scheduled in index order, so block index + (resident CTAs of the grid) starts about when this one ends
-        if (ALIGNED && t == 0) {
-            const long long nb = (long long)blockIdx.x + OLS_L2_AHEAD;
-            if (nb < (long long)gridDim.x) {
-                const long long nvec = nb / blocks_per_vec;
-                const int nblk = (int)(nb - nvec * blocks_per_vec);
-                const long long q0 = (long long)nblk * step + shift - m_first + (OI_M - step);   // first input not shared with its predecessor
-                if (q0 >= 0 && q0 + step <= N) {
-                    const float2* pf = x + (size_t)nvec * (size_t)N + q0;
-                    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(pf), "r"(step * 8) : "memory");
-                }
-            }
-        }
-#endif
         if (p0 >= 0 && p0 + OI_M <= N) {   // block-uniform: no wrap-around inside this block
             const float2* px = xr + p0 + col;
 #pragma unroll
@@ -114,13 +85,11 @@ ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
                 idx += 256; if (idx >= N) idx -= N;
             }
         }
-        if (!(OI_ABLATE & 4)) {
         r16<false>(v);
         r16<false>(u);
         const float4 w = __ldg(reinterpret_cast<const float4*>(tw + col));
         apply_twiddles<true>(v, make_float2(w.x, w.y));
         apply_twiddles<true>(u, make_float2(w.z, w.w));
-        }
         float2* dst = sm + 16 * hi + ((2 * lo) ^ (2 * (hi & 7)));
 #pragma unroll
         for (int s = 0; s < 16; s++)
@@ -137,11 +106,9 @@ ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
             v[b] = make_float2(f.x, f.y);
             u[b] = make_float2(f.z, f.w);
         }
-        if (!(OI_ABLATE & 2)) {
         r16<false>(v);
         r16<false>(u);
         oi_tw2<true, false, 8>(v, u, tw2);
-        }
 #pragma unroll
         for (int s = 0; s < 16; s++) {
             const int k1 = r16_k(s);
@@ -153,11 +120,6 @@ ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
 #pragma unroll 1
     for (int half = 0; half < 2; half++) {
         float2* grp = row + 16 * (lo + 8 * half);
-#if OI_H_EARLY
-        float4 hq[8];      // spectrum values of this half, requested before the shared loads and the transform
-#pragma unroll
-        for (int q = 0; q < 8; q++) hq[q] = tex1Dfetch<float4>(htex, (half * 8 + q) * OI_T + t);
-#endif
         c2 P[16];
 #pragma unroll
         for (int q = 0; q < 8; q++) {
@@ -165,19 +127,15 @@ ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
             P[2 * q] = make_float2(f.x, f.y);
             P[2 * q + 1] = make_float2(f.z, f.w);
         }
-        if (!(OI_ABLATE & 1)) fft_dif<4, false>(P);
+        fft_dif<4, false>(P);
 #pragma unroll
         for (int q = 0; q < 8; q++) {
             // plan layout: [half][q][thread] float4 = H of positions c = 2q, 2q + 1 -> a warp reads 512 contiguous bytes
-#if OI_H_EARLY
-            const float4 h = hq[q];
-#else
-            const float4 h = (OI_ABLATE & 8) ? make_float4(1.f, 0.f, 1.f, 0.f) : OI_H_LDG ? __ldg(hpos + (half * 8 + q) * OI_T + t) : tex1Dfetch<float4>(htex, (half * 8 + q) * OI_T + t);
-#endif
+            const float4 h = tex1Dfetch<float4>(htex, (half * 8 + q) * OI_T + t);
             P[2 * q] = mul(P[2 * q], make_float2(h.x, h.y));
             P[2 * q + 1] = mul(P[2 * q + 1], make_float2(h.z, h.w));
         }
-        if (!(OI_ABLATE & 1)) fft_dit<4, true>(P);
+        fft_dit<4, true>(P);
 #pragma unroll
         for (int q = 0; q < 8; q++)
             *reinterpret_cast<float4*>(grp + 2 * (q ^ lo)) = make_float4(P[2 * q].x, P[2 * q].y, P[2 * q + 1].x, P[2 * q + 1].y);
@@ -191,11 +149,9 @@ ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
             v[k1] = make_float2(f.x, f.y);
             u[k1] = make_float2(f.z, f.w);
         }
-        if (!(OI_ABLATE & 2)) {
         oi_tw2<false, true, 8>(v, u, tw2);
         r16<true>(v);
         r16<true>(u);
-        }
 #pragma unroll
         for (int s = 0; s < 16; s++) {
             const int b = r16_k(s);
@@ -213,13 +169,11 @@ ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
             v[k0] = make_float2(f.x, f.y);
             u[k0] = make_float2(f.z, f.w);
         }
-        if (!(OI_ABLATE & 4)) {
         const float4 w = __ldg(reinterpret_cast<const float4*>(tw + col));
         apply_twiddles<false>(v, make_float2(w.x, -w.y));
         apply_twiddles<false>(u, make_float2(w.z, -w.w));
         r16<true>(v);
         r16<true>(u);
-        }
         // output i = i0 + m, m = col + 256 a - m_first in [0, step) and i < N
         const int mlo = col - m_first;                     // m for a = 0
         int mhi = step;                                    // exclusive bound on m
@@ -308,7 +262,7 @@ int ols4096_prepare(const void* Hs, void* Hpos, size_t L, cudaStream_t st) {
     return 0;
 }
 
-int ols4096_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, const void* Hpos, cudaTextureObject_t htex, cudaStream_t st) {
+int ols4096_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, cudaTextureObject_t htex, cudaStream_t st) {
     if (x == y) { set_last_error("ols4096_convolve: in-place operation is not supported"); return -3; }
     int d, shift, m_first, step;
     olsi_geometry(OI_M, L, &d, &shift, &m_first, &step);
@@ -320,10 +274,10 @@ int ols4096_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, c
     const bool aligned = (N % 2 == 0) && ((reinterpret_cast<uintptr_t>(y) & 15) == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
     if (aligned)
         BDSP_CUDA_OK(launch_pdl(ols4096i_kernel<true>, dim3((unsigned)grid), dim3(OI_T), 0, st, reinterpret_cast<const float2*>(x),
-                                reinterpret_cast<float2*>(y), (int)N, m_first, step, shift, (int)bpv, tw, htex, reinterpret_cast<const float4*>(Hpos)));
+                                reinterpret_cast<float2*>(y), (int)N, m_first, step, shift, (int)bpv, tw, htex));
     else
         BDSP_CUDA_OK(launch_pdl(ols4096i_kernel<false>, dim3((unsigned)grid), dim3(OI_T), 0, st, reinterpret_cast<const float2*>(x),
-                                reinterpret_cast<float2*>(y), (int)N, m_first, step, shift, (int)bpv, tw, htex, reinterpret_cast<const float4*>(Hpos)));
+                                reinterpret_cast<float2*>(y), (int)N, m_first, step, shift, (int)bpv, tw, htex));
     BDSP_LAUNCHED();
     return 0;
 }

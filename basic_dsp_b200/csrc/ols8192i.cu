@@ -30,14 +30,9 @@ namespace bdsp {
 
 using namespace cx;
 
-#ifndef OLS_L2_AHEAD
-#define OLS_L2_AHEAD 0   // blocks ahead (296 = resident CTAs): measured 0.396 vs 0.398 ms without at 2047 taps - off
-#endif
 #define O8_M 8192
 #define O8_T 256
-#ifndef O8_MIN_CTAS
 #define O8_MIN_CTAS 2
-#endif
 #define O8_SMEM_BYTES (O8_M * sizeof(float2))
 
 // twiddle table (float2): [0,512) W8192^col; [512 + 32 k + c] W512^{k c}, k in [0,16), c in [0,32)
@@ -64,22 +59,6 @@ ols8192i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
         const int col = 2 * t;
         // block position p holds x[(p0 + p) mod N], p0 = i0 + shift - m_first  (p0 > -8192, even)
         const int p0 = i0 + shift - m_first;
-#if OLS_L2_AHEAD > 0
-        // one thread asks L2 for the NEW inputs (step points) of the block that takes this CTA's slot next: blocks are
-        // scheduled in index order, so block index + (resident CTAs of the grid) starts about when this one ends
-        if (ALIGNED && t == 0) {
-            const long long nb = (long long)blockIdx.x + OLS_L2_AHEAD;
-            if (nb < (long long)gridDim.x) {
-                const long long nvec = nb / blocks_per_vec;
-                const int nblk = (int)(nb - nvec * blocks_per_vec);
-                const long long q0 = (long long)nblk * step + shift - m_first + (O8_M - step);   // first input not shared with its predecessor
-                if (q0 >= 0 && q0 + step <= N) {
-                    const float2* pf = x + (size_t)nvec * (size_t)N + q0;
-                    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(pf), "r"(step * 8) : "memory");
-                }
-            }
-        }
-#endif
         if (p0 >= 0 && p0 + O8_M <= N) {   // block-uniform: no wrap-around inside this block
             const float2* px = xr + p0 + col;
 #pragma unroll
@@ -290,9 +269,7 @@ long long ols8192_blocks(size_t N, size_t L) {
     return ((long long)N + step - 1) / step;
 }
 
-int ols8192_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, const void* Hpos, cudaTextureObject_t htex,
-                     cudaStream_t st) {
-    (void)Hpos;
+int ols8192_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, cudaTextureObject_t htex, cudaStream_t st) {
     if (x == y) { set_last_error("ols8192_convolve: in-place operation is not supported"); return -3; }
     int d, shift, m_first, step;
     olsi_geometry(O8_M, L, &d, &shift, &m_first, &step);

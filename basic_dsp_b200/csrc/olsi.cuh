@@ -5,47 +5,15 @@
 namespace bdsp {
 using namespace cx;
 
-// block inputs are used once: OI_X_LOAD = 1 (L1::no_allocate) / 2 (ld.global.cg, L2 only) keep them from displacing the
-// spectrum and the twiddles in L1
-#ifndef OI_X_LOAD
-#define OI_X_LOAD 0
-#endif
-__device__ __forceinline__ float4 ld_x4(const float2* p) {
-#if OI_X_LOAD == 1
-    float4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    return r;
-#elif OI_X_LOAD == 2
-    float4 r;
-    asm volatile("ld.global.cg.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    return r;
-#else
-    return __ldg(reinterpret_cast<const float4*>(p));
-#endif
-}
-// stride-16 stage twiddles W256^{k c}, k = 1..15: 0 = fifteen 128-bit table loads per stage (4-5 L1 wavefronts each:
-// 16 % of the kernel's L1 data-pipe traffic, which is its saturated unit), 1 = six loads (k = 1, 2, 3, 4, 8, 12) +
-// nine products, 2 = one load + the power scheme of the stride-256 stages
-// measurement only (results become wrong): bit 0 = no F3|H|I3 arithmetic, 1 = no stride-16 stages' arithmetic, 2 = no
-// stride-256 stages' arithmetic, 3 = no H fetch, 4 = no shared-memory traffic in the middle section
-#ifndef OI_ABLATE
-#define OI_ABLATE 0
-#endif
-#ifndef OI_TW2_MODE
-#define OI_TW2_MODE 1
-#endif
+// two adjacent block inputs as one 128-bit read-only load
+__device__ __forceinline__ float4 ld_x4(const float2* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
+// stride-16 stage twiddles W256^{k c}, k = 1..15: six 128-bit table loads (k = 1, 2, 3, 4, 8, 12) and nine products.
+// Fifteen loads per stage (4-5 L1 wavefronts each) were 16 % of the kernel's L1 data-pipe traffic, which is its saturated
+// unit.
 // v[s] *= W^{k(s)} (CONJ: conjugated), k(s) = SLOTMAP ? r16_k(s) : s, for the two columns held in v / u
 // tw2[STRIDE * k]: float4 = W^{k c}, W^{k (c + 1)} of the thread's two columns
 template <bool SLOTMAP, bool CONJ, int STRIDE>
 __device__ __forceinline__ void oi_tw2(c2 (&v)[16], c2 (&u)[16], const float4* __restrict__ tw2) {
-#if OI_TW2_MODE == 0
-#pragma unroll
-    for (int s = 1; s < 16; s++) {
-        const float4 f = __ldg(tw2 + STRIDE * (SLOTMAP ? r16_k(s) : s));
-        v[s] = CONJ ? mul_conj(v[s], make_float2(f.x, f.y)) : mul(v[s], make_float2(f.x, f.y));
-        u[s] = CONJ ? mul_conj(u[s], make_float2(f.z, f.w)) : mul(u[s], make_float2(f.z, f.w));
-    }
-#elif OI_TW2_MODE == 1
     c2 Av[4], Bv[4], Au[4], Bu[4];
 #pragma unroll
     for (int i = 1; i < 4; i++) {
@@ -62,11 +30,6 @@ __device__ __forceinline__ void oi_tw2(c2 (&v)[16], c2 (&u)[16], const float4* _
         v[s] = mul(v[s], wv);
         u[s] = mul(u[s], wu);
     }
-#else
-    const float4 f = __ldg(tw2 + STRIDE);
-    apply_twiddles<SLOTMAP>(v, make_float2(f.x, CONJ ? -f.y : f.y));
-    apply_twiddles<SLOTMAP>(u, make_float2(f.z, CONJ ? -f.w : f.w));
-#endif
 }
 
 // plan geometry shared by prepare and convolve (block length M): the delay d in {0, 1} samples that the plan folds

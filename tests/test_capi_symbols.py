@@ -83,6 +83,24 @@ def test_product_does_not_import_the_oracle():
                 assert "oracle" not in text.replace("no CPU fallback", ""), os.path.join(dirpath, f)
 
 
+def test_every_cuda_source_is_built():
+    from basic_dsp_b200 import build
+    on_disk = {f for f in os.listdir(build.CSRC) if f.endswith(".cu")}
+    assert on_disk == set(build.SOURCES), (sorted(on_disk - set(build.SOURCES)), sorted(set(build.SOURCES) - on_disk))
+
+
+def test_one_build_one_code_path():
+    """The shipped kernels are the only kernels: no build switches, no environment overrides in the CUDA sources."""
+    from basic_dsp_b200 import build
+    offenders = []
+    for f in sorted(os.listdir(build.CSRC)):
+        if f.endswith((".cu", ".cuh")):
+            for i, line in enumerate(open(os.path.join(build.CSRC, f)), 1):
+                if "getenv" in line or re.match(r"\s*#\s*(if|ifdef|ifndef|elif)\b", line):
+                    offenders.append("%s:%d: %s" % (f, i, line.strip()))
+    assert not offenders, offenders
+
+
 def _build_cpp(tmp_path, libpath):
     exe = str(tmp_path / "host_mirror")
     src = os.path.join(ROOT, "tests", "cpp", "host_mirror.cpp")
