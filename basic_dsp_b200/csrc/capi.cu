@@ -379,47 +379,35 @@ inline void table_consumed() {
 }
 
 // ---- convolution -----------------------------------------------------------------------------------
-// circular FIR / fast convolution dispatch for taps resident on the device
-struct PlanCache {   // where convolve_taps may keep the plan between calls (an impulse-response vector)
-    std::mutex* mu;
-    std::shared_ptr<OlsPlan>* plan;
-    unsigned long long* plan_version;
-    int* plan_complex_signal;
-    unsigned long long version;
-};
+// convolution with taps resident on the device; h: the impulse-response vector that caches the overlap-save plan of
+// these taps between calls, or nullptr (the plan is then made for this call only)
 inline std::shared_ptr<OlsPlan> own_plan(OlsPlan* p) { return std::shared_ptr<OlsPlan>(p, [](OlsPlan* q) { ols_plan_destroy(q); }); }
 
 template <typename T>
-int convolve_taps(Vec<T>* v, const T* h_dev, size_t L, bool h_complex, PlanCache* cache) {
+int convolve_taps(Vec<T>* v, const T* h_dev, size_t L, bool h_complex, Vec<T>* h) {
     const size_t N = points_of(v);
     int rc = ensure_scratch(v, v->len);
     if (rc) return rc;
-    const size_t cl = L - L / 2;
-    const size_t direct_max = h_complex ? 24 : 96;
-    if (L <= direct_max) {
-        rc = fir_convolve<T>(v->d, v->scratch, h_dev, N, 1, L, cl, v->is_complex, h_complex, g_stream);
-    } else if (L <= ols_max_taps<T>()) {
-        std::shared_ptr<OlsPlan> plan;
-        if (cache) {
-            std::lock_guard<std::mutex> lk(*cache->mu);
-            if (*cache->plan && *cache->plan_version == cache->version && *cache->plan_complex_signal == v->is_complex)
-                plan = *cache->plan;
+    std::shared_ptr<OlsPlan> plan;
+    if (conv_needs_plan<T>(L, !h_complex)) {
+        if (h) {
+            std::lock_guard<std::mutex> lk(h->plan_mu);
+            if (h->plan && h->plan_version == h->version && h->plan_complex_signal == v->is_complex)
+                plan = h->plan;
             else {
                 plan = own_plan(ols_plan_create<T>(h_dev, L, !h_complex, v->is_complex != 0, g_stream));
                 if (!plan) return -1;
                 // other streams may use the plan as soon as it is published
                 BDSP_CUDA_OK(cudaStreamSynchronize(g_stream));
-                *cache->plan = plan; *cache->plan_version = cache->version; *cache->plan_complex_signal = v->is_complex;
+                h->plan = plan; h->plan_version = h->version; h->plan_complex_signal = v->is_complex;
             }
         } else {
             plan = own_plan(ols_plan_create<T>(h_dev, L, !h_complex, v->is_complex != 0, g_stream));
             if (!plan) return -1;
         }
-        rc = ols_plan_convolve<T>(plan.get(), v->d, v->scratch, N, 1, !v->is_complex, g_stream);
-        // an uncached plan is destroyed here (ols_plan_destroy synchronises the device first)
-    } else {
-        rc = fft_convolve_full<T>(v->d, v->scratch, h_dev, N, 1, L, !v->is_complex, !h_complex, g_stream);
     }
+    rc = convolve<T>(v->d, v->scratch, N, 1, !v->is_complex, h_dev, L, !h_complex, plan.get(), g_stream);
+    // an uncached plan is destroyed here (ols_plan_destroy synchronises the device first)
     if (rc) return rc;
     trade(v);
     return 0;
@@ -480,8 +468,7 @@ template <typename T> Res<T> op_convolve_signal(Vec<T>* v, Vec<T>* h) {
         if (N) cudaMemsetAsync(v->d, 0, v->len * sizeof(T), g_stream);
         return done(v, 0);
     }
-    PlanCache cache{&h->plan_mu, &h->plan, &h->plan_version, &h->plan_complex_signal, h->version};
-    return done(v, convolve_taps<T>(v, h->d, L, h->is_complex, &cache));
+    return done(v, convolve_taps<T>(v, h->d, L, h->is_complex, h));
 }
 
 // More taps than points: the tap window wraps around the vector (the reference's ReverseWrappingIterator,
@@ -1317,8 +1304,8 @@ int scale_mul_mag_phase(Vec<T>* v, T cre, T cim, const Vec<T>* w, Vec<T>* mag, V
 struct ConvPlan {
     int is64;
     size_t L;
-    OlsPlan* ols;   // overlap-save plan or nullptr
-    void* taps;     // copy of the taps (L complex) for the direct / full-length paths
+    OlsPlan* ols;   // overlap-save plan of the taps, where convolve() needs one
+    void* taps;     // copy of the taps (L complex)
 };
 
 template <typename T> ConvPlan* conv_plan_create(const void* h_dev, size_t L) {
@@ -1328,7 +1315,7 @@ template <typename T> ConvPlan* conv_plan_create(const void* h_dev, size_t L) {
     p->is64 = sizeof(T) == 8; p->L = L; p->ols = nullptr; p->taps = nullptr;
     if (cudaMalloc(&p->taps, L * sizeof(C)) != cudaSuccess) { delete p; return nullptr; }
     cudaMemcpyAsync(p->taps, h_dev, L * sizeof(C), cudaMemcpyDeviceToDevice, g_stream);
-    if (L > 24 && L <= ols_max_taps<T>()) {
+    if (conv_needs_plan<T>(L, 0)) {
         p->ols = ols_plan_create<T>(p->taps, L, 0, true, g_stream);
         if (!p->ols) { cudaFree(p->taps); delete p; return nullptr; }
     }
@@ -1339,9 +1326,7 @@ template <typename T> int conv_rows(const void* in, void* out, size_t points, si
     if (!p || p->is64 != (sizeof(T) == 8)) { set_last_error("conv rows: plan precision mismatch"); return -2; }
     if (points < p->L) return E_ARG_LEN;
     if (!points || !rows) return 0;
-    if (p->ols) return ols_plan_convolve<T>(p->ols, in, out, points, rows, 0, g_stream);
-    if (p->L <= 24) return fir_convolve<T>(in, out, p->taps, points, rows, p->L, p->L - p->L / 2, 1, 1, g_stream);
-    return fft_convolve_full<T>(in, out, p->taps, points, rows, p->L, 0, 0, g_stream);
+    return convolve<T>(in, out, points, rows, 0, p->taps, p->L, 0, p->ols, g_stream);
 }
 
 template <typename T> int fft_rows(const void* in, void* out, size_t points, size_t rows, int flags) {

@@ -6,11 +6,18 @@
 //  convolve_iteration, time_freq/mod.rs:456-473).  They replace the reference's overlap_discard
 // (convolution.rs:304-461), its SIMD FIR (time_freq/mod.rs:531-610) and its OpenCL kernels
 // conv_vecs_r/conv_vecs_c/multiply_vector (gpu_support/ocl/ocl_kernels32.rs).
+#include <math.h>
+
+#include <map>
+#include <mutex>
 #include <type_traits>
+#include <utility>
+#include <vector>
 
 #include "conv.cuh"
 #include "fft.cuh"
 #include "fft_core.cuh"
+#include "olsi.cuh"
 
 namespace bdsp {
 
@@ -97,15 +104,13 @@ template <typename T> size_t ols_block_len(size_t L, bool complex_signal) {
     return m;
 }
 
-template <typename T> size_t ols_max_taps() { return fft_block_max_n<T>() / 2; }
+// largest L the overlap-save blocks take
+template <typename T> static size_t ols_max_taps() { return fft_block_max_n<T>() / 2; }
 
-bool ols4096_applicable(size_t N, size_t L, size_t M);
 int ols4096_prepare(const void* Hs, void* Hpos, size_t L, cudaStream_t st);
 int ols4096_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, cudaTextureObject_t htex, cudaStream_t st);
-bool ols8192_applicable(size_t N, size_t L);
 int ols8192_prepare(const void* Hs, void* Hpos, size_t L, cudaStream_t st);
 int ols8192_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, cudaTextureObject_t htex, cudaStream_t st);
-long long ols8192_blocks(size_t N, size_t L);
 bool ols64_applicable(size_t N, size_t L, size_t M);
 int ols64_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, const void* Hs, cudaStream_t st);
 
@@ -155,15 +160,6 @@ OlsPlan* ols_plan_create(const void* h, size_t L, int h_is_real, bool complex_si
         p->M2 = 8192;
         rc = ols_spectrum<T>(h, L, h_is_real, p->M2, true, &p->Hs2, &p->htex2, st);
     }
-    if (!rc && sizeof(T) == 4 && complex_signal && L > 4094) {
-        const size_t bytes = L * (h_is_real ? sizeof(T) : sizeof(typename CpxOf<T>::type));
-        if (cudaMalloc(&p->taps_dev, bytes) != cudaSuccess ||
-            cudaMemcpyAsync(p->taps_dev, h, bytes, cudaMemcpyDeviceToDevice, st) != cudaSuccess) {
-            cudaGetLastError();
-            if (p->taps_dev) cudaFree(p->taps_dev);
-            p->taps_dev = nullptr;   // not fatal: such plans use the generic blocks
-        }
-    }
     if (rc) { ols_plan_destroy(p); return nullptr; }
     return p;
 }
@@ -178,40 +174,48 @@ void ols_plan_destroy(OlsPlan* p) {
     if (p->htex2) cudaDestroyTextureObject(p->htex2);
     if (p->Hs) cudaFree(p->Hs);
     if (p->Hs2) cudaFree(p->Hs2);
-    if (p->taps_dev) cudaFree(p->taps_dev);
     if (cur != p->device) cudaSetDevice(cur);
     delete p;
 }
 
-// Choice between the two fused block lengths where both apply (2 <= L <= 2046).  Measured on B200, 64 x 2^20 points
-// (profiles/r2_ols_block_choice.txt): per POINT the 4096-point kernel is ~20 % faster (four independently phased CTAs per
-// SM against two), so the 8192-point kernel only wins once its better block efficiency (M - L)/M outweighs that.
-#define BDSP_OLS8192_MIN_TAPS 1450
-#define BDSP_OLS8192_MIN_BLOCKS 592
-
-template <typename T>
-int ols_plan_convolve(const OlsPlan* p, const void* x, void* y, size_t N, size_t batch, int is_real, cudaStream_t st) {
-    typedef typename CpxOf<T>::type C;
-    if (!p || p->is64 != (sizeof(T) == 8)) { set_last_error("ols_convolve: plan precision mismatch"); return -2; }
-    if (x == y) { set_last_error("ols_convolve: in-place operation is not supported"); return -3; }
-    const size_t L = p->L, M = p->M;
-    // c32 responses beyond the fused blocks (4095 .. 8192 taps) on power-of-two vectors with packed multi-pass transforms:
-    // forward transform + inverse transform with the spectrum multiply on its first load (2 x 2 passes over HBM) beats the
-    // generic 16384-point overlap-save blocks (64 x 2^20, 8191 taps: 1.79 ms)
-    if (sizeof(T) == 4 && !is_real && L > 4094 && is_pow2(N) && N >= (1u << 15) && N <= (1u << 24) && p->taps_dev)
-        return fft_convolve_full<T>(x, y, p->taps_dev, N, batch, L, 0, p->h_is_real, st);
-    if (sizeof(T) == 4 && !is_real) {
-        // (ols8192_blocks divides by the block step, which is only positive for applicable lengths)
-        const bool want8 = ols8192_applicable(N, L) && L >= BDSP_OLS8192_MIN_TAPS &&
-                           ols8192_blocks(N, L) * (long long)batch >= BDSP_OLS8192_MIN_BLOCKS;
-        if (p->htex2 && want8)
-            return ols8192_convolve(x, y, N, batch, L, p->htex2, st);
-        if (p->htex && M == 4096 && ols4096_applicable(N, L, M))
-            return ols4096_convolve(x, y, N, batch, L, p->htex, st);
-        if (p->htex && M == 8192 && ols8192_applicable(N, L))
-            return ols8192_convolve(x, y, N, batch, L, p->htex, st);
+const float2* olsi_twiddles(int M) {
+    int d = 0;
+    if (cudaGetDevice(&d) != cudaSuccess) { set_last_error("ols%d: cudaGetDevice failed", M); return nullptr; }
+    static std::mutex mu;
+    static std::map<std::pair<int, int>, float2*> tables;   // (device, M)
+    std::lock_guard<std::mutex> lk(mu);
+    auto it = tables.find({d, M});
+    if (it != tables.end()) return it->second;
+    const int n1 = M / 16, n2 = M / 256;
+    std::vector<float2> h(2 * n1);
+    const long double tau = 2.0L * 3.14159265358979323846264338327950288L;
+    for (int c = 0; c < n1; c++) {
+        h[c].x = (float)cosl(-tau * (long double)c / (long double)M);
+        h[c].y = (float)sinl(-tau * (long double)c / (long double)M);
     }
-    if (sizeof(T) == 8 && !is_real && ols64_applicable(N, L, M)) return ols64_convolve(x, y, N, batch, L, p->Hs, st);   // fused 4096-point c64 blocks
+    for (int k = 0; k < 16; k++)
+        for (int c = 0; c < n2; c++) {
+            const long double a = -tau * (long double)((k * c) % n1) / (long double)n1;
+            h[n1 + n2 * k + c].x = (float)cosl(a);
+            h[n1 + n2 * k + c].y = (float)sinl(a);
+        }
+    float2* dev = nullptr;
+    if (cudaMalloc(&dev, h.size() * sizeof(float2)) != cudaSuccess ||
+        cudaMemcpy(dev, h.data(), h.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess) {
+        if (dev) cudaFree(dev);
+        cudaGetLastError();
+        set_last_error("ols%d: twiddle table allocation failed", M);
+        return nullptr;
+    }
+    tables[{d, M}] = dev;
+    return dev;
+}
+
+// generic overlap-save blocks of the plan's length M
+template <typename T>
+static int ols_generic_convolve(const OlsPlan* p, const void* x, void* y, size_t N, size_t batch, int is_real, cudaStream_t st) {
+    typedef typename CpxOf<T>::type C;
+    const size_t L = p->L, M = p->M;
     const size_t step = M - L + 1;
     const long long bpv = (long long)((N + step - 1) / step);
     const int log2M = ilog2(M);
@@ -337,9 +341,10 @@ fir_kernel(const void* __restrict__ x_, void* __restrict__ y_, const void* __res
 }
 
 template <typename T>
-int fir_convolve(const void* x, void* y, const void* h, size_t N, size_t batch, size_t L, size_t cl, int x_complex,
-                 int h_complex, cudaStream_t st) {
+static int fir_convolve(const void* x, void* y, const void* h, size_t N, size_t batch, size_t L, int x_complex, int h_complex,
+                        cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
+    const size_t cl = L - L / 2;
     if (x == y) { set_last_error("fir_convolve: in-place operation is not supported"); return -3; }
     const long long tpv = (long long)((N + FIR_TILE - 1) / FIR_TILE);
     const size_t W = FIR_TILE + L - 1 + FIR_U + 1;
@@ -401,8 +406,8 @@ __global__ void complex_to_real_kernel(const typename CpxOf<T>::type* __restrict
 }
 
 template <typename T>
-int fft_convolve_full(const void* x, void* y, const void* h, size_t N, size_t batch, size_t L, int is_real,
-                      int h_is_real, cudaStream_t st) {
+static int fft_convolve_full(const void* x, void* y, const void* h, size_t N, size_t batch, size_t L, int is_real,
+                             int h_is_real, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
     const size_t cl = L - L / 2;
     // slots 4 / 5: fft_exec below uses slots 0..2 for its own passes (mixed-radix interleave, chirp-z ping-pong)
@@ -438,12 +443,49 @@ int fft_convolve_full(const void* x, void* y, const void* h, size_t N, size_t ba
     return 0;
 }
 
+// Choice between the two fused block lengths where both apply (2 <= L <= 2046).  Measured on B200, 64 x 2^20 points
+// (profiles/r2_ols_block_choice.txt): per POINT the 4096-point kernel is ~20 % faster (four independently phased CTAs per
+// SM against two), so the 8192-point kernel only wins once its better block efficiency (M - L)/M outweighs that.
+#define BDSP_OLS8192_MIN_TAPS 1450
+#define BDSP_OLS8192_MIN_BLOCKS 592
+
+// direct FIR up to this many taps
+static size_t fir_max_taps(int h_is_real) { return h_is_real ? 96 : 24; }
+
+template <typename T> bool conv_needs_plan(size_t L, int h_is_real) { return L > fir_max_taps(h_is_real) && L <= ols_max_taps<T>(); }
+
+template <typename T>
+int convolve(const void* x, void* y, size_t N, size_t batch, int x_is_real, const void* h, size_t L, int h_is_real,
+             const OlsPlan* p, cudaStream_t st) {
+    if (L <= fir_max_taps(h_is_real)) return fir_convolve<T>(x, y, h, N, batch, L, !x_is_real, !h_is_real, st);
+    if (L > ols_max_taps<T>()) return fft_convolve_full<T>(x, y, h, N, batch, L, x_is_real, h_is_real, st);
+    if (!p || p->is64 != (sizeof(T) == 8) || p->L != L) { set_last_error("convolve: %zu taps need their overlap-save plan", L); return -2; }
+    if (x == y) { set_last_error("ols_convolve: in-place operation is not supported"); return -3; }
+    const size_t M = p->M;
+    if (sizeof(T) == 4 && !x_is_real) {
+        // c32 responses beyond the fused blocks (4095 .. 8192 taps) on power-of-two vectors with packed multi-pass transforms:
+        // forward transform + inverse transform with the spectrum multiply on its first load (2 x 2 passes over HBM) beats
+        // the generic 16384-point overlap-save blocks (64 x 2^20, 8191 taps: 1.79 ms)
+        if (L > 4094 && is_pow2(N) && N >= (1u << 15) && N <= (1u << 24))
+            return fft_convolve_full<T>(x, y, h, N, batch, L, 0, h_is_real, st);
+        // (olsi_blocks divides by the block step, which is only positive for applicable lengths)
+        const bool want8 = olsi_applicable(8192, N, L) && L >= BDSP_OLS8192_MIN_TAPS &&
+                           olsi_blocks(8192, N, L) * (long long)batch >= BDSP_OLS8192_MIN_BLOCKS;
+        if (p->htex2 && want8)
+            return ols8192_convolve(x, y, N, batch, L, p->htex2, st);
+        if (p->htex && M == 4096 && olsi_applicable(4096, N, L))
+            return ols4096_convolve(x, y, N, batch, L, p->htex, st);
+        if (p->htex && M == 8192 && olsi_applicable(8192, N, L))
+            return ols8192_convolve(x, y, N, batch, L, p->htex, st);
+    }
+    if (sizeof(T) == 8 && !x_is_real && ols64_applicable(N, L, M)) return ols64_convolve(x, y, N, batch, L, p->Hs, st);   // fused 4096-point c64 blocks
+    return ols_generic_convolve<T>(p, x, y, N, batch, x_is_real, st);
+}
+
 #define BDSP_INST(T)                                                                                                    \
-    template size_t ols_max_taps<T>();                                                                                  \
     template OlsPlan* ols_plan_create<T>(const void*, size_t, int, bool, cudaStream_t);                                 \
-    template int ols_plan_convolve<T>(const OlsPlan*, const void*, void*, size_t, size_t, int, cudaStream_t);           \
-    template int fir_convolve<T>(const void*, void*, const void*, size_t, size_t, size_t, size_t, int, int, cudaStream_t); \
-    template int fft_convolve_full<T>(const void*, void*, const void*, size_t, size_t, size_t, int, int, cudaStream_t);
+    template bool conv_needs_plan<T>(size_t, int);                                                                      \
+    template int convolve<T>(const void*, void*, size_t, size_t, int, const void*, size_t, int, const OlsPlan*, cudaStream_t);
 BDSP_INST(float)
 BDSP_INST(double)
 #undef BDSP_INST

@@ -4,9 +4,6 @@
 
 namespace bdsp {
 
-// largest L the overlap-save kernels support
-template <typename T> size_t ols_max_taps();
-
 // Overlap-save plan of one impulse response (the reference recomputes this spectrum inside every
 // convolve_signal call, convolution.rs:333-339,419-425).  Immutable after ols_plan_create, so any number of
 // threads / streams of the creating device may convolve with it concurrently.  Destruction synchronises the device.
@@ -22,22 +19,20 @@ struct OlsPlan {
     size_t M2 = 0;
     void* Hs2 = nullptr;
     cudaTextureObject_t htex2 = 0;
-    // c32 responses longer than the fused blocks: the plan's own copy of the taps (L real or complex values) for the
-    // full-length frequency-domain path, which power-of-two vectors take instead of the generic blocks
-    void* taps_dev = nullptr;
 };
 // h: L complex (or real) taps on the device.  complex_signal: the vectors that will be convolved are complex.
 template <typename T> OlsPlan* ols_plan_create(const void* h, size_t L, int h_is_real, bool complex_signal, cudaStream_t st);
 void ols_plan_destroy(OlsPlan* p);
-// y <- centred circular convolution of every one of `batch` vectors of N points (x != y)
-template <typename T> int ols_plan_convolve(const OlsPlan* p, const void* x, void* y, size_t N, size_t batch, int is_real, cudaStream_t st);
-// direct form, y[i] = sum_k x[(i + cl - 1 - k) mod N] h[k]
+
+// true where convolve() runs overlap-save blocks and so needs a plan of h
+template <typename T> bool conv_needs_plan(size_t L, int h_is_real);
+// y <- centred circular convolution y[i] = sum_{k<L} x[(i + cl - 1 - k) mod N] h[k], cl = L - L/2, of every one of
+// `batch` vectors of N points (x != y) with the L taps h (device).  Chooses the direct FIR, an overlap-save kernel or
+// the full-length FFT path.  `plan` is required when conv_needs_plan<T>(L, h_is_real), otherwise ignored: the plan of
+// these taps, made for complex signals when x_is_real is 0 and for real ones otherwise.  h must stay valid until the
+// call's kernels have run.
 template <typename T>
-int fir_convolve(const void* x, void* y, const void* h, size_t N, size_t batch, size_t L, size_t cl, int x_complex,
-                 int h_complex, cudaStream_t st);
-// full-length FFT path (any N, any L <= N)
-template <typename T>
-int fft_convolve_full(const void* x, void* y, const void* h, size_t N, size_t batch, size_t L, int is_real,
-                      int h_is_real, cudaStream_t st);
+int convolve(const void* x, void* y, size_t N, size_t batch, int x_is_real, const void* h, size_t L, int h_is_real,
+             const OlsPlan* plan, cudaStream_t st);
 
 }  // namespace bdsp

@@ -15,12 +15,6 @@
 // Shared layout: point p lives in float2 slot 256 a + 16 b + (c ^ 2 (b & 7)): the 16-byte chunks of a 128-byte row
 // are XOR-swizzled by the row number, which keeps the 128-bit accesses of every quarter-warp in eight different bank
 // windows in all three access patterns, without padding (32 KB per CTA).
-#include <math.h>
-
-#include <map>
-#include <mutex>
-#include <vector>
-
 #include "conv.cuh"
 #include "olsi.cuh"
 
@@ -32,8 +26,7 @@ using namespace cx;
 #define OI_T 128
 #define OI_MIN_CTAS 5
 
-// twiddle table (float2): [0,256) W4096^col; [256 + 16 k + c] W256^{k c}, k, c in [0,16)
-#define OI_TW_C2 (256 + 256)
+// twiddle table olsi_twiddles(4096): [0,256) W4096^col; [256 + 16 k + c] W256^{k c}, k, c in [0,16)
 #define OI_TW2 256
 
 // ALIGNED: rows start on 16-byte boundaries (N even, 16-byte aligned base pointers); together with the even block
@@ -213,46 +206,6 @@ __global__ void ols4096i_permute_h_kernel(const float2* __restrict__ Hs, float2*
     Hpos[2 * ((half * 8 + (c >> 1)) * OI_T + t) + (c & 1)] = h;
 }
 
-namespace {
-std::mutex g_oi_mu;
-std::map<int, float2*> g_oi_tw;  // per device
-
-const float2* ols4096i_twiddles() {
-    int d = 0;
-    if (cudaGetDevice(&d) != cudaSuccess) { set_last_error("ols4096: cudaGetDevice failed"); return nullptr; }
-    std::lock_guard<std::mutex> lk(g_oi_mu);
-    auto it = g_oi_tw.find(d);
-    if (it != g_oi_tw.end()) return it->second;
-    std::vector<float2> h(OI_TW_C2);
-    const long double tau = 2.0L * 3.14159265358979323846264338327950288L;
-    for (int c = 0; c < 256; c++) {
-        h[c].x = (float)cosl(-tau * (long double)c / 4096.0L);
-        h[c].y = (float)sinl(-tau * (long double)c / 4096.0L);
-    }
-    for (int k = 0; k < 16; k++)
-        for (int c = 0; c < 16; c++) {
-            const long double a = -tau * (long double)((k * c) % 256) / 256.0L;
-            h[OI_TW2 + 16 * k + c].x = (float)cosl(a);
-            h[OI_TW2 + 16 * k + c].y = (float)sinl(a);
-        }
-    float2* dev = nullptr;
-    if (cudaMalloc(&dev, OI_TW_C2 * sizeof(float2)) != cudaSuccess ||
-        cudaMemcpy(dev, h.data(), OI_TW_C2 * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess) {
-        if (dev) cudaFree(dev);
-        cudaGetLastError();
-        set_last_error("ols4096: twiddle table allocation failed");
-        return nullptr;
-    }
-    g_oi_tw[d] = dev;
-    return dev;
-}
-}  // namespace
-
-bool ols4096_applicable(size_t N, size_t L, size_t M) {
-    // needs one wrap at most per strided load and 32-bit row indices
-    return M == OI_M && L >= 2 && L <= OI_M / 2 - 2 && N >= OI_M && N < (1ull << 30);
-}
-
 // Hpos: 4096 float2 <- Hs from the plan (FFT_4096(pad(h)) / 4096, natural order)
 int ols4096_prepare(const void* Hs, void* Hpos, size_t L, cudaStream_t st) {
     int d, shift, m_first, step;
@@ -269,7 +222,7 @@ int ols4096_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, c
     const long long bpv = ((long long)N + step - 1) / step;
     const long long grid = bpv * (long long)batch;
     if (grid > 0x7fffffffll) { set_last_error("ols4096_convolve: grid too large"); return -2; }
-    const float2* tw = ols4096i_twiddles();
+    const float2* tw = olsi_twiddles(OI_M);
     if (!tw) return -1;
     const bool aligned = (N % 2 == 0) && ((reinterpret_cast<uintptr_t>(y) & 15) == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
     if (aligned)

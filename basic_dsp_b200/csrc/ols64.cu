@@ -111,13 +111,11 @@ int ols64_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, con
     const double2* tw = twiddle_table<double>();
     if (!tw) return -1001;
     const size_t smem = (size_t)O64_WORDS * sizeof(double2);
-    static bool configured[16] = {};
-    int dev = 0;
-    BDSP_CUDA_OK(cudaGetDevice(&dev));
-    if (dev >= 16 || !configured[dev]) {
+    static PerDeviceOnce configured;
+    if (configured.need()) {
         BDSP_CUDA_OK(cudaFuncSetAttribute(ols64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         BDSP_CUDA_OK(cudaFuncSetAttribute(ols64_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        if (dev < 16) configured[dev] = true;
+        configured.mark();
     }
     ols64_kernel<<<(unsigned)(bpv * batch), O64_T, smem, st>>>(reinterpret_cast<const double2*>(x), reinterpret_cast<double2*>(y), (long long)N,
                                                                (int)L, step, (unsigned)bpv, reinterpret_cast<const double2*>(Hs), tw);

@@ -17,11 +17,7 @@
 // Shared layout: point p lives in float2 slot 512 a + 32 b + (c ^ 2 (b & 7)): the low three bits of the 16-byte chunk
 // index are XOR-swizzled by the row number, which keeps the 128-bit accesses of every quarter-warp in eight different
 // bank windows in all three access patterns, without padding (64 KB per CTA, two CTAs per SM).
-#include <math.h>
-
-#include <map>
 #include <mutex>
-#include <vector>
 
 #include "conv.cuh"
 #include "olsi.cuh"
@@ -35,8 +31,7 @@ using namespace cx;
 #define O8_MIN_CTAS 2
 #define O8_SMEM_BYTES (O8_M * sizeof(float2))
 
-// twiddle table (float2): [0,512) W8192^col; [512 + 32 k + c] W512^{k c}, k in [0,16), c in [0,32)
-#define O8_TW_C2 (512 + 512)
+// twiddle table olsi_twiddles(8192): [0,512) W8192^col; [512 + 32 k + c] W512^{k c}, k in [0,16), c in [0,32)
 #define O8_TW2 512
 
 template <bool ALIGNED>
@@ -211,49 +206,6 @@ __global__ void ols8192i_permute_h_kernel(const float2* __restrict__ Hs, float2*
     Hpos[2 * ((c >> 1) * O8_T + t) + (c & 1)] = h;
 }
 
-namespace {
-std::mutex g_o8_mu;
-struct O8Dev { float2* tw = nullptr; bool attr = false; };
-std::map<int, O8Dev> g_o8;
-
-int o8_device(O8Dev** out) {
-    int d = 0;
-    BDSP_CUDA_OK(cudaGetDevice(&d));
-    std::lock_guard<std::mutex> lk(g_o8_mu);
-    O8Dev& s = g_o8[d];
-    if (!s.tw) {
-        std::vector<float2> h(O8_TW_C2);
-        const long double tau = 2.0L * 3.14159265358979323846264338327950288L;
-        for (int c = 0; c < 512; c++) {
-            h[c].x = (float)cosl(-tau * (long double)c / 8192.0L);
-            h[c].y = (float)sinl(-tau * (long double)c / 8192.0L);
-        }
-        for (int k = 0; k < 16; k++)
-            for (int c = 0; c < 32; c++) {
-                const long double a = -tau * (long double)((k * c) % 512) / 512.0L;
-                h[O8_TW2 + 32 * k + c].x = (float)cosl(a);
-                h[O8_TW2 + 32 * k + c].y = (float)sinl(a);
-            }
-        float2* dev = nullptr;
-        BDSP_CUDA_OK(cudaMalloc(&dev, O8_TW_C2 * sizeof(float2)));
-        BDSP_CUDA_OK(cudaMemcpy(dev, h.data(), O8_TW_C2 * sizeof(float2), cudaMemcpyHostToDevice));
-        s.tw = dev;
-    }
-    if (!s.attr) {
-        BDSP_CUDA_OK(cudaFuncSetAttribute(ols8192i_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)O8_SMEM_BYTES));
-        BDSP_CUDA_OK(cudaFuncSetAttribute(ols8192i_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)O8_SMEM_BYTES));
-        s.attr = true;
-    }
-    *out = &s;
-    return 0;
-}
-}  // namespace
-
-bool ols8192_applicable(size_t N, size_t L) {
-    // one wrap at most per strided load; 32-bit row indices
-    return L >= 2 && L <= O8_M / 2 - 2 && N >= O8_M && N < (1ull << 30);
-}
-
 // Hpos: 8192 float2 <- Hs = FFT_8192(pad(h)) / 8192 (natural order)
 int ols8192_prepare(const void* Hs, void* Hpos, size_t L, cudaStream_t st) {
     int d, shift, m_first, step;
@@ -263,12 +215,6 @@ int ols8192_prepare(const void* Hs, void* Hpos, size_t L, cudaStream_t st) {
     return 0;
 }
 
-long long ols8192_blocks(size_t N, size_t L) {
-    int d, shift, m_first, step;
-    olsi_geometry(O8_M, L, &d, &shift, &m_first, &step);
-    return ((long long)N + step - 1) / step;
-}
-
 int ols8192_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, cudaTextureObject_t htex, cudaStream_t st) {
     if (x == y) { set_last_error("ols8192_convolve: in-place operation is not supported"); return -3; }
     int d, shift, m_first, step;
@@ -276,16 +222,23 @@ int ols8192_convolve(const void* x, void* y, size_t N, size_t batch, size_t L, c
     const long long bpv = ((long long)N + step - 1) / step;
     const long long grid = bpv * (long long)batch;
     if (grid > 0x7fffffffll) { set_last_error("ols8192_convolve: grid too large"); return -2; }
-    O8Dev* dev = nullptr;
-    int rc = o8_device(&dev);
-    if (rc) return rc;
+    const float2* tw = olsi_twiddles(O8_M);
+    if (!tw) return -1;
+    static std::mutex mu;   // launches from threads on different devices: PerDeviceOnce is not thread-safe on its own
+    static PerDeviceOnce configured;
+    std::lock_guard<std::mutex> lk(mu);
+    if (configured.need()) {
+        BDSP_CUDA_OK(cudaFuncSetAttribute(ols8192i_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)O8_SMEM_BYTES));
+        BDSP_CUDA_OK(cudaFuncSetAttribute(ols8192i_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)O8_SMEM_BYTES));
+        configured.mark();
+    }
     const bool aligned = (N % 2 == 0) && ((reinterpret_cast<uintptr_t>(y) & 15) == 0) && ((reinterpret_cast<uintptr_t>(x) & 15) == 0);
     if (aligned)
         ols8192i_kernel<true><<<(unsigned)grid, O8_T, O8_SMEM_BYTES, st>>>(reinterpret_cast<const float2*>(x), reinterpret_cast<float2*>(y),
-                                                                          (int)N, m_first, step, shift, (int)bpv, dev->tw, htex);
+                                                                          (int)N, m_first, step, shift, (int)bpv, tw, htex);
     else
         ols8192i_kernel<false><<<(unsigned)grid, O8_T, O8_SMEM_BYTES, st>>>(reinterpret_cast<const float2*>(x), reinterpret_cast<float2*>(y),
-                                                                           (int)N, m_first, step, shift, (int)bpv, dev->tw, htex);
+                                                                           (int)N, m_first, step, shift, (int)bpv, tw, htex);
     BDSP_LAUNCHED();
     return 0;
 }

@@ -46,4 +46,18 @@ static inline void olsi_geometry(size_t M, size_t L, int* d, int* shift, int* m_
     *step = ((int)M - mf) & ~1;
 }
 
+// the M-point kernel takes N-point vectors and L taps: at most one wrap per strided load, 32-bit row indices
+static inline bool olsi_applicable(size_t M, size_t N, size_t L) { return L >= 2 && L <= M / 2 - 2 && N >= M && N < (1ull << 30); }
+
+// blocks per vector (L must be applicable: the step is only positive then)
+static inline long long olsi_blocks(size_t M, size_t N, size_t L) {
+    int d, shift, m_first, step;
+    olsi_geometry(M, L, &d, &shift, &m_first, &step);
+    return ((long long)N + step - 1) / step;
+}
+
+// twiddle table of the M-point kernel (M = 4096, 8192), built once per device and M (float2):
+// [0, M/16) W_M^c; [M/16 + (M/256) k + c] W_{M/16}^{k c}, k < 16, c < M/256.  nullptr (last error set) on failure.
+const float2* olsi_twiddles(int M);
+
 }  // namespace bdsp

@@ -230,7 +230,7 @@ def ols_peer(x, h, dtype, M, geometry="generic"):
 
 def ols_block(dtype, L, complex_signal, N, rows):
     """(M, geometry) of the block overlap-save path conv.cu takes for these arguments (ols_block_len and the
-    8192-point choice of ols_plan_convolve); None where a FIR or the full-length path runs instead."""
+    8192-point choice of convolve); None where a FIR or the full-length path runs instead."""
     c32 = dtype == np.float32 and complex_signal
     if c32 and 2 <= L <= 2046:
         blocks8 = -(-N // olsi_geometry(8192, L)[2]) if L <= 4094 else 0

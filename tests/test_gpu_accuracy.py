@@ -207,12 +207,12 @@ def test_windowed_fft_accuracy(dtype, n, rows, branch):
 
 # ---- convolution -----------------------------------------------------------------------------------------------------
 def gpu_conv_vec(x, h):
-    """Per-vector convolve_signal (capi.cu convolve_taps)."""
+    """Per-vector convolve_signal (capi.cu convolve_taps -> conv.cu convolve)."""
     return DspVec(x[0]).convolve_signal(DspVec(h)).to_numpy().reshape(1, -1)
 
 
 def gpu_conv_rows(x, h, dtype, off=0):
-    """bdsp_convolve_signal_rows_* (capi.cu conv_rows); off: input and output pointers `off` elements past alignment."""
+    """bdsp_convolve_signal_rows_* (capi.cu conv_rows -> conv.cu convolve); off: input and output pointers `off` elements past alignment."""
     L = bd.lib()
     rows, n = x.shape
     sfx = "c32" if dtype == F32 else "c64"
@@ -242,17 +242,17 @@ def conv_peer(x, h, dtype, kind):
 #   The smallest tap count an overlap-save kernel sees through the C ABI is 25 (complex taps; <= 24 run the FIR) and
 #   97 (real taps on real signals): 1- and 2-tap responses never reach ols4096i / ols64.
 CONV_CASES = [
-    (F32, 5000, 1, 24, "vec", "fir", "FIR c32, 24 complex taps, N >= 2048 + L", "convolve_taps: L <= 24 (complex); fir_kernel big"),
+    (F32, 5000, 1, 24, "vec", "fir", "FIR c32, 24 complex taps, N >= 2048 + L", "convolve: L <= 24 (complex); fir_kernel big"),
     (F32, 2000, 1, 24, "vec", "fir", "FIR c32, 24 complex taps, N < 2048 + L (modulo)", "fir_kernel: N < FIR_TILE + L"),
-    (F64, 5000, 1, 24, "vec", "fir", "FIR c64, 24 complex taps", "convolve_taps: L <= 24"),
+    (F64, 5000, 1, 24, "vec", "fir", "FIR c64, 24 complex taps", "convolve: L <= 24"),
     (F64, 700, 1, 24, "vec", "fir", "FIR c64, N < 2048 + L (modulo)", "fir_kernel: N < FIR_TILE + L"),
-    (F32, 5000, 1, 96, "vec-real", "fir", "FIR f32 real, 96 real taps", "convolve_taps: L <= 96 (real)"),
+    (F32, 5000, 1, 96, "vec-real", "fir", "FIR f32 real, 96 real taps", "convolve: L <= 96 (real)"),
     (F32, 1000, 1, 96, "vec-real", "fir", "FIR f32 real, 96 taps, modulo", "fir_kernel: N < FIR_TILE + L"),
-    (F64, 3000, 1, 96, "vec-real", "fir", "FIR f64 real, 96 real taps", "convolve_taps: L <= 96 (real)"),
-    (F32, 5000, 3, 24, "rows", "fir", "FIR rows c32", "conv_rows: L <= 24 -> fir_convolve batch > 1"),
-    (F32, 1500, 4, 17, "rows", "fir", "FIR rows c32, modulo", "conv_rows: L <= 24, N < FIR_TILE + L"),
-    (F64, 5000, 3, 24, "rows", "fir", "FIR rows c64", "conv_rows: L <= 24"),
-    (F32, 20000, 1, 1023, "vec", "ols", "ols4096i<true> even N", "ols_plan_convolve: M == 4096, ols4096_applicable, aligned"),
+    (F64, 3000, 1, 96, "vec-real", "fir", "FIR f64 real, 96 real taps", "convolve: L <= 96 (real)"),
+    (F32, 5000, 3, 24, "rows", "fir", "FIR rows c32", "convolve: L <= 24 -> fir_convolve batch > 1"),
+    (F32, 1500, 4, 17, "rows", "fir", "FIR rows c32, modulo", "convolve: L <= 24, N < FIR_TILE + L"),
+    (F64, 5000, 3, 24, "rows", "fir", "FIR rows c64", "convolve: L <= 24"),
+    (F32, 20000, 1, 1023, "vec", "ols", "ols4096i<true> even N", "convolve: M == 4096, olsi_applicable(4096), aligned"),
     (F32, 20001, 1, 1023, "vec", "ols", "ols4096i<false> odd N", "ols4096_convolve: N % 2 != 0"),
     (F32, 20000, 1, 25, "vec", "ols", "ols4096i<true> 25 taps", "L > 24 (FIR below)"),
     (F32, 20000, 1, 2046, "vec", "ols", "ols4096i<true> 2046 taps", "ols_block_len: L <= 2046 -> 4096; 8192 blocks*rows < 592"),
@@ -262,37 +262,37 @@ CONV_CASES = [
     (F32, 20000, 3, 25, "rows-offset", "ols", "ols4096i<false> rows, misaligned, 25 taps", "(x | y) & 15"),
     (F32, 20001, 2, 2046, "rows", "ols", "ols4096i<false> rows, odd N, 2046 taps", "N % 2 != 0"),
     (F32, 50000, 1, 2047, "vec", "ols", "ols8192i<true> 2047 taps", "ols_block_len: 2047 <= L <= 4094 -> 8192"),
-    (F32, 50000, 1, 4094, "vec", "ols", "ols8192i<true> 4094 taps", "ols8192_applicable: L <= 4094"),
-    (F32, 1 << 20, 4, 1450, "rows", "ols", "ols8192i for 1450 taps, blocks*rows >= 592", "L >= 1450 && ols8192_blocks * batch >= 592"),
-    (F32, 1 << 20, 1, 1450, "vec", "ols", "ols4096i for 1450 taps, blocks*rows < 592", "ols8192_blocks * batch < 592"),
+    (F32, 50000, 1, 4094, "vec", "ols", "ols8192i<true> 4094 taps", "olsi_applicable(8192): L <= 4094"),
+    (F32, 1 << 20, 4, 1450, "rows", "ols", "ols8192i for 1450 taps, blocks*rows >= 592", "L >= 1450 && olsi_blocks(8192) * batch >= 592"),
+    (F32, 1 << 20, 1, 1450, "vec", "ols", "ols4096i for 1450 taps, blocks*rows < 592", "olsi_blocks(8192) * batch < 592"),
     (F32, 50001, 1, 3000, "vec", "ols", "ols8192i<false> odd N", "ols8192_convolve: N % 2 != 0"),
     (F32, 50000, 2, 3000, "rows-offset", "ols", "ols8192i<false> rows, misaligned", "(x | y) & 15"),
     (F64, 30000, 1, 25, "vec", "ols", "ols64 25 taps", "ols64_applicable: M == 4096, L <= 2048, N >= 4096"),
     (F64, 30000, 1, 1023, "vec", "ols", "ols64 1023 taps", "ols64_applicable"),
     (F64, 30000, 1, 2048, "vec", "ols", "ols64 2048 taps", "ols_block_len: c64 L <= 2048 -> 4096"),
-    (F64, 30000, 3, 1023, "rows", "ols", "ols64 rows", "conv_rows: ols plan, batch > 1"),
+    (F64, 30000, 3, 1023, "rows", "ols", "ols64 rows", "convolve: ols plan, batch > 1"),
     (F64, 4096, 3, 1023, "rows", "ols", "ols64 N = 4096 exactly", "ols64_applicable: N >= 4096"),
     (F64, 30000, 2, 2048, "rows-offset", "ols", "ols64 rows, pointers one element into the buffer", "ols64 has no aligned variant"),
-    (F32, 30000, 1, 1000, "vec-real", "ols", "ols_conv_kernel<float, REAL>", "convolve_taps: real signal -> complex_signal false, generic"),
+    (F32, 30000, 1, 1000, "vec-real", "ols", "ols_conv_kernel<float, REAL>", "convolve_taps: real signal -> plan with complex_signal false, generic"),
     (F64, 30000, 1, 1000, "vec-real", "ols", "ols_conv_kernel<double, REAL>", "real signal, generic"),
-    (F32, 3000, 1, 1000, "vec", "ols", "ols_conv_kernel c32, N < 4096", "ols4096_applicable: N < 4096"),
+    (F32, 3000, 1, 1000, "vec", "ols", "ols_conv_kernel c32, N < 4096", "olsi_applicable(4096): N < 4096"),
     (F32, 1500, 4, 700, "rows", "ols", "ols_conv_kernel c32 rows, N < M/2 (loads wrap twice)", "N < 4096, rows > 1"),
-    (F32, 6000, 2, 3000, "rows", "ols", "ols_conv_kernel c32 rows, M = 8192, N < 8192", "ols8192_applicable: N < 8192"),
+    (F32, 6000, 2, 3000, "rows", "ols", "ols_conv_kernel c32 rows, M = 8192, N < 8192", "olsi_applicable(8192): N < 8192"),
     (F64, 3000, 1, 1000, "vec", "ols", "ols_conv_kernel c64, N < 4096", "ols64_applicable: N < 4096"),
     (F64, 1500, 3, 700, "rows", "ols", "ols_conv_kernel c64 rows, N < M/2", "N < 4096, rows > 1"),
     (F64, 50000, 1, 3000, "vec", "ols", "ols_conv_kernel c64, L > 2048 (M = 8192)", "ols_block_len c64: L > 2048"),
     (F64, 50000, 2, 4000, "rows", "ols", "ols_conv_kernel c64 rows, L > 2048", "ols_block_len c64: L > 2048"),
-    (F32, 1 << 16, 1, 5000, "vec", "full", "full length c32, fused spectrum multiply (taps_dev)",
-     "ols_plan_convolve: L > 4094, pow2 N >= 2^15 -> fft_convolve_full, in_mul"),
-    (F32, 1 << 15, 3, 8000, "rows", "full", "full length c32 rows (taps_dev)", "L > 4094, pow2 N >= 2^15"),
-    (F32, 1 << 16, 1, 6000, "vec-real", "ols", "ols_conv_kernel<float, REAL>, M = 16384", "real signal: the taps_dev path is complex only"),
+    (F32, 1 << 16, 1, 5000, "vec", "full", "full length c32, fused spectrum multiply (4095 .. 8192 taps)",
+     "convolve: c32, L > 4094, pow2 N >= 2^15 -> fft_convolve_full, in_mul"),
+    (F32, 1 << 15, 3, 8000, "rows", "full", "full length c32 rows (4095 .. 8192 taps)", "L > 4094, pow2 N >= 2^15"),
+    (F32, 1 << 16, 1, 6000, "vec-real", "ols", "ols_conv_kernel<float, REAL>, M = 16384", "real signal: the 4095 .. 8192-tap full-length path is complex only"),
     (F32, 16384, 1, 9000, "vec", "full", "full length c32 N = 16384, separate spectrum multiply",
-     "convolve_taps: L > 8192; fft_convolve_full: pow2 N <= 16384 -> spectrum_mul_kernel"),
+     "convolve: L > 8192; fft_convolve_full: pow2 N <= 16384 -> spectrum_mul_kernel"),
     (F32, 3 << 14, 1, 9000, "vec", "full", "full length c32, q*2^k N", "L > 8192, not pow2: in_mul"),
-    (F32, 20000, 2, 9000, "rows", "full", "full length c32 rows, chirp-z N", "conv_rows: L > 8192 -> fft_convolve_full"),
+    (F32, 20000, 2, 9000, "rows", "full", "full length c32 rows, chirp-z N", "convolve: L > 8192 -> fft_convolve_full"),
     (F32, 20000, 1, 5000, "vec", "ols", "ols_conv_kernel c32, M = 16384 (non-pow2 N, L > 4094)", "L > 4094, !is_pow2(N)"),
-    (F64, 40000, 1, 5000, "vec", "full", "full length c64", "convolve_taps: L > ols_max_taps (4096)"),
-    (F64, 1 << 15, 2, 4500, "rows", "full", "full length c64 rows", "conv_rows: no ols plan"),
+    (F64, 40000, 1, 5000, "vec", "full", "full length c64", "convolve: L > ols_max_taps (4096)"),
+    (F64, 1 << 15, 2, 4500, "rows", "full", "full length c64 rows", "convolve: L > ols_max_taps, no ols plan"),
 ]
 
 
