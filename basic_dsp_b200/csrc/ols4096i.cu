@@ -3,11 +3,15 @@
 // (the reference's overlap_discard, convolution.rs:304-461: 2 rustfft calls + a scalar multiply loop per block).
 //
 // Structure (M = 4096 = 16^3, 128 threads, 32 points per thread and stage; block position p = 256 a + 16 b + c):
-//   F1  radix-16 DIF over a, columns (2t, 2t+1) straight from global memory (128-bit loads)        -> smem  | CTA barrier
+//   F1  radix-16 DIF over a, columns (2t, 2t+1) of the input in smem (aligned rows: bulk copies)
+//       or straight from global memory (other rows)                                                 -> smem  | CTA barrier
 //   F2  radix-16 DIF over b inside row a = t >> 3                                                    -> smem  | warp barrier
 //   F3  radix-16 DIF over the 16 contiguous c | * H (position order) | radix-16 DIT  (registers)    -> smem  | warp barrier
 //   I2  radix-16 DIT over b                                                                          -> smem  | CTA barrier
-//   I1  radix-16 DIT over a, valid outputs straight to global memory (128-bit stores)
+//   I1  radix-16 DIT over a, valid outputs to global memory: aligned rows through smem in natural order and one
+//       bulk copy, other rows with direct stores
+// Aligned rows move a block's input and output between global and shared memory by bulk asynchronous copies
+// (cp.async.bulk + mbarrier): no load or store instruction per 16 bytes on the L1 data pipe, the kernel's saturated unit.
 // The forward transform leaves the spectrum digit-reversed, the plan stores H in that order, the inverse consumes it:
 // no reordering pass.  All arithmetic is interleaved-complex packed FP32x2 (cxmath.cuh): two adjacent points travel as
 // one 128-bit word through every global and shared access, so a stage costs 16 + 16 shared-memory instructions per
@@ -30,13 +34,15 @@ using namespace cx;
 #define OI_TW2 256
 
 // ALIGNED: rows start on 16-byte boundaries (N even, 16-byte aligned base pointers); together with the even block
-// offsets chosen by the plan every thread then moves its two adjacent points with one 128-bit access.  `shift` =
+// offsets chosen by the plan every thread then moves its two adjacent points with one 128-bit access, and every piece
+// of a block's input and output is a 16-byte aligned run of a multiple of 16 bytes, as bulk copies require.  `shift` =
 // cl - 1 + d is the (even) distance between a block position's input index and its output index.
 template <bool ALIGNED>
 __global__ void __launch_bounds__(OI_T, OI_MIN_CTAS)
 ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int m_first, int step, int shift,
                 int blocks_per_vec, const float2* __restrict__ tw, cudaTextureObject_t htex) {
-    __shared__ __align__(16) float2 sm[OI_M];
+    __shared__ __align__(128) float2 sm[OI_M];
+    __shared__ __align__(8) unsigned long long bar;
     const int t = threadIdx.x;
     const int vec = blockIdx.x / blocks_per_vec;
     const int blk = blockIdx.x - vec * blocks_per_vec;
@@ -44,27 +50,43 @@ ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
     const float2* xr = x + (size_t)vec * (size_t)N;
     float2* yr = y + (size_t)vec * (size_t)N;
     const int hi = t >> 3, lo = t & 7;         // quarter-warp index / lane inside it
+    // block position p holds x[(p0 + p) mod N], p0 = i0 + shift - m_first  (-4096 < p0 < N - 1, even)
+    const int p0 = i0 + shift - m_first;
     pdl_trigger();                             // the next kernel of the stream may start launching
     pdl_wait();                                // ... and this one touches global memory only after its predecessor is complete
+    if (ALIGNED) {
+        // the block's 32 KB of input land in sm in natural order through one or two bulk copies (two when it wraps
+        // around the end of the vector): no load instruction per 16 bytes on the L1 data pipe, its saturated unit
+        if (t == 0) {
+            const unsigned b = smem_u32(&bar), s = smem_u32(sm);
+            mbar_init(b, 1);
+            mbar_arrive_expect_tx(b, OI_M * 8);
+            const int first = p0 < 0 ? p0 + N : p0;
+            const int n1 = min(OI_M, N - first);
+            bulk_g2s(s, xr + first, 8 * n1, b);
+            if (n1 < OI_M) bulk_g2s(s + 8 * n1, xr, 8 * (OI_M - n1), b);
+        }
+        __syncthreads();                       // the barrier is initialised before anyone waits on it
+        mbar_wait(smem_u32(&bar), 0);
+    }
 
     c2 v[16], u[16];                           // the thread's two columns
     // ------------------------------------------------------------------ F1: over a, columns (2t, 2t+1) = (b = hi, c = 2 lo, 2 lo + 1)
     {
         const int col = 2 * t;
-        // block position p holds x[(p0 + p) mod N], p0 = i0 + shift - m_first  (p0 > -4096, even)
-        const int p0 = i0 + shift - m_first;
-        if (p0 >= 0 && p0 + OI_M <= N) {   // block-uniform: no wrap-around inside this block
+        if (ALIGNED) {
+#pragma unroll
+            for (int a = 0; a < 16; a++) {
+                const float4 ab = *reinterpret_cast<const float4*>(sm + 256 * a + col);
+                v[a] = make_float2(ab.x, ab.y);
+                u[a] = make_float2(ab.z, ab.w);
+            }
+        } else if (p0 >= 0 && p0 + OI_M <= N) {   // block-uniform: no wrap-around inside this block
             const float2* px = xr + p0 + col;
 #pragma unroll
             for (int a = 0; a < 16; a++) {
-                if (ALIGNED) {
-                    const float4 ab = ld_x4(px + 256 * a);
-                    v[a] = make_float2(ab.x, ab.y);
-                    u[a] = make_float2(ab.z, ab.w);
-                } else {
-                    v[a] = __ldg(px + 256 * a);
-                    u[a] = __ldg(px + 256 * a + 1);
-                }
+                v[a] = __ldg(px + 256 * a);
+                u[a] = __ldg(px + 256 * a + 1);
             }
         } else {                             // first / last block of a vector: circular indexing
             int idx = p0 + col;
@@ -83,6 +105,7 @@ ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
         const float4 w = __ldg(reinterpret_cast<const float4*>(tw + col));
         apply_twiddles<true>(v, make_float2(w.x, w.y));
         apply_twiddles<true>(u, make_float2(w.z, w.w));
+        if (ALIGNED) __syncthreads();          // every thread has read the natural-order input before it is overwritten
         float2* dst = sm + 16 * hi + ((2 * lo) ^ (2 * (hi & 7)));
 #pragma unroll
         for (int s = 0; s < 16; s++)
@@ -172,16 +195,24 @@ ols4096i_kernel(const float2* __restrict__ x, float2* __restrict__ y, int N, int
         int mhi = step;                                    // exclusive bound on m
         if (i0 + step > N) mhi = N - i0;                   // last block of the vector
         float2* py = yr + i0 + mlo;
+        // ALIGNED: the valid outputs go to sm in natural order (position m_first + m) and leave through one bulk copy
+        // of the mhi outputs (a 16-byte aligned, even count) instead of a 128-bit store each
+        if (ALIGNED) __syncthreads();                      // every thread has read the swizzled layout
 #pragma unroll
         for (int s = 0; s < 16; s++) {
             const int a = r16_k(s);
             const int m = mlo + 256 * a;
             if (ALIGNED) {
-                if (m >= 0 && m < mhi) *reinterpret_cast<float4*>(py + 256 * a) = make_float4(v[s].x, v[s].y, u[s].x, u[s].y);
+                if (m >= 0 && m < mhi) *reinterpret_cast<float4*>(sm + col + 256 * a) = make_float4(v[s].x, v[s].y, u[s].x, u[s].y);
             } else {
                 if (m >= 0 && m < mhi) py[256 * a] = v[s];
                 if (m + 1 >= 0 && m + 1 < mhi) py[256 * a + 1] = u[s];
             }
+        }
+        if (ALIGNED) {
+            fence_proxy_async_smem();                      // the stores above precede the bulk copy's reads
+            __syncthreads();
+            if (t == 0) bulk_s2g_wait_read(yr + i0, smem_u32(sm + m_first), 8 * mhi);   // sm stays valid until read
         }
     }
 }

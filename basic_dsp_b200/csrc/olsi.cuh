@@ -7,6 +7,38 @@ using namespace cx;
 
 // two adjacent block inputs as one 128-bit read-only load
 __device__ __forceinline__ float4 ld_x4(const float2* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
+
+// --- bulk asynchronous copies between global and shared memory, mbarrier completion (shared addresses as u32) ------
+__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+}
+// one arrival that also announces `bytes` of copies completing on the barrier's current phase
+__device__ __forceinline__ void mbar_arrive_expect_tx(unsigned bar, unsigned bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
+    unsigned done;
+    do {
+        asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
+                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+    } while (!done);
+}
+// bytes: multiple of 16, both addresses 16-byte aligned
+__device__ __forceinline__ void bulk_g2s(unsigned dst, const void* src, unsigned bytes, unsigned bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
+}
+// orders this thread's earlier generic-proxy accesses to shared memory before later async-proxy (bulk copy) accesses
+__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+// shared -> global bulk copy (same rules as bulk_g2s); returns once the copy has READ its shared-memory source, so the
+// buffer may be reused or the CTA may exit
+__device__ __forceinline__ void bulk_s2g_wait_read(void* dst, unsigned src, unsigned bytes) {
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(src), "r"(bytes) : "memory");
+    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+    asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+}
 // stride-16 stage twiddles W256^{k c}, k = 1..15: six 128-bit table loads (k = 1, 2, 3, 4, 8, 12) and nine products.
 // Fifteen loads per stage (4-5 L1 wavefronts each) were 16 % of the kernel's L1 data-pipe traffic, which is its saturated
 // unit.
