@@ -13,6 +13,9 @@
 //
 // ifft_shift / scaling / real->complex are fused into the load of the first pass, fft_shift and
 // magnitude into the store of the last one (FftOpts).
+//
+// fft_route (fft_route.h) is the one place that picks the path, packed kernels of fftp.cu / fftp16k.cu / fftc.cu
+// included; fft_any calls it once per level and switches on the result.
 #include <map>
 #include <memory>
 #include <mutex>
@@ -20,20 +23,24 @@
 
 #include "fft.cuh"
 #include "fft_core.cuh"
+#include "fft_route.h"
 #include "elementwise.cuh"
 
 namespace bdsp {
 
-int fftp_rows1k_try(const void* tmp, void* out, size_t n, size_t rows, bool inverse, size_t out_rot, double scale, bool magnitude,
-                    cudaStream_t st);
-int fftp_three_pass_try(const void* in, void* out, void* tmp, size_t n, size_t rows, bool inverse, size_t in_rot, size_t out_rot,
-                        double scale, bool magnitude, cudaStream_t st, bool real_in, const InMul& im);
-int fftp_two_pass_try(const void* in, void* out, void* tmp, size_t n, size_t rows, bool inverse, size_t in_rot, size_t out_rot,
-                      double scale, bool magnitude, cudaStream_t st, bool real_in, const InMul& im);
-int fftp_try(const void* in, void* out, size_t n, size_t rows, bool inverse, size_t in_rot, size_t out_rot, double scale,
-             bool magnitude, cudaStream_t st);
-int fftp_try_real(const void* in, void* out, size_t n, size_t rows, size_t out_rot, double scale, bool magnitude, cudaStream_t st);
-int fftc_try(const void* in, void* out, size_t n, size_t rows, bool inverse, size_t in_rot, size_t out_rot, double scale, cudaStream_t st);
+// launchers of the packed routes (fftp.cu, fftp16k.cu, fftc.cu): 0 or a negative error
+template <bool RIN>
+int fftp_single(const void* in, void* out, size_t n, size_t groups, bool inverse, bool si, bool so, bool magnitude, double scale,
+                cudaStream_t st);
+int fftp_two_pass(const void* in, void* out, void* tmp, const FftPlan& p, size_t rows, bool inverse, bool si, bool so, bool magnitude,
+                  double scale, bool real_in, const InMul& im, cudaStream_t st);
+int fftp_three_pass(const void* in, void* out, void* tmp, const FftPlan& p, size_t n, size_t rows, bool inverse, bool si, bool so,
+                    bool magnitude, double scale, bool real_in, const InMul& im, cudaStream_t st);
+int fftp_rows_pass(const void* tmp, void* out, int tq, size_t groups, bool inverse, bool so, bool magnitude, float sc, cudaStream_t st,
+                   int n1, int n2c);
+int fftp16k(const void* in, void* out, size_t rows, bool inverse, bool shift_in, bool shift_out, bool magnitude, float scale, cudaStream_t st);
+int fftc65536(const void* in, void* out, size_t rows, bool inverse, bool shift_in, bool shift_out, double scale, cudaStream_t st);
+bool fftc_cluster_ok();
 
 // ------------------------------------------------------------------------------------------
 // per-device state: twiddle tables, workspaces
@@ -146,8 +153,8 @@ void* workspace(size_t bytes, int slot) {
     return s.p[slot];
 }
 
-template <> size_t fft_block_max_n<float>() { return 16384; }
-template <> size_t fft_block_max_n<double>() { return 8192; }
+template <> size_t fft_block_max_n<float>() { return FFT_BLOCK_MAX_C32; }
+template <> size_t fft_block_max_n<double>() { return FFT_BLOCK_MAX_C64; }
 
 // ------------------------------------------------------------------------------------------
 // output addressing shared by all "last pass" kernels
@@ -580,16 +587,6 @@ template <typename T, bool INV>
 int launch_block(const void* in, void* out, size_t n, size_t batch, bool real_in, bool mag, long long in_rot,
                  T scale, const OutMap& om, cudaStream_t st, const InMul& im = InMul()) {
     typedef typename CpxOf<T>::type C;
-    if constexpr (sizeof(T) == 8) {
-        // c64 rows of 1024 / 2048 / 4096 points: the 8-points-per-thread row kernel of fft64t.cuh
-        // (in place only with the plain row layout: a row's loads all precede its stores, rows do not overlap)
-        if (n >= 1024 && n <= 4096 && (in != out || (om.seq_group == 1 && om.oes == 1 && om.group_stride == (long long)n && !real_in && !mag))) {
-            const double2* twt = twiddle_table<double>();
-            if (!twt) return -1001;
-            const int rc = f64t::launch_rows<INV>(in, out, n, batch, real_in, mag, in_rot, (double)scale, om, im, twt, st);
-            if (rc <= 0) { if (!rc) BDSP_LAUNCHED(); return rc; }
-        }
-    }
     const int log2n = ilog2(n);
     // points per CTA for short sequences (BDSP_BLOCK_POINTS): smaller CTAs overlap their load / compute / store phases better
     int nfft = (int)(BDSP_BLOCK_POINTS / n);
@@ -649,20 +646,27 @@ template <typename T> int tile_log2m_max() { return sizeof(T) == 4 ? 10 : 9; }
 #define BDSP_TILE_LANES_F64 8
 template <typename T> long long tile_lanes() { return sizeof(T) == 8 ? BDSP_TILE_LANES_F64 : 8; }
 
-// power-of-two transform of `batch` sequences; handles any supported size
+// power-of-two transform of `batch` sequences with the generic kernels: route C64Rows, Block, Hybrid or Tiles
 template <typename T, bool INV>
-int fft_pow2(const void* in, void* out, size_t n, size_t batch, bool real_in, bool mag, long long in_rot, T scale,
+int fft_pow2(const FftPlan& plan, const void* in, void* out, size_t n, size_t batch, bool real_in, bool mag, long long in_rot, T scale,
              const OutMap& om, void* work, cudaStream_t st, const InMul& im = InMul()) {
-    if (n <= fft_block_max_n<T>()) return launch_block<T, INV>(in, out, n, batch, real_in, mag, in_rot, scale, om, st, im);
+    if constexpr (sizeof(T) == 8) {
+        if (plan.route == FftRoute::C64Rows) {
+            // the 8-points-per-thread row kernel of fft64t.cuh
+            const double2* twt = twiddle_table<double>();
+            if (!twt) return -1001;
+            const int rc = f64t::launch_rows<INV>(in, out, n, batch, real_in, mag, in_rot, (double)scale, om, im, twt, st);
+            if (!rc) BDSP_LAUNCHED();
+            return rc;
+        }
+    }
+    if (plan.route == FftRoute::Block) return launch_block<T, INV>(in, out, n, batch, real_in, mag, in_rot, scale, om, st, im);
     const int L = ilog2(n);
     const int mx = tile_log2m_max<T>();
-    if (sizeof(T) == 4 && L - 10 <= mx && om.seq_group == 1 && om.oes == 1 && om.group_stride == (long long)n && om.rot_n == (long long)n &&
-        (om.rot == 0 || om.rot == (long long)n / 2) && !(INV && (mag || om.rot != 0))) {
-        // c32, n = n1 * 1024 with n1 <= 2^10: generic column pass (any input form: real, rotated, scaled) followed by the
-        // packed four-rows-per-CTA 1024-point pass of fftp.cu
-        typedef typename CpxOf<T>::type C;
+    if (plan.route == FftRoute::Hybrid) {
+        // generic column pass (any input form: real, rotated, scaled) followed by the packed four-rows-per-CTA 1024-point
+        // pass of fftp.cu
         TileParams p;
-        const long long n1 = (long long)n / 1024;
         p.in = in; p.out = work; p.log2m = L - 10;
         // short columns: more lanes per tile so that a CTA still holds >= 2048 points
         p.lanes = 1024; p.ct = (int)tile_lanes<T>(); p.o1_count = 1;
@@ -672,14 +676,9 @@ int fft_pow2(const void* in, void* out, size_t n, size_t batch, bool real_in, bo
         p.tw_n = (long long)n; p.in_rot = in_rot; p.in_n = (long long)n; p.real_input = real_in; p.last = 0; p.magnitude = 0;
         p.om = om;
         p.im = im;
-        (void)n1;
-        if (work != out && work != in) {
-            int rc = launch_tile<T, INV>(p, (long long)batch, scale, st);
-            if (rc) return rc;
-            rc = fftp_rows1k_try(work, out, n, batch, INV, (size_t)om.rot, 1.0, mag, st);
-            if (rc <= 0) return rc;
-            // not covered (alignment): fall through and redo everything with the generic passes
-        }
+        const int rc = launch_tile<T, INV>(p, (long long)batch, scale, st);
+        if (rc) return rc;
+        return fftp_rows_pass(work, out, 4, plan.groups, INV, om.rot != 0, mag, 1.0f, st, plan.n1, 1);
     }
     // (A three-pass variant of this hybrid - two generic column passes + the packed 1024-point pass - was measured
     // slower than three generic passes for 2^21 (2.03 vs 1.73 ms per 2^26 points): short columns make the generic
@@ -729,22 +728,17 @@ int fft_pow2(const void* in, void* out, size_t n, size_t batch, bool real_in, bo
 //   B: inside every row K1: columns of N2 points over stride N3, in place, twiddle W_{N2 N3}^{l k2}
 //   C: rows of N3 points, lanes = K1, transposing store X[K1 + N1 (k2 + N2 k3)]
 // 96 bytes per point (c64) instead of the 160 of "radix-q pre-pass + three passes + interleave pass".
+// Geometry from the route (FftRoute::QThreePass): N1 = plan.n1 = q * 2^a <= ~1024 points per column, N2 = 2^plan.log2n2
+// (1: short enough for no middle pass), N3 = 2^plan.log2n3.
 template <typename T, bool INV>
-int fft_q_three_pass(const void* in, void* out, size_t n, size_t batch, size_t q, bool real_in, bool mag, long long in_rot, T scale,
-                     const OutMap& om, void* work, cudaStream_t st, const InMul& im = InMul()) {
+int fft_q_three_pass(const FftPlan& plan, const void* in, void* out, size_t n, size_t batch, bool real_in, long long in_rot, T scale,
+                     const OutMap& om, void* work, cudaStream_t st, const InMul& im) {
     typedef typename CpxOf<T>::type C;
-    size_t P = n / q;
-    const int k = ilog2(P);
-    const int mx = tile_log2m_max<T>();
-    int a = 8 - (q > 3 ? ilog2(q) - 1 : 0);          // N1 = q * 2^a <= ~1024 points per column
-    if (a < 4) a = 4;
-    int rest = k - a;
-    if (rest < 1 || rest > 2 * mx) return 1;
-    const bool two = rest <= mx;                       // short enough: no middle pass
-    const int b = two ? 0 : (rest + 1) / 2, c = rest - b;
-    const long long N1 = (long long)q << a, N2 = 1ll << b, N3 = 1ll << c;
+    const size_t q = plan.q;
+    const int a = ilog2((size_t)plan.n1 / q), b = plan.log2n2, c = plan.log2n3;
+    const bool two = b == 0;
+    const long long N1 = plan.n1, N2 = 1ll << b, N3 = 1ll << c;
     const long long ct1 = 4;                           // lanes of the first pass: 64-byte (c64) row segments, q * 2^a * 4 points per tile
-    if ((long long)n / N1 % ct1) return 1;
     C* tmp = reinterpret_cast<C*>(work);
     TileParams p;
     p.in = in; p.out = tmp; p.log2m = a; p.q = (int)q;
@@ -774,7 +768,7 @@ int fft_q_three_pass(const void* in, void* out, size_t n, size_t batch, size_t q
     p.o1_count = two ? 1 : N2;
     p.in_lane_stride = (long long)n / N1; p.in_point_stride = 1; p.in_o1_stride = two ? 0 : N3;
     p.out_lane_stride = 1; p.out_point_stride = two ? N1 : N1 * N2; p.out_o1_stride = two ? 0 : N1;
-    p.tw_n = 0; p.in_rot = 0; p.real_input = 0; p.last = 1; p.magnitude = mag;
+    p.tw_n = 0; p.in_rot = 0; p.real_input = 0; p.last = 1; p.magnitude = 0;
     return launch_tile<T, INV>(p, (long long)batch, (T)1, st);
 }
 
@@ -812,6 +806,13 @@ template <typename T, bool INV>
 int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o, void* work, size_t work_bytes,
             cudaStream_t st);
 
+// route of a plain transform that the caller runs on the generic kernels (fft_pow2) directly
+template <typename T>
+FftPlan generic_route(const void* in, void* out, size_t n, size_t batch, bool inverse, bool mag, const void* work) {
+    return fft_route({sizeof(T) == 8, n, batch, inverse, false, mag, 0, 0, 0, reinterpret_cast<uintptr_t>(in), reinterpret_cast<uintptr_t>(out),
+                      reinterpret_cast<uintptr_t>(work), false, true});
+}
+
 // spectrum of the chirp filter for length n (M = padded length), from the cache or computed on `st`
 template <typename T, bool INV>
 int bluestein_filter(size_t n, size_t M, void* w0, cudaStream_t st, std::shared_ptr<BluesteinFilter>* out) {
@@ -830,7 +831,8 @@ int bluestein_filter(size_t n, size_t M, void* w0, cudaStream_t st, std::shared_
     bluestein_filter_kernel<T, INV><<<(unsigned)((M + 255) / 256), 256, 0, st>>>(reinterpret_cast<C*>(f->spec), (long long)n, (long long)M);
     BDSP_LAUNCHED();
     OutMap plain; plain.seq_group = 1; plain.oes = 1; plain.group_stride = (long long)M; plain.rot = 0; plain.rot_n = (long long)M;
-    int rc = fft_pow2<T, false>(f->spec, f->spec, M, 1, false, false, 0, (T)1, plain, w0, st);
+    int rc = fft_pow2<T, false>(generic_route<T>(f->spec, f->spec, M, 1, false, false, w0), f->spec, f->spec, M, 1, false, false, 0, (T)1,
+                                plain, w0, st);
     if (rc) return rc;
     BDSP_CUDA_OK(cudaStreamSynchronize(st));
     std::vector<std::shared_ptr<BluesteinFilter>> evicted;   // destroyed (device sync + free) outside the lock
@@ -897,12 +899,19 @@ int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o,
         BDSP_LAUNCHED();
         im.p = tab; im.kind = 1;
     }
-    // a first-load multiplier (window / spectrum) is carried by the generic kernels, the c64 tile passes and the packed
-    // column passes of the two- and three-pass c32 transforms; the packed single-pass c32 kernels do not take one: in
-    // their throughput regime one elementwise pass + the packed kernel beats the generic kernel with the multiplier fused
-    if (sizeof(T) == 4 && im.kind && is_pow2(n) && n >= 64 && n <= 16384 && n * batch >= (1u << 16)) {
-        const bool to_complex = o.real_input && im.kind == 2;
-        const bool real_rows = o.real_input && !to_complex;
+    // the multi-pass power-of-two transforms need a scratch buffer: the caller's or the pass workspace
+    void* w = work;
+    if (is_pow2(n) && n > fft_block_max_n<T>()) {
+        const size_t need = n * batch * sizeof(C);
+        if (!w || work_bytes < need) { w = workspace(need, 0); if (!w) return -1001; }
+    }
+    const bool si = in_rot != 0, so = om.rot != 0, mag = o.magnitude != 0, real_in = o.real_input != 0;
+    const FftPlan plan = fft_route({sizeof(T) == 8, n, batch, INV, real_in, mag, im.kind, (size_t)in_rot, (size_t)om.rot, reinterpret_cast<uintptr_t>(in),
+                                    reinterpret_cast<uintptr_t>(out), reinterpret_cast<uintptr_t>(w), sizeof(T) == 4 && n == 65536 && fftc_cluster_ok()});
+    switch (plan.route) {
+    case FftRoute::MulPass: {
+        const bool to_complex = real_in && im.kind == 2;
+        const bool real_rows = real_in && !to_complex;
         BDSP_WS(mx, void*, n * batch * (real_rows ? sizeof(T) : sizeof(C)), 2);
         const long long tot = (long long)(n * batch);
         in_mul_rows_kernel<T><<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(in, mx, (long long)n, tot, o.real_input, im);
@@ -912,64 +921,34 @@ int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o,
         if (to_complex) o2.real_input = 0;
         return fft_any<T, INV>(mx, out, n, batch, o2, work, work_bytes, st);
     }
-    if (is_pow2(n)) {
-        if (sizeof(T) == 4 && !im.kind && o.real_input && !INV && in_rot == 0 && n >= 64 && n <= 16384 && n * batch >= (1u << 16)) {
-            // rows of real scalars, single pass: the packed kernel loads the reals directly (4 B read + 8 B written per point)
-            const int rc = fftp_try_real(in, out, n, batch, (size_t)om.rot, o.scale, o.magnitude != 0, st);
-            if (rc <= 0) return rc;
-        }
-        if (sizeof(T) == 4 && o.real_input && (INV || in_rot != 0) && n >= 512 && n <= (1u << 24) && (n >= (1u << 15) || n * batch >= (1u << 18)) &&
-            (n >= 4096 || batch % (4096 / n) == 0)) {
-            // real f32 input in the throughput regime: one complexifying pass (4 B read + 8 B written per point) and the
-            // packed complex passes beat the generic kernels that fuse the conversion into their first load
-            BDSP_WS(cx, C*, n * batch * sizeof(C), 1);
-            int rc = ew_zero_interleave<T>(in, cx, n * batch, 2, 1, st);
-            if (rc) return rc;
-            FftOpts oc = o;
-            oc.real_input = 0;
-            oc.in_mul = im;
-            return fft_any<T, INV>(cx, out, n, batch, oc, work, work_bytes, st);
-        }
-        if (sizeof(T) == 4 && !im.kind && !o.real_input && n >= 64 && n <= 16384) {
-            // packed-FP32x2 kernel (fftp.cu); returns 1 when the configuration is not covered
-            const int rc = fftp_try(in, out, n, batch, INV, (size_t)in_rot, (size_t)om.rot, o.scale, o.magnitude != 0, st);
-            if (rc <= 0) return rc;
-        }
-        void* w = work;
-        if (n > fft_block_max_n<T>()) {
-            size_t need = n * batch * sizeof(C);
-            if (!w || work_bytes < need) { w = workspace(need, 0); if (!w) return -1001; }
-        }
-        if (sizeof(T) == 4 && n == 65536 && !o.real_input && !im.kind && !o.magnitude) {
-            // few 2^16-point vectors: one launch on a 16-CTA cluster, transposition through distributed shared memory (fftc.cu)
-            const int rc = fftc_try(in, out, n, batch, INV, (size_t)in_rot, (size_t)om.rot, o.scale, st);
-            if (rc <= 0) return rc;
-        }
-        if (sizeof(T) == 4 && n >= (1u << 15) && n <= (1u << 20)) {
-            // packed two-pass path (fftp.cu): 16 B/point of traffic per pass
-            const int rc = fftp_two_pass_try(in, out, w, n, batch, INV, (size_t)in_rot, (size_t)om.rot, o.scale, o.magnitude != 0, st, o.real_input != 0, im);
-            if (rc <= 0) return rc;
-        }
-        if (sizeof(T) == 4 && n >= (1u << 21) && n <= (1u << 24)) {
-            // packed three-pass path (fftp.cu)
-            const int rc = fftp_three_pass_try(in, out, w, n, batch, INV, (size_t)in_rot, (size_t)om.rot, o.scale, o.magnitude != 0, st, o.real_input != 0, im);
-            if (rc <= 0) return rc;
-        }
-        return fft_pow2<T, INV>(in, out, n, batch, o.real_input, o.magnitude, in_rot, scale, om, w, st, im);
+    case FftRoute::Complexify: {
+        BDSP_WS(cx, C*, n * batch * sizeof(C), 1);
+        const int rc = ew_zero_interleave<T>(in, cx, n * batch, 2, 1, st);
+        if (rc) return rc;
+        FftOpts oc = o;
+        oc.real_input = 0;
+        oc.in_mul = im;
+        return fft_any<T, INV>(cx, out, n, batch, oc, work, work_bytes, st);
     }
-    // n = q * P with q odd
-    size_t P = 1;
-    while ((n % (2 * P)) == 0) P *= 2;
-    const size_t q = n / P;
-    if (q <= 31 && P >= 2) {
-        size_t need = n * batch * sizeof(C);
-        if (sizeof(T) == 8 && P > fft_block_max_n<T>() && !o.magnitude) {
-            // f64, long q * 2^k: three passes with the radix-q step inside the first one (C5a: 3 * 2^26)
-            void* w = work;
-            if (!w || work_bytes < need || w == in || w == out) { w = workspace(need, 0); if (!w) return -1001; }
-            const int rc = fft_q_three_pass<T, INV>(in, out, n, batch, q, o.real_input != 0, false, in_rot, scale, om, w, st, im);
-            if (rc <= 0) return rc;
-        }
+    case FftRoute::RealRows: return fftp_single<true>(in, out, n, plan.groups, false, false, so, mag, o.scale, st);
+    case FftRoute::Packed: return fftp_single<false>(in, out, n, plan.groups, INV, si, so, mag, o.scale, st);
+    case FftRoute::Packed16k: return fftp16k(in, out, batch, INV, si, so, mag, (float)o.scale, st);
+    case FftRoute::Cluster: return fftc65536(in, out, batch, INV, si, so, o.scale, st);
+    case FftRoute::TwoPass: return fftp_two_pass(in, out, w, plan, batch, INV, si, so, mag, o.scale, real_in, im, st);
+    case FftRoute::ThreePass: return fftp_three_pass(in, out, w, plan, n, batch, INV, si, so, mag, o.scale, real_in, im, st);
+    case FftRoute::C64Rows:
+    case FftRoute::Block:
+    case FftRoute::Hybrid:
+    case FftRoute::Tiles: return fft_pow2<T, INV>(plan, in, out, n, batch, real_in, mag, in_rot, scale, om, w, st, im);
+    case FftRoute::QThreePass: {
+        // f64, long q * 2^k: three passes with the radix-q step inside the first one (C5a: 3 * 2^26)
+        const size_t need = n * batch * sizeof(C);
+        if (!w || work_bytes < need || w == in || w == out) { w = workspace(need, 0); if (!w) return -1001; }
+        return fft_q_three_pass<T, INV>(plan, in, out, n, batch, real_in, in_rot, scale, om, w, st, im);
+    }
+    case FftRoute::QRowsInterleave:
+    case FftRoute::QRows: {
+        const size_t P = plan.P, q = plan.q, need = n * batch * sizeof(C);
         BDSP_WS(w1, C*, need, 1);
         const long long tot = (long long)(P * batch);
         const unsigned qgrid = (unsigned)((tot + 255) / 256);
@@ -978,30 +957,27 @@ int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o,
         else if (q == 7) dft_q_pass_kernel<T, INV, 7><<<qgrid, 256, 0, st>>>(in, w1, 7, (long long)P, (long long)batch, in_rot, o.real_input, scale, im);
         else dft_q_pass_kernel<T, INV, 0><<<qgrid, 256, 0, st>>>(in, w1, (int)q, (long long)P, (long long)batch, in_rot, o.real_input, scale, im);
         BDSP_LAUNCHED();
-        OutMap om2;
-        om2.seq_group = (long long)q; om2.oes = (long long)q; om2.group_stride = (long long)n;
-        om2.rot = om.rot; om2.rot_n = (long long)n;
-        // c32 rows with a packed single-pass kernel (whole groups of 4096 points) in the throughput regime: packed rows +
-        // interleave pass beat the generic kernel with the interleave fused into its stores (3072-point rows: 0.69 ms
-        // vs the three-kernel path per 2^26 points)
-        const bool packed_rows = sizeof(T) == 4 && P >= 256 && P <= fft_block_max_n<T>() && n * batch >= (1u << 18) &&
-                                 (P >= 4096 || (batch * q) % (4096 / P) == 0);
-        if (P > fft_block_max_n<T>() || packed_rows) {
-            // row transforms into a second buffer (natural order), then one interleave pass
-            void* w0 = P > fft_block_max_n<T>() ? workspace(need, 0) : nullptr;
-            if (P > fft_block_max_n<T>() && !w0) return -1001;
-            BDSP_WS(w2, C*, need, 2);
-            OutMap plainP; plainP.seq_group = 1; plainP.oes = 1; plainP.group_stride = (long long)P; plainP.rot = 0; plainP.rot_n = (long long)P;
-            (void)plainP;
-            FftOpts po;   // plain transform of the q*batch rows: takes the packed passes where they exist
-            po.inverse = INV;
-            int rc = fft_any<T, INV>(w1, w2, P, batch * q, po, w0, w0 ? need : 0, st);
-            if (rc) return rc;
-            interleave_q_kernel<T><<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(w2, out, (int)q, (long long)P, (long long)batch, om.rot, o.magnitude);
-            BDSP_LAUNCHED();
-            return 0;
+        if (plan.route == FftRoute::QRows) {
+            // generic rows that store interleaved: result k1 + q*k2 of row (b, k1)
+            OutMap om2;
+            om2.seq_group = (long long)q; om2.oes = (long long)q; om2.group_stride = (long long)n;
+            om2.rot = om.rot; om2.rot_n = (long long)n;
+            return fft_pow2<T, INV>(generic_route<T>(w1, out, P, batch * q, INV, mag, nullptr), w1, out, P, batch * q, false, mag, 0, (T)1,
+                                    om2, nullptr, st);
         }
-        return fft_pow2<T, INV>(w1, out, P, batch * q, false, o.magnitude, 0, (T)1, om2, nullptr, st);
+        // row transforms into a second buffer (natural order), then one interleave pass
+        void* w0 = P > fft_block_max_n<T>() ? workspace(need, 0) : nullptr;
+        if (P > fft_block_max_n<T>() && !w0) return -1001;
+        BDSP_WS(w2, C*, need, 2);
+        FftOpts po;   // plain transform of the q*batch rows: takes the packed passes where they exist
+        po.inverse = INV;
+        const int rc = fft_any<T, INV>(w1, w2, P, batch * q, po, w0, w0 ? need : 0, st);
+        if (rc) return rc;
+        interleave_q_kernel<T><<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(w2, out, (int)q, (long long)P, (long long)batch, om.rot, o.magnitude);
+        BDSP_LAUNCHED();
+        return 0;
+    }
+    case FftRoute::Bluestein: break;
     }
     // Bluestein
     if (n >= (1ull << 31)) { set_last_error("fft: length %zu not supported", n); return -2; }
@@ -1030,7 +1006,7 @@ int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o,
     if (pingpong) { b2 = reinterpret_cast<C*>(workspace(M * batch * sizeof(C), 2)); if (!b2) return -1001; }
     if (w0) rc = fft_any<T, false>(a, a, M, batch, fo, w0, w0_bytes, st);
     else if (pingpong) rc = fft_any<T, false>(a, b2, M, batch, fo, nullptr, 0, st);
-    else rc = fft_pow2<T, false>(a, a, M, batch, false, false, 0, (T)1, plain, w0, st);
+    else rc = fft_pow2<T, false>(generic_route<T>(a, a, M, batch, false, false, w0), a, a, M, batch, false, false, 0, (T)1, plain, w0, st);
     if (rc) return rc;
     // the product with the chirp filter's spectrum (and the 1/M of the inverse) rides on the inverse transform's first
     // load where that transform takes a multiplier; the packed single-pass c32 kernels keep the separate pass
@@ -1045,7 +1021,8 @@ int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o,
     }
     if (w0) rc = fft_any<T, true>(a, a, M, batch, fo, w0, w0_bytes, st);
     else if (pingpong) rc = fft_any<T, true>(b2, a, M, batch, fo, nullptr, 0, st);
-    else rc = fft_pow2<T, true>(a, a, M, batch, false, false, 0, fused_filter ? (T)(1.0 / (double)M) : (T)1, plain, w0, st, fused_filter ? fm : InMul());
+    else rc = fft_pow2<T, true>(generic_route<T>(a, a, M, batch, true, false, w0), a, a, M, batch, false, false, 0,
+                                fused_filter ? (T)(1.0 / (double)M) : (T)1, plain, w0, st, fused_filter ? fm : InMul());
     if (rc) return rc;
     const long long totn = (long long)(n * batch);
     bluestein_post_kernel<T, INV><<<(unsigned)((totn + 255) / 256), 256, 0, st>>>(a, out, (long long)n, (long long)M, (long long)batch, om, o.magnitude);

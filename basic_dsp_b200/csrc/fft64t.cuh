@@ -378,16 +378,14 @@ int launch_row(const void* in, void* out, size_t batch, bool real_in, bool mag, 
     return 0;
 }
 
-// 1: not covered, 0: launched, < 0: error.  The scale is applied to the input by the generic kernel and to the output here
-// (the transform is linear).
+// n = 1024 / 2048 / 4096, batch < 2^31 (FftRoute::C64Rows); 0: launched, < 0: error.  The scale is applied to the input by
+// the generic kernel and to the output here (the transform is linear).
 template <bool INV>
 int launch_rows(const void* in, void* out, size_t n, size_t batch, bool real_in, bool mag, long long in_rot, double scale, const OutMap& om,
                 const InMul& im, const double2* tw, cudaStream_t st) {
-    if (batch > 0x7fffffffull) return 1;
     if (n == 1024) return launch_row<10, INV>(in, out, batch, real_in, mag, in_rot, scale, om, im, tw, st);
     if (n == 2048) return launch_row<11, INV>(in, out, batch, real_in, mag, in_rot, scale, om, im, tw, st);
-    if (n == 4096) return launch_row<12, INV>(in, out, batch, real_in, mag, in_rot, scale, om, im, tw, st);
-    return 1;
+    return launch_row<12, INV>(in, out, batch, real_in, mag, in_rot, scale, om, im, tw, st);
 }
 
 }  // namespace f64t

@@ -103,46 +103,52 @@ fftc65536_kernel(const float2* __restrict__ x, float2* __restrict__ out, int shi
     }
 }
 
-}  // namespace
-
-// 1: not covered (the caller takes the two-pass path), 0: launched, < 0: error
-int fftc_try(const void* in, void* out, size_t n, size_t rows, bool inverse, size_t in_rot, size_t out_rot, double scale, cudaStream_t st) {
-    if (n != 65536 || rows == 0 || rows > 8 || in == out) return 1;
-    if ((in_rot != 0 && in_rot != n / 2) || (out_rot != 0 && out_rot != n / 2)) return 1;
-    if ((reinterpret_cast<uintptr_t>(in) & 7) || (reinterpret_cast<uintptr_t>(out) & 7)) return 1;
-    auto kf = fftc65536_kernel<false>;
-    auto ki = fftc65536_kernel<true>;
-    // per-device configuration; a device / driver that cannot place a 16-CTA cluster takes the two-pass path
-    static int state[16] = {};   // 0: unknown, 1: usable, -1: not usable
-    int dev = 0;
-    BDSP_CUDA_OK(cudaGetDevice(&dev));
+cudaLaunchConfig_t fftc_config(size_t rows, cudaStream_t st, cudaLaunchAttribute* attr) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(FC_CL * rows), 1, 1);
     cfg.blockDim = dim3(FC_T, 1, 1);
     cfg.dynamicSmemBytes = FC_SMEM;
     cfg.stream = st;
-    cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = FC_CL;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if (dev >= 16 || state[dev] == 0) {
-        bool ok = cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FC_SMEM) == cudaSuccess &&
-                  cudaFuncSetAttribute(ki, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FC_SMEM) == cudaSuccess &&
-                  cudaFuncSetAttribute(kf, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess &&
-                  cudaFuncSetAttribute(ki, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
-        int nclusters = 0;
-        if (ok) ok = cudaOccupancyMaxActiveClusters(&nclusters, kf, &cfg) == cudaSuccess && nclusters >= 1;
-        cudaGetLastError();   // a refusal here is not an error of the call: the two-pass path takes over
-        if (dev < 16) state[dev] = ok ? 1 : -1;
-        if (!ok) return 1;
-    }
-    if (dev < 16 && state[dev] < 0) return 1;
-    const int si = in_rot != 0, so = out_rot != 0;
-    if (inverse) BDSP_CUDA_OK(cudaLaunchKernelEx(&cfg, ki, reinterpret_cast<const float2*>(in), reinterpret_cast<float2*>(out), si, so, (float)scale));
-    else BDSP_CUDA_OK(cudaLaunchKernelEx(&cfg, kf, reinterpret_cast<const float2*>(in), reinterpret_cast<float2*>(out), si, so, (float)scale));
+    return cfg;
+}
+
+}  // namespace
+
+// Whether a 16-CTA cluster of the kernel can be placed on the current device (configures the kernel on first use).  A
+// device / driver that cannot place one takes the two-pass path.  Cached for device indices below 16.
+bool fftc_cluster_ok() {
+    static int state[16] = {};   // 0: unknown, 1: usable, -1: not usable
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) { cudaGetLastError(); return false; }
+    if (dev < 16 && state[dev]) return state[dev] > 0;
+    auto kf = fftc65536_kernel<false>;
+    auto ki = fftc65536_kernel<true>;
+    cudaLaunchAttribute attr[1];
+    const cudaLaunchConfig_t cfg = fftc_config(1, nullptr, attr);
+    bool ok = cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FC_SMEM) == cudaSuccess &&
+              cudaFuncSetAttribute(ki, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FC_SMEM) == cudaSuccess &&
+              cudaFuncSetAttribute(kf, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess &&
+              cudaFuncSetAttribute(ki, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
+    int nclusters = 0;
+    if (ok) ok = cudaOccupancyMaxActiveClusters(&nclusters, kf, &cfg) == cudaSuccess && nclusters >= 1;
+    cudaGetLastError();   // a refusal here is not an error of the call: the two-pass path takes over
+    if (dev < 16) state[dev] = ok ? 1 : -1;
+    return ok;
+}
+
+// 1 .. 8 sequences of 65536 points, in != out (FftRoute::Cluster)
+int fftc65536(const void* in, void* out, size_t rows, bool inverse, bool shift_in, bool shift_out, double scale, cudaStream_t st) {
+    cudaLaunchAttribute attr[1];
+    const cudaLaunchConfig_t cfg = fftc_config(rows, st, attr);
+    auto kern = inverse ? fftc65536_kernel<true> : fftc65536_kernel<false>;
+    BDSP_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, reinterpret_cast<const float2*>(in), reinterpret_cast<float2*>(out), (int)shift_in,
+                                    (int)shift_out, (float)scale));
     BDSP_LAUNCHED();
     return 0;
 }

@@ -13,8 +13,8 @@
 //   RIN       the input holds real scalars
 // fftp_col16_kernel / fftp_col256_kernel: first pass(es) of the multi-pass transforms: 16- / 256-point (NH = 2: 32- / 512-point)
 //   columns of 16 adjacent columns per CTA, inter-pass twiddle evaluated with sincospif on exact arguments.
-// Dispatchers: fftp_try (single pass), fftp_try_real, fftp_two_pass_try (2^15..2^20), fftp_three_pass_try (2^21..2^24),
-//   fftp_rows1k_try (packed last pass behind a generic column pass).
+// Launchers, one per route of fft_route.h: fftp_single (complex or real rows), fftp_two_pass (2^15..2^20), fftp_three_pass
+//   (2^21..2^24), fftp_rows_pass (packed last pass, also behind a generic column pass).
 // Replaces rustfft for these lengths (vector/src/vector_types/time_freq/mod.rs:45-58) incl. the fused
 // fft_shift (time_to_freq.rs:163), ifft's scale + ifft_shift (freq_to_time.rs:165-167) and magnitude.
 #include <map>
@@ -665,59 +665,8 @@ int fftp_launch(const void* in, void* out, size_t rows, float scale, cudaStream_
     return 0;
 }
 
-template <int Q>
-int fftp_dispatch_nat(const void* in, void* out, size_t groups, bool inv, bool shift_in, bool shift_out, bool mag, float scale, cudaStream_t st) {
-    if (!inv) {
-        if (mag) return shift_out ? fftp_launch<1, false, false, true, true, false, 0, Q>(in, out, groups, scale, st)
-                                  : fftp_launch<1, false, false, false, true, false, 0, Q>(in, out, groups, scale, st);
-        return shift_out ? fftp_launch<1, false, false, true, false, false, 0, Q>(in, out, groups, scale, st)
-                         : fftp_launch<1, false, false, false, false, false, 0, Q>(in, out, groups, scale, st);
-    }
-    if (mag || shift_out) return 1;
-    return shift_in ? fftp_launch<1, true, true, false, false, false, 0, Q>(in, out, groups, scale, st)
-                    : fftp_launch<1, true, false, false, false, false, 0, Q>(in, out, groups, scale, st);
-}
-
-// rows of 64 / 128 points (fftp_kernel<SQ>): whole groups of 4096 points
-template <int P>
-int fftp_dispatch_short(const void* in, void* out, size_t groups, bool inv, bool shift_in, bool shift_out, bool mag, float scale, cudaStream_t st) {
-    if (!inv) {
-        if (mag) return shift_out ? fftp_launch<1, false, false, true, true, false, 0, 1, false, P>(in, out, groups, scale, st)
-                                  : fftp_launch<1, false, false, false, true, false, 0, 1, false, P>(in, out, groups, scale, st);
-        return shift_out ? fftp_launch<1, false, false, true, false, false, 0, 1, false, P>(in, out, groups, scale, st)
-                         : fftp_launch<1, false, false, false, false, false, 0, 1, false, P>(in, out, groups, scale, st);
-    }
-    if (mag || shift_out) return 1;
-    return shift_in ? fftp_launch<1, true, true, false, false, false, 0, 1, false, P>(in, out, groups, scale, st)
-                    : fftp_launch<1, true, false, false, false, false, 0, 1, false, P>(in, out, groups, scale, st);
-}
-
-template <int R0>
-int fftp_dispatch(const void* in, void* out, size_t rows, bool inv, bool shift_in, bool shift_out, bool mag, float scale,
-                  cudaStream_t st) {
-    if (!inv) {
-        if (mag) return shift_out ? fftp_launch<R0, false, false, true, true>(in, out, rows, scale, st)
-                                  : fftp_launch<R0, false, false, false, true>(in, out, rows, scale, st);
-        return shift_out ? fftp_launch<R0, false, false, true, false>(in, out, rows, scale, st)
-                         : fftp_launch<R0, false, false, false, false>(in, out, rows, scale, st);
-    }
-    if (mag || shift_out) return 1;   // not instantiated: caller falls back to the generic kernel
-    return shift_in ? fftp_launch<R0, true, true, false, false>(in, out, rows, scale, st)
-                    : fftp_launch<R0, true, false, false, false>(in, out, rows, scale, st);
-}
-
-
-// last pass over 4096-point rows, four adjacent rows per 512-thread CTA
-int fftp_rows_pass(const void* tmp, void* out, size_t groups, bool inverse, bool so, bool magnitude, float sc, cudaStream_t st, int n1) {
-    if (inverse) return fftp_launch<4, true, false, false, false, true>(tmp, out, groups, sc, st, n1);
-    if (magnitude) return so ? fftp_launch<4, false, false, true, true, true>(tmp, out, groups, sc, st, n1)
-                             : fftp_launch<4, false, false, false, true, true>(tmp, out, groups, sc, st, n1);
-    return so ? fftp_launch<4, false, false, true, false, true>(tmp, out, groups, sc, st, n1)
-              : fftp_launch<4, false, false, false, false, true>(tmp, out, groups, sc, st, n1);
-}
-
 template <bool INV, bool SI, bool RIN = false>
-int fftp_colpass(const void* in, void* tmp, int n1, int log2n2, size_t rows, cudaStream_t st, const InMul& im = InMul()) {
+int fftp_colpass(const void* in, void* tmp, int n1, int log2n2, size_t rows, cudaStream_t st, const InMul& im) {
     const float* tw = fftp_twiddles();
     if (!tw) return -1001;
     const float2* i2 = reinterpret_cast<const float2*>(in);
@@ -743,187 +692,81 @@ int fftp_colpass(const void* in, void* tmp, int n1, int log2n2, size_t rows, cud
     return 0;
 }
 
-// last pass over rows of 256*Q points, 16/Q adjacent rows per 128-thread CTA
-template <int Q>
-int fftp_rowsq_pass(const void* tmp, void* out, size_t groups, bool inverse, bool so, bool magnitude, float sc, cudaStream_t st, int n1,
-                    int n2c = 1) {
-    if (inverse) return fftp_launch<1, true, false, false, false, true, Q>(tmp, out, groups, sc, st, n1, n2c);
-    if (magnitude) return so ? fftp_launch<1, false, false, true, true, true, Q>(tmp, out, groups, sc, st, n1, n2c)
-                             : fftp_launch<1, false, false, false, true, true, Q>(tmp, out, groups, sc, st, n1, n2c);
-    return so ? fftp_launch<1, false, false, true, false, true, Q>(tmp, out, groups, sc, st, n1, n2c)
-              : fftp_launch<1, false, false, false, false, true, Q>(tmp, out, groups, sc, st, n1, n2c);
+// first pass of the multi-pass transforms; real input comes forward and unrotated only
+int fftp_first_colpass(const void* in, void* tmp, int n1, int log2n2, size_t rows, bool inverse, bool si, bool real_in, const InMul& im,
+                       cudaStream_t st) {
+    if (real_in) return fftp_colpass<false, false, true>(in, tmp, n1, log2n2, rows, st, im);
+    if (inverse) return si ? fftp_colpass<true, true>(in, tmp, n1, log2n2, rows, st, im) : fftp_colpass<true, false>(in, tmp, n1, log2n2, rows, st, im);
+    return si ? fftp_colpass<false, true>(in, tmp, n1, log2n2, rows, st, im) : fftp_colpass<false, false>(in, tmp, n1, log2n2, rows, st, im);
 }
 }  // namespace
 
-// two-pass packed transform for n = 2^16 and 2^20 (tmp: n*rows complex values, distinct from in; may equal out only
-// if out != in).  Returns 1 when the configuration is not covered.
-int fftp_two_pass_try(const void* in, void* out, void* tmp, size_t n, size_t rows, bool inverse, size_t in_rot, size_t out_rot,
-                      double scale, bool magnitude, cudaStream_t st, bool real_in, const InMul& im) {
-    if (real_in && (inverse || in_rot != 0)) return 1;
-    // n = n1 * N2:  2^15 = 32 x 1024, 2^16 = 256 x 256, 2^17 = 256 x 512, 2^18 = 256 x 1024, 2^19 = 512 x 1024, 2^20 = 256 x 4096.
-    // (two adjacent 2048-point rows give only 16-byte store runs: 16 x 2048 took 0.46 ms and 256 x 2048 0.48 ms per 2^26 points)
-    // Last pass: 16/Q adjacent rows of N2 = 256*Q points per 128-thread CTA (Q = N2/256 <= 8), or four 4096-point rows per
-    // 512-thread CTA.
-    int n1, log2n2;
-    switch (n) {
-    case 1u << 15: n1 = 32; log2n2 = 10; break;
-    case 1u << 16: n1 = 256; log2n2 = 8; break;
-    case 1u << 17: n1 = 256; log2n2 = 9; break;
-    case 1u << 18: n1 = 256; log2n2 = 10; break;
-    case 1u << 19: n1 = 512; log2n2 = 10; break;
-    case 1u << 20: n1 = 256; log2n2 = 12; break;
-    default: return 1;
-    }
-    if ((in_rot != 0 && in_rot != n / 2) || (out_rot != 0 && out_rot != n / 2)) return 1;
-    if (inverse && (magnitude || out_rot != 0)) return 1;
-    if ((reinterpret_cast<uintptr_t>(in) & (real_in ? 7 : 15)) || (reinterpret_cast<uintptr_t>(out) & 7) || (reinterpret_cast<uintptr_t>(tmp) & 15)) return 1;
-    if (tmp == in || tmp == out) return 1;
-    const int tq = log2n2 < 12 ? 1 << (log2n2 - 8) : 0;
-    // The 4096-point last pass takes four rows per 512-thread CTA (one CTA per SM, full 32-byte store sectors).  Measured on
-    // B200 (64 x 2^20): 0.453 ms, against 0.494 ms with two rows per 256-thread CTA (16-byte half sectors, two CTAs per SM).
-    const int rpc = tq ? 16 / tq : 4;
-    const size_t groups = rows * (size_t)(n1 / rpc);
-    if (groups > 0x7fffffffull || rows * 4096 > 0x7fffffffull) return 1;
-    const bool si = in_rot != 0, so = out_rot != 0;
+// Last pass of a multi-pass transform, stored at k1 + n1 * k2 (+ n1 * n2c * k3): tq = 0: four adjacent 4096-point rows per
+// 512-thread CTA; tq = Q: 16/Q adjacent rows of 256*Q points per 128-thread CTA.  Also the packed 1024-point pass (tq = 4)
+// behind the generic column pass of FftRoute::Hybrid, which left tmp[k1 * 1024 + n2] (column transform and inter-pass
+// twiddle applied).
+int fftp_rows_pass(const void* tmp, void* out, int tq, size_t groups, bool inverse, bool so, bool magnitude, float sc, cudaStream_t st,
+                   int n1, int n2c) {
+    return fftp_with_flags<true, false>(inverse, false, so, magnitude, [&](auto inv, auto si, auto sho, auto mag) {
+        switch (tq) {
+        case 0: return fftp_launch<4, inv, si, sho, mag, true>(tmp, out, groups, sc, st, n1, n2c);
+        case 1: return fftp_launch<1, inv, si, sho, mag, true, 1>(tmp, out, groups, sc, st, n1, n2c);
+        case 2: return fftp_launch<1, inv, si, sho, mag, true, 2>(tmp, out, groups, sc, st, n1, n2c);
+        case 4: return fftp_launch<1, inv, si, sho, mag, true, 4>(tmp, out, groups, sc, st, n1, n2c);
+        default: return fftp_launch<1, inv, si, sho, mag, true, 8>(tmp, out, groups, sc, st, n1, n2c);
+        }
+    });
+}
+
+// single pass over rows of n = 64 .. 16384 points (FftRoute::Packed); RIN: forward transforms of real scalars (FftRoute::RealRows)
+template <bool RIN>
+int fftp_single(const void* in, void* out, size_t n, size_t groups, bool inverse, bool si, bool so, bool magnitude, double scale,
+                cudaStream_t st) {
     const float sc = (float)scale;
+    return fftp_with_flags<!RIN, !RIN>(inverse, si, so, magnitude, [&](auto inv, auto shi, auto sho, auto mag) {
+        switch (n) {
+        case 64: return fftp_launch<1, inv, shi, sho, mag, false, 0, 1, RIN, 4>(in, out, groups, sc, st);
+        case 128: return fftp_launch<1, inv, shi, sho, mag, false, 0, 1, RIN, 8>(in, out, groups, sc, st);
+        case 256: return fftp_launch<1, inv, shi, sho, mag, false, 0, 1, RIN>(in, out, groups, sc, st);
+        case 512: return fftp_launch<1, inv, shi, sho, mag, false, 0, 2, RIN>(in, out, groups, sc, st);
+        case 1024: return fftp_launch<1, inv, shi, sho, mag, false, 0, 4, RIN>(in, out, groups, sc, st);
+        case 2048: return fftp_launch<1, inv, shi, sho, mag, false, 0, 8, RIN>(in, out, groups, sc, st);
+        case 4096: return fftp_launch<1, inv, shi, sho, mag, false, 0, 0, RIN>(in, out, groups, sc, st);
+        case 8192: return fftp_launch<2, inv, shi, sho, mag, false, 0, 0, RIN>(in, out, groups, sc, st);
+        default: return fftp_launch<4, inv, shi, sho, mag, false, 0, 0, RIN>(in, out, groups, sc, st);
+        }
+    });
+}
+template int fftp_single<false>(const void*, void*, size_t, size_t, bool, bool, bool, bool, double, cudaStream_t);
+template int fftp_single<true>(const void*, void*, size_t, size_t, bool, bool, bool, bool, double, cudaStream_t);
+
+// two-pass transform for n = 2^15 .. 2^20 (FftRoute::TwoPass), n = p.n1 * 2^p.log2n2; tmp holds n*rows complex values
+int fftp_two_pass(const void* in, void* out, void* tmp, const FftPlan& p, size_t rows, bool inverse, bool si, bool so, bool magnitude,
+                  double scale, bool real_in, const InMul& im, cudaStream_t st) {
     // One launch pair over the whole batch.  Measured on B200 (64 x 2^20): 0.448 ms, against 0.571 / 0.596 / 1.18 ms for
     // chunks of sequences whose intermediate (8 bytes per point) is 64 / 32 / 8 MB and could stay in the 126 MB L2 between
     // the passes: launch rate and wave tails cost more than the saved DRAM traffic.
-    int rc;
-    if (real_in) rc = fftp_colpass<false, false, true>(in, tmp, n1, log2n2, rows, st, im);
-    else if (inverse) rc = si ? fftp_colpass<true, true>(in, tmp, n1, log2n2, rows, st, im) : fftp_colpass<true, false>(in, tmp, n1, log2n2, rows, st, im);
-    else rc = si ? fftp_colpass<false, true>(in, tmp, n1, log2n2, rows, st, im) : fftp_colpass<false, false>(in, tmp, n1, log2n2, rows, st, im);
+    const int rc = fftp_first_colpass(in, tmp, p.n1, p.log2n2, rows, inverse, si, real_in, im, st);
     if (rc) return rc;
-    if (tq == 8) return fftp_rowsq_pass<8>(tmp, out, groups, inverse, so, magnitude, sc, st, n1);
-    if (tq == 4) return fftp_rowsq_pass<4>(tmp, out, groups, inverse, so, magnitude, sc, st, n1);
-    if (tq == 2) return fftp_rowsq_pass<2>(tmp, out, groups, inverse, so, magnitude, sc, st, n1);
-    if (tq == 1) return fftp_rowsq_pass<1>(tmp, out, groups, inverse, so, magnitude, sc, st, n1);
-    return fftp_rows_pass(tmp, out, groups, inverse, so, magnitude, sc, st, n1);
+    // The 4096-point last pass takes four rows per 512-thread CTA (one CTA per SM, full 32-byte store sectors).  Measured on
+    // B200 (64 x 2^20): 0.453 ms, against 0.494 ms with two rows per 256-thread CTA (16-byte half sectors, two CTAs per SM).
+    const int tq = p.log2n2 < 12 ? 1 << (p.log2n2 - 8) : 0;
+    return fftp_rows_pass(tmp, out, tq, p.groups, inverse, so, magnitude, (float)scale, st, p.n1, 1);
 }
 
-
-// three-pass packed transform for n = 2^21 .. 2^24:  n = nA * 256 * N3 with nA in {16, 32, 256}:
+// three-pass transform for n = 2^21 .. 2^24 (FftRoute::ThreePass):  n = nA * 256 * N3 with nA = p.n1 in {16, 32, 256}:
 //   pass A: nA-point columns over stride n/nA (+ W_n twiddle), pass B: 256-point columns inside every block of 256*N3
 //   points (exactly the first pass of the two-pass transform of that length, in place), pass C: rows of N3 = 256*Q points,
 //   16/Q rows with consecutive k1 per CTA, stored at k1 + nA*k2 + nA*256*k3.
-int fftp_three_pass_try(const void* in, void* out, void* tmp, size_t n, size_t rows, bool inverse, size_t in_rot, size_t out_rot,
-                        double scale, bool magnitude, cudaStream_t st, bool real_in, const InMul& im) {
-    if (real_in && (inverse || in_rot != 0)) return 1;
-    int nA, log2n3;
-    switch (n) {
-    case 1u << 21: nA = 16; log2n3 = 9; break;
-    case 1u << 22: nA = 16; log2n3 = 10; break;
-    case 1u << 23: nA = 32; log2n3 = 10; break;
-    case 1u << 24: nA = 256; log2n3 = 8; break;
-    default: return 1;
-    }
-    if ((in_rot != 0 && in_rot != n / 2) || (out_rot != 0 && out_rot != n / 2)) return 1;
-    if (inverse && (magnitude || out_rot != 0)) return 1;
-    if ((reinterpret_cast<uintptr_t>(in) & (real_in ? 7 : 15)) || (reinterpret_cast<uintptr_t>(out) & 7) || (reinterpret_cast<uintptr_t>(tmp) & 15)) return 1;
-    if (tmp == in || tmp == out) return 1;
-    const int tq = 1 << (log2n3 - 8);
-    if (rows * (n >> 4) > 0x7fffffffull) return 1;
-    const bool si = in_rot != 0, so = out_rot != 0;
-    int rc;
+int fftp_three_pass(const void* in, void* out, void* tmp, const FftPlan& p, size_t n, size_t rows, bool inverse, bool si, bool so,
+                    bool magnitude, double scale, bool real_in, const InMul& im, cudaStream_t st) {
     int l2 = 0;
-    while (((size_t)nA << l2) < n) l2++;                 // n / nA = 2^l2
-    if (real_in) rc = fftp_colpass<false, false, true>(in, tmp, nA, l2, rows, st, im);
-    else if (inverse) rc = si ? fftp_colpass<true, true>(in, tmp, nA, l2, rows, st, im) : fftp_colpass<true, false>(in, tmp, nA, l2, rows, st, im);
-    else rc = si ? fftp_colpass<false, true>(in, tmp, nA, l2, rows, st, im) : fftp_colpass<false, false>(in, tmp, nA, l2, rows, st, im);
+    while (((size_t)p.n1 << l2) < n) l2++;                 // n / nA = 2^l2
+    int rc = fftp_first_colpass(in, tmp, p.n1, l2, rows, inverse, si, real_in, im, st);
     if (rc) return rc;
-    rc = inverse ? fftp_colpass<true, false>(tmp, tmp, 256, log2n3, rows * (size_t)nA, st) : fftp_colpass<false, false>(tmp, tmp, 256, log2n3, rows * (size_t)nA, st);
+    rc = fftp_first_colpass(tmp, tmp, 256, p.log2n3, rows * (size_t)p.n1, inverse, false, false, InMul(), st);
     if (rc) return rc;
-    const size_t groups = rows * (size_t)(nA / (16 / tq)) * 256;
-    const float sc = (float)scale;
-    if (tq == 8) return fftp_rowsq_pass<8>(tmp, out, groups, inverse, so, magnitude, sc, st, nA, 256);
-    if (tq == 4) return fftp_rowsq_pass<4>(tmp, out, groups, inverse, so, magnitude, sc, st, nA, 256);
-    if (tq == 2) return fftp_rowsq_pass<2>(tmp, out, groups, inverse, so, magnitude, sc, st, nA, 256);
-    return fftp_rowsq_pass<1>(tmp, out, groups, inverse, so, magnitude, sc, st, nA, 256);
-}
-
-// Last pass of a two-pass transform of n = n1 * 1024 points whose first pass (any kernel) left tmp[k1 * 1024 + n2]
-// (k1-th column transform, inter-pass twiddle applied): X[k1 + n1 * k2] = sum_n2 tmp[k1][n2] W_1024^{n2 k2}.
-// Returns 1 when the configuration is not covered.
-int fftp_rows1k_try(const void* tmp, void* out, size_t n, size_t rows, bool inverse, size_t out_rot, double scale, bool magnitude,
-                    cudaStream_t st) {
-    if (n < 4096 || (n & (n - 1)) || n > ((size_t)1 << 30)) return 1;
-    if (out_rot != 0 && out_rot != n / 2) return 1;
-    if (inverse && (magnitude || out_rot != 0)) return 1;
-    if ((reinterpret_cast<uintptr_t>(tmp) & 15) || (reinterpret_cast<uintptr_t>(out) & 7) || tmp == out) return 1;
-    const int n1 = (int)(n / 1024);
-    const size_t groups = rows * (size_t)(n1 / 4);
-    if (groups > 0x7fffffffull) return 1;
-    return fftp_rowsq_pass<4>(tmp, out, groups, inverse, out_rot != 0, magnitude, (float)scale, st, n1);
-}
-
-int fftp16k_try(const void* in, void* out, size_t rows, bool inverse, bool shift_in, bool shift_out, bool magnitude, float scale,
-                cudaStream_t st);
-
-// returns 0 on success, 1 when this configuration is not covered (caller uses the generic kernel)
-int fftp_try(const void* in, void* out, size_t n, size_t rows, bool inverse, size_t in_rot, size_t out_rot, double scale,
-             bool magnitude, cudaStream_t st) {
-    if (n != 64 && n != 128 && n != 256 && n != 512 && n != 1024 && n != 2048 && n != 4096 && n != 8192 && n != 16384) return 1;
-    if ((in_rot != 0 && in_rot != n / 2) || (out_rot != 0 && out_rot != n / 2)) return 1;
-    if (n < 4096) {
-        // several rows per CTA: whole groups of 4096 points only (the caller handles other batch sizes generically)
-        const size_t per = 4096 / n;
-        if (rows % per != 0) return 1;
-        if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(out) & 7) || in == out) return 1;
-        const size_t groups = rows / per;
-        if (groups > 0x7fffffffull) return 1;
-        const bool si = in_rot != 0, so = out_rot != 0;
-        if (n == 64) return fftp_dispatch_short<4>(in, out, groups, inverse, si, so, magnitude, (float)scale, st);
-        if (n == 128) return fftp_dispatch_short<8>(in, out, groups, inverse, si, so, magnitude, (float)scale, st);
-        if (n == 256) return fftp_dispatch_nat<1>(in, out, groups, inverse, si, so, magnitude, (float)scale, st);
-        if (n == 512) return fftp_dispatch_nat<2>(in, out, groups, inverse, si, so, magnitude, (float)scale, st);
-        if (n == 1024) return fftp_dispatch_nat<4>(in, out, groups, inverse, si, so, magnitude, (float)scale, st);
-        return fftp_dispatch_nat<8>(in, out, groups, inverse, si, so, magnitude, (float)scale, st);
-    }
-    if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(out) & 7)) return 1;
-    if (in == out) return 1;   // rows are consumed while other CTAs may still read them only within a row; keep it simple
-    if (rows * 2 > 0x7fffffffull) return 1;
-    const bool si = in_rot != 0, so = out_rot != 0;
-    const float sc = (float)scale;
-    if (n == 4096) return fftp_dispatch<1>(in, out, rows, inverse, si, so, magnitude, sc, st);
-    if (n == 16384 && rows >= 2) {
-        // persistent CTAs with the rolling F3 || F0 pipeline (fftp16k.cu)
-        const int rc = fftp16k_try(in, out, rows, inverse, si, so, magnitude, sc, st);
-        if (rc <= 0) return rc;
-    }
-    if (n == 8192) return fftp_dispatch<2>(in, out, rows, inverse, si, so, magnitude, sc, st);
-    return fftp_dispatch<4>(in, out, rows, inverse, si, so, magnitude, sc, st);
-}
-
-// real-input forward transforms (fftp_kernel<RIN>): rows of `n` real scalars, n in {512 ... 16384}
-template <int R0, int Q, int SQ = 0>
-int fftp_dispatch_real(const void* in, void* out, size_t groups, bool shift_out, bool mag, float scale, cudaStream_t st) {
-    if (mag) return shift_out ? fftp_launch<R0, false, false, true, true, false, 0, Q, true, SQ>(in, out, groups, scale, st)
-                              : fftp_launch<R0, false, false, false, true, false, 0, Q, true, SQ>(in, out, groups, scale, st);
-    return shift_out ? fftp_launch<R0, false, false, true, false, false, 0, Q, true, SQ>(in, out, groups, scale, st)
-                     : fftp_launch<R0, false, false, false, false, false, 0, Q, true, SQ>(in, out, groups, scale, st);
-}
-
-int fftp_try_real(const void* in, void* out, size_t n, size_t rows, size_t out_rot, double scale, bool magnitude, cudaStream_t st) {
-    if (n != 64 && n != 128 && n != 256 && n != 512 && n != 1024 && n != 2048 && n != 4096 && n != 8192 && n != 16384) return 1;
-    if (out_rot != 0 && out_rot != n / 2) return 1;
-    if ((reinterpret_cast<uintptr_t>(in) & 7) || (reinterpret_cast<uintptr_t>(out) & 7) || in == out) return 1;
-    const size_t per = n < 4096 ? 4096 / n : 1;
-    if (rows % per != 0) return 1;
-    const size_t groups = rows / per;
-    if (groups * 2 > 0x7fffffffull) return 1;
-    const bool so = out_rot != 0;
-    const float sc = (float)scale;
-    switch (n) {
-    case 64: return fftp_dispatch_real<1, 1, 4>(in, out, groups, so, magnitude, sc, st);
-    case 128: return fftp_dispatch_real<1, 1, 8>(in, out, groups, so, magnitude, sc, st);
-    case 256: return fftp_dispatch_real<1, 1>(in, out, groups, so, magnitude, sc, st);
-    case 512: return fftp_dispatch_real<1, 2>(in, out, groups, so, magnitude, sc, st);
-    case 1024: return fftp_dispatch_real<1, 4>(in, out, groups, so, magnitude, sc, st);
-    case 2048: return fftp_dispatch_real<1, 8>(in, out, groups, so, magnitude, sc, st);
-    case 4096: return fftp_dispatch_real<1, 0>(in, out, groups, so, magnitude, sc, st);
-    case 8192: return fftp_dispatch_real<2, 0>(in, out, groups, so, magnitude, sc, st);
-    default: return fftp_dispatch_real<4, 0>(in, out, groups, so, magnitude, sc, st);
-    }
+    return fftp_rows_pass(tmp, out, 1 << (p.log2n3 - 8), p.groups, inverse, so, magnitude, (float)scale, st, p.n1, 256);
 }
 
 }  // namespace bdsp

@@ -1,6 +1,9 @@
 // Shared pieces of the packed-FP32x2 FFT kernels (fftp.cu, fftp16k.cu): shared-memory layout and twiddle table offsets.
 #pragma once
+#include <type_traits>
+
 #include "fft.cuh"
+#include "fft_route.h"
 #include "ols4096.cuh"
 
 namespace bdsp {
@@ -29,5 +32,26 @@ __device__ __forceinline__ int fp_rot(int row, int g) { return (((g >> 1) + (row
 
 // per-device table (nullptr and last error set on failure)
 const float* fftp_twiddles();
+
+// Calls launch(INV, SHIFT_IN, SHIFT_OUT, MAG) with std::bool_constant arguments for the variant a packed kernel has.  Every
+// packed kernel has the four forward variants (fft_shift and magnitude on the store, nothing on the load); HAS_INV adds the
+// plain inverse one, HAS_INV_SI the inverse one with ifft_shift on the load.  A combination without a kernel is an error.
+template <bool HAS_INV, bool HAS_INV_SI, typename L>
+int fftp_with_flags(bool inv, bool si, bool so, bool mag, const L& launch) {
+    const std::true_type y;
+    const std::false_type n;
+    if (!inv && !si) {
+        if (mag) return so ? launch(n, n, y, y) : launch(n, n, n, y);
+        return so ? launch(n, n, y, n) : launch(n, n, n, n);
+    }
+    if constexpr (HAS_INV) {
+        if (inv && !so && !mag) {
+            if constexpr (HAS_INV_SI) { if (si) return launch(y, y, n, n); }
+            if (!si) return launch(y, n, n, n);
+        }
+    }
+    set_last_error("fftp: no kernel for inverse %d, ifft_shift %d, fft_shift %d, magnitude %d", (int)inv, (int)si, (int)so, (int)mag);
+    return -2;
+}
 
 }  // namespace bdsp

@@ -242,19 +242,11 @@ int f16_launch(const void* in, void* out, size_t rows, float scale, cudaStream_t
 
 int sm_count();
 
-// rows of 16384 c32 points; returns 1 when the configuration is not covered
-int fftp16k_try(const void* in, void* out, size_t rows, bool inverse, bool shift_in, bool shift_out, bool magnitude, float scale,
-                cudaStream_t st) {
-    if (!inverse) {
-        if (shift_in) return 1;
-        if (magnitude) return shift_out ? f16_launch<false, false, true, true>(in, out, rows, scale, st)
-                                        : f16_launch<false, false, false, true>(in, out, rows, scale, st);
-        return shift_out ? f16_launch<false, false, true, false>(in, out, rows, scale, st)
-                         : f16_launch<false, false, false, false>(in, out, rows, scale, st);
-    }
-    if (magnitude || shift_out) return 1;
-    return shift_in ? f16_launch<true, true, false, false>(in, out, rows, scale, st)
-                    : f16_launch<true, false, false, false>(in, out, rows, scale, st);
+// rows of 16384 c32 points (FftRoute::Packed16k)
+int fftp16k(const void* in, void* out, size_t rows, bool inverse, bool shift_in, bool shift_out, bool magnitude, float scale, cudaStream_t st) {
+    return fftp_with_flags<true, true>(inverse, shift_in, shift_out, magnitude, [&](auto inv, auto si, auto so, auto mag) {
+        return f16_launch<inv, si, so, mag>(in, out, rows, scale, st);
+    });
 }
 
 }  // namespace bdsp

@@ -111,66 +111,76 @@ def gpu_fft(x, flags, dtype, off=0, inplace=False, window=None):
     return out.get((rows, n))
 
 
-# (dtype, n, rows, flags, variant, branch, selecting condition)
+# (dtype, n, rows, flags, variant, branch, selecting condition, route)
 #   variant: "" | "offset" (input and output one element past a 16-byte boundary) | "inplace" (in == out)
+#   route: what fft_route (csrc/fft_route.h) picks, level by level ("mul-pass > packed"); a dict maps flags to routes where
+#   they differ (None: the other flags).  Checked without a GPU by test_fft_route.py.
 FFT_CASES = []
 
 
-def fc(dtype, n, rows, flags, branch, cond, variant=""):
+def fc(dtype, n, rows, flags, branch, cond, route, variant=""):
     for f in flags:
-        FFT_CASES.append(pytest.param(dtype, n, rows, f, variant, branch, cond,
+        FFT_CASES.append(pytest.param(dtype, n, rows, f, variant, branch, cond, route,
                                       id="%s-%d-x%d-f%d%s" % ("c32" if dtype == F32 else "c64", n, rows, f, "-" + variant if variant else "")))
 
 
 _SP = {64: "fftp SQ=4", 128: "fftp SQ=8", 256: "fftp NATQ=1", 512: "fftp NATQ=2", 1024: "fftp NATQ=4", 2048: "fftp NATQ=8",
-       4096: "fftp_dispatch<1,1>", 8192: "fftp_dispatch<2,1>"}
+       4096: "fftp R0=1", 8192: "fftp R0=2"}
+PACKED = {None: "packed", REAL: "real-rows"}
 for n, name in _SP.items():
     # rows = 2^16 / n: a multiple of 4096 / n, and n * rows >= 2^16 for the real-input kernel
     fc(F32, n, 65536 // n, ALL_FLAGS, "packed single pass " + name,
-       "fft.cu fft_any: c32 pow2 64 <= n <= 16384, no in_mul -> fftp_try; n < 4096: rows % (4096/n) == 0; "
-       "REAL: fftp_try_real, n*rows >= 2^16")
+       "fft_route: c32 pow2 64 <= n <= 16384, no in_mul, in != out, in & 15 == 0; n < 4096: rows % (4096/n) == 0; "
+       "REAL: real-rows, n*rows >= 2^16", PACKED)
     if n < 4096:
-        fc(F32, n, 4096 // n + 1, ALL_FLAGS, "generic fall-back of " + name, "fftp_try: rows % (4096/n) != 0 -> fft_pow2 block kernel")
-    fc(F32, n, 4096 // n if n < 4096 else 2, (0, SH, INV, INV | SH), "generic fall-back of " + name, "fftp_try: in == out", "inplace")
+        fc(F32, n, 4096 // n + 1, ALL_FLAGS, "generic fall-back of " + name, "fft_route: rows % (4096/n) != 0 -> block kernel", "block")
+    fc(F32, n, 4096 // n if n < 4096 else 2, (0, SH, INV, INV | SH), "generic fall-back of " + name, "fft_route: in == out", "block",
+       "inplace")
     fc(F32, n, 4096 // n if n < 4096 else 2, ALL_FLAGS, "generic fall-back of " + name,
-       "fftp_try: in & 15 (fftp_try_real: in & 7) -> generic kernels", "offset")
-fc(F32, 16384, 4, ALL_FLAGS, "packed 16384 persistent (fftp16k)", "fftp_try: n == 16384 && rows >= 2 -> fftp16k_try")
-fc(F32, 16384, 1, ALL_FLAGS[:5], "packed 16384 non-persistent fftp_dispatch<4,1>", "fftp_try: n == 16384 && rows == 1")
-fc(F32, 16384, 2, (0, SH, INV, INV | SH), "generic fall-back of 16384", "fftp_try: in == out", "inplace")
-fc(F32, 16384, 2, ALL_FLAGS, "generic fall-back of 16384", "fftp_try: in & 15", "offset")
-fc(F32, 1 << 16, 1, (0, SH, INV, INV | SH), "2^16 cluster kernel (fftc)", "fft.cu: n == 65536, !real, !mag, fftc_try: rows <= 8, in != out")
-fc(F32, 1 << 16, 8, (0, SH, INV, INV | SH), "2^16 cluster kernel (fftc)", "fftc_try: rows <= 8")
-fc(F32, 1 << 16, 9, ALL_FLAGS, "packed two-pass 2^16 (N1 = 256)", "fftc_try: rows > 8 -> fftp_two_pass_try")
-fc(F32, 1 << 15, 4, ALL_FLAGS, "packed two-pass 2^15 (N1 = 32)", "fft.cu: 2^15 <= n <= 2^20 -> fftp_two_pass_try")
-fc(F32, 1 << 19, 2, ALL_FLAGS, "packed two-pass 2^19 (N1 = 512)", "fftp_two_pass_try n1 = 512")
-fc(F32, 1 << 20, 2, ALL_FLAGS, "packed two-pass 2^20 (N1 = 256, 4096-point rows)", "fftp_two_pass_try n1 = 256, log2n2 = 12")
-fc(F32, 1 << 20, 1, (0,), "generic two-pass 2^20 (misaligned)", "fftp_two_pass_try: in & 15 -> fft_pow2 tiles", "offset")
-fc(F32, 1 << 21, 2, ALL_FLAGS, "packed three-pass 2^21 (nA = 16)", "fft.cu: 2^21 <= n <= 2^24 -> fftp_three_pass_try")
-fc(F32, 1 << 23, 1, (0, INV | SH), "packed three-pass 2^23 (nA = 32)", "fftp_three_pass_try nA = 32")
-fc(F32, 1 << 24, 1, (0, INV | SH), "packed three-pass 2^24 (nA = 256)", "fftp_three_pass_try nA = 256")
+       "fft_route: in & 15 (real rows: in & 7) -> generic kernels", "block", "offset")
+fc(F32, 16384, 4, ALL_FLAGS, "packed 16384 persistent (fftp16k)", "fft_route: n == 16384 && rows >= 2 -> packed-16k",
+   {None: "packed-16k", REAL: "real-rows"})
+fc(F32, 16384, 1, ALL_FLAGS[:5], "packed 16384 non-persistent fftp R0=4", "fft_route: n == 16384 && rows == 1", "packed")
+fc(F32, 16384, 2, (0, SH, INV, INV | SH), "generic fall-back of 16384", "fft_route: in == out", "block", "inplace")
+fc(F32, 16384, 2, ALL_FLAGS, "generic fall-back of 16384", "fft_route: in & 15", "block", "offset")
+fc(F32, 1 << 16, 1, (0, SH, INV, INV | SH), "2^16 cluster kernel (fftc)", "fft_route: n == 65536, !real, !mag, rows <= 8, in != out",
+   "cluster")
+fc(F32, 1 << 16, 8, (0, SH, INV, INV | SH), "2^16 cluster kernel (fftc)", "fft_route: rows <= 8", "cluster")
+fc(F32, 1 << 16, 9, ALL_FLAGS, "packed two-pass 2^16 (N1 = 256)", "fft_route: rows > 8 -> two-pass", "two-pass")
+fc(F32, 1 << 15, 4, ALL_FLAGS, "packed two-pass 2^15 (N1 = 32)", "fft_route: 2^15 <= n <= 2^20 -> two-pass", "two-pass")
+fc(F32, 1 << 19, 2, ALL_FLAGS, "packed two-pass 2^19 (N1 = 512)", "fft_route: two-pass n1 = 512", "two-pass")
+fc(F32, 1 << 20, 2, ALL_FLAGS, "packed two-pass 2^20 (N1 = 256, 4096-point rows)", "fft_route: two-pass n1 = 256, log2n2 = 12", "two-pass")
+fc(F32, 1 << 20, 1, (0,), "generic column pass + packed 1024-point rows 2^20 (misaligned)",
+   "fft_route: in & 15 -> no two-pass; out & 7 == 0, work & 15 == 0 -> hybrid", "hybrid", "offset")
+fc(F32, 1 << 21, 2, ALL_FLAGS, "packed three-pass 2^21 (nA = 16)", "fft_route: 2^21 <= n <= 2^24 -> three-pass", "three-pass")
+fc(F32, 1 << 23, 1, (0, INV | SH), "packed three-pass 2^23 (nA = 32)", "fft_route: three-pass nA = 32", "three-pass")
+fc(F32, 1 << 24, 1, (0, INV | SH), "packed three-pass 2^24 (nA = 256)", "fft_route: three-pass nA = 256", "three-pass")
 fc(F32, 3 << 12, 24, (0, SH, INV | SH, SH | MAG), "q = 3: radix-3 pass + packed rows + interleave",
-   "fft.cu: q <= 31, packed_rows: P >= 256, n*batch >= 2^18")
-fc(F32, 15 << 10, 2, (0, SH, INV | SH, SH | MAG), "q = 15: radix-q pass + generic rows", "fft.cu: q <= 31, !packed_rows")
-fc(F32, 31 << 15, 1, (0, SH, INV | SH, SH | MAG), "q = 31: radix-q pass + two-pass rows + interleave", "fft.cu: P > fft_block_max_n")
-fc(F32, 1001, 5, ALL_FLAGS, "chirp-z (M = 2048: separate filter multiply)", "fft.cu: q > 31 -> Bluestein, M <= 16384")
-fc(F32, 10007 * 3, 2, ALL_FLAGS, "chirp-z (M = 2^16: filter fused into in_mul)", "fft.cu: Bluestein, M > 16384")
-fc(F64, 512, 8, ALL_FLAGS, "c64 fft_block_kernel", "fft_pow2: n <= 8192, launch_block: not 1024/2048/4096")
-fc(F64, 8192, 3, ALL_FLAGS, "c64 fft_block_kernel", "fft_pow2: n <= 8192")
+   "fft_route: q <= 31, packed rows: P >= 256, n*batch >= 2^18", "q-rows-interleave > packed")
+fc(F32, 15 << 10, 2, (0, SH, INV | SH, SH | MAG), "q = 15: radix-q pass + generic rows", "fft_route: q <= 31, no packed rows", "q-rows")
+fc(F32, 31 << 15, 1, (0, SH, INV | SH, SH | MAG), "q = 31: radix-q pass + two-pass rows + interleave", "fft_route: P > fft_block_max_n",
+   "q-rows-interleave > two-pass")
+fc(F32, 1001, 5, ALL_FLAGS, "chirp-z (M = 2048: separate filter multiply)", "fft_route: q > 31 -> Bluestein, M <= 16384", "bluestein")
+fc(F32, 10007 * 3, 2, ALL_FLAGS, "chirp-z (M = 2^16: filter fused into in_mul)", "fft_route: Bluestein, M > 16384", "bluestein")
+fc(F64, 512, 8, ALL_FLAGS, "c64 fft_block_kernel", "fft_route: n <= 8192, not 1024/2048/4096 -> block", "block")
+fc(F64, 8192, 3, ALL_FLAGS, "c64 fft_block_kernel", "fft_route: n <= 8192", "block")
 for n in (1024, 2048, 4096):
-    fc(F64, n, 4, ALL_FLAGS, "c64 f64_row_kernel", "fft64t.cuh launch_rows: n in {1024, 2048, 4096}")
-fc(F64, 1024, 4, (0, INV | SH), "c64 f64_row_kernel (misaligned)", "launch_rows takes any alignment", "offset")
-fc(F64, 1 << 15, 2, ALL_FLAGS, "c64 two-pass f64_tile_kernel", "fft_pow2: n > 8192, ceil(log2 n / 9) == 2")
-fc(F64, 1 << 18, 1, (0, INV | SH, SH | MAG), "c64 two-pass f64_tile_kernel", "log2 n = 18")
-fc(F64, 1 << 20, 1, (0, INV | SH, SH | MAG, REAL), "c64 three-pass f64_tile_kernel", "fft_pow2: ceil(log2 n / 9) == 3")
-fc(F64, 3 << 16, 1, (0, SH, INV | SH, REAL), "c64 3*2^k, folded radix-3 first pass", "fft.cu: f64, P > 8192, !mag -> fft_q_three_pass")
-fc(F64, 15 << 8, 3, (0, SH, INV | SH, SH | MAG), "c64 q*2^k, radix-q pass + block rows", "fft.cu: q <= 31, P <= 8192")
-fc(F64, 31 << 10, 2, (0, INV | SH, SH | MAG), "c64 q*2^k, radix-q pass + f64_row rows", "fft.cu: q <= 31, P = 1024")
-fc(F64, 1001, 3, ALL_FLAGS, "c64 chirp-z", "fft.cu: q > 31 -> Bluestein")
-fc(F64, 10007 * 3, 1, (0, SH, INV | SH), "c64 chirp-z (M = 2^16, tiles)", "Bluestein, M > 8192")
+    fc(F64, n, 4, ALL_FLAGS, "c64 f64_row_kernel", "fft_route: f64, n in {1024, 2048, 4096} -> c64-rows", "c64-rows")
+fc(F64, 1024, 4, (0, INV | SH), "c64 f64_row_kernel (misaligned)", "c64-rows take any alignment", "c64-rows", "offset")
+fc(F64, 1 << 15, 2, ALL_FLAGS, "c64 two-pass f64_tile_kernel", "fft_pow2 tiles: n > 8192, ceil(log2 n / 9) == 2", "tiles")
+fc(F64, 1 << 18, 1, (0, INV | SH, SH | MAG), "c64 two-pass f64_tile_kernel", "log2 n = 18", "tiles")
+fc(F64, 1 << 20, 1, (0, INV | SH, SH | MAG, REAL), "c64 three-pass f64_tile_kernel", "fft_pow2 tiles: ceil(log2 n / 9) == 3", "tiles")
+fc(F64, 3 << 16, 1, (0, SH, INV | SH, REAL), "c64 3*2^k, folded radix-3 first pass", "fft_route: f64, P > 8192, !mag -> q-three-pass",
+   "q-three-pass")
+fc(F64, 15 << 8, 3, (0, SH, INV | SH, SH | MAG), "c64 q*2^k, radix-q pass + block rows", "fft_route: q <= 31, P <= 8192 -> q-rows", "q-rows")
+fc(F64, 31 << 10, 2, (0, INV | SH, SH | MAG), "c64 q*2^k, radix-q pass + f64_row rows", "fft_route: q <= 31, P = 1024; rows: c64-rows",
+   "q-rows")
+fc(F64, 1001, 3, ALL_FLAGS, "c64 chirp-z", "fft_route: q > 31 -> Bluestein", "bluestein")
+fc(F64, 10007 * 3, 1, (0, SH, INV | SH), "c64 chirp-z (M = 2^16, tiles)", "Bluestein, M > 8192", "bluestein")
 
 
-@pytest.mark.parametrize("dtype,n,rows,flags,variant,branch,cond", FFT_CASES)
-def test_fft_rows_accuracy(dtype, n, rows, flags, variant, branch, cond):
+@pytest.mark.parametrize("dtype,n,rows,flags,variant,branch,cond,route", FFT_CASES)
+def test_fft_rows_accuracy(dtype, n, rows, flags, variant, branch, cond, route):
     rng = np.random.default_rng(n * 131 + rows * 7 + flags)
     x = rand_c(rng, (rows, n), dtype)
     if flags & REAL:
@@ -184,17 +194,21 @@ def test_fft_rows_accuracy(dtype, n, rows, flags, variant, branch, cond):
     assert_scaled_exact(lambda xs: gpu_fft(xs, flags, dtype, off, inplace), x, got, dtype, ulps=1 if flags & MAG else 0)
 
 
-# windowed_fft (Blackman-Harris through in_mul) on one length of each multi-kernel family
-@pytest.mark.parametrize("dtype,n,rows,branch", [
-    (F32, 4096, 16, "single pass: in_mul_rows_kernel + packed kernel (n*rows >= 2^16)"),
-    (F32, 1 << 16, 2, "packed two-pass, window on the column pass"),
-    (F32, 1 << 21, 1, "packed three-pass, window on pass A"),
-    (F32, 3 << 15, 1, "q*2^k: window in the radix-q pass"),
-    (F32, 10007, 2, "chirp-z: window in bluestein_pre_kernel"),
-    (F64, 1 << 15, 2, "c64 tiles"),
-    (F64, 3 << 14, 1, "c64 folded radix-3"),
-    (F64, 10007, 1, "c64 chirp-z"),
-])
+# windowed_fft (Blackman-Harris through in_mul) on one length of each multi-kernel family: (dtype, n, rows, branch, route)
+WINDOWED_CASES = [
+    (F32, 4096, 16, "single pass: in_mul_rows_kernel + packed kernel (n*rows >= 2^16)", "mul-pass > packed"),
+    (F32, 1 << 16, 2, "packed two-pass, window on the column pass", "two-pass"),
+    (F32, 1 << 21, 1, "packed three-pass, window on pass A", "three-pass"),
+    (F32, 3 << 15, 1, "q*2^k: window in the radix-q pass", "q-rows-interleave > two-pass"),
+    (F32, 10007, 2, "chirp-z: window in bluestein_pre_kernel", "bluestein"),
+    (F64, 1 << 15, 2, "c64 tiles", "tiles"),
+    (F64, 3 << 14, 1, "c64 folded radix-3", "q-three-pass"),
+    (F64, 10007, 1, "c64 chirp-z", "bluestein"),
+]
+
+
+@pytest.mark.parametrize("dtype,n,rows,branch", [c[:4] for c in WINDOWED_CASES],
+                         ids=["%s-%d-%d-%s" % (np.dtype(c[0]).name, c[1], c[2], c[3]) for c in WINDOWED_CASES])
 def test_windowed_fft_accuracy(dtype, n, rows, branch):
     rng = np.random.default_rng(n + rows)
     x = rand_c(rng, (rows, n), dtype)
