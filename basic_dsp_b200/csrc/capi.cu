@@ -7,6 +7,7 @@
 #include <map>
 #include <memory>
 #include <mutex>
+#include <optional>
 #include <vector>
 
 #include "../../include/basic_dsp_b200.h"
@@ -122,7 +123,27 @@ template <typename T> bool meta_agrees(const Vec<T>* a, const Vec<T>* b) {
 }
 
 // ---- transforms ------------------------------------------------------------------------------------
-template <typename T> Res<T> op_fft(Vec<T>* v, bool inverse, bool shifted, bool magnitude, const InMul* in_mul = nullptr) {
+// built-in windows: 0 triangular, 1 hamming, 2 blackman-harris; any other kind is rectangular (interop/src/lib.rs:153-164)
+const int RECTANGULAR = 3;
+
+// Options of a transform of `points` points.  shift: fft_shift on the store of a forward transform (freq.rs:85-87), or
+// scale(1/points) -> ifft_shift on the load of an inverse one; a built-in window rides on the load.
+template <typename T> FftOpts fft_opts(size_t points, bool inverse, bool shift, bool magnitude, bool real_input, int window) {
+    FftOpts o;
+    o.inverse = inverse;
+    o.real_input = real_input;
+    o.magnitude = magnitude;
+    if (shift && points) {
+        if (inverse) { o.in_rot = points / 2; o.scale = (double)((T)1 / (T)points); }
+        else o.out_rot = points / 2;
+    }
+    if (window >= 0 && window < RECTANGULAR) { o.in_mul.kind = 3; o.in_mul.arg = window; }
+    return o;
+}
+
+// window_table: a host-built window table multiplied in on the load, instead of a built-in window
+template <typename T>
+Res<T> op_fft(Vec<T>* v, bool inverse, bool shifted, bool magnitude, int window = RECTANGULAR, const T* window_table = nullptr) {
     // time_to_freq.rs:136-165, freq_to_time.rs:138-168, time_freq/mod.rs:32-63
     const int want_domain = inverse ? 1 : 0;
     if (v->domain != want_domain) {
@@ -132,17 +153,9 @@ template <typename T> Res<T> op_fft(Vec<T>* v, bool inverse, bool shifted, bool 
         return done(v, 0);
     }
     const size_t points = points_of(v);
-    FftOpts o;
-    o.inverse = inverse;
-    o.real_input = !v->is_complex;
-    o.magnitude = magnitude;
-    if (in_mul) o.in_mul = *in_mul;
+    FftOpts o = fft_opts<T>(points, inverse, shifted, magnitude, !v->is_complex, window);
+    if (window_table) { o.in_mul.p = window_table; o.in_mul.kind = 1; }
     if (points) {
-        if (shifted && !inverse) o.out_rot = points / 2;                       // fft_shift (freq.rs:85-87)
-        if (shifted && inverse) {                                              // ifft: scale -> ifft_shift -> plain_ifft
-            o.in_rot = points / 2;
-            o.scale = (double)((T)1 / (T)points);
-        }
         const size_t out_scalars = magnitude ? points : 2 * points;
         int rc = ensure_scratch(v, 2 * points);
         if (!rc) rc = fft_exec<T>(v->d, v->scratch, points, 1, o, nullptr, 0, g_stream);
@@ -313,33 +326,21 @@ template <typename T> T host_rc(T x, T rolloff) {
     T arg = two * rolloff * x;
     return (T)sin(pi_x) * (T)cos(pi_x * rolloff) / pi_x / (one - (arg * arg));
 }
-template <typename T> T host_sinc_freq(T x) { return (T)fabs(x) <= (T)1 ? (T)1 : (T)0; }
-template <typename T> T host_rc_freq(T x, T rolloff) {
-    const T one = 1, two = 2, pi = (T)M_PI;
-    T ax = (T)fabs(x);
-    if (ax <= (one - rolloff)) return one;
-    if (((one - rolloff) < ax) && (ax <= (one + rolloff)))
-        return one / two * (one + (T)cos(pi / rolloff * (ax - (one - rolloff)) / two));
-    return (T)0;
-}
 
-// generic host evaluator: built-in kinds or a C callback
+// A real impulse or frequency response: the built-in `kind` (0 sinc, 1 raised cosine with `rolloff`) when `fn` is null,
+// else the C callback fn(data, x).  Built-in frequency responses are evaluated on the device, so the host evaluates only
+// callbacks and the built-in impulse responses of tap tables.
 template <typename T> struct RealFn {
-    int kind = 0;        // 0 sinc, 1 raised cosine, 2 callback
+    int kind = 0;
     T rolloff = 0;
     T (*fn)(const void*, T) = nullptr;
     const void* data = nullptr;
-    bool freq = false;   // evaluate the frequency response instead of the impulse response
-    T operator()(T x) const {
-        if (kind == 2) return fn(data, x);
-        if (freq) return kind == 0 ? host_sinc_freq<T>(x) : host_rc_freq<T>(x, rolloff);
-        return kind == 0 ? host_sinc<T>(x) : host_rc<T>(x, rolloff);
-    }
+    T operator()(T x) const { return fn ? fn(data, x) : kind == 0 ? host_sinc<T>(x) : host_rc<T>(x, rolloff); }
 };
 
-// Small host-built tables (tap tables, custom frequency responses) go through a per-thread grow-only
-// pinned staging buffer + device buffer, so that a call does no cudaMalloc/cudaFree and never blocks on
-// the GPU: the copy is queued on the caller's stream, the consumer kernel follows on the same stream.
+// Small host-built tables go through a grow-only pinned staging buffer + device buffer per host thread and device, so
+// that a call does no cudaMalloc/cudaFree and never blocks on the GPU: the copy is queued on the caller's stream, the
+// consumer kernel follows on the same stream.
 struct TableStage {
     void* dev = nullptr;
     void* host = nullptr;
@@ -347,10 +348,10 @@ struct TableStage {
     cudaEvent_t copied = nullptr;   // staging buffer has been read by the last copy
     cudaEvent_t used = nullptr;     // device buffer has been consumed by the last kernel
 };
-thread_local TableStage g_stage;
+thread_local std::map<int, TableStage> g_stage;   // by device
 
-template <typename T> int upload_table(const std::vector<T>& h, T** dev) {
-    TableStage& s = g_stage;
+template <typename T> int stage_table(int dev, const std::vector<T>& h, TableStage** stage) {
+    TableStage& s = g_stage[dev];
     const size_t need = (h.size() ? h.size() : 1) * sizeof(T);
     if (!s.copied) {
         BDSP_CUDA_OK(cudaEventCreateWithFlags(&s.copied, cudaEventDisableTiming));
@@ -370,13 +371,89 @@ template <typename T> int upload_table(const std::vector<T>& h, T** dev) {
     memcpy(s.host, h.data(), h.size() * sizeof(T));
     BDSP_CUDA_OK(cudaMemcpyAsync(s.dev, s.host, h.size() * sizeof(T), cudaMemcpyHostToDevice, g_stream));
     BDSP_CUDA_OK(cudaEventRecord(s.copied, g_stream));
-    *dev = reinterpret_cast<T*>(s.dev);
+    *stage = &s;
     return 0;
 }
-// call after the kernel that reads the table has been launched
-inline void table_consumed() {
-    if (g_stage.used) cudaEventRecord(g_stage.used, g_stream);
+
+// ---- cache of tap tables built from the BUILT-IN functions -----------------------------------------------------------
+// Repeated calls with the same parameters (the usual streaming use) skip the host evaluation and the upload.
+// Keyed by everything the table depends on; tables live in device memory until the process ends (<= 64 entries
+// per process, then the cache stops growing).  Callback functions are never cached.
+struct TableKey {
+    int dev, is64, what, kind, flag;
+    double rolloff, a, b;
+    size_t n0, n1;
+    bool operator<(const TableKey& o) const {
+        if (dev != o.dev) return dev < o.dev;
+        if (is64 != o.is64) return is64 < o.is64;
+        if (what != o.what) return what < o.what;
+        if (kind != o.kind) return kind < o.kind;
+        if (flag != o.flag) return flag < o.flag;
+        if (rolloff != o.rolloff) return rolloff < o.rolloff;
+        if (a != o.a) return a < o.a;
+        if (b != o.b) return b < o.b;
+        if (n0 != o.n0) return n0 < o.n0;
+        return n1 < o.n1;
+    }
+};
+std::mutex g_table_mu;
+std::map<TableKey, std::pair<void*, size_t>> g_table_cache;
+
+// the key of a table of `f`: built-in functions are cached by parameter set, callbacks are not (nullptr)
+template <typename T> const TableKey* cache_key(const RealFn<T>& f, TableKey* key) {
+    if (f.fn) return nullptr;
+    key->kind = f.kind;
+    key->rolloff = (double)f.rolloff;
+    return key;
 }
+
+// A host-built table on the device for the kernels launched while this object is in scope.  With a key, the table is
+// taken from or added to the cache; otherwise, or when the cache is full, build() is staged, and the staging buffer is
+// marked consumed when this object goes out of scope, i.e. after the consuming launch.
+template <typename T> class DeviceTable {
+  public:
+    const T* p = nullptr;
+    size_t count = 0;   // T scalars
+    int rc = 0;
+    template <typename Build> DeviceTable(const TableKey* key, Build build) {
+        int dev = 0;
+        cudaGetDevice(&dev);
+        TableKey k = {};
+        if (key) {
+            k = *key;
+            k.dev = dev;
+            k.is64 = sizeof(T) == 8;
+            std::lock_guard<std::mutex> lk(g_table_mu);
+            auto it = g_table_cache.find(k);
+            if (it != g_table_cache.end()) {
+                p = reinterpret_cast<const T*>(it->second.first);
+                count = it->second.second;
+                return;
+            }
+        }
+        const std::vector<T> tab = build();
+        count = tab.size();
+        if (key && cache_insert(k, tab)) return;
+        rc = stage_table(dev, tab, &stage_);
+        if (!rc) p = reinterpret_cast<const T*>(stage_->dev);
+    }
+    ~DeviceTable() { if (stage_) cudaEventRecord(stage_->used, g_stream); }
+    DeviceTable(const DeviceTable&) = delete;
+    DeviceTable& operator=(const DeviceTable&) = delete;
+
+  private:
+    TableStage* stage_ = nullptr;
+    bool cache_insert(const TableKey& k, const std::vector<T>& tab) {
+        std::lock_guard<std::mutex> lk(g_table_mu);
+        if (g_table_cache.size() >= 64) return false;
+        void* dev = nullptr;
+        if (cudaMalloc(&dev, tab.size() * sizeof(T)) != cudaSuccess) return false;
+        if (cudaMemcpy(dev, tab.data(), tab.size() * sizeof(T), cudaMemcpyHostToDevice) != cudaSuccess) { cudaFree(dev); return false; }
+        g_table_cache[k] = std::make_pair(dev, tab.size());
+        p = reinterpret_cast<const T*>(dev);
+        return true;
+    }
+};
 
 // ---- convolution -----------------------------------------------------------------------------------
 // convolution with taps resident on the device; h: the impulse-response vector that caches the overlap-save plan of
@@ -413,51 +490,6 @@ int convolve_taps(Vec<T>* v, const T* h_dev, size_t L, bool h_complex, Vec<T>* h
     return 0;
 }
 
-// ---- cache of tap / response tables built from the BUILT-IN functions (kind 0 / 1) ----------------------
-// Repeated calls with the same parameters (the usual streaming use) skip the host evaluation and the upload.
-// Keyed by everything the table depends on; tables live in device memory until the process ends (<= 64 entries
-// per process, then the cache stops growing).  Callback functions are never cached.
-struct TableKey {
-    int dev, is64, what, kind, flag;
-    double rolloff, a, b;
-    size_t n0, n1;
-    bool operator<(const TableKey& o) const {
-        if (dev != o.dev) return dev < o.dev;
-        if (is64 != o.is64) return is64 < o.is64;
-        if (what != o.what) return what < o.what;
-        if (kind != o.kind) return kind < o.kind;
-        if (flag != o.flag) return flag < o.flag;
-        if (rolloff != o.rolloff) return rolloff < o.rolloff;
-        if (a != o.a) return a < o.a;
-        if (b != o.b) return b < o.b;
-        if (n0 != o.n0) return n0 < o.n0;
-        return n1 < o.n1;
-    }
-};
-std::mutex g_table_mu;
-std::map<TableKey, std::pair<void*, size_t>> g_table_cache;
-
-template <typename T> const T* table_cache_find(TableKey key, size_t* count) {
-    cudaGetDevice(&key.dev);
-    key.is64 = sizeof(T) == 8;
-    std::lock_guard<std::mutex> lk(g_table_mu);
-    auto it = g_table_cache.find(key);
-    if (it == g_table_cache.end()) return nullptr;
-    *count = it->second.second;
-    return reinterpret_cast<const T*>(it->second.first);
-}
-template <typename T> const T* table_cache_insert(TableKey key, const std::vector<T>& tab) {
-    cudaGetDevice(&key.dev);
-    key.is64 = sizeof(T) == 8;
-    std::lock_guard<std::mutex> lk(g_table_mu);
-    if (g_table_cache.size() >= 64) return nullptr;
-    void* dev = nullptr;
-    if (cudaMalloc(&dev, tab.size() * sizeof(T)) != cudaSuccess) return nullptr;
-    if (cudaMemcpy(dev, tab.data(), tab.size() * sizeof(T), cudaMemcpyHostToDevice) != cudaSuccess) { cudaFree(dev); return nullptr; }
-    g_table_cache[key] = std::make_pair(dev, tab.size());
-    return reinterpret_cast<const T*>(dev);
-}
-
 template <typename T> Res<T> op_convolve_signal(Vec<T>* v, Vec<T>* h) {
     // convolution.rs:477-542
     if (!meta_agrees(v, h)) return done(v, E_META);
@@ -488,6 +520,35 @@ template <typename T> void fold_taps(std::vector<T>& taps, size_t N, size_t widt
     taps.swap(folded);
 }
 
+// convolve_function_priv taps (time_freq/mod.rs:174-213): y[i] = sum_{m=-L..L} x[i+m] f(-m*ratio) == circular FIR with
+// h[k] = f(-(L-k)*ratio), k = 0..2L (centre cl = L+1); eval(x, out) writes the `width` scalars of f(x)
+template <typename T, typename Eval> std::vector<T> priv_taps(size_t L, T ratio, int width, Eval eval) {
+    std::vector<T> h(width * (2 * L + 1));
+    T j = -(T)L;
+    for (size_t q = 0; q < 2 * L + 1; q++) { eval(-j * ratio, &h[width * (2 * L - q)]); j = j + (T)1; }
+    return h;
+}
+
+// ratio * f(j/mx * ratio) on the grid j = -mx..: multiply_function_priv with is_fft_shifted = false
+// (time_freq/mod.rs:612-723); eval(x, out) writes the `width` scalars of f(x)
+template <typename T, typename Eval> std::vector<T> freq_resp_table(size_t points, T ratio, int width, Eval eval) {
+    std::vector<T> tab(width * points);
+    const size_t offset = points % 2;
+    const T mx = (T)(points - offset) / (T)2;
+    T j = -(T)(points - offset) / (T)2;
+    for (size_t i = 0; i < points; i++) {
+        T* t = &tab[width * i];
+        eval(j / mx * ratio, t);
+        for (int c = 0; c < width; c++) t[c] = ratio * t[c];
+        j = j + (T)1;
+    }
+    return tab;
+}
+
+template <typename T, typename CT> auto complex_eval(CT (*fn)(const void*, T), const void* data) {
+    return [=](T x, T* out) { const CT c = fn(data, x); out[0] = c.re; out[1] = c.im; };
+}
+
 template <typename T> Res<T> op_convolve_fn(Vec<T>* v, const RealFn<T>& f, T ratio, size_t len) {
     // convolution.rs:136-192 (real impulse response)
     if (v->domain != 0) { mark_invalid(v); return done(v, 0); }   // assert_time!
@@ -496,38 +557,22 @@ template <typename T> Res<T> op_convolve_fn(Vec<T>* v, const RealFn<T>& f, T rat
     const T ratio_inv = (T)1 / ratio;
     const bool simd_branch = len <= 202 && v->len > 2000 && (T)fabs((T)round(ratio_inv) - ratio_inv) < (T)1e-6 && ratio > (T)0.5;
     TableKey key = {};
-    key.what = 1; key.kind = f.kind; key.flag = simd_branch; key.rolloff = (double)f.rolloff; key.a = (double)ratio; key.n0 = len; key.n1 = N;
-    if (f.kind != 2) {
-        size_t cnt = 0;
-        const T* cached = table_cache_find<T>(key, &cnt);
-        if (cached) return done(v, convolve_taps<T>(v, cached, cnt, false, nullptr));
-    }
-    std::vector<T> taps;
-    if (simd_branch) {
-        // taps f(j/ratio), j = -len..len, handed to convolve_signal (convolution.rs:151-172).
-        // Deviation Q4: for real vectors the reference fills only every second tap.
-        T j = -(T)len;
-        for (size_t q = 0; q < 2 * len + 1; q++) { taps.push_back(f(j * ratio_inv)); j = j + (T)1; }
-    } else {
-        // convolve_function_priv (time_freq/mod.rs:174-213): y[i] = sum_{m=-L..L} x[i+m] f(-m*ratio)
-        // == circular FIR with h[k] = f(-(L-k)*ratio), k = 0..2L (centre cl = L+1)
-        const size_t L = len > N ? N : len;
-        std::vector<T> t(2 * L + 1);
-        T j = -(T)L;
-        for (size_t q = 0; q < 2 * L + 1; q++) { t[q] = f(-j * ratio); j = j + (T)1; }
-        taps.assign(t.rbegin(), t.rend());
-    }
-    fold_taps(taps, N, 1);
-    if (f.kind != 2) {
-        const T* cached = table_cache_insert<T>(key, taps);
-        if (cached) return done(v, convolve_taps<T>(v, cached, taps.size(), false, nullptr));
-    }
-    T* h_dev = nullptr;
-    int rc = upload_table(taps, &h_dev);
-    if (rc) return done(v, rc);
-    rc = convolve_taps<T>(v, h_dev, taps.size(), false, nullptr);
-    table_consumed();
-    return done(v, rc);
+    key.what = 1; key.flag = simd_branch; key.a = (double)ratio; key.n0 = len; key.n1 = N;
+    DeviceTable<T> taps(cache_key(f, &key), [&] {
+        std::vector<T> h;
+        if (simd_branch) {
+            // taps f(j/ratio), j = -len..len, handed to convolve_signal (convolution.rs:151-172).
+            // Deviation Q4: for real vectors the reference fills only every second tap.
+            T j = -(T)len;
+            for (size_t q = 0; q < 2 * len + 1; q++) { h.push_back(f(j * ratio_inv)); j = j + (T)1; }
+        } else {
+            h = priv_taps<T>(len > N ? N : len, ratio, 1, [&](T x, T* out) { *out = f(x); });
+        }
+        fold_taps(h, N, 1);
+        return h;
+    });
+    if (taps.rc) return done(v, taps.rc);
+    return done(v, convolve_taps<T>(v, taps.p, taps.count, false, nullptr));
 }
 
 template <typename T, typename CT>
@@ -538,22 +583,13 @@ Res<T> op_convolve_cfn(Vec<T>* v, CT (*fn)(const void*, T), const void* data, T 
     if (v->domain != 0) { mark_invalid(v); return done(v, 0); }
     const size_t N = points_of(v);
     if (N == 0) return done(v, 0);
-    const size_t L = len > N ? N : len;
-    std::vector<T> t(2 * (2 * L + 1));
-    T j = -(T)L;
-    for (size_t q = 0; q < 2 * L + 1; q++) {
-        CT c = fn(data, -j * ratio);
-        size_t k = 2 * L - q;  // reversed: h[k] = f(-(L-k)*ratio)
-        t[2 * k] = c.re; t[2 * k + 1] = c.im;
-        j = j + (T)1;
-    }
-    fold_taps(t, N, 2);   // 2L + 1 > N: the window wraps around the vector, as in the reference
-    T* h_dev = nullptr;
-    int rc = upload_table(t, &h_dev);
-    if (rc) return done(v, rc);
-    rc = convolve_taps<T>(v, h_dev, t.size() / 2, true, nullptr);
-    table_consumed();
-    return done(v, rc);
+    DeviceTable<T> taps(nullptr, [&] {
+        std::vector<T> h = priv_taps<T>(len > N ? N : len, ratio, 2, complex_eval<T, CT>(fn, data));
+        fold_taps(h, N, 2);   // 2L + 1 > N: the window wraps around the vector, as in the reference
+        return h;
+    });
+    if (taps.rc) return done(v, taps.rc);
+    return done(v, convolve_taps<T>(v, taps.p, taps.count / 2, true, nullptr));
 }
 
 template <typename T> Res<T> op_mul_freq_resp(Vec<T>* v, const RealFn<T>& f, T ratio) {
@@ -561,21 +597,10 @@ template <typename T> Res<T> op_mul_freq_resp(Vec<T>* v, const RealFn<T>& f, T r
     if (v->domain != 1) { mark_invalid(v); return done(v, 0); }
     const size_t points = points_of(v);
     if (!points) return done(v, 0);
-    int rc;
-    if (f.kind != 2) {
-        rc = ew_mul_freq_resp<T>(v->d, points, v->is_complex, f.kind, (double)f.rolloff, (double)ratio, g_stream);
-    } else {
-        std::vector<T> tab(points);
-        const size_t offset = points % 2;
-        const T mx = (T)(points - offset) / (T)2;
-        T j = -(T)(points - offset) / (T)2;
-        for (size_t i = 0; i < points; i++) { tab[i] = ratio * f(j / mx * ratio); j = j + (T)1; }
-        T* dev = nullptr;
-        rc = upload_table(tab, &dev);
-        if (!rc) rc = ew_mul_table<T>(v->d, dev, points, v->is_complex, 0, g_stream);
-        table_consumed();
-    }
-    return done(v, rc);
+    if (!f.fn) return done(v, ew_mul_freq_resp<T>(v->d, points, v->is_complex, f.kind, (double)f.rolloff, (double)ratio, g_stream));
+    DeviceTable<T> tab(nullptr, [&] { return freq_resp_table<T>(points, ratio, 1, [&](T x, T* out) { *out = f(x); }); });
+    if (tab.rc) return done(v, tab.rc);
+    return done(v, ew_mul_table<T>(v->d, tab.p, points, v->is_complex, 0, g_stream));
 }
 
 template <typename T, typename CT>
@@ -583,63 +608,41 @@ Res<T> op_mul_freq_resp_c(Vec<T>* v, CT (*fn)(const void*, T), const void* data,
     if (!v->is_complex || v->domain != 1) { mark_invalid(v); return done(v, 0); }
     const size_t points = points_of(v);
     if (!points) return done(v, 0);
-    std::vector<T> tab(2 * points);
-    const size_t offset = points % 2;
-    const T mx = (T)(points - offset) / (T)2;
-    T j = -(T)(points - offset) / (T)2;
-    for (size_t i = 0; i < points; i++) {
-        CT c = fn(data, j / mx * ratio);
-        tab[2 * i] = ratio * c.re; tab[2 * i + 1] = ratio * c.im;
-        j = j + (T)1;
-    }
-    T* dev = nullptr;
-    int rc = upload_table(tab, &dev);
-    if (!rc) rc = ew_mul_table<T>(v->d, dev, points, 1, 1, g_stream);
-    table_consumed();
-    return done(v, rc);
+    DeviceTable<T> tab(nullptr, [&] { return freq_resp_table<T>(points, ratio, 2, complex_eval<T, CT>(fn, data)); });
+    if (tab.rc) return done(v, tab.rc);
+    return done(v, ew_mul_table<T>(v->d, tab.p, points, 1, 1, g_stream));
 }
 
 // ---- SURVEY 8(f) rows: windows, correlation, reverse, decimatei --------------------------------------
-template <typename T> T host_window(int kind, size_t n, size_t length) {
-    // window_functions.rs:25-129, interop translate_to_window_function (lib.rs:153-164)
-    const T one = 1, two = 2, pi = (T)M_PI;
-    const T nn = (T)n, ln = (T)length;
-    if (kind == 0) return one - (T)fabs((nn - (ln - one) / two) / (ln / two));
-    if (kind == 1) { const T alpha = (T)0.54; return alpha - (one - alpha) * (T)cos(two * pi * nn / (ln - one)); }
-    if (kind == 2)
-        return (T)0.35875 - (T)0.48829 * (T)cos(two * pi * nn / (ln - one)) + (T)0.14128 * (T)cos((T)4 * pi * nn / (ln - one)) -
-               (T)0.01168 * (T)cos((T)6 * pi * nn / (ln - one));
-    return one;
-}
-
-// built-in window kind, or a foreign callback window(data, i, points) (facade32.rs:1030-1044)
+// built-in window kind (evaluated on the device), or a foreign callback window fn(data, i, points) (facade32.rs:1030-1044)
 template <typename T> struct WinFn {
-    int kind = 3;
+    int kind = RECTANGULAR;
     T (*fn)(const void*, size_t, size_t) = nullptr;
     const void* data = nullptr;
     bool symmetric = true;
-    T operator()(size_t i, size_t points) const { return fn ? fn(data, i, points) : host_window<T>(kind, i, points); }
 };
 
-template <typename T> Res<T> op_window_fn(Vec<T>* v, const WinFn<T>& w, bool unapply) {
-    // time.rs:33-66 + multiply_window_priv (vector_types/mod.rs:528-598): symmetric windows evaluate the
-    // first half and mirror it
-    if (v->domain != 0) { mark_invalid(v); return done(v, 0); }
-    const size_t points = points_of(v);
-    if (!points) return done(v, 0);
-    // built-in windows are evaluated on the device (no host work, no table); callbacks through a host-built table
-    if (!w.fn) return done(v, ew_window<T>(v->d, points, v->is_complex, w.kind < 0 || w.kind > 2 ? 3 : w.kind, unapply, g_stream));
+// table of a callback window (multiply_window_priv, vector_types/mod.rs:528-598): symmetric windows evaluate the first half
+// and mirror it; unapply multiplies by the reciprocal
+template <typename T> std::vector<T> window_table(const WinFn<T>& w, size_t points, bool unapply) {
     std::vector<T> tab(points);
     for (size_t i = 0; i < points; i++) {
         const size_t j = !w.symmetric || i < (points + 1) / 2 ? i : points - 1 - i;
-        const T x = w(j, points);
+        const T x = w.fn(w.data, j, points);
         tab[i] = unapply ? (T)1 / x : x;
     }
-    T* dev = nullptr;
-    int rc = upload_table(tab, &dev);
-    if (!rc) rc = ew_mul_table<T>(v->d, dev, points, v->is_complex, 0, g_stream);
-    table_consumed();
-    return done(v, rc);
+    return tab;
+}
+
+template <typename T> Res<T> op_window_fn(Vec<T>* v, const WinFn<T>& w, bool unapply) {
+    // time.rs:33-66
+    if (v->domain != 0) { mark_invalid(v); return done(v, 0); }
+    const size_t points = points_of(v);
+    if (!points) return done(v, 0);
+    if (!w.fn) return done(v, ew_window<T>(v->d, points, v->is_complex, w.kind < 0 || w.kind > 2 ? RECTANGULAR : w.kind, unapply, g_stream));
+    DeviceTable<T> tab(nullptr, [&] { return window_table<T>(w, points, unapply); });
+    if (tab.rc) return done(v, tab.rc);
+    return done(v, ew_mul_table<T>(v->d, tab.p, points, v->is_complex, 0, g_stream));
 }
 template <typename T> Res<T> op_window(Vec<T>* v, int kind, bool unapply) {
     WinFn<T> w; w.kind = kind;
@@ -652,25 +655,10 @@ template <typename T> Res<T> op_windowed_fft_fn(Vec<T>* v, const WinFn<T>& w) {
     // callback windows come from the host-built table.
     if (v->domain != 0) { mark_invalid(v); return op_fft(v, false, true, false); }
     const size_t points = points_of(v);
-    if (!points) return op_fft(v, false, true, false);
-    InMul im;
-    if (!w.fn) {
-        im.kind = 3; im.arg = w.kind < 0 || w.kind > 2 ? 3 : w.kind;
-        if (im.arg == 3) im.kind = 0;   // rectangular
-        return op_fft(v, false, true, false, &im);
-    }
-    std::vector<T> tab(points);
-    for (size_t i = 0; i < points; i++) {
-        const size_t j = !w.symmetric || i < (points + 1) / 2 ? i : points - 1 - i;
-        tab[i] = w(j, points);
-    }
-    T* dev = nullptr;
-    int rc = upload_table(tab, &dev);
-    if (rc) return done(v, rc);
-    im.p = dev; im.kind = 1;
-    Res<T> r = op_fft(v, false, true, false, &im);
-    table_consumed();
-    return r;
+    if (!points || !w.fn) return op_fft(v, false, true, false, w.kind);
+    DeviceTable<T> tab(nullptr, [&] { return window_table<T>(w, points, false); });
+    if (tab.rc) return done(v, tab.rc);
+    return op_fft(v, false, true, false, RECTANGULAR, tab.p);
 }
 template <typename T> Res<T> op_windowed_ifft_fn(Vec<T>* v, const WinFn<T>& w) {
     Res<T> r = op_fft(v, true, true, false);
@@ -747,75 +735,77 @@ template <typename T> Res<T> op_decimatei(Vec<T>* v, uint32_t factor, uint32_t d
 }
 
 // ---- interpolation ---------------------------------------------------------------------------------
+// Shape and path of interpolatef (interpolation.rs:387-482) on `len` scalars, for the vector and the row API alike.
+struct InterpfShape {
+    size_t conv_len;     // clamped to half the points
+    size_t new_len;      // output scalars: round(len * factor), made even
+    size_t new_points;
+    bool poly;           // polyphase tap tables with the integer factor F; else per-output taps
+    int F;
+};
+template <typename T> int interpf_shape(size_t len, bool is_complex, T factor, size_t conv_len, InterpfShape* s) {
+    const size_t points = is_complex ? len / 2 : len;
+    s->conv_len = conv_len > points / 2 ? points / 2 : conv_len;
+    const double nl = round((double)((T)len * factor));
+    if (!(nl >= 0)) return E_ARG_LEN;
+    s->new_len = (size_t)nl;
+    s->new_len += s->new_len % 2;
+    s->new_points = is_complex ? s->new_len / 2 : s->new_len;
+    const bool integer = (T)fabs((T)round(factor) - factor) < (T)1e-6;
+    s->poly = s->conv_len <= 202 && s->new_len >= 2000 && integer;
+    s->F = s->poly ? (int)round(factor) : 0;
+    return 0;
+}
+
 // Tap tables of the polyphase interpolatef path on the device: [2][F][2L+3] (interior, edge) over the window superset
-// n = r-L-1+jj, jj in [0, 2L+3).  Built-in responses are cached by parameter set; callbacks go through the staging buffer
-// (call table_consumed() after the consuming kernel).
-template <typename T> int interp_tap_tables(const RealFn<T>& f, T delay, int F, int L, const T** tab_dev) {
-    const int J = 2 * L + 3;
+// n = r-L-1+jj, jj in [0, 2L+3).
+template <typename T> DeviceTable<T> interp_tap_tables(const RealFn<T>& f, T delay, int F, int L) {
     TableKey key = {};
-    key.what = 2; key.kind = f.kind; key.rolloff = (double)f.rolloff; key.a = (double)delay; key.n0 = (size_t)F; key.n1 = (size_t)L;
-    size_t cnt = 0;
-    const T* cached = f.kind != 2 ? table_cache_find<T>(key, &cnt) : nullptr;
-    if (cached) { *tab_dev = cached; return 0; }
-    // function_to_vectors (interpolation.rs:133-181): v_s[k] = f(j_k - s/F), j_0 = -(L-1) + delay
-    std::vector<T> vs((size_t)F * (2 * L + 1));
-    for (int s = 0; s < F; s++) {
-        T offset = (T)s / (T)F;
-        T j = -((T)L - (T)1) + delay;
-        for (int k = 0; k < 2 * L + 1; k++) { vs[(size_t)s * (2 * L + 1) + k] = f(j - offset); j = j + (T)1; }
-    }
-    std::vector<T> tab((size_t)2 * F * J, (T)0);
-    for (int s = 0; s < F; s++) {
-        T* ti = &tab[(size_t)s * J];                    // interior (interpolation.rs:244-275)
-        if (s == 0) { for (int jj = 0; jj <= 2 * L; jj++) ti[jj] = vs[2 * L - jj]; }
-        else { for (int jj = 1; jj <= 2 * L + 1; jj++) ti[jj] = vs[(size_t)(F - s) * (2 * L + 1) + (2 * L + 1 - jj)]; }
-        T* te = &tab[(size_t)(F + s) * J];              // edges (interpolation.rs:293-315)
-        for (int k = 0; k <= 2 * L; k++) te[k + 2] = vs[(size_t)s * (2 * L + 1) + k];
-    }
-    cached = f.kind != 2 ? table_cache_insert<T>(key, tab) : nullptr;
-    if (cached) { *tab_dev = cached; return 0; }
-    T* dev = nullptr;
-    const int rc = upload_table(tab, &dev);
-    *tab_dev = dev;
-    return rc;
+    key.what = 2; key.a = (double)delay; key.n0 = (size_t)F; key.n1 = (size_t)L;
+    return DeviceTable<T>(cache_key(f, &key), [&] {
+        const int J = 2 * L + 3;
+        // function_to_vectors (interpolation.rs:133-181): v_s[k] = f(j_k - s/F), j_0 = -(L-1) + delay
+        std::vector<T> vs((size_t)F * (2 * L + 1));
+        for (int s = 0; s < F; s++) {
+            T offset = (T)s / (T)F;
+            T j = -((T)L - (T)1) + delay;
+            for (int k = 0; k < 2 * L + 1; k++) { vs[(size_t)s * (2 * L + 1) + k] = f(j - offset); j = j + (T)1; }
+        }
+        std::vector<T> tab((size_t)2 * F * J, (T)0);
+        for (int s = 0; s < F; s++) {
+            T* ti = &tab[(size_t)s * J];                    // interior (interpolation.rs:244-275)
+            if (s == 0) { for (int jj = 0; jj <= 2 * L; jj++) ti[jj] = vs[2 * L - jj]; }
+            else { for (int jj = 1; jj <= 2 * L + 1; jj++) ti[jj] = vs[(size_t)(F - s) * (2 * L + 1) + (2 * L + 1 - jj)]; }
+            T* te = &tab[(size_t)(F + s) * J];              // edges (interpolation.rs:293-315)
+            for (int k = 0; k <= 2 * L; k++) te[k + 2] = vs[(size_t)s * (2 * L + 1) + k];
+        }
+        return tab;
+    });
 }
 
 template <typename T> Res<T> op_interpolatef(Vec<T>* v, const RealFn<T>& f, T factor, T delay, size_t conv_len) {
     // interpolation.rs:387-482
     delay = delay / v->delta;
-    const size_t len = v->len;
     const size_t N = points_of(v);
-    const size_t points_half = N / 2;
-    if (conv_len > points_half) conv_len = points_half;
-    const double nl = round((double)((T)len * factor));
-    if (!(nl >= 0) || N == 0) return done(v, N == 0 ? 0 : E_ARG_LEN);
-    size_t new_len = (size_t)nl;
-    new_len += new_len % 2;
-    const size_t new_points = v->is_complex ? new_len / 2 : new_len;
-    int rc = ensure_scratch(v, new_len);
+    if (N == 0) return done(v, 0);
+    InterpfShape s;
+    int rc = interpf_shape<T>(v->len, v->is_complex != 0, factor, conv_len, &s);
+    if (!rc) rc = ensure_scratch(v, s.new_len);
     if (rc) return done(v, rc);
-    const bool integer = (T)fabs((T)round(factor) - factor) < (T)1e-6;
-    if (conv_len <= 202 && new_len >= 2000 && integer) {
-        const int F = (int)round(factor);
-        const int L = (int)conv_len;
-        const T* tab = nullptr;
-        rc = interp_tap_tables<T>(f, delay, F, L, &tab);
-        if (!rc) rc = interp_poly<T>(v->d, v->scratch, tab, N, new_points, F, L, v->is_complex, g_stream);
-        table_consumed();
+    if (s.poly) {
+        DeviceTable<T> tab = interp_tap_tables<T>(f, delay, s.F, (int)s.conv_len);
+        rc = tab.rc ? tab.rc : interp_poly<T>(v->d, v->scratch, tab.p, N, s.new_points, s.F, (int)s.conv_len, v->is_complex, g_stream);
     } else {
-        if (f.kind == 2) return done(v, E_ARG_LEN);   // custom callback + per-output taps: not supported on the device
-        rc = interp_frac<T>(v->d, v->scratch, N, new_points, (double)factor, (double)delay, (int)conv_len, f.kind,
+        if (f.fn) return done(v, E_ARG_LEN);   // custom callback + per-output taps: not supported on the device
+        rc = interp_frac<T>(v->d, v->scratch, N, s.new_points, (double)factor, (double)delay, (int)s.conv_len, f.kind,
                             (double)f.rolloff, v->is_complex, g_stream);
     }
     if (rc) return done(v, rc);
     trade(v);
-    v->len = new_len;
+    v->len = s.new_len;
     return done(v, 0);
 }
 
-// multiplier table of multiply_function_priv with is_fft_shifted = true (time_freq/mod.rs:612-723, fft_swap_x :67-78):
-// ratio * f(swap(x_i) * ratio); symmetric functions are evaluated for the first half and mirrored
-// (execute_sym_pairs_with_range, threading.rs:552-612)
 template <typename T> std::vector<T> shifted_response_table(const RealFn<T>& f, bool is_symmetric, size_t points, T ratio) {
     std::vector<T> tab(points);
     const size_t offset = points % 2;
@@ -858,15 +848,12 @@ template <typename T> Res<T> op_interpolatei(Vec<T>* v, const RealFn<T>& f, bool
     FftOpts fw;
     rc = fft_exec<T>(v->d, v->scratch, points, 1, fw, nullptr, 0, g_stream);
     if (rc) return done(v, rc);
-    if (f.kind != 2 && is_symmetric) {
-        // built-in responses: evaluated on the device (no O(points) host work, no table upload)
+    if (!f.fn) {
+        // built-in responses (always symmetric): evaluated on the device (no O(points) host work, no table upload)
         rc = ew_mul_shifted_resp<T>(v->scratch, points, f.kind, (double)f.rolloff, (double)(T)factor, g_stream);
     } else {
-        std::vector<T> tab = shifted_response_table<T>(f, is_symmetric, points, (T)factor);
-        T* dev = nullptr;
-        rc = upload_table(tab, &dev);
-        if (!rc) rc = ew_mul_table<T>(v->scratch, dev, points, 1, 0, g_stream);
-        table_consumed();
+        DeviceTable<T> tab(nullptr, [&] { return shifted_response_table<T>(f, is_symmetric, points, (T)factor); });
+        rc = tab.rc ? tab.rc : ew_mul_table<T>(v->scratch, tab.p, points, 1, 0, g_stream);
     }
     if (rc) return done(v, rc);
     FftOpts inv;
@@ -905,18 +892,15 @@ template <typename T> Res<T> op_interpolate(Vec<T>* v, const RealFn<T>* f, bool 
     if (!rc) rc = reserve(&v->d, &v->cap, big, false, 0);
     if (rc) return done(v, rc);
     // spectrum in the scratch -> re-binned spectrum in d
-    T* dev = nullptr;
-    bool have_table = false;
+    std::optional<DeviceTable<T>> tab;
     double scale = 1.0;
     int use_scale = 0;
     int resp_kind = -1;
     if (dest_points > n) {
-        if (f && f->kind != 2 && is_symmetric) resp_kind = f->kind;      // built-in response: evaluated on the device
+        if (f && !f->fn) resp_kind = f->kind;      // built-in response (always symmetric): evaluated on the device
         else if (f) {
-            std::vector<T> tab = shifted_response_table<T>(*f, is_symmetric, dest_points, factor);
-            rc = upload_table(tab, &dev);
-            if (rc) return done(v, rc);
-            have_table = true;
+            tab.emplace(nullptr, [&] { return shifted_response_table<T>(*f, is_symmetric, dest_points, factor); });
+            if (tab->rc) return done(v, tab->rc);
         } else { scale = (double)factor; use_scale = 1; }
     } else if (dest_points < n) {
         scale = (double)((T)(2 * dest_points) / (T)(2 * n));
@@ -924,9 +908,8 @@ template <typename T> Res<T> op_interpolate(Vec<T>* v, const RealFn<T>* f, bool 
     }
     const T pi = (T)M_PI;
     const T phase_inc = (T)2 * pi * (delay / delta_t) / (T)n;
-    rc = ew_resample_spectrum<T>(v->scratch, v->d, n, dest_points, dev, scale, use_scale, (double)phase_inc, delay != (T)0, resp_kind,
+    rc = ew_resample_spectrum<T>(v->scratch, v->d, n, dest_points, tab ? tab->p : nullptr, scale, use_scale, (double)phase_inc, delay != (T)0, resp_kind,
                                  f ? (double)f->rolloff : 0.0, (double)factor, g_stream);
-    if (have_table) table_consumed();
     if (rc) return done(v, rc);
     FftOpts inv;
     inv.inverse = 1;
@@ -1330,20 +1313,11 @@ template <typename T> int conv_rows(const void* in, void* out, size_t points, si
 }
 
 template <typename T> int fft_rows(const void* in, void* out, size_t points, size_t rows, int flags) {
-    FftOpts o;
-    o.inverse = (flags & BDSP_F_INVERSE) != 0;
-    o.magnitude = (flags & BDSP_F_MAGNITUDE) != 0;
-    o.real_input = (flags & BDSP_F_REAL_INPUT) != 0;
-    if ((flags & BDSP_F_SHIFT) && points) {
-        if (o.inverse) { o.in_rot = points / 2; o.scale = (double)((T)1 / (T)points); }
-        else o.out_rot = points / 2;
-    }
+    const bool inverse = (flags & BDSP_F_INVERSE) != 0;
     const int wk = (flags >> 8) & 15;   // BDSP_F_WINDOW(kind): every row is multiplied by the window on the way in (windowed_fft per row)
-    if (wk) {
-        if (o.inverse) { set_last_error("fft rows: a window applies to forward transforms only"); return -2; }
-        const int kind = wk - 1;
-        if (kind >= 0 && kind <= 2) { o.in_mul.kind = 3; o.in_mul.arg = kind; }
-    }
+    if (wk && inverse) { set_last_error("fft rows: a window applies to forward transforms only"); return -2; }
+    const FftOpts o = fft_opts<T>(points, inverse, (flags & BDSP_F_SHIFT) != 0, (flags & BDSP_F_MAGNITUDE) != 0,
+                                  (flags & BDSP_F_REAL_INPUT) != 0, wk ? wk - 1 : RECTANGULAR);
     return fft_exec<T>(in, out, points, rows, o, nullptr, 0, g_stream);
 }
 
@@ -1362,40 +1336,34 @@ int chain_rows(void* v, const void* w, void* mag, void* phase, size_t points, si
     return ew_scale_mul_mag_phase<T>(v, w, mag, phase, points * rows, (double)cre, (double)cim, cim != (T)0, write_back, g_stream);
 }
 // interpolatef (interpolation.rs:387-482) with a built-in impulse response on `rows` rows of `points` points (complex or
-// real), integer factor (the polyphase path): the tap tables are built once, every row is one kernel launch.
+// real): the polyphase path's tap tables are built once, every row is one kernel launch.
 // out: rows * new_points points, new_points as interpolatef32 computes it.  Returns the reference's error codes.
 template <typename T>
 int interp_rows(const void* in, void* out, size_t points, size_t rows, int is_complex, int kind, T rolloff, T factor, T delay,
                 size_t conv_len, size_t* new_points_out) {
     typedef typename CpxOf<T>::type C;
-    const size_t len = is_complex ? 2 * points : points;
-    if (conv_len > points / 2) conv_len = points / 2;
-    const double nl = round((double)((T)len * factor));
-    if (!(nl >= 0)) return E_ARG_LEN;
-    size_t new_len = (size_t)nl;
-    new_len += new_len % 2;
-    const size_t new_points = is_complex ? new_len / 2 : new_len;
-    if (new_points_out) *new_points_out = new_points;
+    InterpfShape s;
+    int rc = interpf_shape<T>(is_complex ? 2 * points : points, is_complex != 0, factor, conv_len, &s);
+    if (rc) return rc;
+    if (new_points_out) *new_points_out = s.new_points;
     if (!points || !rows) return 0;
-    const bool integer = (T)fabs((T)round(factor) - factor) < (T)1e-6;
     RealFn<T> f;
     f.kind = kind == 0 ? 0 : 1;
     f.rolloff = rolloff;
-    const size_t in_stride = (is_complex ? sizeof(C) : sizeof(T)) * points, out_stride = (is_complex ? sizeof(C) : sizeof(T)) * new_points;
-    if (conv_len <= 202 && new_len >= 2000 && integer) {
-        const int F = (int)round(factor), L = (int)conv_len;
-        const T* tab = nullptr;
-        int rc = interp_tap_tables<T>(f, delay, F, L, &tab);
+    const size_t esz = is_complex ? sizeof(C) : sizeof(T);
+    const char* x = reinterpret_cast<const char*>(in);
+    char* y = reinterpret_cast<char*>(out);
+    const int L = (int)s.conv_len;
+    if (s.poly) {
+        DeviceTable<T> tab = interp_tap_tables<T>(f, delay, s.F, L);
+        rc = tab.rc;
         for (size_t r = 0; r < rows && !rc; r++)
-            rc = interp_poly<T>(reinterpret_cast<const char*>(in) + r * in_stride, reinterpret_cast<char*>(out) + r * out_stride, tab, points,
-                                new_points, F, L, is_complex, g_stream);
-        table_consumed();
+            rc = interp_poly<T>(x + r * esz * points, y + r * esz * s.new_points, tab.p, points, s.new_points, s.F, L, is_complex, g_stream);
         return rc;
     }
-    int rc = 0;
     for (size_t r = 0; r < rows && !rc; r++)
-        rc = interp_frac<T>(reinterpret_cast<const char*>(in) + r * in_stride, reinterpret_cast<char*>(out) + r * out_stride, points, new_points,
-                            (double)factor, (double)delay, (int)conv_len, f.kind, (double)rolloff, is_complex, g_stream);
+        rc = interp_frac<T>(x + r * esz * points, y + r * esz * s.new_points, points, s.new_points, (double)factor, (double)delay, L,
+                            f.kind, (double)rolloff, is_complex, g_stream);
     return rc;
 }
 
@@ -1565,18 +1533,18 @@ template <typename R, typename T> static inline R as_res(Res<T> r) {
         return as_res<RES>(op_convolve_fn<T>(VEC(v), f, ratio, len));                                         \
     }                                                                                                                  \
     extern "C" RES convolve_real##S(HV* v, RFN fn, const void* data, uint8_t, T ratio, size_t len) {                   \
-        RealFn<T> f; f.kind = 2; f.fn = fn; f.data = data;                                                             \
+        RealFn<T> f; f.fn = fn; f.data = data;                                                                         \
         return as_res<RES>(op_convolve_fn<T>(VEC(v), f, ratio, len));                                         \
     }                                                                                                                  \
     extern "C" RES convolve_complex##S(HV* v, CFN fn, const void* data, uint8_t, T ratio, size_t len) {                \
         return as_res<RES>(op_convolve_cfn<T, CPLX>(VEC(v), fn, data, ratio, len));                                    \
     }                                                                                                                  \
     extern "C" RES multiply_frequency_response##S(HV* v, int32_t kind, T rolloff, T ratio) {                           \
-        RealFn<T> f; f.kind = kind == 0 ? 0 : 1; f.rolloff = rolloff; f.freq = true;                                   \
+        RealFn<T> f; f.kind = kind == 0 ? 0 : 1; f.rolloff = rolloff;                                                  \
         return as_res<RES>(op_mul_freq_resp<T>(VEC(v), f, ratio));                                                     \
     }                                                                                                                  \
     extern "C" RES multiply_frequency_response_real##S(HV* v, RFN fn, const void* data, uint8_t, T ratio) {            \
-        RealFn<T> f; f.kind = 2; f.fn = fn; f.data = data; f.freq = true;                                              \
+        RealFn<T> f; f.fn = fn; f.data = data;                                                                         \
         return as_res<RES>(op_mul_freq_resp<T>(VEC(v), f, ratio));                                                     \
     }                                                                                                                  \
     extern "C" RES multiply_frequency_response_complex##S(HV* v, CFN fn, const void* data, uint8_t, T ratio) {         \
@@ -1587,24 +1555,24 @@ template <typename R, typename T> static inline R as_res(Res<T> r) {
         return as_res<RES>(op_interpolatef<T>(VEC(v), f, factor, delay, len));                                         \
     }                                                                                                                  \
     extern "C" RES interpolatef_custom##S(HV* v, RFN fn, const void* data, uint8_t, T factor, T delay, size_t len) {   \
-        RealFn<T> f; f.kind = 2; f.fn = fn; f.data = data;                                                             \
+        RealFn<T> f; f.fn = fn; f.data = data;                                                                         \
         return as_res<RES>(op_interpolatef<T>(VEC(v), f, factor, delay, len));                                         \
     }                                                                                                                  \
     extern "C" RES interpolate_lin##S(HV* v, T factor, T delay) { return as_res<RES>(op_interpolate_lin(VEC(v), factor, delay)); } \
     extern "C" RES interpolatei##S(HV* v, int32_t kind, T rolloff, int32_t factor) {                                  \
-        RealFn<T> f; f.kind = kind == 0 ? 0 : 1; f.rolloff = rolloff; f.freq = true;                                   \
+        RealFn<T> f; f.kind = kind == 0 ? 0 : 1; f.rolloff = rolloff;                                                  \
         return as_res<RES>(op_interpolatei<T>(VEC(v), f, true, (uint32_t)factor));                                     \
     }                                                                                                                  \
     extern "C" RES interpolatei_custom##S(HV* v, RFN fn, const void* data, uint8_t is_symmetric, int32_t factor) {     \
-        RealFn<T> f; f.kind = 2; f.fn = fn; f.data = data; f.freq = true;                                              \
+        RealFn<T> f; f.fn = fn; f.data = data;                                                                         \
         return as_res<RES>(op_interpolatei<T>(VEC(v), f, is_symmetric != 0, (uint32_t)factor));                        \
     }                                                                                                                  \
     extern "C" RES interpolate##S(HV* v, int32_t kind, T rolloff, size_t dest_points, T delay) {                       \
-        RealFn<T> f; f.kind = kind == 0 ? 0 : 1; f.rolloff = rolloff; f.freq = true;                                   \
+        RealFn<T> f; f.kind = kind == 0 ? 0 : 1; f.rolloff = rolloff;                                                  \
         return as_res<RES>(op_interpolate<T>(VEC(v), &f, true, dest_points, delay));                                   \
     }                                                                                                                  \
     extern "C" RES interpolate_custom##S(HV* v, RFN fn, const void* data, uint8_t is_symmetric, size_t dest_points, T delay) { \
-        RealFn<T> f; f.kind = 2; f.fn = fn; f.data = data; f.freq = true;                                              \
+        RealFn<T> f; f.fn = fn; f.data = data;                                                                         \
         return as_res<RES>(op_interpolate<T>(VEC(v), &f, is_symmetric != 0, dest_points, delay));                      \
     }                                                                                                                  \
     extern "C" RES interpft##S(HV* v, size_t dest_points) { return as_res<RES>(op_interpolate<T>(VEC(v), nullptr, true, dest_points, (T)0)); } \

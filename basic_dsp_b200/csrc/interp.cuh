@@ -6,7 +6,7 @@
 
 namespace bdsp {
 
-// tab_dev: [2][F][2L+3] tap tables (interior, edge) built by the host, see capi.cu build_interp_tables()
+// tab_dev: [2][F][2L+3] tap tables (interior, edge) built by the host, see capi.cu interp_tap_tables()
 template <typename T>
 int interp_poly(const void* x, void* y, const T* tab_dev, size_t N, size_t new_points, int F, int L, int is_complex,
                 cudaStream_t st);

@@ -284,6 +284,23 @@ def test_interpolatef_rows(dtype, cplx_):
         assert o.rel_l2(got[r], ref) <= tol(4096, dtype)
         # identical to the per-vector trait call
         assert np.array_equal(got[r], DspVec(xr[r].copy()).interpolatef(bd.SINC, 0.0, float(F), 0.0, conv_len).to_numpy())
+    # both sides of every condition of the path rule (polyphase: conv_len <= 202, new_len >= 2000, integer factor)
+    ulp = float(np.spacing(dtype(4)))
+    near, off = (4 + ulp, 4 + 3 * ulp) if dtype == np.float32 else (4 + 5e-7, 4 + 2e-6)
+    shapes = [(3000, 2.5, 12, False), (3000, 2.0, 202, True), (3000, 2.0, 203, False), (3000, near, 12, True), (3000, off, 12, False)]
+    shapes += [(333, 3.0, 12, False), (500, 2.0, 12, True)] if cplx_ else [(999, 2.0, 12, False), (1000, 2.0, 12, True)]   # new_len 1998, 2000
+    for points, factor, conv_len, poly in shapes:
+        rows, scalars = 2, (2 if cplx_ else 1) * points
+        new_len = o.interpolatef_new_len(scalars, factor, dtype)
+        assert o.interpolatef_uses_fast_path(min(conv_len, points // 2), new_len, factor, dtype) == poly
+        x = rand_c(rng, points * rows, dtype) if cplx_ else rng.uniform(-10, 10, points * rows).astype(dtype)
+        xv, out = DspVec(x), DspVec.zeros(new_len * rows, is_complex=cplx_, dtype=dtype)
+        rc = getattr(L, "bdsp_interpolatef_rows" + sfx)(dptr(xv), dptr(out), points, rows, 1 if cplx_ else 0, bd.SINC, 0.0, factor, 0.25,
+                                                        conv_len, ctypes.byref(npts))
+        assert rc == 0 and npts.value == new_len // (2 if cplx_ else 1), (points, factor, conv_len)
+        got = out.to_numpy().reshape(rows, npts.value)
+        for r, xr in enumerate(x.reshape(rows, points)):
+            assert np.array_equal(got[r], DspVec(xr.copy()).interpolatef(bd.SINC, 0.0, factor, 0.25, conv_len).to_numpy()), (points, factor, conv_len)
 
 
 def test_convolve_complex_callback_wraps_around_short_vectors():
@@ -463,7 +480,7 @@ def test_windowed_fft_rows(n, rows, dtype):
 
 def test_two_devices_in_one_process():
     """One process driving two devices (bdsp_set_device): kernels that need more than 48 KB of dynamic shared memory are
-    configured per device, plans / tables / workspaces are per device."""
+    configured per device, plans / tables / staging buffers / workspaces are per device."""
     if bd.device_count() < 2:
         pytest.skip("needs two GPUs")
     L = bd.lib()
@@ -487,6 +504,11 @@ def test_two_devices_in_one_process():
             assert o.rel_l2(DspVec(xd).plain_fft().to_numpy(), o.plain_fft(xd)) <= tol(xd.size, np.float64)
             r = rng.uniform(-1, 1, 20001).astype(np.float32)
             DspVec(r).interpolatef(bd.SINC, 0.0, 4.0, 0.0, 12).to_numpy()
+            # a callback window: its table is staged in this device's memory
+            xw = rand_c(rng, 1001, np.float32)
+            w = np.array([np.float32(1.0 + i / 1001) for i in range(1001)])
+            got = DspVec(xw).custom_window("apply_custom_window", lambda i, p: 1.0 + i / p, is_symmetric=False).to_numpy()
+            assert o.rel_l2(got, xw * w) < 1e-6
             assert abs(DspVec(r).sum() - float(np.sum(r.astype(np.float64)))) < 1e-2
     finally:
         L.bdsp_set_device(0)
