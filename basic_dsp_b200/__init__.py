@@ -233,6 +233,8 @@ def _declare(lib):
     for s in ("32", "64"):
         f = getattr(lib, "bdsp_fft_rows_c" + s)
         f.restype, f.argtypes = c_int32, [c_void_p, c_void_p, c_size_t, c_size_t, c_int32]
+        f = getattr(lib, "bdsp_fft_frames_c" + s)
+        f.restype, f.argtypes = c_int32, [c_void_p, c_void_p, c_size_t, c_size_t, c_size_t, c_int32]
         f = getattr(lib, "bdsp_conv_plan_create_c" + s)
         f.restype, f.argtypes = c_void_p, [c_void_p, c_size_t]
         f = getattr(lib, "bdsp_convolve_signal_rows_c" + s)

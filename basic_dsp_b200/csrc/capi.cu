@@ -1321,6 +1321,27 @@ template <typename T> int fft_rows(const void* in, void* out, size_t points, siz
     return fft_exec<T>(in, out, points, rows, o, nullptr, 0, g_stream);
 }
 
+// fft_rows over `frames` frames of one signal, frame f = the `points` points from point f*hop on (short-time analysis)
+template <typename T> int fft_frames(const void* in, void* out, size_t points, size_t hop, size_t frames, int flags) {
+    if (flags & BDSP_F_INVERSE) { set_last_error("fft frames: frames are analysis frames, BDSP_F_INVERSE is not accepted"); return -2; }
+    if (!hop) { set_last_error("fft frames: hop must be at least 1"); return -2; }
+    if (!points || !frames) return 0;
+    const bool real = (flags & BDSP_F_REAL_INPUT) != 0, mag = (flags & BDSP_F_MAGNITUDE) != 0;
+    const size_t in_esz = real ? sizeof(T) : 2 * sizeof(T), out_esz = mag ? sizeof(T) : 2 * sizeof(T);
+    const size_t max = ~(size_t)0;
+    if (frames - 1 > (max - points) / hop || ((frames - 1) * hop + points) > max / in_esz || frames > max / points / out_esz) {
+        set_last_error("fft frames: %zu frames of %zu points, hop %zu overflow the address space", frames, points, hop);
+        return -2;
+    }
+    const uintptr_t i0 = reinterpret_cast<uintptr_t>(in), o0 = reinterpret_cast<uintptr_t>(out);
+    const size_t in_bytes = ((frames - 1) * hop + points) * in_esz, out_bytes = frames * points * out_esz;
+    if (i0 < o0 + out_bytes && o0 < i0 + in_bytes) { set_last_error("fft frames: the output overlaps the input"); return -3; }
+    const int wk = (flags >> 8) & 15;
+    FftOpts o = fft_opts<T>(points, false, (flags & BDSP_F_SHIFT) != 0, mag, real, wk ? wk - 1 : RECTANGULAR);
+    o.in_stride = hop;
+    return fft_exec<T>(in, out, points, frames, o, nullptr, 0, g_stream);
+}
+
 // ---- batched (matrix-row) forms: the reference's MatrixMxN applies the vector operation to every row in turn
 // (matrix/src/time_freq.rs:52-74, matrix/src/complex.rs:18-26); rows sit back to back in device memory ----------------------
 // magnitude (hypot, complex_to_real.rs:376) / phase (atan2, :402) / magnitude_squared of `rows` rows: elementwise, so the
@@ -1702,6 +1723,12 @@ extern "C" int32_t bdsp_stream_sync(void* s) { BDSP_CUDA_OK(cudaStreamSynchroniz
 
 extern "C" int32_t bdsp_fft_rows_c32(const void* in, void* out, size_t points, size_t rows, int32_t flags) { return fft_rows<float>(in, out, points, rows, flags); }
 extern "C" int32_t bdsp_fft_rows_c64(const void* in, void* out, size_t points, size_t rows, int32_t flags) { return fft_rows<double>(in, out, points, rows, flags); }
+extern "C" int32_t bdsp_fft_frames_c32(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags) {
+    return fft_frames<float>(in, out, points, hop, frames, flags);
+}
+extern "C" int32_t bdsp_fft_frames_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags) {
+    return fft_frames<double>(in, out, points, hop, frames, flags);
+}
 extern "C" BdspConvPlan* bdsp_conv_plan_create_c32(const void* h, size_t L) { return reinterpret_cast<BdspConvPlan*>(conv_plan_create<float>(h, L)); }
 extern "C" BdspConvPlan* bdsp_conv_plan_create_c64(const void* h, size_t L) { return reinterpret_cast<BdspConvPlan*>(conv_plan_create<double>(h, L)); }
 extern "C" void bdsp_conv_plan_destroy(BdspConvPlan* plan) {

@@ -32,6 +32,9 @@ namespace bdsp {
 template <bool RIN>
 int fftp_single(const void* in, void* out, size_t n, size_t groups, bool inverse, bool si, bool so, bool magnitude, double scale,
                 cudaStream_t st);
+template <bool RIN>
+int fftp_frames(const void* in, void* out, size_t n, size_t groups, size_t hop, const float* win, bool so, bool magnitude, double scale,
+                cudaStream_t st);
 int fftp_two_pass(const void* in, void* out, void* tmp, const FftPlan& p, size_t rows, bool inverse, bool si, bool so, bool magnitude,
                   double scale, bool real_in, const InMul& im, cudaStream_t st);
 int fftp_three_pass(const void* in, void* out, void* tmp, const FftPlan& p, size_t n, size_t rows, bool inverse, bool si, bool so,
@@ -101,10 +104,11 @@ template <> const double2* twiddle_table<double>() { DeviceState* s = dev_state(
 // default stream, where their multi-kernel operations may interleave, so scratch buffers are never shared between
 // threads (the reference is safe for concurrent use of distinct vectors).  The calling thread binds its stream with
 // workspace_bind_stream (capi: bdsp_set_stream).  Slots: 0..3 the transforms and reductions, 4..5 the full-length
-// convolution (its buffers stay live across nested fft_exec calls, which use 0..2).
+// convolution (its buffers stay live across nested fft_exec calls, which use 0..2), 6 the gathered frames of
+// FftRoute::FramePass (live across the transform that is routed again, which may use 0..3).
 namespace {
 thread_local cudaStream_t tl_ws_stream = nullptr;
-constexpr int WS_SLOTS = 6;
+constexpr int WS_SLOTS = 7;
 struct WsSet { void* p[WS_SLOTS] = {}; size_t bytes[WS_SLOTS] = {}; };
 struct WsMap {
     std::map<std::pair<int, cudaStream_t>, WsSet> m;
@@ -883,6 +887,15 @@ __global__ void in_mul_rows_kernel(const void* __restrict__ in_, void* __restric
     else reinterpret_cast<C*>(out_)[i] = v;
 }
 
+// out[f][p] = in[f * hop + p]: frames of a strided input laid back to back (FftRoute::FramePass), E = real or complex point
+template <typename E>
+__global__ void gather_frames_kernel(const E* __restrict__ in, E* __restrict__ out, long long n, long long hop, long long total) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const long long f = i / n;
+    out[i] = in[f * hop + (i - f * n)];
+}
+
 template <typename T, bool INV>
 int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o, void* work, size_t work_bytes,
             cudaStream_t st) {
@@ -907,8 +920,27 @@ int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o,
     }
     const bool si = in_rot != 0, so = om.rot != 0, mag = o.magnitude != 0, real_in = o.real_input != 0;
     const FftPlan plan = fft_route({sizeof(T) == 8, n, batch, INV, real_in, mag, im.kind, (size_t)in_rot, (size_t)om.rot, reinterpret_cast<uintptr_t>(in),
-                                    reinterpret_cast<uintptr_t>(out), reinterpret_cast<uintptr_t>(w), sizeof(T) == 4 && n == 65536 && fftc_cluster_ok()});
+                                    reinterpret_cast<uintptr_t>(out), reinterpret_cast<uintptr_t>(w), sizeof(T) == 4 && n == 65536 && fftc_cluster_ok(),
+                                    false, o.in_stride});
     switch (plan.route) {
+    case FftRoute::FramePass: {
+        // the frames back to back in a slot that no route of the rows uses, then those rows exactly as fft_exec takes them
+        const long long tot = (long long)(n * batch), hop = (long long)o.in_stride;
+        const unsigned grid = (unsigned)((tot + 255) / 256);
+        BDSP_WS(fr, void*, n * batch * (real_in ? sizeof(T) : sizeof(C)), 6);
+        if (real_in) gather_frames_kernel<T><<<grid, 256, 0, st>>>(static_cast<const T*>(in), static_cast<T*>(fr), (long long)n, hop, tot);
+        else gather_frames_kernel<C><<<grid, 256, 0, st>>>(static_cast<const C*>(in), static_cast<C*>(fr), (long long)n, hop, tot);
+        BDSP_LAUNCHED();
+        FftOpts o2 = o;
+        o2.in_stride = n;
+        o2.in_mul = im;   // the window table is already written
+        return fft_any<T, INV>(fr, out, n, batch, o2, work, work_bytes, st);
+    }
+    case FftRoute::PackedFrames: {
+        const float* win = static_cast<const float*>(im.kind ? im.p : nullptr);   // kind 1: n real scalars
+        if (real_in) return fftp_frames<true>(in, out, n, plan.groups, o.in_stride, win, so, mag, o.scale, st);
+        return fftp_frames<false>(in, out, n, plan.groups, o.in_stride, win, so, mag, o.scale, st);
+    }
     case FftRoute::MulPass: {
         const bool to_complex = real_in && im.kind == 2;
         const bool real_rows = real_in && !to_complex;

@@ -14,10 +14,13 @@ struct FftOpts {
     InMul in_mul;           // multiply input element g of every sequence by a table entry / window value while loading
                             // (windowed_fft: time_to_freq.rs:167-175; spectrum multiply of the frequency-domain
                             // convolution: convolution.rs:427-429,444-446) - no separate pass over memory
+    size_t in_stride = 0;   // points between the starts of consecutive input sequences; 0 means n
 };
 
 // Transforms `batch` sequences of n complex points (sequence b at element offset b*n; real input:
-// b*n scalars).  `work` must hold n*batch complex values when the transform needs a scratch pass
+// b*n scalars).  With opts.in_stride = s (not 0 or n), sequence b is the n points (scalars) that start at
+// point b*s instead: overlapping or spaced frames of one signal, the last one ending at (batch-1)*s + n; such a
+// call must not write into its input.  `work` must hold n*batch complex values when the transform needs a scratch pass
 // (n > block limit or non power of two); pass nullptr to use the library's grow-only workspace.
 // in == out is allowed.  Returns 0 or a negative error code (see set_last_error()).
 template <typename T>

@@ -1,6 +1,7 @@
 // Which kernels run one level of an FFT (fft.cu fft_any): the one place that picks the path.  Plain C++ (no CUDA), so that
-// the routing table can be checked without a GPU (tests/cpp/fft_route_driver.cpp).  The rules apply in the order of
-// FftRoute; the first one that matches wins.
+// the routing table can be checked without a GPU (tests/cpp/fft_route_driver.cpp, tests/cpp/fft_frames_route_driver.cpp).
+// A strided input (FftRouteIn::in_stride other than 0 or n) takes one of the two frame routes; every other input the
+// rules apply to in the order of FftRoute, and the first one that matches wins.
 #pragma once
 #include <cstddef>
 #include <cstdint>
@@ -24,6 +25,9 @@ enum class FftRoute {
     QRowsInterleave, // radix-q pass, rows of P points routed again into a second buffer, interleave pass
     QRows,           // radix-q pass, generic rows that store interleaved
     Bluestein,       // chirp-z
+    PackedFrames,    // strided frames: packed single pass with the frame addressing and the multiplier on its first load
+                     // (fftp_kernel<FRAMES>)
+    FramePass,       // strided frames: gather_frames_kernel copies them back to back, the copy is routed again
 };
 
 struct FftRouteIn {
@@ -36,6 +40,7 @@ struct FftRouteIn {
     uintptr_t work = 0;            // scratch of the multi-pass routes (n = 2^k > fft_block_max_n), 0 when none is needed
     bool cluster_ok = false;       // the 16-CTA cluster kernel can be placed on this device
     bool generic_only = false;     // the generic kernels only: rows with a strided output map, the Bluestein sub-transforms
+    size_t in_stride = 0;          // points between the starts of consecutive input sequences; 0 means n
 };
 
 struct FftPlan {
@@ -61,6 +66,18 @@ inline FftPlan fft_route(const FftRouteIn& a) {
     const bool half_rot = (a.in_rot == 0 || a.in_rot == n / 2) && (a.out_rot == 0 || a.out_rot == n / 2);
     const bool inv_store = !(a.inverse && (a.magnitude || a.out_rot != 0));
     const bool pow2 = n && !(n & (n - 1));
+    if (a.in_stride != 0 && a.in_stride != n) {
+        // Frames that overlap or leave gaps: fused where fft_route would take Packed or RealRows (after MulPass) for the
+        // same frames laid back to back, and where every frame start keeps the alignment of the paired loads (even stride:
+        // 16 B for complex points, 8 B for real scalars).  Everything else is gathered first and then routed as rows.
+        const size_t per = n >= 64 && n < 4096 ? 4096 / n : 1;
+        const bool grid_ok = a.real_input ? rows / per * 2 <= FFT_GRID_MAX : (n < 4096 ? rows / per : rows * 2) <= FFT_GRID_MAX;
+        if (c32 && !a.inverse && pow2 && n >= 64 && n <= 8192 && a.in_rot == 0 && half_rot && (a.in_mul == 0 || a.in_mul == 1) &&
+            n * rows >= (1u << 16) && rows % per == 0 && grid_ok && aligned(a.in, a.real_input ? 8 : 16) && aligned(a.out, 8) &&
+            a.in_stride % 2 == 0 && a.in != a.out)
+            return {FftRoute::PackedFrames, rows / per};
+        return {FftRoute::FramePass};
+    }
     if (pow2 && !a.generic_only) {
         // the packed single-pass kernels take no first-load multiplier: in their throughput regime one elementwise pass +
         // the packed kernel beats the generic kernel with the multiplier fused

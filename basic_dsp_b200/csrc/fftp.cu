@@ -11,9 +11,10 @@
 //   ROWS      last pass of a multi-pass transform: four adjacent 4096-point rows per CTA, transposing store
 //   TQ = Q    last pass with 16/Q adjacent rows of 256*Q points per CTA (128 threads), transposing store
 //   RIN       the input holds real scalars
+//   FRAMES    the sequences are strided frames of one signal, with an optional window multiplied in on the first load
 // fftp_col16_kernel / fftp_col256_kernel: first pass(es) of the multi-pass transforms: 16- / 256-point (NH = 2: 32- / 512-point)
 //   columns of 16 adjacent columns per CTA, inter-pass twiddle evaluated with sincospif on exact arguments.
-// Launchers, one per route of fft_route.h: fftp_single (complex or real rows), fftp_two_pass (2^15..2^20), fftp_three_pass
+// Launchers, one per route of fft_route.h: fftp_single (complex or real rows), fftp_frames (strided frames), fftp_two_pass (2^15..2^20), fftp_three_pass
 //   (2^21..2^24), fftp_rows_pass (packed last pass, also behind a generic column pass).
 // Replaces rustfft for these lengths (vector/src/vector_types/time_freq/mod.rs:45-58) incl. the fused
 // fft_shift (time_to_freq.rs:163), ifft's scale + ifft_shift (freq_to_time.rs:165-167) and magnitude.
@@ -40,10 +41,17 @@ using namespace ols16;
 // NATQ = Q in {1, 2, 4, 8} (R0 = 1, no ROWS): the CTA's 4096 contiguous points are 16/Q independent rows of 256*Q points
 // (k0 = q + Q*row); the first stage is a radix-Q butterfly inside every row, results are stored in natural order.
 // Batched 512 / 1024 / 2048-point transforms with the structure of the 4096-point kernel.
+// FRAMES = true (forward, no ROWS, n <= 8192): the sequences are frames of one signal that start `hop` points apart (hop
+// even): point p of the CTA's N points is read from x[(row * (N / n) + p / n) * hop + p % n], n the sequence length, and,
+// when `win` is not null, multiplied by win[p % n] as it is loaded.  The product is rounded on its own (__fmul_rn), as the
+// separate multiplier pass (fft.cu in_mul_rows_kernel) rounds it, so that the result is the one of that pass followed by the
+// plain kernel.
 #define FP_MINB256 2   // CTAs per SM for the 256-thread 8192-point kernel
-template <int R0, bool INV, bool SHIFT_IN, bool SHIFT_OUT, bool MAG, bool ROWS, int TQ = 0, int NATQ = 0, bool RIN = false, int SQ = 0>
+template <int R0, bool INV, bool SHIFT_IN, bool SHIFT_OUT, bool MAG, bool ROWS, int TQ = 0, int NATQ = 0, bool RIN = false, int SQ = 0,
+          bool FRAMES = false>
 __global__ void __launch_bounds__(128 * R0, R0 == 2 ? FP_MINB256 : 4 / R0)
-fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long rows, float scale, const float* __restrict__ tw, int n1, int n2c) {
+fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long rows, float scale, const float* __restrict__ tw, int n1, int n2c,
+            long long hop, const float* __restrict__ win) {
     constexpr int NSB = R0;               // sub-blocks (4096-point transforms) owned by this CTA
     constexpr int NT = 128 * NSB;         // threads
     constexpr int N = 4096 * R0;
@@ -74,7 +82,28 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
 
     // two adjacent points starting at complex element pointer gp: {re0, im0, re1, im1}
     auto ldpair = [&](const float2* gp) -> float4 {
-        if constexpr (RIN) {
+        if constexpr (FRAMES) {
+            constexpr int FN = SQ ? 16 * SQ : NATQ ? 256 * NATQ : N;   // frame length
+            const int p = (int)(gp - xr);
+            const long long src = ((long long)seq * (N / FN) + p / FN) * hop + p % FN;
+            float4 v;
+            if constexpr (RIN) {
+                const float2 r = __ldg(reinterpret_cast<const float2*>(reinterpret_cast<const float*>(x) + src));
+                v = make_float4(r.x, 0.f, r.y, 0.f);
+            } else {
+                v = __ldg(reinterpret_cast<const float4*>(x + src));
+            }
+            if (win) {
+                const float2 w = __ldg(reinterpret_cast<const float2*>(win + p % FN));
+                v.x = __fmul_rn(v.x, w.x);
+                v.z = __fmul_rn(v.z, w.y);
+                if constexpr (!RIN) {
+                    v.y = __fmul_rn(v.y, w.x);
+                    v.w = __fmul_rn(v.w, w.y);
+                }
+            }
+            return v;
+        } else if constexpr (RIN) {
             const float2 r = __ldg(reinterpret_cast<const float2*>(reinterpret_cast<const float*>(x) + (gp - x)));
             return make_float4(r.x, 0.f, r.y, 0.f);
         } else {
@@ -648,10 +677,12 @@ const float* fftp_twiddles() {
 
 namespace {
 
-template <int R0, bool INV, bool SI, bool SO, bool MAG, bool ROWS = false, int TQ = 0, int NATQ = 0, bool RIN = false, int SQ = 0>
-int fftp_launch(const void* in, void* out, size_t rows, float scale, cudaStream_t st, int n1 = 1, int n2c = 1) {
+template <int R0, bool INV, bool SI, bool SO, bool MAG, bool ROWS = false, int TQ = 0, int NATQ = 0, bool RIN = false, int SQ = 0,
+          bool FRAMES = false>
+int fftp_launch(const void* in, void* out, size_t rows, float scale, cudaStream_t st, int n1 = 1, int n2c = 1, size_t hop = 0,
+                const float* win = nullptr) {
     const size_t smem = (size_t)2 * R0 * FP_B_OF(R0) * sizeof(float);
-    auto kern = fftp_kernel<R0, INV, SI, SO, MAG, ROWS, TQ, NATQ, RIN, SQ>;
+    auto kern = fftp_kernel<R0, INV, SI, SO, MAG, ROWS, TQ, NATQ, RIN, SQ, FRAMES>;
     static PerDeviceOnce configured;   // per instantiation and device
     if (configured.need()) {
         BDSP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -659,7 +690,8 @@ int fftp_launch(const void* in, void* out, size_t rows, float scale, cudaStream_
     }
     const float* tw = fftp_twiddles();
     if (!tw) return -1001;
-    kern<<<(unsigned)rows, 128 * R0, smem, st>>>(reinterpret_cast<const float2*>(in), out, (long long)rows, scale, tw, n1, n2c);
+    kern<<<(unsigned)rows, 128 * R0, smem, st>>>(reinterpret_cast<const float2*>(in), out, (long long)rows, scale, tw, n1, n2c,
+                                                  (long long)hop, win);
     BDSP_CUDA_OK(cudaGetLastError());
     BDSP_LAUNCHED();
     return 0;
@@ -739,6 +771,28 @@ int fftp_single(const void* in, void* out, size_t n, size_t groups, bool inverse
 }
 template int fftp_single<false>(const void*, void*, size_t, size_t, bool, bool, bool, bool, double, cudaStream_t);
 template int fftp_single<true>(const void*, void*, size_t, size_t, bool, bool, bool, bool, double, cudaStream_t);
+
+// forward single pass over frames of n = 64 .. 8192 points that start `hop` points apart (FftRoute::PackedFrames), with an
+// optional table of n real multipliers (the window) on the first load; RIN: the frames hold real scalars
+template <bool RIN>
+int fftp_frames(const void* in, void* out, size_t n, size_t groups, size_t hop, const float* win, bool so, bool magnitude, double scale,
+                cudaStream_t st) {
+    const float sc = (float)scale;
+    return fftp_with_flags<false, false>(false, false, so, magnitude, [&](auto inv, auto shi, auto sho, auto mag) {
+        switch (n) {
+        case 64: return fftp_launch<1, inv, shi, sho, mag, false, 0, 1, RIN, 4, true>(in, out, groups, sc, st, 1, 1, hop, win);
+        case 128: return fftp_launch<1, inv, shi, sho, mag, false, 0, 1, RIN, 8, true>(in, out, groups, sc, st, 1, 1, hop, win);
+        case 256: return fftp_launch<1, inv, shi, sho, mag, false, 0, 1, RIN, 0, true>(in, out, groups, sc, st, 1, 1, hop, win);
+        case 512: return fftp_launch<1, inv, shi, sho, mag, false, 0, 2, RIN, 0, true>(in, out, groups, sc, st, 1, 1, hop, win);
+        case 1024: return fftp_launch<1, inv, shi, sho, mag, false, 0, 4, RIN, 0, true>(in, out, groups, sc, st, 1, 1, hop, win);
+        case 2048: return fftp_launch<1, inv, shi, sho, mag, false, 0, 8, RIN, 0, true>(in, out, groups, sc, st, 1, 1, hop, win);
+        case 4096: return fftp_launch<1, inv, shi, sho, mag, false, 0, 0, RIN, 0, true>(in, out, groups, sc, st, 1, 1, hop, win);
+        default: return fftp_launch<2, inv, shi, sho, mag, false, 0, 0, RIN, 0, true>(in, out, groups, sc, st, 1, 1, hop, win);
+        }
+    });
+}
+template int fftp_frames<false>(const void*, void*, size_t, size_t, size_t, const float*, bool, bool, double, cudaStream_t);
+template int fftp_frames<true>(const void*, void*, size_t, size_t, size_t, const float*, bool, bool, double, cudaStream_t);
 
 // two-pass transform for n = 2^15 .. 2^20 (FftRoute::TwoPass), n = p.n1 * 2^p.log2n2; tmp holds n*rows complex values
 int fftp_two_pass(const void* in, void* out, void* tmp, const FftPlan& p, size_t rows, bool inverse, bool si, bool so, bool magnitude,

@@ -510,6 +510,16 @@ BdspVecResult64 bdsp_fft_magnitude64(BdspVec64* vector);
                                                      * (matrix/src/time_freq.rs:69-74, time_to_freq.rs:167-175) */
 int32_t bdsp_fft_rows_c32(const void* in, void* out, size_t points, size_t rows, int32_t flags);
 int32_t bdsp_fft_rows_c64(const void* in, void* out, size_t points, size_t rows, int32_t flags);
+/* Windowed transforms of overlapping (or spaced) frames of one signal: a short-time Fourier transform / spectrogram.
+ * Frame f is the `points` points (complex, or real scalars with BDSP_F_REAL_INPUT) that start at point f*hop of `in`,
+ * which must hold (frames-1)*hop + points points: frames = 1 + (len - points) / hop, no padding, no centring; hop > points
+ * skips the samples between frames.  Row f of `out` is byte for byte what bdsp_fft_rows_* writes for the same points,
+ * frames and flags when the frames lie back to back; BDSP_F_WINDOW(kind) | BDSP_F_MAGNITUDE gives a spectrogram.
+ * flags: BDSP_F_SHIFT, BDSP_F_MAGNITUDE, BDSP_F_REAL_INPUT, BDSP_F_WINDOW(kind).  Returns 0; -2 for BDSP_F_INVERSE, hop == 0
+ * or sizes that overflow size_t; -3 when the input range and the output overlap (bdsp_last_error says which).
+ * points == 0 or frames == 0 returns 0 without a launch. */
+int32_t bdsp_fft_frames_c32(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
+int32_t bdsp_fft_frames_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
 /* convolve_signal for every row with one impulse response of h_points complex taps (device pointer);
  * `plan` caches the impulse-response spectrum between calls (create once, reuse, destroy) */
 typedef struct BdspConvPlan BdspConvPlan;
