@@ -22,6 +22,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BASIC_DSP_B200_LIB", os.path.join(_HERE, "libbasic_dsp_b200.so"))
 
 F_INVERSE, F_SHIFT, F_MAGNITUDE, F_REAL_INPUT = 1, 2, 4, 8
+F_REAL_OUTPUT = 16   # bdsp_ifft_frames_*: the output holds the real parts of the synthesis as scalars
 
 
 def F_WINDOW(kind):
@@ -233,8 +234,9 @@ def _declare(lib):
     for s in ("32", "64"):
         f = getattr(lib, "bdsp_fft_rows_c" + s)
         f.restype, f.argtypes = c_int32, [c_void_p, c_void_p, c_size_t, c_size_t, c_int32]
-        f = getattr(lib, "bdsp_fft_frames_c" + s)
-        f.restype, f.argtypes = c_int32, [c_void_p, c_void_p, c_size_t, c_size_t, c_size_t, c_int32]
+        for name in ("bdsp_fft_frames_c", "bdsp_ifft_frames_c"):
+            f = getattr(lib, name + s)
+            f.restype, f.argtypes = c_int32, [c_void_p, c_void_p, c_size_t, c_size_t, c_size_t, c_int32]
         f = getattr(lib, "bdsp_conv_plan_create_c" + s)
         f.restype, f.argtypes = c_void_p, [c_void_p, c_size_t]
         f = getattr(lib, "bdsp_convolve_signal_rows_c" + s)

@@ -1342,6 +1342,36 @@ template <typename T> int fft_frames(const void* in, void* out, size_t points, s
     return fft_exec<T>(in, out, points, frames, o, nullptr, 0, g_stream);
 }
 
+// the inverse of fft_frames: inverse rows scaled by 1/points, then the least-squares overlap-add of the frames under the
+// synthesis window (torch.istft(center=False), scipy.signal.istft) into (frames-1)*hop + points points
+template <typename T> int ifft_frames(const void* in, void* out, size_t points, size_t hop, size_t frames, int flags) {
+    const int unknown = flags & ~(BDSP_F_SHIFT | BDSP_F_REAL_OUTPUT | (15 << 8));   // (15 << 8): every BDSP_F_WINDOW(kind)
+    if (unknown) {
+        const char* name = (unknown & BDSP_F_INVERSE) ? "BDSP_F_INVERSE" : (unknown & BDSP_F_MAGNITUDE) ? "BDSP_F_MAGNITUDE"
+                         : (unknown & BDSP_F_REAL_INPUT) ? "BDSP_F_REAL_INPUT" : nullptr;
+        if (name) set_last_error("ifft frames: %s is not accepted (BDSP_F_SHIFT, BDSP_F_REAL_OUTPUT, BDSP_F_WINDOW(kind) are)", name);
+        else set_last_error("ifft frames: unknown flag bits 0x%x", (unsigned)unknown);
+        return -2;
+    }
+    if (!hop) { set_last_error("ifft frames: hop must be at least 1"); return -2; }
+    if (!points || !frames) return 0;
+    if (hop > points) { set_last_error("ifft frames: hop %zu > %zu points leaves samples that no frame covers", hop, points); return -2; }
+    const bool real_out = (flags & BDSP_F_REAL_OUTPUT) != 0;
+    const size_t in_esz = 2 * sizeof(T), out_esz = real_out ? sizeof(T) : 2 * sizeof(T);
+    // hop <= points: the output's (frames-1)*hop + points points are at most the input's frames*points
+    if (frames > ~(size_t)0 / points / in_esz) {
+        set_last_error("ifft frames: %zu frames of %zu points overflow the address space", frames, points);
+        return -2;
+    }
+    const uintptr_t i0 = reinterpret_cast<uintptr_t>(in), o0 = reinterpret_cast<uintptr_t>(out);
+    const size_t in_bytes = frames * points * in_esz, out_bytes = ((frames - 1) * hop + points) * out_esz;
+    if (i0 < o0 + out_bytes && o0 < i0 + in_bytes) { set_last_error("ifft frames: the output overlaps the input"); return -3; }
+    const int wk = (flags >> 8) & 15;
+    FftOpts o = fft_opts<T>(points, true, (flags & BDSP_F_SHIFT) != 0, false, false, wk ? wk - 1 : RECTANGULAR);
+    o.scale = (double)((T)1 / (T)points);   // ifft()'s 1/points, with or without the shift
+    return ifft_frames_exec<T>(in, out, points, hop, frames, o, real_out, g_stream);
+}
+
 // ---- batched (matrix-row) forms: the reference's MatrixMxN applies the vector operation to every row in turn
 // (matrix/src/time_freq.rs:52-74, matrix/src/complex.rs:18-26); rows sit back to back in device memory ----------------------
 // magnitude (hypot, complex_to_real.rs:376) / phase (atan2, :402) / magnitude_squared of `rows` rows: elementwise, so the
@@ -1728,6 +1758,12 @@ extern "C" int32_t bdsp_fft_frames_c32(const void* in, void* out, size_t points,
 }
 extern "C" int32_t bdsp_fft_frames_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags) {
     return fft_frames<double>(in, out, points, hop, frames, flags);
+}
+extern "C" int32_t bdsp_ifft_frames_c32(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags) {
+    return ifft_frames<float>(in, out, points, hop, frames, flags);
+}
+extern "C" int32_t bdsp_ifft_frames_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags) {
+    return ifft_frames<double>(in, out, points, hop, frames, flags);
 }
 extern "C" BdspConvPlan* bdsp_conv_plan_create_c32(const void* h, size_t L) { return reinterpret_cast<BdspConvPlan*>(conv_plan_create<float>(h, L)); }
 extern "C" BdspConvPlan* bdsp_conv_plan_create_c64(const void* h, size_t L) { return reinterpret_cast<BdspConvPlan*>(conv_plan_create<double>(h, L)); }

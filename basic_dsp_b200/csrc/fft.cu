@@ -104,8 +104,9 @@ template <> const double2* twiddle_table<double>() { DeviceState* s = dev_state(
 // default stream, where their multi-kernel operations may interleave, so scratch buffers are never shared between
 // threads (the reference is safe for concurrent use of distinct vectors).  The calling thread binds its stream with
 // workspace_bind_stream (capi: bdsp_set_stream).  Slots: 0..3 the transforms and reductions, 4..5 the full-length
-// convolution (its buffers stay live across nested fft_exec calls, which use 0..2), 6 the gathered frames of
-// FftRoute::FramePass (live across the transform that is routed again, which may use 0..3).
+// convolution (its buffers stay live across nested fft_exec calls, which use 0..2), 6 the frame buffers of the frame
+// entry points: the gathered frames of FftRoute::FramePass and the inverse rows of ifft_frames_exec (live across the
+// transform that fills or reads them, which may use 0..3).
 namespace {
 thread_local cudaStream_t tl_ws_stream = nullptr;
 constexpr int WS_SLOTS = 7;
@@ -896,6 +897,35 @@ __global__ void gather_frames_kernel(const E* __restrict__ in, E* __restrict__ o
     out[i] = in[f * hop + (i - f * n)];
 }
 
+// out[t] = sum_f w[p] y[f][p] / sum_f w[p]^2, p = t - f * hop, over the frames f that cover point t in ascending order:
+// the least-squares overlap-add of bdsp_ifft_frames_* (win == nullptr: w = 1, the mean of the covering frames).  The sums
+// start from the first frame's terms, so a point that one frame covers without a window is that frame's value bit for bit.
+// Neighbouring threads read neighbouring points of every frame, each frame value once; no atomics, so every call writes
+// the same bytes.
+template <typename T, bool REAL_OUT>
+__global__ void overlap_add_kernel(const typename CpxOf<T>::type* __restrict__ y, const T* __restrict__ win, void* __restrict__ out,
+                                   long long n, long long hop, long long frames, long long len) {
+    typedef typename CpxOf<T>::type C;
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= len) return;
+    long long f = t < n ? 0 : (t - n) / hop + 1;
+    const long long f_hi = min(t / hop, frames - 1);
+    long long p = t - f * hop;
+    C v = y[f * n + p];
+    T w = win ? win[p] : (T)1;
+    C num = mk<T>(w * v.x, w * v.y);
+    T den = w * w;
+    for (++f, p -= hop; f <= f_hi; ++f, p -= hop) {
+        v = y[f * n + p];
+        w = win ? win[p] : (T)1;
+        num.x += w * v.x;
+        num.y += w * v.y;
+        den += w * w;
+    }
+    if (REAL_OUT) reinterpret_cast<T*>(out)[t] = num.x / den;
+    else reinterpret_cast<C*>(out)[t] = mk<T>(num.x / den, num.y / den);
+}
+
 template <typename T, bool INV>
 int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o, void* work, size_t work_bytes,
             cudaStream_t st) {
@@ -1074,5 +1104,34 @@ int fft_exec(const void* in, void* out, size_t n, size_t batch, const FftOpts& o
 
 template int fft_exec<float>(const void*, void*, size_t, size_t, const FftOpts&, void*, size_t, cudaStream_t);
 template int fft_exec<double>(const void*, void*, size_t, size_t, const FftOpts&, void*, size_t, cudaStream_t);
+
+template <typename T>
+int ifft_frames_exec(const void* in, void* out, size_t n, size_t hop, size_t frames, const FftOpts& opts, bool real_out,
+                     cudaStream_t stream) {
+    typedef typename CpxOf<T>::type C;
+    if (n == 0 || frames == 0) return 0;
+    // the inverse rows into a slot that no route of the rows uses; it stays live across their transform (slots 0..3)
+    BDSP_WS(y, C*, n * frames * sizeof(C), 6);
+    FftOpts rows = opts;
+    rows.in_mul = InMul();
+    const int rc = fft_exec<T>(in, y, n, frames, rows, nullptr, 0, stream);
+    if (rc) return rc;
+    const T* win = nullptr;
+    if (opts.in_mul.kind == 3) {
+        BDSP_WS(tab, T*, n * sizeof(T), 3);
+        window_table_kernel<T><<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(tab, (long long)n, opts.in_mul.arg);
+        BDSP_LAUNCHED();
+        win = tab;
+    }
+    const long long len = (long long)((frames - 1) * hop + n);
+    const unsigned grid = (unsigned)((len + 255) / 256);
+    if (real_out) overlap_add_kernel<T, true><<<grid, 256, 0, stream>>>(y, win, out, (long long)n, (long long)hop, (long long)frames, len);
+    else overlap_add_kernel<T, false><<<grid, 256, 0, stream>>>(y, win, out, (long long)n, (long long)hop, (long long)frames, len);
+    BDSP_LAUNCHED();
+    return 0;
+}
+
+template int ifft_frames_exec<float>(const void*, void*, size_t, size_t, size_t, const FftOpts&, bool, cudaStream_t);
+template int ifft_frames_exec<double>(const void*, void*, size_t, size_t, size_t, const FftOpts&, bool, cudaStream_t);
 
 }  // namespace bdsp

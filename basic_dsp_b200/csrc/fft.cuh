@@ -27,6 +27,15 @@ template <typename T>
 int fft_exec(const void* in, void* out, size_t n, size_t batch, const FftOpts& opts, void* work,
              size_t work_bytes, cudaStream_t stream);
 
+// Inverse short-time transform: the inverse transforms of `frames` spectra of n points (back to back in `in`) under `opts`
+// (inverse, scale, in_rot), then their least-squares overlap-add at `hop` points apart into (frames-1)*hop + n points of
+// `out`: out[t] = sum_f w[t-f*hop] y_f[t-f*hop] / sum_f w[t-f*hop]^2.  opts.in_mul (kind 3, a built-in window, or none) is the
+// synthesis window w, applied in the overlap-add rather than on the transform's load.  real_out: `out` holds the real parts
+// as scalars.  Needs hop <= n, so that a frame covers every point, and `out` apart from `in`.  Returns 0 or a negative error.
+template <typename T>
+int ifft_frames_exec(const void* in, void* out, size_t n, size_t hop, size_t frames, const FftOpts& opts, bool real_out,
+                     cudaStream_t stream);
+
 // largest n the single-CTA shared-memory kernel handles for this precision
 template <typename T> size_t fft_block_max_n();
 

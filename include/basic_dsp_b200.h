@@ -520,6 +520,21 @@ int32_t bdsp_fft_rows_c64(const void* in, void* out, size_t points, size_t rows,
  * points == 0 or frames == 0 returns 0 without a launch. */
 int32_t bdsp_fft_frames_c32(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
 int32_t bdsp_fft_frames_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
+#define BDSP_F_REAL_OUTPUT 16 /* bdsp_ifft_frames_*: out holds real scalars, the real part of the synthesis */
+/* The inverse of bdsp_fft_frames_*: a signal from the spectra of its overlapping frames (inverse short-time Fourier
+ * transform).  `in` holds `frames` rows of `points` complex spectra back to back (what bdsp_fft_frames_* writes without
+ * BDSP_F_MAGNITUDE); `out` receives len = (frames-1)*hop + points points, complex or, with BDSP_F_REAL_OUTPUT, the real
+ * parts as scalars (the imaginary parts are dropped, Hermitian symmetry is not checked).  Weighted overlap-add with
+ * least-squares normalisation, as torch.istft(center=False) and scipy.signal.istft:
+ *   y_f = ifft(X_f) / points (BDSP_F_SHIFT: X_f ifft-shifted first, the inverse of the forward call's BDSP_F_SHIFT),
+ *   out[t] = sum_f w[t-f*hop] y_f[t-f*hop] / sum_f w[t-f*hop]^2 over the frames that cover t,
+ * w = the built-in window BDSP_F_WINDOW(kind), or 1 without it (out[t] = the mean of the frames that cover t).  So
+ * bdsp_ifft_frames(bdsp_fft_frames(x, W), W) returns x within rounding for every hop <= points.
+ * flags: BDSP_F_SHIFT, BDSP_F_REAL_OUTPUT, BDSP_F_WINDOW(kind).  Returns 0; -2 for any other flag (bdsp_last_error names
+ * it), hop == 0, hop > points (samples that no frame covers) or sizes that overflow size_t; -3 when the output range and
+ * the input range overlap.  points == 0 or frames == 0 returns 0 without a launch. */
+int32_t bdsp_ifft_frames_c32(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
+int32_t bdsp_ifft_frames_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
 /* convolve_signal for every row with one impulse response of h_points complex taps (device pointer);
  * `plan` caches the impulse-response spectrum between calls (create once, reuse, destroy) */
 typedef struct BdspConvPlan BdspConvPlan;
