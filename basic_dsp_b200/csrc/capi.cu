@@ -1469,10 +1469,10 @@ template <typename R, typename T> static inline R as_res(Res<T> r) {
     extern "C" RES diff##S(HV* v) { return as_res<RES>(op_diff<T>(VEC(v), false)); }                                   \
     extern "C" RES diff_with_start##S(HV* v) { return as_res<RES>(op_diff<T>(VEC(v), true)); }                         \
     extern "C" RES cum_sum##S(HV* v) { return as_res<RES>(op_cum_sum<T>(VEC(v))); }                                    \
-    extern "C" RES add_smaller_vector##S(HV* v, const HV* o) { return as_res<RES>(op_binary_smaller<T>(VEC(v), CVEC(o), 0)); } \
-    extern "C" RES sub_smaller_vector##S(HV* v, const HV* o) { return as_res<RES>(op_binary_smaller<T>(VEC(v), CVEC(o), 1)); } \
-    extern "C" RES mul_smaller_vector##S(HV* v, const HV* o) { return as_res<RES>(op_binary_smaller<T>(VEC(v), CVEC(o), 2)); } \
-    extern "C" RES div_smaller_vector##S(HV* v, const HV* o) { return as_res<RES>(op_binary_smaller<T>(VEC(v), CVEC(o), 3)); } \
+    extern "C" RES add_smaller_vector##S(HV* v, const HV* o) { return as_res<RES>(op_binary_smaller<T>(VEC(v), CVEC(o), EW_ADD)); } \
+    extern "C" RES sub_smaller_vector##S(HV* v, const HV* o) { return as_res<RES>(op_binary_smaller<T>(VEC(v), CVEC(o), EW_SUB)); } \
+    extern "C" RES mul_smaller_vector##S(HV* v, const HV* o) { return as_res<RES>(op_binary_smaller<T>(VEC(v), CVEC(o), EW_MUL)); } \
+    extern "C" RES div_smaller_vector##S(HV* v, const HV* o) { return as_res<RES>(op_binary_smaller<T>(VEC(v), CVEC(o), EW_DIV)); } \
     extern "C" int32_t get_real_imag##S(HV* v, HV* re, HV* im) { return op_get_real_imag<T>(VEC(v), VEC(re), VEC(im)); } \
     extern "C" RES set_real_imag##S(HV* v, const HV* re, const HV* im) { return as_res<RES>(op_set_pair<T>(VEC(v), CVEC(re), CVEC(im), false)); } \
     extern "C" RES set_mag_phase##S(HV* v, const HV* m, const HV* p) { return as_res<RES>(op_set_pair<T>(VEC(v), CVEC(m), CVEC(p), true)); } \

@@ -60,18 +60,32 @@ template <typename C> __device__ __forceinline__ C cmul(C a, C b) {
 }
 template <typename C> __device__ __forceinline__ C cconj(C a) { a.y = -a.y; return a; }
 
-// exact-rounding product (ac-bd, ad+bc): every operation individually rounded, no FMA.  This is
-// what the reference's CPU path computes (num-complex Mul, simd_extensions/fallback.rs:195-203).
-__device__ __forceinline__ float2 cmul_nofma(float2 a, float2 b) {
-    float2 r;
-    r.x = __fsub_rn(__fmul_rn(a.x, b.x), __fmul_rn(a.y, b.y));
-    r.y = __fadd_rn(__fmul_rn(a.x, b.y), __fmul_rn(a.y, b.x));
+// --- the reference's CPU arithmetic: every product, sum, difference and quotient rounded on its own (no FMA contraction),
+// so that elementwise results follow the reference operation by operation --------------------------------------------
+__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+__device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ float sub_rn(float a, float b) { return __fsub_rn(a, b); }
+__device__ __forceinline__ double sub_rn(double a, double b) { return __dsub_rn(a, b); }
+__device__ __forceinline__ float div_rn(float a, float b) { return __fdiv_rn(a, b); }
+__device__ __forceinline__ double div_rn(double a, double b) { return __ddiv_rn(a, b); }
+
+// num-complex Mul (ac-bd, ad+bc) in that arithmetic (simd_extensions/fallback.rs:195-203)
+template <typename C> __device__ __forceinline__ C cmul_nofma(C a, C b) {
+    C r;
+    r.x = sub_rn(mul_rn(a.x, b.x), mul_rn(a.y, b.y));
+    r.y = add_rn(mul_rn(a.x, b.y), mul_rn(a.y, b.x));
     return r;
 }
-__device__ __forceinline__ double2 cmul_nofma(double2 a, double2 b) {
-    double2 r;
-    r.x = __dsub_rn(__dmul_rn(a.x, b.x), __dmul_rn(a.y, b.y));
-    r.y = __dadd_rn(__dmul_rn(a.x, b.y), __dmul_rn(a.y, b.x));
+// num-complex Div (a * conj(b)) / |b|^2 in that arithmetic
+template <typename C> __device__ __forceinline__ C cdiv_nofma(C a, C b) {
+    const auto ns = add_rn(mul_rn(b.x, b.x), mul_rn(b.y, b.y));
+    const auto re = add_rn(mul_rn(a.x, b.x), mul_rn(a.y, b.y));
+    const auto im = sub_rn(mul_rn(a.y, b.x), mul_rn(a.x, b.y));
+    C r;
+    r.x = div_rn(re, ns);
+    r.y = div_rn(im, ns);
     return r;
 }
 
@@ -143,6 +157,25 @@ __device__ __forceinline__ typename CpxOf<T>::type unit_root(unsigned long long 
     return mk<T>(c, sign < 0 ? -s : s);
 }
 
+int sm_count();
+
+// grid-stride kernels: blocks of 256 threads for `items` work items, one item per thread up to 16 blocks per SM
+constexpr int GRID_STRIDE_THREADS = 256;
+inline unsigned grid_stride_blocks(long long items) {
+    long long g = (items + GRID_STRIDE_THREADS - 1) / GRID_STRIDE_THREADS;
+    const long long cap = (long long)sm_count() * 16;
+    if (g > cap) g = cap;
+    if (g < 1) g = 1;
+    return (unsigned)g;
+}
+// launches a grid-stride kernel over `items` work items on `st` and counts the launch
+template <typename... KArgs, typename... Args>
+inline int launch_grid_stride(void (*kernel)(KArgs...), long long items, cudaStream_t st, Args... args) {
+    kernel<<<grid_stride_blocks(items), GRID_STRIDE_THREADS, 0, st>>>(args...);
+    BDSP_LAUNCHED();
+    return 0;
+}
+
 static inline int ilog2(size_t v) {
     int l = 0;
     while ((1ull << (l + 1)) <= v) l++;
@@ -154,7 +187,5 @@ static inline size_t next_pow2(size_t v) {
     while (p < v) p <<= 1;
     return p;
 }
-
-int sm_count();
 
 }  // namespace bdsp

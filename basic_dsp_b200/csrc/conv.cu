@@ -15,6 +15,7 @@
 #include <vector>
 
 #include "conv.cuh"
+#include "elementwise.cuh"
 #include "fft.cuh"
 #include "fft_core.cuh"
 #include "olsi.cuh"
@@ -385,27 +386,6 @@ __global__ void pad_roll_h_kernel(const void* __restrict__ h_, typename CpxOf<T>
 }
 
 template <typename T>
-__global__ void spectrum_mul_kernel(typename CpxOf<T>::type* __restrict__ X, const typename CpxOf<T>::type* __restrict__ H,
-                                    long long N, long long batch, T scale) {
-    long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (gid >= N * batch) return;
-    typename CpxOf<T>::type v = cmul(X[gid], H[gid % N]);
-    v.x *= scale; v.y *= scale;
-    X[gid] = v;
-}
-
-template <typename T>
-__global__ void real_to_complex_kernel(const T* __restrict__ in, typename CpxOf<T>::type* __restrict__ out, long long n) {
-    long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (gid < n) out[gid] = mk<T>(in[gid], (T)0);
-}
-template <typename T>
-__global__ void complex_to_real_kernel(const typename CpxOf<T>::type* __restrict__ in, T* __restrict__ out, long long n) {
-    long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (gid < n) out[gid] = in[gid].x;
-}
-
-template <typename T>
 static int fft_convolve_full(const void* x, void* y, const void* h, size_t N, size_t batch, size_t L, int is_real,
                              int h_is_real, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
@@ -422,15 +402,14 @@ static int fft_convolve_full(const void* x, void* y, const void* h, size_t N, si
     fx.real_input = is_real;
     rc = fft_exec<T>(x, X, N, batch, fx, nullptr, 0, st);
     if (rc) return rc;
-    const long long tot = (long long)(N * batch);
     // spectrum multiply (convolution.rs:427-429,444-446) and the 1/N of the inverse: fused into the first load of the
     // inverse transform (FftOpts::in_mul) wherever that transform carries a multiplier - every length except c32 powers of
     // two up to 16384, whose packed single-pass kernels keep the separate pass
     FftOpts inv;
     inv.inverse = 1;
     if (sizeof(T) == 4 && is_pow2(N) && N >= 64 && N <= 16384) {
-        spectrum_mul_kernel<T><<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(X, Hf, (long long)N, (long long)batch, (T)(1.0 / (double)N));
-        BDSP_LAUNCHED();
+        rc = ew_spectrum_mul_rows<T>(X, Hf, N, batch, 1.0 / (double)N, st);
+        if (rc) return rc;
     } else {
         inv.in_mul.p = Hf; inv.in_mul.kind = 2;
         inv.scale = 1.0 / (double)N;
@@ -438,9 +417,7 @@ static int fft_convolve_full(const void* x, void* y, const void* h, size_t N, si
     if (!is_real) return fft_exec<T>(X, y, N, batch, inv, nullptr, 0, st);
     rc = fft_exec<T>(X, X, N, batch, inv, nullptr, 0, st);
     if (rc) return rc;
-    complex_to_real_kernel<T><<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(X, reinterpret_cast<T*>(y), tot);
-    BDSP_LAUNCHED();
-    return 0;
+    return ew_complex_to_real<T>(C2R_REAL, X, y, N * batch, st);
 }
 
 // Choice between the two fused block lengths where both apply (2 <= L <= 2046).  Measured on B200, 64 x 2^20 points

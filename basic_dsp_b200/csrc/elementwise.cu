@@ -3,50 +3,25 @@
 //
 // Reference: vector/src/vector_types/general/elementary.rs:283-360,420-455,540-589 and
 // vector/src/vector_types/complex/complex_to_real.rs:374-478,595-712.  Arithmetic follows the
-// reference's CPU path operation by operation (no FMA contraction: __fmul_rn/__fadd_rn), so results
+// reference's CPU path operation by operation (no FMA contraction: mul_rn/add_rn of common.cuh), so results
 // are within the 4-ulp budget of BASELINE.json (bit-identical for the ring operations).
 // All kernels are grid-stride, 16 B per thread per access where alignment allows.
 #include "elementwise.cuh"
 
 namespace bdsp {
 
-template <typename T> struct Arith;
-template <> struct Arith<float> {
-    static __device__ __forceinline__ float mul(float a, float b) { return __fmul_rn(a, b); }
-    static __device__ __forceinline__ float add(float a, float b) { return __fadd_rn(a, b); }
-    static __device__ __forceinline__ float sub(float a, float b) { return __fsub_rn(a, b); }
-    static __device__ __forceinline__ float div(float a, float b) { return __fdiv_rn(a, b); }
-    static __device__ __forceinline__ float sqrt_(float a) { return __fsqrt_rn(a); }
-    static __device__ __forceinline__ float hypot_(float a, float b) { return hypotf(a, b); }
-    static __device__ __forceinline__ float atan2_(float a, float b) { return atan2f(a, b); }
-};
-template <> struct Arith<double> {
-    static __device__ __forceinline__ double mul(double a, double b) { return __dmul_rn(a, b); }
-    static __device__ __forceinline__ double add(double a, double b) { return __dadd_rn(a, b); }
-    static __device__ __forceinline__ double sub(double a, double b) { return __dsub_rn(a, b); }
-    static __device__ __forceinline__ double div(double a, double b) { return __ddiv_rn(a, b); }
-    static __device__ __forceinline__ double sqrt_(double a) { return __dsqrt_rn(a); }
-    static __device__ __forceinline__ double hypot_(double a, double b) { return hypot(a, b); }
-    static __device__ __forceinline__ double atan2_(double a, double b) { return atan2(a, b); }
-};
-
-static inline unsigned ew_grid(long long work_items, int threads) {
-    long long g = (work_items + threads - 1) / threads;
-    long long cap = (long long)sm_count() * 16;
-    if (g > cap) g = cap;
-    if (g < 1) g = 1;
-    return (unsigned)g;
-}
+// correctly rounded square root in T (norm and argument: the float / double overloads of hypot and atan2)
+__device__ __forceinline__ float sqrt_rn(float a) { return __fsqrt_rn(a); }
+__device__ __forceinline__ double sqrt_rn(double a) { return __dsqrt_rn(a); }
 
 // ---- unary ops on T scalars (real scale / offset) ------------------------------------------------
 template <typename T, int OP>
 __global__ void scalar_op_kernel(const T* __restrict__ in, T* __restrict__ out, long long n, T c) {
-    typedef Arith<T> A;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (; i < n; i += stride) {
         T v = in[i];
-        out[i] = OP == EW_SCALE ? A::mul(v, c) : A::add(v, c);
+        out[i] = OP == EW_SCALE ? mul_rn(v, c) : add_rn(v, c);
     }
 }
 
@@ -55,14 +30,13 @@ template <typename T, int OP>
 __global__ void complex_const_kernel(const typename CpxOf<T>::type* __restrict__ in,
                                      typename CpxOf<T>::type* __restrict__ out, long long n, T cre, T cim) {
     typedef typename CpxOf<T>::type C;
-    typedef Arith<T> A;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
     const C c = mk<T>(cre, cim);
     for (; i < n; i += stride) {
         C v = in[i];
         if (OP == EW_SCALE) v = cmul_nofma(v, c);
-        else if (OP == EW_OFFSET) { v.x = A::add(v.x, cre); v.y = A::add(v.y, cim); }
+        else if (OP == EW_OFFSET) { v.x = add_rn(v.x, cre); v.y = add_rn(v.y, cim); }
         else if (OP == EW_CONJ) v.y = -v.y;
         out[i] = v;
     }
@@ -71,48 +45,26 @@ __global__ void complex_const_kernel(const typename CpxOf<T>::type* __restrict__
 // ---- binary vector ops --------------------------------------------------------------------------------
 template <typename T, int OP>
 __global__ void binary_real_kernel(const T* __restrict__ a, const T* __restrict__ b, T* __restrict__ out, long long n) {
-    typedef Arith<T> A;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
-    for (; i < n; i += stride) {
-        T x = a[i], y = b[i], r;
-        if (OP == EW_ADD) r = A::add(x, y);
-        else if (OP == EW_SUB) r = A::sub(x, y);
-        else if (OP == EW_MUL) r = A::mul(x, y);
-        else r = A::div(x, y);
-        out[i] = r;
-    }
-}
-
-template <typename T> __device__ __forceinline__ typename CpxOf<T>::type cdiv_ref(typename CpxOf<T>::type a, typename CpxOf<T>::type b) {
-    // num-complex Div: (a * conj(b)) / |b|^2, component-wise, no FMA
-    typedef Arith<T> A;
-    T ns = A::add(A::mul(b.x, b.x), A::mul(b.y, b.y));
-    T re = A::add(A::mul(a.x, b.x), A::mul(a.y, b.y));
-    T im = A::sub(A::mul(a.y, b.x), A::mul(a.x, b.y));
-    return mk<T>(A::div(re, ns), A::div(im, ns));
+    for (; i < n; i += stride) out[i] = ew_real_op<OP>(a[i], b[i]);
 }
 
 template <typename T, int OP>
 __global__ void binary_complex_kernel(const typename CpxOf<T>::type* __restrict__ a,
                                       const typename CpxOf<T>::type* __restrict__ b,
                                       typename CpxOf<T>::type* __restrict__ out, long long n) {
-    typedef typename CpxOf<T>::type C;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
-    for (; i < n; i += stride) {
-        C x = a[i], y = b[i];
-        out[i] = OP == EW_MUL ? cmul_nofma(x, y) : cdiv_ref<T>(x, y);
-    }
+    for (; i < n; i += stride) out[i] = ew_complex_op<OP>(a[i], b[i]);
 }
 
 // ---- complex -> real ------------------------------------------------------------------------------------
 template <typename T, int OP> __device__ __forceinline__ T c2r(typename CpxOf<T>::type v) {
-    typedef Arith<T> A;
-    if (OP == C2R_MAG_HYPOT) return A::hypot_(v.x, v.y);
-    if (OP == C2R_MAG_SQRT) return A::sqrt_(A::add(A::mul(v.x, v.x), A::mul(v.y, v.y)));
-    if (OP == C2R_MAG_SQ) return A::add(A::mul(v.x, v.x), A::mul(v.y, v.y));
-    if (OP == C2R_PHASE) return A::atan2_(v.y, v.x);
+    if (OP == C2R_MAG_HYPOT) return hypot(v.x, v.y);
+    if (OP == C2R_MAG_SQRT) return sqrt_rn(add_rn(mul_rn(v.x, v.x), mul_rn(v.y, v.y)));
+    if (OP == C2R_MAG_SQ) return add_rn(mul_rn(v.x, v.x), mul_rn(v.y, v.y));
+    if (OP == C2R_PHASE) return atan2(v.y, v.x);
     if (OP == C2R_REAL) return v.x;
     return v.y;
 }
@@ -131,13 +83,12 @@ __global__ void complex_to_real_kernel(const typename CpxOf<T>::type* __restrict
 
 template <typename T>
 __global__ void mag_phase_kernel(const typename CpxOf<T>::type* __restrict__ in, T* __restrict__ mag, T* __restrict__ ph, long long n) {
-    typedef Arith<T> A;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (; i < n; i += stride) {
         typename CpxOf<T>::type v = in[i];
-        mag[i] = A::hypot_(v.x, v.y);   // Complex::to_polar = (norm, arg), complex_to_real.rs:707
-        ph[i] = A::atan2_(v.y, v.x);
+        mag[i] = hypot(v.x, v.y);   // Complex::to_polar = (norm, arg), complex_to_real.rs:707
+        ph[i] = atan2(v.y, v.x);
     }
 }
 
@@ -147,18 +98,17 @@ template <typename T, bool WRITE_V>
 __global__ void scale_mul_mag_phase_kernel(typename CpxOf<T>::type* __restrict__ v, const typename CpxOf<T>::type* __restrict__ w,
                                            T* __restrict__ mag, T* __restrict__ ph, long long n, T cre, T cim, int complex_scale) {
     typedef typename CpxOf<T>::type C;
-    typedef Arith<T> A;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
     const C c = mk<T>(cre, cim);
     for (; i < n; i += stride) {
         C x = v[i];
         if (complex_scale) x = cmul_nofma(x, c);
-        else { x.x = A::mul(x.x, cre); x.y = A::mul(x.y, cre); }
+        else { x.x = mul_rn(x.x, cre); x.y = mul_rn(x.y, cre); }
         x = cmul_nofma(x, w[i]);
         if (WRITE_V) v[i] = x;
-        mag[i] = A::hypot_(x.x, x.y);
-        ph[i] = A::atan2_(x.y, x.x);
+        mag[i] = hypot(x.x, x.y);
+        ph[i] = atan2(x.y, x.x);
     }
 }
 
@@ -224,14 +174,13 @@ __global__ void fill_kernel(T* __restrict__ out, long long n, T v) {
 // conv_types.rs:434-449,498-505): X[i] *= ratio * f((j/max) * ratio), j = i - (points - points%2)/2
 template <typename T>
 __global__ void mul_freq_resp_kernel(T* __restrict__ data, long long points, int is_complex, int kind, T rolloff, T ratio) {
-    typedef Arith<T> A;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
     const long long offset = points % 2;
     const T mx = (T)(points - offset) / (T)2;
     for (; i < points; i += stride) {
-        T j = A::add(-mx, (T)i);
-        T x = A::mul(A::div(j, mx), ratio);
+        T j = add_rn(-mx, (T)i);
+        T x = mul_rn(div_rn(j, mx), ratio);
         T ax = fabs(x);
         T f;
         if (kind == 0) f = ax <= (T)1 ? (T)1 : (T)0;
@@ -248,7 +197,7 @@ __global__ void mul_freq_resp_kernel(T* __restrict__ data, long long points, int
             v = cmul_nofma(v, mk<T>(f, (T)0));
             reinterpret_cast<typename CpxOf<T>::type*>(data)[i] = v;
         } else {
-            data[i] = A::mul(A::mul(data[i], ratio), f);
+            data[i] = mul_rn(mul_rn(data[i], ratio), f);
         }
     }
 }
@@ -258,24 +207,22 @@ __global__ void mul_freq_resp_kernel(T* __restrict__ data, long long points, int
 // evaluated for the first half and mirrored, vector_types/mod.rs:528-598), evaluated on the device in precision T
 template <typename T>
 __global__ void window_kernel(T* __restrict__ data, long long points, int is_complex, int kind, int unapply) {
-    typedef Arith<T> A;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (; i < points; i += stride) {
         const long long j = i < (points + 1) / 2 ? i : points - 1 - i;
         T w = window_value_dev<T>(kind, j, points);
-        if (unapply) w = A::div((T)1, w);
+        if (unapply) w = div_rn((T)1, w);
         if (is_complex) {
             typedef typename CpxOf<T>::type C;
             reinterpret_cast<C*>(data)[i] = cmul_nofma(reinterpret_cast<C*>(data)[i], mk<T>(w, (T)0));
-        } else data[i] = A::mul(data[i], w);
+        } else data[i] = mul_rn(data[i], w);
     }
 }
 
 // X[i] *= table[i] (complex or real table) - host-evaluated custom responses / windows
 template <typename T>
 __global__ void mul_table_kernel(T* __restrict__ data, const T* __restrict__ table, long long points, int is_complex, int table_complex) {
-    typedef Arith<T> A;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (; i < points; i += stride) {
@@ -284,7 +231,7 @@ __global__ void mul_table_kernel(T* __restrict__ data, const T* __restrict__ tab
             C v = reinterpret_cast<C*>(data)[i];
             C t = table_complex ? reinterpret_cast<const C*>(table)[i] : mk<T>(table[i], (T)0);
             reinterpret_cast<C*>(data)[i] = cmul_nofma(v, t);
-        } else data[i] = A::mul(data[i], table[i]);
+        } else data[i] = mul_rn(data[i], table[i]);
     }
 }
 
@@ -329,7 +276,6 @@ __global__ void resample_spectrum_kernel(const typename CpxOf<T>::type* __restri
                                          long long n, long long dest, const T* __restrict__ table, T scale, int use_scale,
                                          double phase_inc, int use_phase, int resp_kind, T resp_rolloff, T resp_ratio) {
     typedef typename CpxOf<T>::type C;
-    typedef Arith<T> A;
     long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (; k < dest; k += stride) {
@@ -352,7 +298,7 @@ __global__ void resample_spectrum_kernel(const typename CpxOf<T>::type* __restri
             }
             if (table) { const T w = table[k]; v = cmul_nofma(v, mk<T>(w, (T)0)); }
             else if (resp_kind >= 0) v = cmul_nofma(v, mk<T>(shifted_resp_dev<T>(k, dest, resp_kind, resp_rolloff, resp_ratio), (T)0));
-            if (use_scale) { v.x = A::mul(v.x, scale); v.y = A::mul(v.y, scale); }
+            if (use_scale) { v.x = mul_rn(v.x, scale); v.y = mul_rn(v.y, scale); }
         }
         out[k] = v;
     }
@@ -383,177 +329,174 @@ __global__ void mul_cexp_kernel(typename CpxOf<T>::type* __restrict__ data, long
     }
 }
 
+// spectrum product of a fast convolution over rows: a[r * M + i] = a[r * M + i] * bspec[i] * scale.  Contraction allowed,
+// as in the transforms around it; one thread per point.
+template <typename T>
+__global__ void spectrum_mul_rows_kernel(typename CpxOf<T>::type* __restrict__ a,
+                                         const typename CpxOf<T>::type* __restrict__ bspec, long long M,
+                                         long long batch, T scale) {
+    typedef typename CpxOf<T>::type C;
+    long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= M * batch) return;
+    C v = cmul(a[gid], bspec[gid % M]);
+    v.x *= scale; v.y *= scale;
+    a[gid] = v;
+}
+
 // ------------------------------------------------------------------------------------------
 // host wrappers
 // ------------------------------------------------------------------------------------------
 template <typename T>
 int ew_scalar(int op, const void* in, void* out, size_t n_scalars, double c, cudaStream_t st) {
     const T* i = reinterpret_cast<const T*>(in); T* o = reinterpret_cast<T*>(out);
-    unsigned g = ew_grid((long long)n_scalars, 256);
-    if (op == EW_SCALE) scalar_op_kernel<T, EW_SCALE><<<g, 256, 0, st>>>(i, o, (long long)n_scalars, (T)c);
-    else scalar_op_kernel<T, EW_OFFSET><<<g, 256, 0, st>>>(i, o, (long long)n_scalars, (T)c);
-    BDSP_LAUNCHED();
-    return 0;
+    const long long n = (long long)n_scalars;
+    if (op == EW_SCALE) return launch_grid_stride(scalar_op_kernel<T, EW_SCALE>, n, st, i, o, n, (T)c);
+    return launch_grid_stride(scalar_op_kernel<T, EW_OFFSET>, n, st, i, o, n, (T)c);
 }
 
 template <typename T>
 int ew_complex_const(int op, const void* in, void* out, size_t points, double re, double im, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
     const C* i = reinterpret_cast<const C*>(in); C* o = reinterpret_cast<C*>(out);
-    unsigned g = ew_grid((long long)points, 256);
-    if (op == EW_SCALE) complex_const_kernel<T, EW_SCALE><<<g, 256, 0, st>>>(i, o, (long long)points, (T)re, (T)im);
-    else if (op == EW_OFFSET) complex_const_kernel<T, EW_OFFSET><<<g, 256, 0, st>>>(i, o, (long long)points, (T)re, (T)im);
-    else complex_const_kernel<T, EW_CONJ><<<g, 256, 0, st>>>(i, o, (long long)points, (T)re, (T)im);
-    BDSP_LAUNCHED();
-    return 0;
+    const long long n = (long long)points;
+    if (op == EW_SCALE) return launch_grid_stride(complex_const_kernel<T, EW_SCALE>, n, st, i, o, n, (T)re, (T)im);
+    if (op == EW_OFFSET) return launch_grid_stride(complex_const_kernel<T, EW_OFFSET>, n, st, i, o, n, (T)re, (T)im);
+    return launch_grid_stride(complex_const_kernel<T, EW_CONJ>, n, st, i, o, n, (T)re, (T)im);
 }
 
 template <typename T>
 int ew_binary(int op, const void* a, const void* b, void* out, size_t n_scalars, int is_complex, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
     if (is_complex && (op == EW_MUL || op == EW_DIV)) {
-        unsigned g = ew_grid((long long)(n_scalars / 2), 256);
-        if (op == EW_MUL) binary_complex_kernel<T, EW_MUL><<<g, 256, 0, st>>>(reinterpret_cast<const C*>(a), reinterpret_cast<const C*>(b), reinterpret_cast<C*>(out), (long long)(n_scalars / 2));
-        else binary_complex_kernel<T, EW_DIV><<<g, 256, 0, st>>>(reinterpret_cast<const C*>(a), reinterpret_cast<const C*>(b), reinterpret_cast<C*>(out), (long long)(n_scalars / 2));
-    } else {
-        const T* x = reinterpret_cast<const T*>(a); const T* y = reinterpret_cast<const T*>(b); T* o = reinterpret_cast<T*>(out);
-        unsigned g = ew_grid((long long)n_scalars, 256);
-        if (op == EW_ADD) binary_real_kernel<T, EW_ADD><<<g, 256, 0, st>>>(x, y, o, (long long)n_scalars);
-        else if (op == EW_SUB) binary_real_kernel<T, EW_SUB><<<g, 256, 0, st>>>(x, y, o, (long long)n_scalars);
-        else if (op == EW_MUL) binary_real_kernel<T, EW_MUL><<<g, 256, 0, st>>>(x, y, o, (long long)n_scalars);
-        else binary_real_kernel<T, EW_DIV><<<g, 256, 0, st>>>(x, y, o, (long long)n_scalars);
+        const C* x = reinterpret_cast<const C*>(a); const C* y = reinterpret_cast<const C*>(b); C* o = reinterpret_cast<C*>(out);
+        const long long n = (long long)(n_scalars / 2);
+        if (op == EW_MUL) return launch_grid_stride(binary_complex_kernel<T, EW_MUL>, n, st, x, y, o, n);
+        return launch_grid_stride(binary_complex_kernel<T, EW_DIV>, n, st, x, y, o, n);
     }
-    BDSP_LAUNCHED();
-    return 0;
+    // complex add / sub are the real ops on the interleaved scalars
+    const T* x = reinterpret_cast<const T*>(a); const T* y = reinterpret_cast<const T*>(b); T* o = reinterpret_cast<T*>(out);
+    const long long n = (long long)n_scalars;
+    if (op == EW_ADD) return launch_grid_stride(binary_real_kernel<T, EW_ADD>, n, st, x, y, o, n);
+    if (op == EW_SUB) return launch_grid_stride(binary_real_kernel<T, EW_SUB>, n, st, x, y, o, n);
+    if (op == EW_MUL) return launch_grid_stride(binary_real_kernel<T, EW_MUL>, n, st, x, y, o, n);
+    return launch_grid_stride(binary_real_kernel<T, EW_DIV>, n, st, x, y, o, n);
 }
 
 template <typename T>
 int ew_complex_to_real(int op, const void* in, void* out, size_t points, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
     const C* i = reinterpret_cast<const C*>(in); T* o = reinterpret_cast<T*>(out);
-    unsigned g = ew_grid((long long)points, 256);
     const long long n = (long long)points;
     switch (op) {
-        case C2R_MAG_HYPOT: complex_to_real_kernel<T, C2R_MAG_HYPOT><<<g, 256, 0, st>>>(i, o, n); break;
-        case C2R_MAG_SQRT: complex_to_real_kernel<T, C2R_MAG_SQRT><<<g, 256, 0, st>>>(i, o, n); break;
-        case C2R_MAG_SQ: complex_to_real_kernel<T, C2R_MAG_SQ><<<g, 256, 0, st>>>(i, o, n); break;
-        case C2R_PHASE: complex_to_real_kernel<T, C2R_PHASE><<<g, 256, 0, st>>>(i, o, n); break;
-        case C2R_REAL: complex_to_real_kernel<T, C2R_REAL><<<g, 256, 0, st>>>(i, o, n); break;
-        default: complex_to_real_kernel<T, C2R_IMAG><<<g, 256, 0, st>>>(i, o, n); break;
+        case C2R_MAG_HYPOT: return launch_grid_stride(complex_to_real_kernel<T, C2R_MAG_HYPOT>, n, st, i, o, n);
+        case C2R_MAG_SQRT: return launch_grid_stride(complex_to_real_kernel<T, C2R_MAG_SQRT>, n, st, i, o, n);
+        case C2R_MAG_SQ: return launch_grid_stride(complex_to_real_kernel<T, C2R_MAG_SQ>, n, st, i, o, n);
+        case C2R_PHASE: return launch_grid_stride(complex_to_real_kernel<T, C2R_PHASE>, n, st, i, o, n);
+        case C2R_REAL: return launch_grid_stride(complex_to_real_kernel<T, C2R_REAL>, n, st, i, o, n);
+        default: return launch_grid_stride(complex_to_real_kernel<T, C2R_IMAG>, n, st, i, o, n);
     }
-    BDSP_LAUNCHED();
-    return 0;
 }
 
 template <typename T>
 int ew_mag_phase(const void* in, void* mag, void* phase, size_t points, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
-    mag_phase_kernel<T><<<ew_grid((long long)points, 256), 256, 0, st>>>(reinterpret_cast<const C*>(in), reinterpret_cast<T*>(mag), reinterpret_cast<T*>(phase), (long long)points);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(mag_phase_kernel<T>, (long long)points, st, reinterpret_cast<const C*>(in), reinterpret_cast<T*>(mag),
+                              reinterpret_cast<T*>(phase), (long long)points);
 }
 
 template <typename T>
 int ew_scale_mul_mag_phase(void* v, const void* w, void* mag, void* phase, size_t points, double cre, double cim,
                            int complex_scale, int write_v, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
-    unsigned g = ew_grid((long long)points, 256);
-    if (write_v) scale_mul_mag_phase_kernel<T, true><<<g, 256, 0, st>>>(reinterpret_cast<C*>(v), reinterpret_cast<const C*>(w), reinterpret_cast<T*>(mag), reinterpret_cast<T*>(phase), (long long)points, (T)cre, (T)cim, complex_scale);
-    else scale_mul_mag_phase_kernel<T, false><<<g, 256, 0, st>>>(reinterpret_cast<C*>(v), reinterpret_cast<const C*>(w), reinterpret_cast<T*>(mag), reinterpret_cast<T*>(phase), (long long)points, (T)cre, (T)cim, complex_scale);
-    BDSP_LAUNCHED();
-    return 0;
+    auto run = [&](auto kernel) {
+        return launch_grid_stride(kernel, (long long)points, st, reinterpret_cast<C*>(v), reinterpret_cast<const C*>(w),
+                                  reinterpret_cast<T*>(mag), reinterpret_cast<T*>(phase), (long long)points, (T)cre, (T)cim, complex_scale);
+    };
+    return write_v ? run(scale_mul_mag_phase_kernel<T, true>) : run(scale_mul_mag_phase_kernel<T, false>);
 }
 
 template <typename T>
 int ew_rotate(const void* in, void* out, size_t n_elems, size_t rot, int esz, cudaStream_t st) {
-    rotate_kernel<T><<<ew_grid((long long)(n_elems * esz), 256), 256, 0, st>>>(reinterpret_cast<const T*>(in), reinterpret_cast<T*>(out), (long long)n_elems, (long long)rot, esz);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(rotate_kernel<T>, (long long)(n_elems * esz), st, reinterpret_cast<const T*>(in), reinterpret_cast<T*>(out),
+                              (long long)n_elems, (long long)rot, esz);
 }
 
 template <typename T>
 int ew_zero_interleave(const void* in, void* out, size_t n_elems, int factor, int esz, cudaStream_t st) {
-    zero_interleave_kernel<T><<<ew_grid((long long)(n_elems * factor * esz), 256), 256, 0, st>>>(reinterpret_cast<const T*>(in), reinterpret_cast<T*>(out), (long long)n_elems, factor, esz);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(zero_interleave_kernel<T>, (long long)(n_elems * factor * esz), st, reinterpret_cast<const T*>(in),
+                              reinterpret_cast<T*>(out), (long long)n_elems, factor, esz);
 }
 
 template <typename T> int ew_reverse(const void* in, void* out, size_t n_elems, int esz, cudaStream_t st) {
-    reverse_kernel<T><<<ew_grid((long long)(n_elems * esz), 256), 256, 0, st>>>(reinterpret_cast<const T*>(in), reinterpret_cast<T*>(out), (long long)n_elems, esz);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(reverse_kernel<T>, (long long)(n_elems * esz), st, reinterpret_cast<const T*>(in), reinterpret_cast<T*>(out),
+                              (long long)n_elems, esz);
 }
 
 template <typename T> int ew_decimate(const void* in, void* out, size_t out_elems, size_t factor, size_t delay, int esz, cudaStream_t st) {
-    decimate_kernel<T><<<ew_grid((long long)(out_elems * esz), 256), 256, 0, st>>>(reinterpret_cast<const T*>(in), reinterpret_cast<T*>(out), (long long)out_elems, (long long)factor, (long long)delay, esz);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(decimate_kernel<T>, (long long)(out_elems * esz), st, reinterpret_cast<const T*>(in), reinterpret_cast<T*>(out),
+                              (long long)out_elems, (long long)factor, (long long)delay, esz);
 }
 
 template <typename T> int ew_fill(void* out, size_t n, double v, cudaStream_t st) {
-    fill_kernel<T><<<ew_grid((long long)n, 256), 256, 0, st>>>(reinterpret_cast<T*>(out), (long long)n, (T)v);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(fill_kernel<T>, (long long)n, st, reinterpret_cast<T*>(out), (long long)n, (T)v);
 }
 
 template <typename T>
 int ew_mul_freq_resp(void* data, size_t points, int is_complex, int kind, double rolloff, double ratio, cudaStream_t st) {
-    mul_freq_resp_kernel<T><<<ew_grid((long long)points, 256), 256, 0, st>>>(reinterpret_cast<T*>(data), (long long)points, is_complex, kind, (T)rolloff, (T)ratio);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(mul_freq_resp_kernel<T>, (long long)points, st, reinterpret_cast<T*>(data), (long long)points, is_complex, kind,
+                              (T)rolloff, (T)ratio);
 }
-
 
 template <typename T>
 int ew_window(void* data, size_t points, int is_complex, int kind, int unapply, cudaStream_t st) {
     if (!points) return 0;
-    window_kernel<T><<<ew_grid((long long)points, 256), 256, 0, st>>>(reinterpret_cast<T*>(data), (long long)points, is_complex, kind, unapply);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(window_kernel<T>, (long long)points, st, reinterpret_cast<T*>(data), (long long)points, is_complex, kind, unapply);
 }
 
 template <typename T>
 int ew_mul_table(void* data, const void* table, size_t points, int is_complex, int table_complex, cudaStream_t st) {
-    mul_table_kernel<T><<<ew_grid((long long)points, 256), 256, 0, st>>>(reinterpret_cast<T*>(data), reinterpret_cast<const T*>(table), (long long)points, is_complex, table_complex);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(mul_table_kernel<T>, (long long)points, st, reinterpret_cast<T*>(data), reinterpret_cast<const T*>(table),
+                              (long long)points, is_complex, table_complex);
 }
-
 
 template <typename T>
 int ew_resample_spectrum(const void* in, void* out, size_t n, size_t dest, const void* table, double scale, int use_scale,
                          double phase_inc, int use_phase, int resp_kind, double resp_rolloff, double resp_ratio, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
     if (!dest) return 0;
-    resample_spectrum_kernel<T><<<ew_grid((long long)dest, 256), 256, 0, st>>>(reinterpret_cast<const C*>(in), reinterpret_cast<C*>(out),
-        (long long)n, (long long)dest, reinterpret_cast<const T*>(table), (T)scale, use_scale, phase_inc, use_phase, resp_kind,
-        (T)resp_rolloff, (T)resp_ratio);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(resample_spectrum_kernel<T>, (long long)dest, st, reinterpret_cast<const C*>(in), reinterpret_cast<C*>(out),
+                              (long long)n, (long long)dest, reinterpret_cast<const T*>(table), (T)scale, use_scale, phase_inc, use_phase,
+                              resp_kind, (T)resp_rolloff, (T)resp_ratio);
 }
 
 template <typename T>
 int ew_mul_shifted_resp(void* data, size_t points, int kind, double rolloff, double ratio, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
     if (!points) return 0;
-    mul_shifted_resp_kernel<T><<<ew_grid((long long)points, 256), 256, 0, st>>>(reinterpret_cast<C*>(data), (long long)points, kind, (T)rolloff, (T)ratio);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(mul_shifted_resp_kernel<T>, (long long)points, st, reinterpret_cast<C*>(data), (long long)points, kind,
+                              (T)rolloff, (T)ratio);
 }
 
 template <typename T>
 int ew_mirror(const void* in, void* out, size_t points, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
     if (!points) return 0;
-    mirror_kernel<T><<<ew_grid((long long)(2 * points - 1), 256), 256, 0, st>>>(reinterpret_cast<const C*>(in), reinterpret_cast<C*>(out), (long long)points);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(mirror_kernel<T>, (long long)(2 * points - 1), st, reinterpret_cast<const C*>(in), reinterpret_cast<C*>(out),
+                              (long long)points);
 }
 template <typename T>
 int ew_mul_cexp(void* data, size_t points, double a, double b, cudaStream_t st) {
     typedef typename CpxOf<T>::type C;
     if (!points) return 0;
-    mul_cexp_kernel<T><<<ew_grid((long long)points, 256), 256, 0, st>>>(reinterpret_cast<C*>(data), (long long)points, a, b);
+    return launch_grid_stride(mul_cexp_kernel<T>, (long long)points, st, reinterpret_cast<C*>(data), (long long)points, a, b);
+}
+
+template <typename T>
+int ew_spectrum_mul_rows(void* x, const void* h, size_t n, size_t rows, double scale, cudaStream_t st) {
+    typedef typename CpxOf<T>::type C;
+    const long long tot = (long long)(n * rows);
+    spectrum_mul_rows_kernel<T><<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(reinterpret_cast<C*>(x), reinterpret_cast<const C*>(h),
+                                                                                (long long)n, (long long)rows, (T)scale);
     BDSP_LAUNCHED();
     return 0;
 }
@@ -576,7 +519,8 @@ int ew_mul_cexp(void* data, size_t points, double a, double b, cudaStream_t st) 
     template int ew_decimate<T>(const void*, void*, size_t, size_t, size_t, int, cudaStream_t);           \
     template int ew_mul_freq_resp<T>(void*, size_t, int, int, double, double, cudaStream_t);              \
     template int ew_window<T>(void*, size_t, int, int, int, cudaStream_t);                                \
-    template int ew_mul_table<T>(void*, const void*, size_t, int, int, cudaStream_t);
+    template int ew_mul_table<T>(void*, const void*, size_t, int, int, cudaStream_t);                     \
+    template int ew_spectrum_mul_rows<T>(void*, const void*, size_t, size_t, double, cudaStream_t);
 BDSP_INST(float)
 BDSP_INST(double)
 #undef BDSP_INST

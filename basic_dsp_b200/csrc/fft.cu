@@ -553,18 +553,6 @@ __global__ void bluestein_filter_kernel(typename CpxOf<T>::type* __restrict__ bf
     bfilt[i] = v;
 }
 
-template <typename T>
-__global__ void pointwise_mul_bcast_kernel(typename CpxOf<T>::type* __restrict__ a,
-                                           const typename CpxOf<T>::type* __restrict__ bspec, long long M,
-                                           long long batch, T scale) {
-    typedef typename CpxOf<T>::type C;
-    long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (gid >= M * batch) return;
-    C v = cmul(a[gid], bspec[gid % M]);
-    v.x *= scale; v.y *= scale;
-    a[gid] = v;
-}
-
 template <typename T, bool INV>
 __global__ void bluestein_post_kernel(const typename CpxOf<T>::type* __restrict__ c, void* __restrict__ out_,
                                       long long n, long long M, long long batch, OutMap om, int magnitude) {
@@ -1076,8 +1064,8 @@ int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o,
     InMul fm; fm.p = bspec; fm.kind = 2;
     const bool fused_filter = !(sizeof(T) == 4 && M >= 64 && M <= 16384);
     if (!fused_filter) {
-        pointwise_mul_bcast_kernel<T><<<(unsigned)((totM + 255) / 256), 256, 0, st>>>(b2, bspec, (long long)M, (long long)batch, (T)(1.0 / (double)M));
-        BDSP_LAUNCHED();
+        rc = ew_spectrum_mul_rows<T>(b2, bspec, M, batch, 1.0 / (double)M, st);
+        if (rc) return rc;
     } else {
         fo.in_mul = fm; fo.scale = 1.0 / (double)M;
     }

@@ -240,8 +240,6 @@ int f16_launch(const void* in, void* out, size_t rows, float scale, cudaStream_t
 }
 }  // namespace
 
-int sm_count();
-
 // rows of 16384 c32 points (FftRoute::Packed16k)
 int fftp16k(const void* in, void* out, size_t rows, bool inverse, bool shift_in, bool shift_out, bool magnitude, float scale, cudaStream_t st) {
     return fftp_with_flags<true, true>(inverse, shift_in, shift_out, magnitude, [&](auto inv, auto si, auto so, auto mag) {

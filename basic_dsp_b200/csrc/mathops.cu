@@ -11,115 +11,100 @@
 #include <math_constants.h>
 
 #include "common.cuh"
+#include "elementwise.cuh"
 #include "mathops.cuh"
 
 namespace bdsp {
-int sm_count();
-
 namespace {
 
-template <typename T> struct C2 { T re, im; };
-template <typename T> __device__ __forceinline__ C2<T> mkc(T a, T b) { C2<T> r; r.re = a; r.im = b; return r; }
-
-// individually rounded products / sums (no contraction) so that results follow the reference's
-// operation order
-__device__ __forceinline__ float mul_(float a, float b) { return __fmul_rn(a, b); }
-__device__ __forceinline__ double mul_(double a, double b) { return __dmul_rn(a, b); }
-__device__ __forceinline__ float add_(float a, float b) { return __fadd_rn(a, b); }
-__device__ __forceinline__ double add_(double a, double b) { return __dadd_rn(a, b); }
-__device__ __forceinline__ float sub_(float a, float b) { return __fsub_rn(a, b); }
-__device__ __forceinline__ double sub_(double a, double b) { return __dsub_rn(a, b); }
-__device__ __forceinline__ float div_(float a, float b) { return __fdiv_rn(a, b); }
-__device__ __forceinline__ double div_(double a, double b) { return __ddiv_rn(a, b); }
-
-template <typename T> __device__ __forceinline__ C2<T> c_mul(C2<T> a, C2<T> b) {
-    return mkc(sub_(mul_(a.re, b.re), mul_(a.im, b.im)), add_(mul_(a.re, b.im), mul_(a.im, b.re)));
-}
 __device__ __forceinline__ void sc_(float x, float* s, float* c) { sincosf(x, s, c); }
 __device__ __forceinline__ void sc_(double x, double* s, double* c) { sincos(x, s, c); }
-template <typename T> __device__ __forceinline__ C2<T> c_from_polar(T r, T th) {
+template <typename T> __device__ __forceinline__ typename CpxOf<T>::type c_from_polar(T r, T th) {
     T s, c;
     sc_(th, &s, &c);
-    return mkc(mul_(r, c), mul_(r, s));
+    return mk<T>(mul_rn(r, c), mul_rn(r, s));
 }
-template <typename T> __device__ __forceinline__ C2<T> c_ln(C2<T> a) { return mkc((T)log(hypot(a.re, a.im)), (T)atan2(a.im, a.re)); }
-template <typename T> __device__ __forceinline__ C2<T> c_sqrt(C2<T> a) {
+template <typename T> __device__ __forceinline__ typename CpxOf<T>::type c_ln(typename CpxOf<T>::type a) {
+    return mk<T>((T)log(hypot(a.x, a.y)), (T)atan2(a.y, a.x));
+}
+template <typename T> __device__ __forceinline__ typename CpxOf<T>::type c_sqrt(typename CpxOf<T>::type a) {
     // num-complex Complex::sqrt: exact branches for purely real / purely imaginary input
-    if (a.im == (T)0) {
-        if (!signbit(a.re)) return mkc((T)sqrt(a.re), a.im);
-        const T im = (T)sqrt(-a.re);
-        return mkc((T)0, signbit(a.im) ? -im : im);
+    if (a.y == (T)0) {
+        if (!signbit(a.x)) return mk<T>((T)sqrt(a.x), a.y);
+        const T im = (T)sqrt(-a.x);
+        return mk<T>((T)0, signbit(a.y) ? -im : im);
     }
-    if (a.re == (T)0) {
-        const T x = (T)sqrt(div_((T)fabs(a.im), (T)2));
-        return mkc(x, signbit(a.im) ? -x : x);
+    if (a.x == (T)0) {
+        const T x = (T)sqrt(div_rn((T)fabs(a.y), (T)2));
+        return mk<T>(x, signbit(a.y) ? -x : x);
     }
-    return c_from_polar((T)sqrt(hypot(a.re, a.im)), div_((T)atan2(a.im, a.re), (T)2));
+    return c_from_polar((T)sqrt(hypot(a.x, a.y)), div_rn((T)atan2(a.y, a.x), (T)2));
 }
 
-template <typename T> __device__ C2<T> complex_fn(int op, C2<T> z, T arg, T ln_arg) {
-    const T re = z.re, im = z.im;
+template <typename T> __device__ typename CpxOf<T>::type complex_fn(int op, typename CpxOf<T>::type z, T arg, T ln_arg) {
+    typedef typename CpxOf<T>::type C;
+    const T re = z.x, im = z.y;
     switch (op) {
-    case M_SIN: return mkc(mul_((T)sin(re), (T)cosh(im)), mul_((T)cos(re), (T)sinh(im)));
-    case M_COS: return mkc(mul_((T)cos(re), (T)cosh(im)), mul_(-(T)sin(re), (T)sinh(im)));
+    case M_SIN: return mk<T>(mul_rn((T)sin(re), (T)cosh(im)), mul_rn((T)cos(re), (T)sinh(im)));
+    case M_COS: return mk<T>(mul_rn((T)cos(re), (T)cosh(im)), mul_rn(-(T)sin(re), (T)sinh(im)));
     case M_TAN: {
-        const T tr = add_(re, re), ti = add_(im, im);
-        const T d = add_((T)cos(tr), (T)cosh(ti));
-        return mkc(div_((T)sin(tr), d), div_((T)sinh(ti), d));
+        const T tr = add_rn(re, re), ti = add_rn(im, im);
+        const T d = add_rn((T)cos(tr), (T)cosh(ti));
+        return mk<T>(div_rn((T)sin(tr), d), div_rn((T)sinh(ti), d));
     }
-    case M_SINH: return mkc(mul_((T)sinh(re), (T)cos(im)), mul_((T)cosh(re), (T)sin(im)));
-    case M_COSH: return mkc(mul_((T)cosh(re), (T)cos(im)), mul_((T)sinh(re), (T)sin(im)));
+    case M_SINH: return mk<T>(mul_rn((T)sinh(re), (T)cos(im)), mul_rn((T)cosh(re), (T)sin(im)));
+    case M_COSH: return mk<T>(mul_rn((T)cosh(re), (T)cos(im)), mul_rn((T)sinh(re), (T)sin(im)));
     case M_TANH: {
-        const T tr = add_(re, re), ti = add_(im, im);
-        const T d = add_((T)cosh(tr), (T)cos(ti));
-        return mkc(div_((T)sinh(tr), d), div_((T)sin(ti), d));
+        const T tr = add_rn(re, re), ti = add_rn(im, im);
+        const T d = add_rn((T)cosh(tr), (T)cos(ti));
+        return mk<T>(div_rn((T)sinh(tr), d), div_rn((T)sin(ti), d));
     }
     case M_ASIN: {   // -i ln(sqrt(1 - z^2) + i z)
-        const C2<T> zz = c_mul(z, z);
-        const C2<T> s = c_sqrt(mkc(sub_((T)1, zz.re), sub_((T)0, zz.im)));
-        const C2<T> w = c_ln(mkc(sub_(s.re, im), add_(s.im, re)));
-        return mkc(w.im, -w.re);
+        const C zz = cmul_nofma(z, z);
+        const C s = c_sqrt<T>(mk<T>(sub_rn((T)1, zz.x), sub_rn((T)0, zz.y)));
+        const C w = c_ln<T>(mk<T>(sub_rn(s.x, im), add_rn(s.y, re)));
+        return mk<T>(w.y, -w.x);
     }
     case M_ACOS: {   // -i ln(i sqrt(1 - z^2) + z)
-        const C2<T> zz = c_mul(z, z);
-        const C2<T> s = c_sqrt(mkc(sub_((T)1, zz.re), sub_((T)0, zz.im)));
-        const C2<T> w = c_ln(mkc(add_(-s.im, re), add_(s.re, im)));
-        return mkc(w.im, -w.re);
+        const C zz = cmul_nofma(z, z);
+        const C s = c_sqrt<T>(mk<T>(sub_rn((T)1, zz.x), sub_rn((T)0, zz.y)));
+        const C w = c_ln<T>(mk<T>(add_rn(-s.y, re), add_rn(s.x, im)));
+        return mk<T>(w.y, -w.x);
     }
     case M_ATAN: {   // (ln(1 + i z) - ln(1 - i z)) / (2 i)
-        if (re == (T)0 && im == (T)1) return mkc((T)0, (T)CUDART_INF);
-        if (re == (T)0 && im == (T)-1) return mkc((T)0, -(T)CUDART_INF);
-        const C2<T> a = c_ln(mkc(sub_((T)1, im), add_((T)0, re)));
-        const C2<T> b = c_ln(mkc(add_((T)1, im), sub_((T)0, re)));
-        return mkc(div_(sub_(a.im, b.im), (T)2), -div_(sub_(a.re, b.re), (T)2));
+        if (re == (T)0 && im == (T)1) return mk<T>((T)0, (T)CUDART_INF);
+        if (re == (T)0 && im == (T)-1) return mk<T>((T)0, -(T)CUDART_INF);
+        const C a = c_ln<T>(mk<T>(sub_rn((T)1, im), add_rn((T)0, re)));
+        const C b = c_ln<T>(mk<T>(add_rn((T)1, im), sub_rn((T)0, re)));
+        return mk<T>(div_rn(sub_rn(a.y, b.y), (T)2), -div_rn(sub_rn(a.x, b.x), (T)2));
     }
     case M_ASINH: {  // ln(z + sqrt(1 + z^2))
-        const C2<T> zz = c_mul(z, z);
-        const C2<T> s = c_sqrt(mkc(add_((T)1, zz.re), add_((T)0, zz.im)));
-        return c_ln(mkc(add_(re, s.re), add_(im, s.im)));
+        const C zz = cmul_nofma(z, z);
+        const C s = c_sqrt<T>(mk<T>(add_rn((T)1, zz.x), add_rn((T)0, zz.y)));
+        return c_ln<T>(mk<T>(add_rn(re, s.x), add_rn(im, s.y)));
     }
     case M_ACOSH: {  // 2 ln(sqrt((z + 1) / 2) + sqrt((z - 1) / 2))
-        const C2<T> a = c_sqrt(mkc(div_(add_(re, (T)1), (T)2), div_(im, (T)2)));
-        const C2<T> b = c_sqrt(mkc(div_(sub_(re, (T)1), (T)2), div_(im, (T)2)));
-        const C2<T> w = c_ln(mkc(add_(a.re, b.re), add_(a.im, b.im)));
-        return mkc(mul_((T)2, w.re), mul_((T)2, w.im));
+        const C a = c_sqrt<T>(mk<T>(div_rn(add_rn(re, (T)1), (T)2), div_rn(im, (T)2)));
+        const C b = c_sqrt<T>(mk<T>(div_rn(sub_rn(re, (T)1), (T)2), div_rn(im, (T)2)));
+        const C w = c_ln<T>(mk<T>(add_rn(a.x, b.x), add_rn(a.y, b.y)));
+        return mk<T>(mul_rn((T)2, w.x), mul_rn((T)2, w.y));
     }
     case M_ATANH: {  // (ln(1 + z) - ln(1 - z)) / 2
-        if (re == (T)1 && im == (T)0) return mkc((T)CUDART_INF, (T)0);
-        if (re == (T)-1 && im == (T)0) return mkc(-(T)CUDART_INF, (T)0);
-        const C2<T> a = c_ln(mkc(add_((T)1, re), add_((T)0, im)));
-        const C2<T> b = c_ln(mkc(sub_((T)1, re), sub_((T)0, im)));
-        return mkc(div_(sub_(a.re, b.re), (T)2), div_(sub_(a.im, b.im), (T)2));
+        if (re == (T)1 && im == (T)0) return mk<T>((T)CUDART_INF, (T)0);
+        if (re == (T)-1 && im == (T)0) return mk<T>(-(T)CUDART_INF, (T)0);
+        const C a = c_ln<T>(mk<T>(add_rn((T)1, re), add_rn((T)0, im)));
+        const C b = c_ln<T>(mk<T>(sub_rn((T)1, re), sub_rn((T)0, im)));
+        return mk<T>(div_rn(sub_rn(a.x, b.x), (T)2), div_rn(sub_rn(a.y, b.y), (T)2));
     }
-    case M_SQRT: return c_sqrt(z);
-    case M_SQUARE: return c_mul(z, z);
-    case M_LN: return c_ln(z);
+    case M_SQRT: return c_sqrt<T>(z);
+    case M_SQUARE: return cmul_nofma(z, z);
+    case M_LN: return c_ln<T>(z);
     case M_EXP: return c_from_polar((T)exp(re), im);
     case M_POWF:
-        if (arg == (T)0) return mkc((T)1, (T)0);
-        return c_from_polar((T)pow(hypot(re, im), arg), mul_((T)atan2(im, re), arg));
-    case M_LOG: return mkc(div_((T)log(hypot(re, im)), ln_arg), div_((T)atan2(im, re), ln_arg));
-    case M_EXPF: return c_from_polar((T)pow(arg, re), mul_(im, ln_arg));
+        if (arg == (T)0) return mk<T>((T)1, (T)0);
+        return c_from_polar((T)pow(hypot(re, im), arg), mul_rn((T)atan2(im, re), arg));
+    case M_LOG: return mk<T>(div_rn((T)log(hypot(re, im)), ln_arg), div_rn((T)atan2(im, re), ln_arg));
+    case M_EXPF: return c_from_polar((T)pow(arg, re), mul_rn(im, ln_arg));
     default: return z;
     }
 }
@@ -139,12 +124,12 @@ template <typename T> __device__ T real_fn(int op, T x, T arg, T ln_arg) {
     case M_ACOSH: return (T)acosh(x);
     case M_ATANH: return (T)atanh(x);
     case M_SQRT: return (T)sqrt(x);
-    case M_SQUARE: return mul_(x, x);
+    case M_SQUARE: return mul_rn(x, x);
     case M_LN: return (T)log(x);
     case M_EXP: return (T)exp(x);
     case M_ABS: return (T)fabs(x);
     case M_POWF: return (T)pow(x, arg);
-    case M_LOG: return div_((T)log(x), ln_arg);
+    case M_LOG: return div_rn((T)log(x), ln_arg);
     case M_EXPF: return (T)pow(arg, x);
     case M_WRAP: return (T)fmod(x, arg);
     default: return x;
@@ -170,8 +155,9 @@ __global__ void math_real_kernel(T* __restrict__ data, long long n, int op, T ar
     if (t < n) data[t] = real_fn<T>(op, data[t], arg, ln_arg);
 }
 template <typename T>
-__global__ void math_complex_kernel(C2<T>* __restrict__ data, long long n, int op, T arg, T ln_arg) {
-    constexpr int W = 16 / sizeof(C2<T>) > 0 ? 16 / sizeof(C2<T>) : 1;   // 2 (f32) or 1 (f64)
+__global__ void math_complex_kernel(typename CpxOf<T>::type* __restrict__ data, long long n, int op, T arg, T ln_arg) {
+    typedef typename CpxOf<T>::type C;
+    constexpr int W = 16 / sizeof(C);   // 2 (f32) or 1 (f64)
     const long long nv = n / W;
     const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
@@ -180,21 +166,13 @@ __global__ void math_complex_kernel(C2<T>* __restrict__ data, long long n, int o
         Pack<T> p = dv[i];
 #pragma unroll
         for (int k = 0; k < W; k++) {
-            const C2<T> r = complex_fn<T>(op, mkc(p.v[2 * k], p.v[2 * k + 1]), arg, ln_arg);
-            p.v[2 * k] = r.re; p.v[2 * k + 1] = r.im;
+            const C r = complex_fn<T>(op, mk<T>(p.v[2 * k], p.v[2 * k + 1]), arg, ln_arg);
+            p.v[2 * k] = r.x; p.v[2 * k + 1] = r.y;
         }
         dv[i] = p;
     }
     const long long t = nv * W + tid;
     if (t < n) data[t] = complex_fn<T>(op, data[t], arg, ln_arg);
-}
-
-unsigned grid_for(long long items, int threads) {
-    long long g = (items + threads - 1) / threads;
-    const long long cap = (long long)sm_count() * 16;
-    if (g > cap) g = cap;
-    if (g < 1) g = 1;
-    return (unsigned)g;
 }
 
 // ---- unwrap: loop-carried through rounded values -> one warp, lane 0 walks 128-element tiles staged in
@@ -203,7 +181,7 @@ template <typename T>
 __global__ void unwrap_kernel(T* __restrict__ data, long long n, T divisor) {
     __shared__ T tile[2][1024];
     const int lane = threadIdx.x;
-    const T half = div_(divisor, (T)2);
+    const T half = div_rn(divisor, (T)2);
     T prev = (T)0;
     const long long tiles = (n + 1023) / 1024;
     for (int k = lane; k < 1024 && k < n; k += 32) tile[0][k] = data[k];
@@ -224,9 +202,9 @@ __global__ void unwrap_kernel(T* __restrict__ data, long long n, T divisor) {
             if (t == 0) { prev = tile[cur][0]; j0 = 1; }
             for (int j = j0; j < cnt; j++) {
                 T v = tile[cur][j];
-                T diff = sub_(v, prev);
-                if (diff > half) { diff = sub_((T)fmod(diff, divisor), divisor); v = add_(prev, diff); }
-                else if (diff < -half) { diff = add_((T)fmod(diff, divisor), divisor); v = add_(prev, diff); }
+                T diff = sub_rn(v, prev);
+                if (diff > half) { diff = sub_rn((T)fmod(diff, divisor), divisor); v = add_rn(prev, diff); }
+                else if (diff < -half) { diff = add_rn((T)fmod(diff, divisor), divisor); v = add_rn(prev, diff); }
                 tile[cur][j] = v;
                 prev = v;
             }
@@ -248,8 +226,8 @@ __global__ void diff_kernel(const T* __restrict__ in, T* __restrict__ out, long 
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (; i < n_out; i += stride) {
-        if (with_start) out[i] = i < step ? in[i] : sub_(in[i], in[i - step]);
-        else out[i] = sub_(in[i + step], in[i]);
+        if (with_start) out[i] = i < step ? in[i] : sub_rn(in[i], in[i - step]);
+        else out[i] = sub_rn(in[i + step], in[i]);
     }
 }
 
@@ -287,14 +265,14 @@ __global__ void __launch_bounds__(CS_THREADS) cumsum_totals_kernel(const T* __re
     for (int l = 0; l < LANES; l++) {
         T s = (T)0;
 #pragma unroll
-        for (int k = 0; k < CS_PER; k++) s = add_(s, v[k * LANES + l]);
+        for (int k = 0; k < CS_PER; k++) s = add_rn(s, v[k * LANES + l]);
         sh[l][threadIdx.x] = s;
     }
     __syncthreads();
     for (int off = CS_THREADS / 2; off > 0; off >>= 1) {
         if (threadIdx.x < off)
 #pragma unroll
-            for (int l = 0; l < LANES; l++) sh[l][threadIdx.x] = add_(sh[l][threadIdx.x], sh[l][threadIdx.x + off]);
+            for (int l = 0; l < LANES; l++) sh[l][threadIdx.x] = add_rn(sh[l][threadIdx.x], sh[l][threadIdx.x + off]);
         __syncthreads();
     }
     if (threadIdx.x < LANES) totals[(long long)threadIdx.x * gridDim.x + blockIdx.x] = sh[threadIdx.x][0];
@@ -307,18 +285,18 @@ __global__ void __launch_bounds__(1024) cumsum_scan_totals_kernel(T* __restrict_
     const long long per = (nblocks + 1023) / 1024;
     const long long b0 = (long long)threadIdx.x * per;
     T s = (T)0;
-    for (long long b = b0; b < b0 + per && b < nblocks; b++) s = add_(s, t[b]);
+    for (long long b = b0; b < b0 + per && b < nblocks; b++) s = add_rn(s, t[b]);
     sh[threadIdx.x] = s;
     __syncthreads();
     for (int off = 1; off < 1024; off <<= 1) {
         T add = (T)0;
         if (threadIdx.x >= off) add = sh[threadIdx.x - off];
         __syncthreads();
-        if (threadIdx.x >= off) sh[threadIdx.x] = add_(sh[threadIdx.x], add);
+        if (threadIdx.x >= off) sh[threadIdx.x] = add_rn(sh[threadIdx.x], add);
         __syncthreads();
     }
     T run = threadIdx.x ? sh[threadIdx.x - 1] : (T)0;
-    for (long long b = b0; b < b0 + per && b < nblocks; b++) { const T v = t[b]; t[b] = run; run = add_(run, v); }
+    for (long long b = b0; b < b0 + per && b < nblocks; b++) { const T v = t[b]; t[b] = run; run = add_rn(run, v); }
 }
 template <typename T, int LANES>
 __global__ void __launch_bounds__(CS_THREADS) cumsum_apply_kernel(const T* __restrict__ in, T* __restrict__ out, const T* __restrict__ totals,
@@ -331,7 +309,7 @@ __global__ void __launch_bounds__(CS_THREADS) cumsum_apply_kernel(const T* __res
     for (int l = 0; l < LANES; l++) {
         T s = (T)0;
 #pragma unroll
-        for (int k = 0; k < CS_PER; k++) { s = add_(s, v[k * LANES + l]); v[k * LANES + l] = s; }
+        for (int k = 0; k < CS_PER; k++) { s = add_rn(s, v[k * LANES + l]); v[k * LANES + l] = s; }
         sh[l][threadIdx.x] = s;
     }
     __syncthreads();
@@ -343,15 +321,15 @@ __global__ void __launch_bounds__(CS_THREADS) cumsum_apply_kernel(const T* __res
         __syncthreads();
         if (threadIdx.x >= off)
 #pragma unroll
-            for (int l = 0; l < LANES; l++) sh[l][threadIdx.x] = add_(sh[l][threadIdx.x], add[l]);
+            for (int l = 0; l < LANES; l++) sh[l][threadIdx.x] = add_rn(sh[l][threadIdx.x], add[l]);
         __syncthreads();
     }
     T offset[LANES];
 #pragma unroll
     for (int l = 0; l < LANES; l++)
-        offset[l] = add_(totals[(long long)l * gridDim.x + blockIdx.x], threadIdx.x ? sh[l][threadIdx.x - 1] : (T)0);
+        offset[l] = add_rn(totals[(long long)l * gridDim.x + blockIdx.x], threadIdx.x ? sh[l][threadIdx.x - 1] : (T)0);
 #pragma unroll
-    for (int k = 0; k < CS_PER * LANES; k++) v[k] = add_(offset[k % LANES], v[k]);
+    for (int k = 0; k < CS_PER * LANES; k++) v[k] = add_rn(offset[k % LANES], v[k]);
     constexpr int W = 16 / sizeof(T);
     constexpr int NP = CS_PER * LANES / W;
     if (base + CS_PER <= points) {
@@ -370,29 +348,16 @@ __global__ void __launch_bounds__(CS_THREADS) cumsum_apply_kernel(const T* __res
     }
 }
 
-// ---- binary op with a shorter, repeated operand ---------------------------------------------------------
-template <typename T>
-__global__ void smaller_kernel(T* __restrict__ data, const T* __restrict__ w, long long points, long long w_points, int op, int is_complex) {
+// ---- binary op with a shorter, repeated operand: data[i] = data[i] OP w[i % w_points] (points) -----------------------
+template <typename T, int OP, bool CPX>
+__global__ void smaller_kernel(T* __restrict__ data, const T* __restrict__ w, long long points, long long w_points) {
+    typedef typename CpxOf<T>::type C;
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (; i < points; i += stride) {
         const long long j = i % w_points;
-        if (!is_complex) {
-            const T a = data[i], b = w[j];
-            data[i] = op == 0 ? add_(a, b) : op == 1 ? sub_(a, b) : op == 2 ? mul_(a, b) : div_(a, b);
-        } else {
-            C2<T> a = reinterpret_cast<C2<T>*>(data)[i];
-            const C2<T> b = reinterpret_cast<const C2<T>*>(w)[j];
-            C2<T> r;
-            if (op == 0) r = mkc(add_(a.re, b.re), add_(a.im, b.im));
-            else if (op == 1) r = mkc(sub_(a.re, b.re), sub_(a.im, b.im));
-            else if (op == 2) r = c_mul(a, b);
-            else {   // num-complex Div: (a * conj(b)) / |b|^2, each term rounded
-                const T ns = add_(mul_(b.re, b.re), mul_(b.im, b.im));
-                r = mkc(div_(add_(mul_(a.re, b.re), mul_(a.im, b.im)), ns), div_(sub_(mul_(a.im, b.re), mul_(a.re, b.im)), ns));
-            }
-            reinterpret_cast<C2<T>*>(data)[i] = r;
-        }
+        if (CPX) reinterpret_cast<C*>(data)[i] = ew_complex_op<OP>(reinterpret_cast<const C*>(data)[i], reinterpret_cast<const C*>(w)[j]);
+        else data[i] = ew_real_op<OP>(data[i], w[j]);
     }
 }
 
@@ -414,10 +379,11 @@ __global__ void split_merge_kernel(T* __restrict__ whole, PartPtrs<T> parts, int
 
 // ---- set_real_imag / set_mag_phase ------------------------------------------------------------------------
 template <typename T>
-__global__ void compose_kernel(const T* __restrict__ a, const T* __restrict__ b, C2<T>* __restrict__ out, long long points, int polar) {
+__global__ void compose_kernel(const T* __restrict__ a, const T* __restrict__ b, typename CpxOf<T>::type* __restrict__ out, long long points,
+                               int polar) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long stride = (long long)gridDim.x * blockDim.x;
-    for (; i < points; i += stride) out[i] = polar ? c_from_polar(a[i], b[i]) : mkc(a[i], b[i]);
+    for (; i < points; i += stride) out[i] = polar ? c_from_polar(a[i], b[i]) : mk<T>(a[i], b[i]);
 }
 
 // ---- interpolate_hermite -----------------------------------------------------------------------------------
@@ -430,7 +396,7 @@ __global__ void hermite_kernel(const T* __restrict__ x, T* __restrict__ y, long 
     const long long end = start + 1;
     const T half = (T)0.5, c15 = (T)1.5, two = (T)2, c25 = (T)2.5;
     for (; k < dest_len; k += stride) {
-        const T rounded = add_(div_(ctr(k, (T)0), F), d);
+        const T rounded = add_rn(div_rn(ctr(k, (T)0), F), d);
         const T bf = (T)floor(rounded);
         long long b = (long long)bf;
         T y0, y1, y2, y3;
@@ -438,7 +404,7 @@ __global__ void hermite_kernel(const T* __restrict__ x, T* __restrict__ y, long 
             if (b < 0) b = 0;
             if (b > n - 3) b = n - 3;                    // the reference asserts b == 0 here; clamp instead of panicking
             y1 = x[b]; y2 = x[b + 1]; y3 = x[b + 2];
-            y0 = sub_(y1, sub_(y2, y1));
+            y0 = sub_rn(y1, sub_rn(y2, y1));
         } else if (k < dest_len - end) {
             if (b < 1) b = 1;
             if (b > n - 3) b = n - 3;
@@ -447,14 +413,14 @@ __global__ void hermite_kernel(const T* __restrict__ x, T* __restrict__ y, long 
             if (b < 1) b = 1;
             if (b > n - 1) b = n - 1;
             y0 = x[b - 1]; y1 = x[b];
-            y2 = b < n - 1 ? x[b + 1] : add_(y1, sub_(y1, y0));
-            y3 = b < n - 2 ? x[b + 2] : add_(y2, sub_(y2, y1));
+            y2 = b < n - 1 ? x[b + 1] : add_rn(y1, sub_rn(y1, y0));
+            y3 = b < n - 2 ? x[b + 2] : add_rn(y2, sub_rn(y2, y1));
         }
-        const T xx = sub_(rounded, bf), x2 = mul_(xx, xx);
-        const T a0 = add_(sub_(add_(mul_(-half, y0), mul_(c15, y1)), mul_(c15, y2)), mul_(half, y3));
-        const T a1 = sub_(add_(sub_(y0, mul_(c25, y1)), mul_(two, y2)), mul_(half, y3));
-        const T a2 = add_(mul_(-half, y0), mul_(half, y2));
-        y[k] = add_(add_(add_(mul_(mul_(a0, xx), x2), mul_(a1, x2)), mul_(a2, xx)), y1);
+        const T xx = sub_rn(rounded, bf), x2 = mul_rn(xx, xx);
+        const T a0 = add_rn(sub_rn(add_rn(mul_rn(-half, y0), mul_rn(c15, y1)), mul_rn(c15, y2)), mul_rn(half, y3));
+        const T a1 = sub_rn(add_rn(sub_rn(y0, mul_rn(c25, y1)), mul_rn(two, y2)), mul_rn(half, y3));
+        const T a2 = add_rn(mul_rn(-half, y0), mul_rn(half, y2));
+        y[k] = add_rn(add_rn(add_rn(mul_rn(mul_rn(a0, xx), x2), mul_rn(a1, x2)), mul_rn(a2, xx)), y1);
     }
 }
 
@@ -467,8 +433,10 @@ int math_unary(int op, void* data, size_t elems, int is_complex, double arg, cud
     T ln_arg;   // `base.ln()` evaluated in T
     if (sizeof(T) == 4) ln_arg = (T)logf((float)a); else ln_arg = (T)log((double)a);
     const long long items = (long long)elems * (is_complex ? 2 : 1) * (long long)sizeof(T) / 16 + 1;
-    if (is_complex) math_complex_kernel<T><<<grid_for(items, 256), 256, 0, st>>>(reinterpret_cast<C2<T>*>(data), (long long)elems, op, a, ln_arg);
-    else math_real_kernel<T><<<grid_for(items, 256), 256, 0, st>>>(reinterpret_cast<T*>(data), (long long)elems, op, a, ln_arg);
+    const unsigned grid = grid_stride_blocks(items);
+    if (is_complex)
+        math_complex_kernel<T><<<grid, GRID_STRIDE_THREADS, 0, st>>>(reinterpret_cast<typename CpxOf<T>::type*>(data), (long long)elems, op, a, ln_arg);
+    else math_real_kernel<T><<<grid, GRID_STRIDE_THREADS, 0, st>>>(reinterpret_cast<T*>(data), (long long)elems, op, a, ln_arg);
     BDSP_LAUNCHED();
     return 0;
 }
@@ -484,9 +452,8 @@ int math_unwrap(void* data, size_t n, double divisor, cudaStream_t st) {
 template <typename T>
 int math_diff(const void* in, void* out, size_t n_out_scalars, int step, int with_start, cudaStream_t st) {
     if (!n_out_scalars) return 0;
-    diff_kernel<T><<<grid_for((long long)n_out_scalars, 256), 256, 0, st>>>(reinterpret_cast<const T*>(in), reinterpret_cast<T*>(out), (long long)n_out_scalars, step, with_start);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(diff_kernel<T>, (long long)n_out_scalars, st, reinterpret_cast<const T*>(in), reinterpret_cast<T*>(out),
+                              (long long)n_out_scalars, step, with_start);
 }
 
 size_t math_cumsum_workspace(size_t points, int lanes, size_t elem_size) {
@@ -516,9 +483,20 @@ int math_cumsum(const void* in, void* out, void* work, size_t points, int lanes,
 template <typename T>
 int math_binary_smaller(int op, void* data, const void* w, size_t points, size_t w_points, int is_complex, cudaStream_t st) {
     if (!points) return 0;
-    smaller_kernel<T><<<grid_for((long long)points, 256), 256, 0, st>>>(reinterpret_cast<T*>(data), reinterpret_cast<const T*>(w), (long long)points, (long long)w_points, op, is_complex);
-    BDSP_LAUNCHED();
-    return 0;
+    auto run = [&](auto kernel) {
+        return launch_grid_stride(kernel, (long long)points, st, reinterpret_cast<T*>(data), reinterpret_cast<const T*>(w), (long long)points,
+                                  (long long)w_points);
+    };
+    if (is_complex) {
+        if (op == EW_ADD) return run(smaller_kernel<T, EW_ADD, true>);
+        if (op == EW_SUB) return run(smaller_kernel<T, EW_SUB, true>);
+        if (op == EW_MUL) return run(smaller_kernel<T, EW_MUL, true>);
+        return run(smaller_kernel<T, EW_DIV, true>);
+    }
+    if (op == EW_ADD) return run(smaller_kernel<T, EW_ADD, false>);
+    if (op == EW_SUB) return run(smaller_kernel<T, EW_SUB, false>);
+    if (op == EW_MUL) return run(smaller_kernel<T, EW_MUL, false>);
+    return run(smaller_kernel<T, EW_DIV, false>);
 }
 
 template <typename T>
@@ -527,25 +505,21 @@ int math_split_merge(void* whole, void* const* parts, int nparts, size_t elems, 
     if (nparts > 64) { set_last_error("split_into / merge: at most 64 parts"); return 7; }
     PartPtrs<T> pp;
     for (int i = 0; i < nparts; i++) pp.p[i] = reinterpret_cast<T*>(parts[i]);
-    split_merge_kernel<T><<<grid_for((long long)elems, 256), 256, 0, st>>>(reinterpret_cast<T*>(whole), pp, nparts, (long long)elems, esz, merge);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(split_merge_kernel<T>, (long long)elems, st, reinterpret_cast<T*>(whole), pp, nparts, (long long)elems, esz, merge);
 }
 
 template <typename T>
 int math_compose(const void* a, const void* b, void* out, size_t points, int polar, cudaStream_t st) {
     if (!points) return 0;
-    compose_kernel<T><<<grid_for((long long)points, 256), 256, 0, st>>>(reinterpret_cast<const T*>(a), reinterpret_cast<const T*>(b), reinterpret_cast<C2<T>*>(out), (long long)points, polar);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(compose_kernel<T>, (long long)points, st, reinterpret_cast<const T*>(a), reinterpret_cast<const T*>(b),
+                              reinterpret_cast<typename CpxOf<T>::type*>(out), (long long)points, polar);
 }
 
 template <typename T>
 int math_hermite(const void* x, void* y, size_t n, size_t dest_len, size_t start, double factor, double delay, cudaStream_t st) {
     if (!dest_len) return 0;
-    hermite_kernel<T><<<grid_for((long long)dest_len, 256), 256, 0, st>>>(reinterpret_cast<const T*>(x), reinterpret_cast<T*>(y), (long long)n, (long long)dest_len, (long long)start, (T)factor, (T)delay);
-    BDSP_LAUNCHED();
-    return 0;
+    return launch_grid_stride(hermite_kernel<T>, (long long)dest_len, st, reinterpret_cast<const T*>(x), reinterpret_cast<T*>(y), (long long)n,
+                              (long long)dest_len, (long long)start, (T)factor, (T)delay);
 }
 
 #define BDSP_INST(T)                                                                                   \

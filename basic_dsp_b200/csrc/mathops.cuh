@@ -17,7 +17,7 @@ template <typename T> int math_unwrap(void* data, size_t n, double divisor, cuda
 template <typename T> int math_diff(const void* in, void* out, size_t n_out_scalars, int step, int with_start, cudaStream_t st);
 size_t math_cumsum_workspace(size_t points, int lanes, size_t elem_size);
 template <typename T> int math_cumsum(const void* in, void* out, void* work, size_t points, int lanes, cudaStream_t st);
-// op: 0 add, 1 sub, 2 mul, 3 div; operand element i % w_points
+// op: EW_ADD, EW_SUB, EW_MUL or EW_DIV (elementwise.cuh); operand element i % w_points
 template <typename T> int math_binary_smaller(int op, void* data, const void* w, size_t points, size_t w_points, int is_complex, cudaStream_t st);
 template <typename T> int math_split_merge(void* whole, void* const* parts, int nparts, size_t elems, int esz, int merge, cudaStream_t st);
 template <typename T> int math_compose(const void* a, const void* b, void* out, size_t points, int polar, cudaStream_t st);

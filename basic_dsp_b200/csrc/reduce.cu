@@ -16,7 +16,6 @@
 #include "mathops.cuh"
 
 namespace bdsp {
-int sm_count();
 void* workspace(size_t bytes, int slot);
 
 namespace {

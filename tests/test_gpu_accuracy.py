@@ -301,7 +301,7 @@ CONV_CASES = [
     (F32, 1 << 15, 3, 8000, "rows", "full", "full length c32 rows (4095 .. 8192 taps)", "L > 4094, pow2 N >= 2^15"),
     (F32, 1 << 16, 1, 6000, "vec-real", "ols", "ols_conv_kernel<float, REAL>, M = 16384", "real signal: the 4095 .. 8192-tap full-length path is complex only"),
     (F32, 16384, 1, 9000, "vec", "full", "full length c32 N = 16384, separate spectrum multiply",
-     "convolve: L > 8192; fft_convolve_full: pow2 N <= 16384 -> spectrum_mul_kernel"),
+     "convolve: L > 8192; fft_convolve_full: pow2 N <= 16384 -> ew_spectrum_mul_rows"),
     (F32, 3 << 14, 1, 9000, "vec", "full", "full length c32, q*2^k N", "L > 8192, not pow2: in_mul"),
     (F32, 20000, 2, 9000, "rows", "full", "full length c32 rows, chirp-z N", "convolve: L > 8192 -> fft_convolve_full"),
     (F32, 20000, 1, 5000, "vec", "ols", "ols_conv_kernel c32, M = 16384 (non-pow2 N, L > 4094)", "L > 4094, !is_pow2(N)"),
