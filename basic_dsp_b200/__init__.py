@@ -23,6 +23,8 @@ LIB_PATH = os.environ.get("BASIC_DSP_B200_LIB", os.path.join(_HERE, "libbasic_ds
 
 F_INVERSE, F_SHIFT, F_MAGNITUDE, F_REAL_INPUT = 1, 2, 4, 8
 F_REAL_OUTPUT = 16   # bdsp_ifft_frames_*: the output holds the real parts of the synthesis as scalars
+F_ONESIDED = 32         # bdsp_welch_*: real input only, points/2 + 1 bins, interior bins doubled
+F_POWER_SPECTRUM = 64   # bdsp_welch_*: scaling 1/(sum w)^2 (power per bin) instead of the density 1/(fs sum w^2)
 
 
 def F_WINDOW(kind):
@@ -237,6 +239,8 @@ def _declare(lib):
         for name in ("bdsp_fft_frames_c", "bdsp_ifft_frames_c"):
             f = getattr(lib, name + s)
             f.restype, f.argtypes = c_int32, [c_void_p, c_void_p, c_size_t, c_size_t, c_size_t, c_int32]
+        f = getattr(lib, "bdsp_welch_c" + s)
+        f.restype, f.argtypes = c_int32, [c_void_p, c_void_p, c_size_t, c_size_t, c_size_t, c_int32, c_float if s == "32" else c_double]
         f = getattr(lib, "bdsp_conv_plan_create_c" + s)
         f.restype, f.argtypes = c_void_p, [c_void_p, c_size_t]
         f = getattr(lib, "bdsp_convolve_signal_rows_c" + s)

@@ -1372,6 +1372,40 @@ template <typename T> int ifft_frames(const void* in, void* out, size_t points, 
     return ifft_frames_exec<T>(in, out, points, hop, frames, o, real_out, g_stream);
 }
 
+// Welch's averaged periodogram of a signal's frames (scipy.signal.welch with detrend=False, MATLAB pwelch): the frames of
+// fft_frames, |X|^2 averaged over them and scaled as a density or a power spectrum, two-sided or one-sided
+template <typename T> int welch(const void* in, void* out, size_t points, size_t hop, size_t frames, int flags, double fs) {
+    const int known = BDSP_F_REAL_INPUT | BDSP_F_SHIFT | (15 << 8) | BDSP_F_ONESIDED | BDSP_F_POWER_SPECTRUM;   // (15 << 8): BDSP_F_WINDOW(kind)
+    const int unknown = flags & ~known;
+    if (unknown) {
+        const char* name = (unknown & BDSP_F_INVERSE) ? "BDSP_F_INVERSE" : (unknown & BDSP_F_MAGNITUDE) ? "BDSP_F_MAGNITUDE"
+                         : (unknown & BDSP_F_REAL_OUTPUT) ? "BDSP_F_REAL_OUTPUT" : nullptr;
+        if (name) set_last_error("welch: %s is not accepted (BDSP_F_REAL_INPUT, BDSP_F_SHIFT, BDSP_F_WINDOW(kind), BDSP_F_ONESIDED, "
+                                 "BDSP_F_POWER_SPECTRUM are)", name);
+        else set_last_error("welch: unknown flag bits 0x%x", (unsigned)unknown);
+        return -2;
+    }
+    const bool real = (flags & BDSP_F_REAL_INPUT) != 0, shift = (flags & BDSP_F_SHIFT) != 0, onesided = (flags & BDSP_F_ONESIDED) != 0;
+    const bool power = (flags & BDSP_F_POWER_SPECTRUM) != 0;
+    if (onesided && !real) { set_last_error("welch: BDSP_F_ONESIDED needs BDSP_F_REAL_INPUT (a complex signal has no symmetric spectrum)"); return -2; }
+    if (onesided && shift) { set_last_error("welch: BDSP_F_ONESIDED and BDSP_F_SHIFT exclude each other"); return -2; }
+    if (!hop) { set_last_error("welch: hop must be at least 1"); return -2; }
+    if (!power && !(isfinite(fs) && fs > 0)) { set_last_error("welch: the sampling rate fs must be finite and > 0"); return -2; }
+    if (!points || !frames) return 0;
+    const size_t in_esz = real ? sizeof(T) : 2 * sizeof(T);
+    const size_t max = ~(size_t)0;
+    if (frames - 1 > (max - points) / hop || ((frames - 1) * hop + points) > max / in_esz || points > max / sizeof(T)) {
+        set_last_error("welch: %zu frames of %zu points, hop %zu overflow the address space", frames, points, hop);
+        return -2;
+    }
+    const uintptr_t i0 = reinterpret_cast<uintptr_t>(in), o0 = reinterpret_cast<uintptr_t>(out);
+    const size_t in_bytes = ((frames - 1) * hop + points) * in_esz, out_bytes = (onesided ? points / 2 + 1 : points) * sizeof(T);
+    if (i0 < o0 + out_bytes && o0 < i0 + in_bytes) { set_last_error("welch: the output overlaps the input"); return -3; }
+    const int wk = (flags >> 8) & 15;
+    const FftOpts o = fft_opts<T>(points, false, shift, false, real, wk ? wk - 1 : RECTANGULAR);
+    return welch_exec<T>(in, static_cast<T*>(out), points, hop, frames, o, onesided, power, fs, g_stream);
+}
+
 // ---- batched (matrix-row) forms: the reference's MatrixMxN applies the vector operation to every row in turn
 // (matrix/src/time_freq.rs:52-74, matrix/src/complex.rs:18-26); rows sit back to back in device memory ----------------------
 // magnitude (hypot, complex_to_real.rs:376) / phase (atan2, :402) / magnitude_squared of `rows` rows: elementwise, so the
@@ -1764,6 +1798,12 @@ extern "C" int32_t bdsp_ifft_frames_c32(const void* in, void* out, size_t points
 }
 extern "C" int32_t bdsp_ifft_frames_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags) {
     return ifft_frames<double>(in, out, points, hop, frames, flags);
+}
+extern "C" int32_t bdsp_welch_c32(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags, float fs) {
+    return welch<float>(in, out, points, hop, frames, flags, (double)fs);
+}
+extern "C" int32_t bdsp_welch_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags, double fs) {
+    return welch<double>(in, out, points, hop, frames, flags, fs);
 }
 extern "C" BdspConvPlan* bdsp_conv_plan_create_c32(const void* h, size_t L) { return reinterpret_cast<BdspConvPlan*>(conv_plan_create<float>(h, L)); }
 extern "C" BdspConvPlan* bdsp_conv_plan_create_c64(const void* h, size_t L) { return reinterpret_cast<BdspConvPlan*>(conv_plan_create<double>(h, L)); }

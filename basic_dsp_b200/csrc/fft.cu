@@ -35,6 +35,9 @@ int fftp_single(const void* in, void* out, size_t n, size_t groups, bool inverse
 template <bool RIN>
 int fftp_frames(const void* in, void* out, size_t n, size_t groups, size_t hop, const float* win, bool so, bool magnitude, double scale,
                 cudaStream_t st);
+template <bool RIN>
+int fftp_frames_psum(const void* in, float* part, size_t n, size_t groups, size_t ctas, size_t hop, size_t frames, const float* win,
+                     cudaStream_t st);
 int fftp_two_pass(const void* in, void* out, void* tmp, const FftPlan& p, size_t rows, bool inverse, bool si, bool so, bool magnitude,
                   double scale, bool real_in, const InMul& im, cudaStream_t st);
 int fftp_three_pass(const void* in, void* out, void* tmp, const FftPlan& p, size_t n, size_t rows, bool inverse, bool si, bool so,
@@ -106,10 +109,11 @@ template <> const double2* twiddle_table<double>() { DeviceState* s = dev_state(
 // workspace_bind_stream (capi: bdsp_set_stream).  Slots: 0..3 the transforms and reductions, 4..5 the full-length
 // convolution (its buffers stay live across nested fft_exec calls, which use 0..2), 6 the frame buffers of the frame
 // entry points: the gathered frames of FftRoute::FramePass and the inverse rows of ifft_frames_exec (live across the
-// transform that fills or reads them, which may use 0..3).
+// transform that fills or reads them, which may use 0..3), 7..8 welch_exec: 7 a chunk of frame spectra (filled by a frame
+// transform, which may use 0..3 and 6), 8 the window sums and the partial rows (live across every chunk).
 namespace {
 thread_local cudaStream_t tl_ws_stream = nullptr;
-constexpr int WS_SLOTS = 7;
+constexpr int WS_SLOTS = 9;
 struct WsSet { void* p[WS_SLOTS] = {}; size_t bytes[WS_SLOTS] = {}; };
 struct WsMap {
     std::map<std::pair<int, cudaStream_t>, WsSet> m;
@@ -914,6 +918,70 @@ __global__ void overlap_add_kernel(const typename CpxOf<T>::type* __restrict__ y
     else reinterpret_cast<C*>(out)[t] = mk<T>(num.x / den, num.y / den);
 }
 
+// sums[0] = sum w, sums[1] = sum w^2 over the n entries of a window table, in double: one block, a fixed order
+template <typename T>
+__global__ void __launch_bounds__(1024) window_sums_kernel(const T* __restrict__ w, long long n, double* __restrict__ sums) {
+    __shared__ double s1[1024], s2[1024];
+    double a = 0, b = 0;
+    for (long long i = threadIdx.x; i < n; i += 1024) {
+        const double v = (double)w[i];
+        a += v;
+        b += v * v;
+    }
+    s1[threadIdx.x] = a;
+    s2[threadIdx.x] = b;
+    for (int h = 512; h > 0; h >>= 1) {
+        __syncthreads();
+        if ((int)threadIdx.x < h) {
+            s1[threadIdx.x] += s1[threadIdx.x + h];
+            s2[threadIdx.x] += s2[threadIdx.x + h];
+        }
+    }
+    if (threadIdx.x == 0) { sums[0] = s1[0]; sums[1] = s2[0]; }
+}
+
+// part[i] (+)= sum |spec[j]|^2 over j = i, i + slabs * n, ... < frames * n: slab s = i / n of the partial rows takes the
+// frames s, s + slabs, ... of the chunk, bin i % n.  |X|^2 is rounded in T, the sum kept in double; the first chunk stores.
+template <typename T>
+__global__ void welch_accumulate_kernel(const typename CpxOf<T>::type* __restrict__ spec, double* __restrict__ part, long long n,
+                                        long long frames, long long slabs, int first) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= slabs * n || i >= frames * n) return;
+    double s = first ? 0.0 : part[i];
+#pragma unroll 4
+    for (long long j = i; j < frames * n; j += slabs * n) {
+        const typename CpxOf<T>::type v = spec[j];
+        s += (double)add_rn(mul_rn(v.x, v.x), mul_rn(v.y, v.y));
+    }
+    part[i] = s;
+}
+
+// Output j of bdsp_welch_*: bin k = j (shift: (j + n - n/2) mod n), the sum of part[r * stride + k] over the `rows` partial
+// rows in double (32 bins x 8 lanes per block: lane y takes rows y, y + 8, ..., the lanes are added in order), times
+// 1 / (frames * fs * sum w^2), or 1 / (frames * (sum w)^2) with `power`; onesided: bins 0 .. n/2, doubled but for 0 and the
+// Nyquist bin of an even n.  sums: the window sums of window_sums_kernel, null without a window (both n).
+template <typename T, typename P>
+__global__ void __launch_bounds__(256) welch_final_kernel(const P* __restrict__ part, long long rows, long long stride, const double* __restrict__ sums,
+                                                          T* __restrict__ out, long long n, long long nout, int shift, int onesided, int power,
+                                                          double fs, long long frames) {
+    __shared__ double lane[8][33];
+    const long long j = (long long)blockIdx.x * 32 + threadIdx.x;
+    const long long k = shift ? (j + n - n / 2) % n : j;
+    double s = 0;
+    if (j < nout) {
+#pragma unroll 4
+        for (long long r = threadIdx.y; r < rows; r += 8) s += (double)part[r * stride + k];
+    }
+    lane[threadIdx.y][threadIdx.x] = s;
+    __syncthreads();
+    if (threadIdx.y != 0 || j >= nout) return;
+    for (int y = 1; y < 8; y++) s += lane[y][threadIdx.x];
+    const double sw = sums ? sums[0] : (double)n, sw2 = sums ? sums[1] : (double)n;
+    double v = s / ((double)frames * (power ? sw * sw : fs * sw2));
+    if (onesided && k != 0 && 2 * k != n) v *= 2;
+    out[j] = (T)v;
+}
+
 template <typename T, bool INV>
 int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o, void* work, size_t work_bytes,
             cudaStream_t st) {
@@ -1121,5 +1189,74 @@ int ifft_frames_exec(const void* in, void* out, size_t n, size_t hop, size_t fra
 
 template int ifft_frames_exec<float>(const void*, void*, size_t, size_t, size_t, const FftOpts&, bool, cudaStream_t);
 template int ifft_frames_exec<double>(const void*, void*, size_t, size_t, size_t, const FftOpts&, bool, cudaStream_t);
+
+template <typename T>
+int welch_exec(const void* in, T* out, size_t n, size_t hop, size_t frames, const FftOpts& opts, bool onesided, bool power_spectrum, double fs,
+               cudaStream_t stream) {
+    typedef typename CpxOf<T>::type C;
+    if (n == 0 || frames == 0) return 0;
+    const bool real_in = opts.real_input != 0;
+    const size_t esz = real_in ? sizeof(T) : sizeof(C);
+    const WelchPlan plan = welch_route(sizeof(T) == 8, n, hop, frames, real_in, reinterpret_cast<uintptr_t>(in));
+    // the partial rows: fused, `ctas` rows of N floats (N = 4096 * R0); otherwise `slabs` rows of n doubles, about 2^18
+    // accumulating threads (each with four loads in flight) whatever n is.  Chunks of at most WELCH_CHUNK_POINTS spectrum
+    // points bound the memory.
+    constexpr size_t WELCH_CHUNK_POINTS = (size_t)1 << 24, WELCH_ACC_THREADS = (size_t)1 << 18;
+    const size_t N = n < 4096 ? 4096 : n;
+    const size_t chunk = n >= WELCH_CHUNK_POINTS ? 1 : (WELCH_CHUNK_POINTS / n < frames ? WELCH_CHUNK_POINTS / n : frames);
+    const size_t slabs = (WELCH_ACC_THREADS + n - 1) / n < chunk ? (WELCH_ACC_THREADS + n - 1) / n : chunk;
+    const size_t part_bytes = plan.fused ? plan.ctas * N * sizeof(float) : slabs * n * sizeof(double);
+    BDSP_WS(ws, char*, 2 * sizeof(double) + part_bytes, 8);
+    double* sums = reinterpret_cast<double*>(ws);
+    void* part = ws + 2 * sizeof(double);
+    const T* win = nullptr;
+    if (opts.in_mul.kind == 3) {
+        BDSP_WS(tab, T*, n * sizeof(T), 3);
+        window_table_kernel<T><<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(tab, (long long)n, opts.in_mul.arg);
+        BDSP_LAUNCHED();
+        window_sums_kernel<T><<<1, 1024, 0, stream>>>(tab, (long long)n, sums);
+        BDSP_LAUNCHED();
+        win = tab;
+    }
+    const size_t nout = onesided ? n / 2 + 1 : n;
+    const dim3 block(32, 8);
+    const unsigned grid = (unsigned)((nout + 31) / 32);
+    const int shift = opts.out_rot != 0;
+    if constexpr (sizeof(T) == 4) {   // welch_route fuses c32 only
+        if (plan.fused) {
+            const int rc = real_in ? fftp_frames_psum<true>(in, static_cast<float*>(part), n, plan.groups, plan.ctas, hop, frames, win, stream)
+                                   : fftp_frames_psum<false>(in, static_cast<float*>(part), n, plan.groups, plan.ctas, hop, frames, win, stream);
+            if (rc) return rc;
+            welch_final_kernel<T, float><<<grid, block, 0, stream>>>(static_cast<const float*>(part), (long long)plan.ctas, (long long)N,
+                                                                     win ? sums : nullptr, out, (long long)n, (long long)nout, shift, onesided,
+                                                                     power_spectrum, fs, (long long)frames);
+            BDSP_LAUNCHED();
+            return 0;
+        }
+    }
+    // every chunk: the frame transform (fft_exec's routes for strided frames, the window table as its multiplier) into
+    // slot 7, then |X|^2 added into the partial rows
+    BDSP_WS(spec, C*, chunk * n * sizeof(C), 7);
+    FftOpts o;
+    o.real_input = opts.real_input;
+    o.in_stride = hop;
+    if (win) { o.in_mul.p = win; o.in_mul.kind = 1; }
+    for (size_t f0 = 0; f0 < frames; f0 += chunk) {
+        const size_t cf = frames - f0 < chunk ? frames - f0 : chunk;
+        const int rc = fft_exec<T>(static_cast<const char*>(in) + f0 * hop * esz, spec, n, cf, o, nullptr, 0, stream);
+        if (rc) return rc;
+        const long long threads = (long long)(slabs * n);
+        welch_accumulate_kernel<T><<<(unsigned)((threads + 255) / 256), 256, 0, stream>>>(spec, static_cast<double*>(part), (long long)n,
+                                                                                        (long long)cf, (long long)slabs, f0 == 0);
+        BDSP_LAUNCHED();
+    }
+    welch_final_kernel<T, double><<<grid, block, 0, stream>>>(static_cast<const double*>(part), (long long)slabs, (long long)n, win ? sums : nullptr,
+                                                              out, (long long)n, (long long)nout, shift, onesided, power_spectrum, fs, (long long)frames);
+    BDSP_LAUNCHED();
+    return 0;
+}
+
+template int welch_exec<float>(const void*, float*, size_t, size_t, size_t, const FftOpts&, bool, bool, double, cudaStream_t);
+template int welch_exec<double>(const void*, double*, size_t, size_t, size_t, const FftOpts&, bool, bool, double, cudaStream_t);
 
 }  // namespace bdsp

@@ -36,6 +36,16 @@ template <typename T>
 int ifft_frames_exec(const void* in, void* out, size_t n, size_t hop, size_t frames, const FftOpts& opts, bool real_out,
                      cudaStream_t stream);
 
+// Welch's averaged periodogram (bdsp_welch_*): out[k] = scale / frames * sum_f |DFT(w x_f)[k]|^2 over the `frames` frames x_f
+// of n points (real scalars with opts.real_input) that start f*hop points apart; w = the built-in window of opts.in_mul
+// (kind 3) or 1, scale = 1 / (fs sum w^2), or 1 / (sum w)^2 with power_spectrum.  out holds n values in fftfreq order
+// (opts.out_rot != 0: fftshift order), or with onesided bins 0 .. n/2, all but bin 0 and the Nyquist bin of an even n
+// doubled.  Bit-reproducible: no atomics, every sum in an order fixed by n, hop, frames and the options.  Returns 0 or a
+// negative error.
+template <typename T>
+int welch_exec(const void* in, T* out, size_t n, size_t hop, size_t frames, const FftOpts& opts, bool onesided, bool power_spectrum,
+               double fs, cudaStream_t stream);
+
 // largest n the single-CTA shared-memory kernel handles for this precision
 template <typename T> size_t fft_block_max_n();
 

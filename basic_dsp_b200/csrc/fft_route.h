@@ -1,5 +1,6 @@
 // Which kernels run one level of an FFT (fft.cu fft_any): the one place that picks the path.  Plain C++ (no CUDA), so that
-// the routing table can be checked without a GPU (tests/cpp/fft_route_driver.cpp, tests/cpp/fft_frames_route_driver.cpp).
+// the routing table can be checked without a GPU (tests/cpp/fft_route_driver.cpp, tests/cpp/fft_frames_route_driver.cpp,
+// tests/cpp/welch_route_driver.cpp for welch_route below).
 // A strided input (FftRouteIn::in_stride other than 0 or n) takes one of the two frame routes; every other input the
 // rules apply to in the order of FftRoute, and the first one that matches wins.
 #pragma once
@@ -165,6 +166,28 @@ inline FftPlan fft_route(const FftRouteIn& a) {
     const bool packed_rows = c32 && p.P >= 256 && p.P <= block_max && n * rows >= (1u << 18) && (p.P >= 4096 || rows * p.q % (4096 / p.P) == 0);
     p.route = p.P > block_max || packed_rows ? FftRoute::QRowsInterleave : FftRoute::QRows;
     return p;
+}
+
+// Welch power sums (fft.cu welch_exec, bdsp_welch_*): fused into the packed frames kernel (fftp_kernel<FRAMES, PSUM>) for c32
+// frames of a power-of-two n in [64, 8192], an even hop and the paired loads' alignment (16 B complex, 8 B real), within
+// the grid limit.  Unlike PackedFrames there is no whole-group condition (the missing frames of the last group load zeros)
+// and no out != in (the kernel writes a workspace).  `ctas` CTAs loop over the `groups` groups of N / n frames (N = 4096,
+// or 8192), each summing into its own partial row of N floats: a function of n and the frame count only, so that the
+// order of every sum, and with it the result, does not depend on the device.  WELCH_CTAS is the B200's residency, 148
+// SMs x 4 CTAs of 128 threads (2 of 256 threads for 8192 points): one wave, 9.7 MB of partial rows in the 126 MB L2.
+struct WelchPlan {
+    bool fused = false;
+    size_t groups = 0, ctas = 0;
+};
+constexpr size_t WELCH_CTAS = 592, WELCH_CTAS_8192 = 296;
+
+inline WelchPlan welch_route(bool f64, size_t n, size_t hop, size_t frames, bool real_input, uintptr_t in) {
+    const size_t per = n >= 64 && n < 4096 ? 4096 / n : 1;
+    const size_t groups = frames / per + (frames % per != 0);
+    const bool pow2 = n && !(n & (n - 1));
+    if (f64 || !pow2 || n < 64 || n > 8192 || hop % 2 != 0 || (in & (real_input ? 7 : 15)) != 0 || groups > FFT_GRID_MAX) return {};
+    const size_t cap = n == 8192 ? WELCH_CTAS_8192 : WELCH_CTAS;
+    return {true, groups, groups < cap ? groups : cap};
 }
 
 }  // namespace bdsp

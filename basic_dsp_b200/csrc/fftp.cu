@@ -12,9 +12,11 @@
 //   TQ = Q    last pass with 16/Q adjacent rows of 256*Q points per CTA (128 threads), transposing store
 //   RIN       the input holds real scalars
 //   FRAMES    the sequences are strided frames of one signal, with an optional window multiplied in on the first load
+//   PSUM      (with FRAMES) Welch's power sum: |X|^2 added into a partial row per CTA instead of stored
 // fftp_col16_kernel / fftp_col256_kernel: first pass(es) of the multi-pass transforms: 16- / 256-point (NH = 2: 32- / 512-point)
 //   columns of 16 adjacent columns per CTA, inter-pass twiddle evaluated with sincospif on exact arguments.
-// Launchers, one per route of fft_route.h: fftp_single (complex or real rows), fftp_frames (strided frames), fftp_two_pass (2^15..2^20), fftp_three_pass
+// Launchers, one per route of fft_route.h: fftp_single (complex or real rows), fftp_frames (strided frames), fftp_frames_psum
+//   (Welch power sums, welch_route), fftp_two_pass (2^15..2^20), fftp_three_pass
 //   (2^21..2^24), fftp_rows_pass (packed last pass, also behind a generic column pass).
 // Replaces rustfft for these lengths (vector/src/vector_types/time_freq/mod.rs:45-58) incl. the fused
 // fft_shift (time_to_freq.rs:163), ifft's scale + ifft_shift (freq_to_time.rs:165-167) and magnitude.
@@ -46,12 +48,17 @@ using namespace ols16;
 // when `win` is not null, multiplied by win[p % n] as it is loaded.  The product is rounded on its own (__fmul_rn), as the
 // separate multiplier pass (fft.cu in_mul_rows_kernel) rounds it, so that the result is the one of that pass followed by the
 // plain kernel.
+// PSUM = true (with FRAMES): Welch's power sum.  `rows` counts the groups of N / n frames, of which only the first `frames`
+// frames exist: a frame index >= frames loads nothing and transforms zeros, so the last group may be incomplete.  Instead of
+// storing X, F3 adds |X|^2 (the MAG epilogue's pfma, without the sqrt) into the CTA's partial row out[blockIdx.x * N + k]:
+// every slot has one owner thread, the CTA's first row stores and later rows add, and after the last row the CTA sums its
+// N / n frames' slots into the first n (fixed order, no atomics).  No scale, no fft_shift: welch_final_kernel applies them.
 #define FP_MINB256 2   // CTAs per SM for the 256-thread 8192-point kernel
 template <int R0, bool INV, bool SHIFT_IN, bool SHIFT_OUT, bool MAG, bool ROWS, int TQ = 0, int NATQ = 0, bool RIN = false, int SQ = 0,
-          bool FRAMES = false>
+          bool FRAMES = false, bool PSUM = false>
 __global__ void __launch_bounds__(128 * R0, R0 == 2 ? FP_MINB256 : 4 / R0)
 fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long rows, float scale, const float* __restrict__ tw, int n1, int n2c,
-            long long hop, const float* __restrict__ win) {
+            long long hop, const float* __restrict__ win, long long frames) {
     constexpr int NSB = R0;               // sub-blocks (4096-point transforms) owned by this CTA
     constexpr int NT = 128 * NSB;         // threads
     constexpr int N = 4096 * R0;
@@ -85,7 +92,9 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
         if constexpr (FRAMES) {
             constexpr int FN = SQ ? 16 * SQ : NATQ ? 256 * NATQ : N;   // frame length
             const int p = (int)(gp - xr);
-            const long long src = ((long long)seq * (N / FN) + p / FN) * hop + p % FN;
+            const long long fr = (long long)seq * (N / FN) + p / FN;
+            if constexpr (PSUM) { if (fr >= frames) return make_float4(0.f, 0.f, 0.f, 0.f); }
+            const long long src = fr * hop + p % FN;
             float4 v;
             if constexpr (RIN) {
                 const float2 r = __ldg(reinterpret_cast<const float2*>(reinterpret_cast<const float*>(x) + src));
@@ -383,7 +392,18 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
                             : R1K ? kbase + (size_t)(RPC * grp + (k0 % RPC)) + kst * (size_t)((k0 / RPC) + TQ * k1)
                                 : kbase + (ROWS ? (size_t)(NSB * grp + lsb) : (size_t)lsb) + kst * (size_t)(k0 + 16 * k1);
         const size_t k2s = SQ ? (size_t)SQ : NATQ ? (size_t)(16 * NATQ) : R1K ? (size_t)(16 * TQ) * kst : (size_t)256 * kst;
-        if constexpr (MAG) {
+        if constexpr (PSUM) {
+            float* o = reinterpret_cast<float*>(out_) + (size_t)blockIdx.x * N + klow;
+            const bool first = row == (long long)blockIdx.x;
+#pragma unroll
+            for (int m = 0; m < 8; m++) {
+                const pk m2 = pfma(P[m].re, P[m].re, pmul(P[m].im, P[m].im));
+                float* a = o + k2s * bitrev4(2 * m);
+                float* b = o + k2s * bitrev4(2 * m + 1);
+                *a = first ? m2.x : *a + m2.x;
+                *b = first ? m2.y : *b + m2.y;
+            }
+        } else if constexpr (MAG) {
             float* o = reinterpret_cast<float*>(out_) + seq * seq_len + klow;
 #pragma unroll
             for (int m = 0; m < 8; m++) {
@@ -404,6 +424,19 @@ fftp_kernel(const float2* __restrict__ x, void* __restrict__ out_, long long row
     }
     if (row + row_step < rows) __syncthreads();   // the next row's F0 overwrites the shared memory F3 just read
     }  // rows
+    if constexpr (PSUM) {
+        constexpr int FN = SQ ? 16 * SQ : NATQ ? 256 * NATQ : N;
+        if constexpr (N / FN > 1) {
+            __syncthreads();   // the slots other threads of this CTA wrote
+            float* o = reinterpret_cast<float*>(out_) + (size_t)blockIdx.x * N;
+            for (int k = t; k < FN; k += NT) {
+                float s = o[k];
+#pragma unroll 4
+                for (int j = 1; j < N / FN; j++) s += o[j * FN + k];
+                o[k] = s;
+            }
+        }
+    }
 }
 
 
@@ -677,12 +710,13 @@ const float* fftp_twiddles() {
 
 namespace {
 
+// grid: CTAs that loop over the rows (0: one CTA per row); frames: fftp_kernel<PSUM>'s frame count
 template <int R0, bool INV, bool SI, bool SO, bool MAG, bool ROWS = false, int TQ = 0, int NATQ = 0, bool RIN = false, int SQ = 0,
-          bool FRAMES = false>
+          bool FRAMES = false, bool PSUM = false>
 int fftp_launch(const void* in, void* out, size_t rows, float scale, cudaStream_t st, int n1 = 1, int n2c = 1, size_t hop = 0,
-                const float* win = nullptr) {
+                const float* win = nullptr, size_t frames = 0, size_t grid = 0) {
     const size_t smem = (size_t)2 * R0 * FP_B_OF(R0) * sizeof(float);
-    auto kern = fftp_kernel<R0, INV, SI, SO, MAG, ROWS, TQ, NATQ, RIN, SQ, FRAMES>;
+    auto kern = fftp_kernel<R0, INV, SI, SO, MAG, ROWS, TQ, NATQ, RIN, SQ, FRAMES, PSUM>;
     static PerDeviceOnce configured;   // per instantiation and device
     if (configured.need()) {
         BDSP_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -690,8 +724,8 @@ int fftp_launch(const void* in, void* out, size_t rows, float scale, cudaStream_
     }
     const float* tw = fftp_twiddles();
     if (!tw) return -1001;
-    kern<<<(unsigned)rows, 128 * R0, smem, st>>>(reinterpret_cast<const float2*>(in), out, (long long)rows, scale, tw, n1, n2c,
-                                                  (long long)hop, win);
+    kern<<<(unsigned)(grid ? grid : rows), 128 * R0, smem, st>>>(reinterpret_cast<const float2*>(in), out, (long long)rows, scale, tw, n1,
+                                                                 n2c, (long long)hop, win, (long long)frames);
     BDSP_CUDA_OK(cudaGetLastError());
     BDSP_LAUNCHED();
     return 0;
@@ -793,6 +827,27 @@ int fftp_frames(const void* in, void* out, size_t n, size_t groups, size_t hop, 
 }
 template int fftp_frames<false>(const void*, void*, size_t, size_t, size_t, const float*, bool, bool, double, cudaStream_t);
 template int fftp_frames<true>(const void*, void*, size_t, size_t, size_t, const float*, bool, bool, double, cudaStream_t);
+
+// Welch power sums over frames of n = 64 .. 8192 points that start `hop` points apart (welch_route): `groups` groups of N / n
+// frames (N = 4096, or 8192), the last one possibly incomplete; `ctas` CTAs each leave the sums of their groups' |X|^2 in
+// part[cta * N + k], k < n.  win: n real multipliers on the first load, or null; RIN: the frames hold real scalars
+template <bool RIN>
+int fftp_frames_psum(const void* in, float* part, size_t n, size_t groups, size_t ctas, size_t hop, size_t frames, const float* win,
+                     cudaStream_t st) {
+    switch (n) {
+    case 64: return fftp_launch<1, false, false, false, false, false, 0, 1, RIN, 4, true, true>(in, part, groups, 1.f, st, 1, 1, hop, win, frames, ctas);
+    case 128: return fftp_launch<1, false, false, false, false, false, 0, 1, RIN, 8, true, true>(in, part, groups, 1.f, st, 1, 1, hop, win, frames, ctas);
+    case 256: return fftp_launch<1, false, false, false, false, false, 0, 1, RIN, 0, true, true>(in, part, groups, 1.f, st, 1, 1, hop, win, frames, ctas);
+    case 512: return fftp_launch<1, false, false, false, false, false, 0, 2, RIN, 0, true, true>(in, part, groups, 1.f, st, 1, 1, hop, win, frames, ctas);
+    case 1024: return fftp_launch<1, false, false, false, false, false, 0, 4, RIN, 0, true, true>(in, part, groups, 1.f, st, 1, 1, hop, win, frames, ctas);
+    case 2048: return fftp_launch<1, false, false, false, false, false, 0, 8, RIN, 0, true, true>(in, part, groups, 1.f, st, 1, 1, hop, win, frames, ctas);
+    case 4096: return fftp_launch<1, false, false, false, false, false, 0, 0, RIN, 0, true, true>(in, part, groups, 1.f, st, 1, 1, hop, win, frames, ctas);
+    case 8192: return fftp_launch<2, false, false, false, false, false, 0, 0, RIN, 0, true, true>(in, part, groups, 1.f, st, 1, 1, hop, win, frames, ctas);
+    default: set_last_error("fftp_frames_psum: no kernel for %zu points", n); return -2;
+    }
+}
+template int fftp_frames_psum<false>(const void*, float*, size_t, size_t, size_t, size_t, size_t, const float*, cudaStream_t);
+template int fftp_frames_psum<true>(const void*, float*, size_t, size_t, size_t, size_t, size_t, const float*, cudaStream_t);
 
 // two-pass transform for n = 2^15 .. 2^20 (FftRoute::TwoPass), n = p.n1 * 2^p.log2n2; tmp holds n*rows complex values
 int fftp_two_pass(const void* in, void* out, void* tmp, const FftPlan& p, size_t rows, bool inverse, bool si, bool so, bool magnitude,

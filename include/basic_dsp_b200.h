@@ -535,6 +535,24 @@ int32_t bdsp_fft_frames_c64(const void* in, void* out, size_t points, size_t hop
  * the input range overlap.  points == 0 or frames == 0 returns 0 without a launch. */
 int32_t bdsp_ifft_frames_c32(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
 int32_t bdsp_ifft_frames_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
+#define BDSP_F_ONESIDED 32        /* bdsp_welch_*: real input only, points/2 + 1 bins, interior bins doubled */
+#define BDSP_F_POWER_SPECTRUM 64  /* bdsp_welch_*: scaling 1/(sum w)^2 (power per bin) instead of the density 1/(fs sum w^2) */
+/* Welch's averaged periodogram of a device signal (scipy.signal.welch with detrend=False, MATLAB pwelch): the power
+ * spectrum estimate from the frames of bdsp_fft_frames_* (frame f = the `points` points, or real scalars with
+ * BDSP_F_REAL_INPUT, that start at point f*hop; no padding, no centring, hop > points allowed):
+ *   out[k] = scale / frames * sum_f |X_f[k]|^2,  X_f = DFT(w * frame f),
+ * w = the built-in window BDSP_F_WINDOW(kind), or 1 without it; scale = 1/(fs sum w^2) (density, the default) or, with
+ * BDSP_F_POWER_SPECTRUM, 1/(sum w)^2 (fs is then ignored).  `out` receives `points` real values (float for c32, double
+ * for c64) in np.fft.fftfreq order, fftshift order with BDSP_F_SHIFT; with BDSP_F_ONESIDED (real input only) points/2 + 1
+ * values, bins 0 .. points/2, each doubled but bin 0 and the Nyquist bin of an even `points`.  The sums run in a fixed
+ * order without atomics: repeated calls, on any device, give the same bytes.  The frames' spectra are never stored
+ * whole: the workspace stays bounded whatever `frames` is.
+ * flags: BDSP_F_REAL_INPUT, BDSP_F_SHIFT, BDSP_F_WINDOW(kind), BDSP_F_ONESIDED, BDSP_F_POWER_SPECTRUM.  Returns 0; -2 for
+ * any other flag (bdsp_last_error names it), BDSP_F_ONESIDED without BDSP_F_REAL_INPUT or with BDSP_F_SHIFT, hop == 0,
+ * fs not finite or not > 0 (unless BDSP_F_POWER_SPECTRUM), sizes that overflow size_t; -3 when the output overlaps the
+ * input range.  points == 0 or frames == 0 returns 0 without a launch and leaves `out` untouched. */
+int32_t bdsp_welch_c32(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags, float fs);
+int32_t bdsp_welch_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags, double fs);
 /* convolve_signal for every row with one impulse response of h_points complex taps (device pointer);
  * `plan` caches the impulse-response spectrum between calls (create once, reuse, destroy) */
 typedef struct BdspConvPlan BdspConvPlan;
