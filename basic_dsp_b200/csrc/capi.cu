@@ -1372,38 +1372,79 @@ template <typename T> int ifft_frames(const void* in, void* out, size_t points, 
     return ifft_frames_exec<T>(in, out, points, hop, frames, o, real_out, g_stream);
 }
 
+// The checks shared by the averaged-spectrum entry points (welch, csd, coherence), in this order: the flags (`known` are
+// accepted and listed in `accepted`; any other is named), BDSP_F_ONESIDED only with BDSP_F_REAL_INPUT and without
+// BDSP_F_SHIFT, hop >= 1, fs finite and > 0 where it is used, sizes that fit size_t.  Returns -2 with bdsp_last_error set,
+// or 0 with the byte counts of one input signal and of the output (out_esz bytes per output value); both 0 for an empty
+// call (points or frames 0).
+template <typename T>
+int spectrum_args(const char* fn, int flags, int known, const char* accepted, size_t points, size_t hop, size_t frames, bool fs_used,
+                  double fs, size_t out_esz, size_t* in_bytes, size_t* out_bytes) {
+    *in_bytes = *out_bytes = 0;
+    const int unknown = flags & ~known;
+    if (unknown) {
+        const char* name = (unknown & BDSP_F_INVERSE) ? "BDSP_F_INVERSE" : (unknown & BDSP_F_MAGNITUDE) ? "BDSP_F_MAGNITUDE"
+                         : (unknown & BDSP_F_REAL_OUTPUT) ? "BDSP_F_REAL_OUTPUT" : (unknown & BDSP_F_POWER_SPECTRUM) ? "BDSP_F_POWER_SPECTRUM"
+                         : nullptr;
+        if (name) set_last_error("%s: %s is not accepted (%s are)", fn, name, accepted);
+        else set_last_error("%s: unknown flag bits 0x%x", fn, (unsigned)unknown);
+        return -2;
+    }
+    const bool real = (flags & BDSP_F_REAL_INPUT) != 0, shift = (flags & BDSP_F_SHIFT) != 0, onesided = (flags & BDSP_F_ONESIDED) != 0;
+    if (onesided && !real) { set_last_error("%s: BDSP_F_ONESIDED needs BDSP_F_REAL_INPUT (a complex signal has no symmetric spectrum)", fn); return -2; }
+    if (onesided && shift) { set_last_error("%s: BDSP_F_ONESIDED and BDSP_F_SHIFT exclude each other", fn); return -2; }
+    if (!hop) { set_last_error("%s: hop must be at least 1", fn); return -2; }
+    if (fs_used && !(isfinite(fs) && fs > 0)) { set_last_error("%s: the sampling rate fs must be finite and > 0", fn); return -2; }
+    if (!points || !frames) return 0;
+    const size_t in_esz = real ? sizeof(T) : 2 * sizeof(T);
+    const size_t max = ~(size_t)0;
+    if (frames - 1 > (max - points) / hop || ((frames - 1) * hop + points) > max / in_esz || points > max / out_esz) {
+        set_last_error("%s: %zu frames of %zu points, hop %zu overflow the address space", fn, frames, points, hop);
+        return -2;
+    }
+    *in_bytes = ((frames - 1) * hop + points) * in_esz;
+    *out_bytes = (onesided ? points / 2 + 1 : points) * out_esz;
+    return 0;
+}
+
+static bool ranges_overlap(const void* a, size_t a_bytes, const void* b, size_t b_bytes) {
+    const uintptr_t a0 = reinterpret_cast<uintptr_t>(a), b0 = reinterpret_cast<uintptr_t>(b);
+    return a0 < b0 + b_bytes && b0 < a0 + a_bytes;
+}
+
 // Welch's averaged periodogram of a signal's frames (scipy.signal.welch with detrend=False, MATLAB pwelch): the frames of
 // fft_frames, |X|^2 averaged over them and scaled as a density or a power spectrum, two-sided or one-sided
 template <typename T> int welch(const void* in, void* out, size_t points, size_t hop, size_t frames, int flags, double fs) {
     const int known = BDSP_F_REAL_INPUT | BDSP_F_SHIFT | (15 << 8) | BDSP_F_ONESIDED | BDSP_F_POWER_SPECTRUM;   // (15 << 8): BDSP_F_WINDOW(kind)
-    const int unknown = flags & ~known;
-    if (unknown) {
-        const char* name = (unknown & BDSP_F_INVERSE) ? "BDSP_F_INVERSE" : (unknown & BDSP_F_MAGNITUDE) ? "BDSP_F_MAGNITUDE"
-                         : (unknown & BDSP_F_REAL_OUTPUT) ? "BDSP_F_REAL_OUTPUT" : nullptr;
-        if (name) set_last_error("welch: %s is not accepted (BDSP_F_REAL_INPUT, BDSP_F_SHIFT, BDSP_F_WINDOW(kind), BDSP_F_ONESIDED, "
-                                 "BDSP_F_POWER_SPECTRUM are)", name);
-        else set_last_error("welch: unknown flag bits 0x%x", (unsigned)unknown);
-        return -2;
-    }
-    const bool real = (flags & BDSP_F_REAL_INPUT) != 0, shift = (flags & BDSP_F_SHIFT) != 0, onesided = (flags & BDSP_F_ONESIDED) != 0;
     const bool power = (flags & BDSP_F_POWER_SPECTRUM) != 0;
-    if (onesided && !real) { set_last_error("welch: BDSP_F_ONESIDED needs BDSP_F_REAL_INPUT (a complex signal has no symmetric spectrum)"); return -2; }
-    if (onesided && shift) { set_last_error("welch: BDSP_F_ONESIDED and BDSP_F_SHIFT exclude each other"); return -2; }
-    if (!hop) { set_last_error("welch: hop must be at least 1"); return -2; }
-    if (!power && !(isfinite(fs) && fs > 0)) { set_last_error("welch: the sampling rate fs must be finite and > 0"); return -2; }
-    if (!points || !frames) return 0;
-    const size_t in_esz = real ? sizeof(T) : 2 * sizeof(T);
-    const size_t max = ~(size_t)0;
-    if (frames - 1 > (max - points) / hop || ((frames - 1) * hop + points) > max / in_esz || points > max / sizeof(T)) {
-        set_last_error("welch: %zu frames of %zu points, hop %zu overflow the address space", frames, points, hop);
-        return -2;
-    }
-    const uintptr_t i0 = reinterpret_cast<uintptr_t>(in), o0 = reinterpret_cast<uintptr_t>(out);
-    const size_t in_bytes = ((frames - 1) * hop + points) * in_esz, out_bytes = (onesided ? points / 2 + 1 : points) * sizeof(T);
-    if (i0 < o0 + out_bytes && o0 < i0 + in_bytes) { set_last_error("welch: the output overlaps the input"); return -3; }
+    size_t in_bytes, out_bytes;
+    const int rc = spectrum_args<T>("welch", flags, known, "BDSP_F_REAL_INPUT, BDSP_F_SHIFT, BDSP_F_WINDOW(kind), BDSP_F_ONESIDED, BDSP_F_POWER_SPECTRUM",
+                                    points, hop, frames, !power, fs, sizeof(T), &in_bytes, &out_bytes);
+    if (rc || !in_bytes) return rc;
+    if (ranges_overlap(in, in_bytes, out, out_bytes)) { set_last_error("welch: the output overlaps the input"); return -3; }
     const int wk = (flags >> 8) & 15;
-    const FftOpts o = fft_opts<T>(points, false, shift, false, real, wk ? wk - 1 : RECTANGULAR);
-    return welch_exec<T>(in, static_cast<T*>(out), points, hop, frames, o, onesided, power, fs, g_stream);
+    const FftOpts o = fft_opts<T>(points, false, (flags & BDSP_F_SHIFT) != 0, false, (flags & BDSP_F_REAL_INPUT) != 0, wk ? wk - 1 : RECTANGULAR);
+    return welch_exec<T>(in, static_cast<T*>(out), points, hop, frames, o, (flags & BDSP_F_ONESIDED) != 0, power, fs, g_stream);
+}
+
+// Cross-spectral density (scipy.signal.csd with detrend=False) or, with `coherence`, the magnitude-squared coherence
+// (scipy.signal.coherence) of two signals' frames, each framed as welch frames its input.  x and y are only read, so they
+// may be the same buffer; the output may overlap neither.
+template <typename T> int cross_spectrum(const void* x, const void* y, void* out, size_t points, size_t hop, size_t frames, int flags,
+                                         double fs, bool coherence) {
+    const char* fn = coherence ? "coherence" : "csd";
+    const int known = BDSP_F_REAL_INPUT | BDSP_F_SHIFT | (15 << 8) | BDSP_F_ONESIDED | (coherence ? 0 : BDSP_F_POWER_SPECTRUM);
+    const bool power = (flags & BDSP_F_POWER_SPECTRUM) != 0;
+    size_t in_bytes, out_bytes;
+    const int rc = spectrum_args<T>(fn, flags, known, coherence ? "BDSP_F_REAL_INPUT, BDSP_F_SHIFT, BDSP_F_WINDOW(kind), BDSP_F_ONESIDED"
+                                                                : "BDSP_F_REAL_INPUT, BDSP_F_SHIFT, BDSP_F_WINDOW(kind), BDSP_F_ONESIDED, BDSP_F_POWER_SPECTRUM",
+                                    points, hop, frames, !coherence && !power, fs, coherence ? sizeof(T) : 2 * sizeof(T), &in_bytes, &out_bytes);
+    if (rc || !in_bytes) return rc;
+    if (ranges_overlap(x, in_bytes, out, out_bytes)) { set_last_error("%s: the output overlaps x", fn); return -3; }
+    if (ranges_overlap(y, in_bytes, out, out_bytes)) { set_last_error("%s: the output overlaps y", fn); return -3; }
+    const int wk = (flags >> 8) & 15;
+    const FftOpts o = fft_opts<T>(points, false, (flags & BDSP_F_SHIFT) != 0, false, (flags & BDSP_F_REAL_INPUT) != 0, wk ? wk - 1 : RECTANGULAR);
+    return csd_exec<T>(x, y, out, points, hop, frames, o, (flags & BDSP_F_ONESIDED) != 0, power, fs, coherence, g_stream);
 }
 
 // ---- batched (matrix-row) forms: the reference's MatrixMxN applies the vector operation to every row in turn
@@ -1804,6 +1845,18 @@ extern "C" int32_t bdsp_welch_c32(const void* in, void* out, size_t points, size
 }
 extern "C" int32_t bdsp_welch_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags, double fs) {
     return welch<double>(in, out, points, hop, frames, flags, fs);
+}
+extern "C" int32_t bdsp_csd_c32(const void* x, const void* y, void* out, size_t points, size_t hop, size_t frames, int32_t flags, float fs) {
+    return cross_spectrum<float>(x, y, out, points, hop, frames, flags, (double)fs, false);
+}
+extern "C" int32_t bdsp_csd_c64(const void* x, const void* y, void* out, size_t points, size_t hop, size_t frames, int32_t flags, double fs) {
+    return cross_spectrum<double>(x, y, out, points, hop, frames, flags, fs, false);
+}
+extern "C" int32_t bdsp_coherence_c32(const void* x, const void* y, void* out, size_t points, size_t hop, size_t frames, int32_t flags) {
+    return cross_spectrum<float>(x, y, out, points, hop, frames, flags, 1.0, true);
+}
+extern "C" int32_t bdsp_coherence_c64(const void* x, const void* y, void* out, size_t points, size_t hop, size_t frames, int32_t flags) {
+    return cross_spectrum<double>(x, y, out, points, hop, frames, flags, 1.0, true);
 }
 extern "C" BdspConvPlan* bdsp_conv_plan_create_c32(const void* h, size_t L) { return reinterpret_cast<BdspConvPlan*>(conv_plan_create<float>(h, L)); }
 extern "C" BdspConvPlan* bdsp_conv_plan_create_c64(const void* h, size_t L) { return reinterpret_cast<BdspConvPlan*>(conv_plan_create<double>(h, L)); }

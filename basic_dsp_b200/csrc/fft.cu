@@ -109,8 +109,9 @@ template <> const double2* twiddle_table<double>() { DeviceState* s = dev_state(
 // workspace_bind_stream (capi: bdsp_set_stream).  Slots: 0..3 the transforms and reductions, 4..5 the full-length
 // convolution (its buffers stay live across nested fft_exec calls, which use 0..2), 6 the frame buffers of the frame
 // entry points: the gathered frames of FftRoute::FramePass and the inverse rows of ifft_frames_exec (live across the
-// transform that fills or reads them, which may use 0..3), 7..8 welch_exec: 7 a chunk of frame spectra (filled by a frame
-// transform, which may use 0..3 and 6), 8 the window sums and the partial rows (live across every chunk).
+// transform that fills or reads them, which may use 0..3), 7..8 welch_exec and csd_exec: 7 a chunk of frame spectra
+// (csd_exec: the chunk spectra of x, then of y; filled by frame transforms, which may use 0..3 and 6), 8 the window sums
+// and the partial rows (live across every chunk).
 namespace {
 thread_local cudaStream_t tl_ws_stream = nullptr;
 constexpr int WS_SLOTS = 9;
@@ -982,6 +983,71 @@ __global__ void __launch_bounds__(256) welch_final_kernel(const P* __restrict__ 
     out[j] = (T)v;
 }
 
+// part[c * rows + i] (+)= the sums over the frames s, s + slabs, ... < frames of the chunk at bin k (rows = slabs * nout,
+// slab s = i / nout, k = i % nout): c = 0, 1 Re and Im of conj(X[k]) Y[k]; with COH c = 2, 3 |X[k]|^2 and |Y[k]|^2 (formed
+// as welch_accumulate_kernel forms |X|^2).  Every product and sum of a frame's term is rounded in T on its own, so that
+// csd(x, x) has an imaginary part of exactly 0 and csd(y, x) = conj(csd(x, y)) byte for byte; the sums over frames are
+// kept in double.  The first chunk stores.
+template <typename T, bool COH>
+__global__ void csd_accumulate_kernel(const typename CpxOf<T>::type* __restrict__ xs, const typename CpxOf<T>::type* __restrict__ ys,
+                                      double* __restrict__ part, long long n, long long nout, long long frames, long long slabs, int first) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long rows = slabs * nout, s = i / nout;
+    if (i >= rows || s >= frames) return;
+    double re = 0, im = 0, xx = 0, yy = 0;
+    if (!first) {
+        re = part[i];
+        im = part[rows + i];
+        if (COH) { xx = part[2 * rows + i]; yy = part[3 * rows + i]; }
+    }
+#pragma unroll 4
+    for (long long j = s * n + (i - s * nout); j < frames * n; j += slabs * n) {
+        const typename CpxOf<T>::type a = xs[j], b = ys[j];
+        re += (double)add_rn(mul_rn(a.x, b.x), mul_rn(a.y, b.y));
+        im += (double)sub_rn(mul_rn(a.x, b.y), mul_rn(a.y, b.x));
+        if (COH) {
+            xx += (double)add_rn(mul_rn(a.x, a.x), mul_rn(a.y, a.y));
+            yy += (double)add_rn(mul_rn(b.x, b.x), mul_rn(b.y, b.y));
+        }
+    }
+    part[i] = re;
+    part[rows + i] = im;
+    if (COH) { part[2 * rows + i] = xx; part[3 * rows + i] = yy; }
+}
+
+// Output j of bdsp_csd_* / bdsp_coherence_*: bin k = j (shift: (j + n - n/2) mod n); each sum of csd_accumulate_kernel
+// added over the `rows` partial rows of nout bins in welch_final_kernel's order.  csd: the complex value scaled and folded
+// as welch_final_kernel does; COH: |Sxy|^2 / (Sxx Syy) in double, NaN where x or y has no power.
+template <typename T, bool COH>
+__global__ void __launch_bounds__(256) csd_final_kernel(const double* __restrict__ part, long long rows, const double* __restrict__ sums,
+                                                        void* __restrict__ out, long long n, long long nout, int shift, int onesided, int power,
+                                                        double fs, long long frames) {
+    constexpr int K = COH ? 4 : 2;
+    __shared__ double lane[K][8][33];
+    const long long j = (long long)blockIdx.x * 32 + threadIdx.x;
+    const long long k = shift ? (j + n - n / 2) % n : j, comp = rows * nout;
+    double s[K] = {};
+    if (j < nout) {
+#pragma unroll 4
+        for (long long r = threadIdx.y; r < rows; r += 8)
+            for (int c = 0; c < K; c++) s[c] += part[c * comp + r * nout + k];
+    }
+    for (int c = 0; c < K; c++) lane[c][threadIdx.y][threadIdx.x] = s[c];
+    __syncthreads();
+    if (threadIdx.y != 0 || j >= nout) return;
+    for (int y = 1; y < 8; y++)
+        for (int c = 0; c < K; c++) s[c] += lane[c][y][threadIdx.x];
+    if (COH) {
+        static_cast<T*>(out)[j] = (T)(add_rn(mul_rn(s[0], s[0]), mul_rn(s[1], s[1])) / mul_rn(s[2], s[3]));
+        return;
+    }
+    const double sw = sums ? sums[0] : (double)n, sw2 = sums ? sums[1] : (double)n;
+    const double den = (double)frames * (power ? sw * sw : fs * sw2);
+    double re = s[0] / den, im = s[1] / den;
+    if (onesided && k != 0 && 2 * k != n) { re *= 2; im *= 2; }
+    static_cast<typename CpxOf<T>::type*>(out)[j] = mk<T>((T)re, (T)im);
+}
+
 template <typename T, bool INV>
 int fft_any(const void* in, void* out, size_t n, size_t batch, const FftOpts& o, void* work, size_t work_bytes,
             cudaStream_t st) {
@@ -1190,6 +1256,22 @@ int ifft_frames_exec(const void* in, void* out, size_t n, size_t hop, size_t fra
 template int ifft_frames_exec<float>(const void*, void*, size_t, size_t, size_t, const FftOpts&, bool, cudaStream_t);
 template int ifft_frames_exec<double>(const void*, void*, size_t, size_t, size_t, const FftOpts&, bool, cudaStream_t);
 
+// The window table of opts (built-in window, kind 3) in slot 3, the multiplier of the frame transforms of welch_exec and
+// csd_exec, and with `sums` its sums (window_sums_kernel); *win stays null without a window
+template <typename T>
+int spectrum_window(const FftOpts& opts, size_t n, double* sums, const T** win, cudaStream_t stream) {
+    if (opts.in_mul.kind != 3) return 0;
+    BDSP_WS(tab, T*, n * sizeof(T), 3);
+    window_table_kernel<T><<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(tab, (long long)n, opts.in_mul.arg);
+    BDSP_LAUNCHED();
+    if (sums) {
+        window_sums_kernel<T><<<1, 1024, 0, stream>>>(tab, (long long)n, sums);
+        BDSP_LAUNCHED();
+    }
+    *win = tab;
+    return 0;
+}
+
 template <typename T>
 int welch_exec(const void* in, T* out, size_t n, size_t hop, size_t frames, const FftOpts& opts, bool onesided, bool power_spectrum, double fs,
                cudaStream_t stream) {
@@ -1210,14 +1292,7 @@ int welch_exec(const void* in, T* out, size_t n, size_t hop, size_t frames, cons
     double* sums = reinterpret_cast<double*>(ws);
     void* part = ws + 2 * sizeof(double);
     const T* win = nullptr;
-    if (opts.in_mul.kind == 3) {
-        BDSP_WS(tab, T*, n * sizeof(T), 3);
-        window_table_kernel<T><<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(tab, (long long)n, opts.in_mul.arg);
-        BDSP_LAUNCHED();
-        window_sums_kernel<T><<<1, 1024, 0, stream>>>(tab, (long long)n, sums);
-        BDSP_LAUNCHED();
-        win = tab;
-    }
+    if (const int rc = spectrum_window<T>(opts, n, sums, &win, stream)) return rc;
     const size_t nout = onesided ? n / 2 + 1 : n;
     const dim3 block(32, 8);
     const unsigned grid = (unsigned)((nout + 31) / 32);
@@ -1258,5 +1333,53 @@ int welch_exec(const void* in, T* out, size_t n, size_t hop, size_t frames, cons
 
 template int welch_exec<float>(const void*, float*, size_t, size_t, size_t, const FftOpts&, bool, bool, double, cudaStream_t);
 template int welch_exec<double>(const void*, double*, size_t, size_t, size_t, const FftOpts&, bool, bool, double, cudaStream_t);
+
+template <typename T>
+int csd_exec(const void* x, const void* y, void* out, size_t n, size_t hop, size_t frames, const FftOpts& opts, bool onesided,
+             bool power_spectrum, double fs, bool coherence, cudaStream_t stream) {
+    typedef typename CpxOf<T>::type C;
+    if (n == 0 || frames == 0) return 0;
+    const size_t esz = opts.real_input ? sizeof(T) : sizeof(C);
+    const CsdPlan plan = csd_plan(sizeof(T) == 8, n, frames);
+    // slot 8: the window sums, then 2 (coherence: 4) sums of `slabs` partial rows of the nout output bins
+    const size_t nout = onesided ? n / 2 + 1 : n, rows = plan.slabs * nout;
+    BDSP_WS(ws, double*, (2 + (coherence ? 4 : 2) * rows) * sizeof(double), 8);
+    double* sums = ws;
+    const T* win = nullptr;
+    if (const int rc = spectrum_window<T>(opts, n, coherence ? nullptr : sums, &win, stream)) return rc;
+    // every chunk: the frame transforms of x and of y (fft_exec's routes for strided frames, the window table as their
+    // multiplier) into the two halves of slot 7, then the cross sums added into the partial rows
+    BDSP_WS(xs, C*, 2 * plan.chunk * n * sizeof(C), 7);
+    C* ys = xs + plan.chunk * n;
+    FftOpts o;
+    o.real_input = opts.real_input;
+    o.in_stride = hop;
+    if (win) { o.in_mul.p = win; o.in_mul.kind = 1; }
+    const unsigned acc_grid = (unsigned)((rows + 255) / 256);
+    for (size_t f0 = 0; f0 < frames; f0 += plan.chunk) {
+        const size_t cf = frames - f0 < plan.chunk ? frames - f0 : plan.chunk;
+        int rc = fft_exec<T>(static_cast<const char*>(x) + f0 * hop * esz, xs, n, cf, o, nullptr, 0, stream);
+        if (rc) return rc;
+        rc = fft_exec<T>(static_cast<const char*>(y) + f0 * hop * esz, ys, n, cf, o, nullptr, 0, stream);
+        if (rc) return rc;
+        if (coherence) csd_accumulate_kernel<T, true><<<acc_grid, 256, 0, stream>>>(xs, ys, ws + 2, (long long)n, (long long)nout, (long long)cf,
+                                                                                    (long long)plan.slabs, f0 == 0);
+        else csd_accumulate_kernel<T, false><<<acc_grid, 256, 0, stream>>>(xs, ys, ws + 2, (long long)n, (long long)nout, (long long)cf,
+                                                                          (long long)plan.slabs, f0 == 0);
+        BDSP_LAUNCHED();
+    }
+    const dim3 block(32, 8);
+    const unsigned grid = (unsigned)((nout + 31) / 32);
+    const int shift = opts.out_rot != 0;
+    if (coherence) csd_final_kernel<T, true><<<grid, block, 0, stream>>>(ws + 2, (long long)plan.slabs, nullptr, out, (long long)n, (long long)nout,
+                                                                         shift, onesided, 0, 0.0, (long long)frames);
+    else csd_final_kernel<T, false><<<grid, block, 0, stream>>>(ws + 2, (long long)plan.slabs, win ? sums : nullptr, out, (long long)n,
+                                                                (long long)nout, shift, onesided, power_spectrum, fs, (long long)frames);
+    BDSP_LAUNCHED();
+    return 0;
+}
+
+template int csd_exec<float>(const void*, const void*, void*, size_t, size_t, size_t, const FftOpts&, bool, bool, double, bool, cudaStream_t);
+template int csd_exec<double>(const void*, const void*, void*, size_t, size_t, size_t, const FftOpts&, bool, bool, double, bool, cudaStream_t);
 
 }  // namespace bdsp

@@ -46,6 +46,15 @@ template <typename T>
 int welch_exec(const void* in, T* out, size_t n, size_t hop, size_t frames, const FftOpts& opts, bool onesided, bool power_spectrum,
                double fs, cudaStream_t stream);
 
+// Cross-spectral density (bdsp_csd_*) of the frames x_f and y_f, taken from x and from y as welch_exec takes them:
+// out[k] = scale / frames * sum_f conj(X_f[k]) Y_f[k], X_f = DFT(w x_f), Y_f = DFT(w y_f), complex, with welch_exec's scale,
+// order and one-sided fold.  With `coherence` (bdsp_coherence_*): out[k] = |sum_f conj(X_f) Y_f|^2 / (sum_f |X_f|^2
+// sum_f |Y_f|^2), real, unscaled (power_spectrum and fs unused), NaN where x or y has no power.  x and y may overlap; out
+// may not overlap either.  Bit-reproducible, and the workspace stays bounded whatever `frames` is (fft_route.h csd_plan).
+template <typename T>
+int csd_exec(const void* x, const void* y, void* out, size_t n, size_t hop, size_t frames, const FftOpts& opts, bool onesided,
+             bool power_spectrum, double fs, bool coherence, cudaStream_t stream);
+
 // largest n the single-CTA shared-memory kernel handles for this precision
 template <typename T> size_t fft_block_max_n();
 

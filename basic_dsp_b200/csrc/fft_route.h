@@ -190,4 +190,27 @@ inline WelchPlan welch_route(bool f64, size_t n, size_t hop, size_t frames, bool
     return {true, groups, groups < cap ? groups : cap};
 }
 
+// Cross-spectral density and coherence (fft.cu csd_exec, bdsp_csd_* / bdsp_coherence_*): the frames of x and of y are
+// transformed chunk by chunk (fft_exec with the frame stride, the routes of bdsp_fft_frames_*) into two chunk spectra at
+// fixed workspace addresses, then summed into `slabs` partial rows.  A chunk holds at most CSD_CHUNK_POINTS spectrum points
+// per signal (one frame when n is larger) and, for c32 below 4096 points, a whole number of groups of 4096 / n frames, so
+// that every chunk but the last keeps the packed frames route where the frames take it.  CSD_CHUNK_POINTS = 2^24: of 2^20 ...
+// 2^24 on a B200 at 1000 W (profiles/r3_csd.txt) the fastest for six of the eight outputs of the four benchmark workloads
+// and within 1 % of the fastest for the other two.  Chunks small enough for both c32 chunk spectra to fit the 126 MB L2
+// (2^22, 64 MB) did not pay: 8 % slower on 1024-point frames of a 2^28-sample signal, 14 % on 4096-point frames, as every
+// chunk adds its launches and the tails of three kernels.  About CSD_ACC_THREADS threads sum the partial rows.
+struct CsdPlan {
+    size_t chunk = 0, slabs = 0;   // frames per chunk, partial rows
+};
+constexpr size_t CSD_CHUNK_POINTS = (size_t)1 << 24, CSD_ACC_THREADS = (size_t)1 << 18;
+
+inline CsdPlan csd_plan(bool f64, size_t n, size_t frames) {
+    if (n == 0 || frames == 0) return {};
+    const size_t per = !f64 && n >= 64 && n < 4096 ? 4096 / n : 1;
+    const size_t whole = n > CSD_CHUNK_POINTS ? 1 : CSD_CHUNK_POINTS / n / per * per;
+    const size_t chunk = whole < frames ? whole : frames;
+    const size_t slabs = (CSD_ACC_THREADS + n - 1) / n;
+    return {chunk, slabs < chunk ? slabs : chunk};
+}
+
 }  // namespace bdsp

@@ -535,8 +535,10 @@ int32_t bdsp_fft_frames_c64(const void* in, void* out, size_t points, size_t hop
  * the input range overlap.  points == 0 or frames == 0 returns 0 without a launch. */
 int32_t bdsp_ifft_frames_c32(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
 int32_t bdsp_ifft_frames_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
-#define BDSP_F_ONESIDED 32        /* bdsp_welch_*: real input only, points/2 + 1 bins, interior bins doubled */
-#define BDSP_F_POWER_SPECTRUM 64  /* bdsp_welch_*: scaling 1/(sum w)^2 (power per bin) instead of the density 1/(fs sum w^2) */
+#define BDSP_F_ONESIDED 32        /* bdsp_welch_*, bdsp_csd_*, bdsp_coherence_*: real input only, points/2 + 1 bins, interior
+                                     bins doubled (coherence: not doubled, the doubling cancels) */
+#define BDSP_F_POWER_SPECTRUM 64  /* bdsp_welch_*, bdsp_csd_*: scaling 1/(sum w)^2 (power per bin) instead of the density
+                                     1/(fs sum w^2) */
 /* Welch's averaged periodogram of a device signal (scipy.signal.welch with detrend=False, MATLAB pwelch): the power
  * spectrum estimate from the frames of bdsp_fft_frames_* (frame f = the `points` points, or real scalars with
  * BDSP_F_REAL_INPUT, that start at point f*hop; no padding, no centring, hop > points allowed):
@@ -553,6 +555,32 @@ int32_t bdsp_ifft_frames_c64(const void* in, void* out, size_t points, size_t ho
  * input range.  points == 0 or frames == 0 returns 0 without a launch and leaves `out` untouched. */
 int32_t bdsp_welch_c32(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags, float fs);
 int32_t bdsp_welch_c64(const void* in, void* out, size_t points, size_t hop, size_t frames, int32_t flags, double fs);
+/* Cross-spectral density of two device signals (scipy.signal.csd with detrend=False): the frames of x and of y are taken
+ * as bdsp_welch_* takes its input's (frame f = the `points` points, or real scalars with BDSP_F_REAL_INPUT, that start at
+ * point f*hop of each signal), and
+ *   out[k] = scale / frames * sum_f conj(X_f[k]) * Y_f[k],  X_f = DFT(w * frame f of x),  Y_f = DFT(w * frame f of y),
+ * with bdsp_welch_*'s window w, scale, order and one-sided fold.  `out` receives complex values (interleaved float2 for
+ * c32, double2 for c64): `points` of them, or points/2 + 1 with BDSP_F_ONESIDED.  The sums run in a fixed order without
+ * atomics: repeated calls, on any device, give the same bytes; the workspace stays bounded whatever `frames` is.
+ * x and y are only read and may be the same buffer.
+ * flags: BDSP_F_REAL_INPUT, BDSP_F_SHIFT, BDSP_F_WINDOW(kind), BDSP_F_ONESIDED, BDSP_F_POWER_SPECTRUM.  Returns 0; -2 for
+ * any other flag (bdsp_last_error names it), BDSP_F_ONESIDED without BDSP_F_REAL_INPUT or with BDSP_F_SHIFT, hop == 0,
+ * fs not finite or not > 0 (unless BDSP_F_POWER_SPECTRUM), sizes that overflow size_t; -3 when the output overlaps the
+ * range of x or of y.  points == 0 or frames == 0 returns 0 without a launch and leaves `out` untouched. */
+int32_t bdsp_csd_c32(const void* x, const void* y, void* out, size_t points, size_t hop, size_t frames, int32_t flags, float fs);
+int32_t bdsp_csd_c64(const void* x, const void* y, void* out, size_t points, size_t hop, size_t frames, int32_t flags, double fs);
+/* Magnitude-squared coherence of two device signals (scipy.signal.coherence with detrend=False), over the frames of
+ * bdsp_csd_*:
+ *   out[k] = |sum_f conj(X_f[k]) Y_f[k]|^2 / (sum_f |X_f[k]|^2 * sum_f |Y_f[k]|^2),
+ * in [0, 1]; NaN in a bin where x or y has no power.  The scale and the one-sided doubling cancel, so there is no fs.
+ * `out` receives `points` real values (float for c32, double for c64), or points/2 + 1 with BDSP_F_ONESIDED, in the order
+ * of bdsp_csd_*.  Same guarantees as bdsp_csd_*.
+ * flags: BDSP_F_REAL_INPUT, BDSP_F_SHIFT, BDSP_F_WINDOW(kind), BDSP_F_ONESIDED.  Returns 0; -2 for any other flag
+ * (BDSP_F_POWER_SPECTRUM included), BDSP_F_ONESIDED without BDSP_F_REAL_INPUT or with BDSP_F_SHIFT, hop == 0, sizes that
+ * overflow size_t; -3 when the output overlaps the range of x or of y.  points == 0 or frames == 0 returns 0 without a
+ * launch and leaves `out` untouched. */
+int32_t bdsp_coherence_c32(const void* x, const void* y, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
+int32_t bdsp_coherence_c64(const void* x, const void* y, void* out, size_t points, size_t hop, size_t frames, int32_t flags);
 /* convolve_signal for every row with one impulse response of h_points complex taps (device pointer);
  * `plan` caches the impulse-response spectrum between calls (create once, reuse, destroy) */
 typedef struct BdspConvPlan BdspConvPlan;
