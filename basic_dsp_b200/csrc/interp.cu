@@ -160,7 +160,8 @@ interp_poly_tiled_kernel(const void* __restrict__ x_, void* __restrict__ y_, con
 // Real f32, F <= 4 (BASELINE config C4a): 8 positions x 4 phases per thread, everything packed FP32x2.
 // The input window is stored DUPLICATED ({x, x} pairs) so that one 64-bit shared load yields the splat
 // operand of FFMA2 without a MOV; per tap and thread: 1 LDS.128 (4 taps, warp-uniform) + 1 LDS.64 +
-// 16 FFMA2 for 32 outputs.
+// 16 FFMA2 for 32 outputs.  y16: y is 16-byte aligned, so F == 4 can be written with float4 stores (the row entry point
+// accepts any float-aligned output).
 // ------------------------------------------------------------------------------------------
 // threads per CTA: small CTAs keep the barrier-separated load / compute / store phases of different CTAs overlapping on
 // the SM.  Measured on B200 (C4a, 2^24 samples x4): 256 threads 0.160 ms, 128: 0.142, 64: 0.133, 32: 0.136 while the vector's last
@@ -177,7 +178,7 @@ __device__ __forceinline__ int ipf_skew(int i) { return i + (i >> IPF_LRP); }
 
 __global__ void __launch_bounds__(IPF_THREADS, 1024 / IPF_THREADS)
 interp_poly_f32_kernel(const float* __restrict__ x, float* __restrict__ y, const float* __restrict__ tab, long long N,
-                       long long new_points, int F, int L, long long scalar_len) {
+                       long long new_points, int F, int L, long long scalar_len, bool y16) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int J = 2 * L + 3;
     const int JI = 2 * L + 2;                                  // the last window slot has no interior tap
@@ -278,7 +279,7 @@ interp_poly_f32_kernel(const float* __restrict__ x, float* __restrict__ y, const
     }
     __syncthreads();
     float* yo = y + r0 * F;
-    if (F == 4) {   // 32 outputs per staging row: no integer division in the copy-out loop; 16-byte stores
+    if (F == 4 && y16) {   // 32 outputs per staging row: no integer division in the copy-out loop; 16-byte stores (y 16-byte aligned)
 #pragma unroll
         for (int it = 0; it < IPF_RP; it++) {
             const int o = 4 * (threadIdx.x + IPF_THREADS * it);
@@ -357,7 +358,8 @@ int interp_poly(const void* x, void* y, const T* tab_dev, size_t N, size_t new_p
             }
             interp_poly_f32_kernel<<<(unsigned)grid, IPF_THREADS, smem, st>>>(reinterpret_cast<const float*>(x), reinterpret_cast<float*>(y),
                                                                               reinterpret_cast<const float*>(tab_dev), (long long)N,
-                                                                              (long long)new_points, F, L, scalar_len);
+                                                                              (long long)new_points, F, L, scalar_len,
+                                                                              (reinterpret_cast<uintptr_t>(y) & 15) == 0);
         }
         else { if (F <= 4) BDSP_IP2(false, 4, 4); else BDSP_IP2(false, 8, 2); }
 #undef BDSP_IP2

@@ -610,7 +610,9 @@ int32_t bdsp_scale_mul_mag_phase_rows_c64(void* v, const void* w, void* magnitud
 /* interpolatef32 (facade32.rs:1334) on every one of `rows` rows of `points` points (is_complex: interleaved complex
  * points, else real scalars) with a built-in impulse response (0 Sinc, else RaisedCosine(rolloff)); delay is in samples
  * (delta = 1).  out must hold rows * new_points points, new_points = round(len * factor) rounded up to even in scalars
- * (interpolation.rs:406-410), also returned through *new_points (may be NULL).  The tap tables are built once. */
+ * (interpolation.rs:406-410), also returned through *new_points (may be NULL).  The tap tables are built once.  in and
+ * out may be any pointers aligned to their element type (float / double, or its complex pair); the kernels pick 16-byte
+ * stores only where out allows them. */
 int32_t bdsp_interpolatef_rows32(const void* in, void* out, size_t points, size_t rows, int32_t is_complex, int32_t impulse_response,
                                  float rolloff, float interpolation_factor, float delay, size_t len, size_t* new_points);
 int32_t bdsp_interpolatef_rows64(const void* in, void* out, size_t points, size_t rows, int32_t is_complex, int32_t impulse_response,

@@ -11,6 +11,8 @@ a GPU result with
 and asserts that the GPU's error is within a small factor of the peer's error, both for the whole row (`rel`) and for its
 worst element (`elmax`, relative to the row's RMS).
 """
+import ctypes
+import ctypes.util
 import math
 
 import numpy as np
@@ -245,3 +247,132 @@ def ols_block(dtype, L, complex_signal, N, rows):
     while m < 4 * max(L - 1, 1):
         m *= 2
     return min(max(m, 4096), 16384 if dtype == np.float32 else 8192), "generic"
+
+
+# ---- interpolation ---------------------------------------------------------------------------------------------------
+# interpolatef (dsp_oracle.interpolatef's formulas) with every output written as a sum over a window of 2L + 1 input
+# points in ascending order, y[i] = sum_k x[(start_i + k) mod N] * taps_i[k]:
+#   * polyphase path (integer factor F): the taps are the host-built tables in T, edge outputs (the first and last
+#     (2L + 1) F) start at i // F - L + 1 with v_s, s = i % F; interior outputs at ceil(i / F) - L - 1 with v_s reversed,
+#     s = (F - i % F) % F;
+#   * per-output path: start floor(i / F) - L, taps f(j + k) with j = -L - frac + delay, all in T.
+# The reference accumulates in float64 (f32 results) or long double (f64 results), the peer in T, tap by tap.
+_LIBM = None
+
+
+def _libm():
+    global _LIBM
+    if _LIBM is None:
+        _LIBM = ctypes.CDLL(ctypes.util.find_library("m"))
+        for name in ("sinf", "cosf"):
+            getattr(_LIBM, name).restype = ctypes.c_float
+            getattr(_LIBM, name).argtypes = [ctypes.c_float]
+    return _LIBM
+
+
+def impulse(kind, rolloff, dtype):
+    """Built-in impulse response (0 Sinc, else RaisedCosine(rolloff)) as the library's host code evaluates it (capi.cu
+    host_sinc / host_rc): every operation rounded to `dtype`, sin and cos from the C library.  numpy's float32 sin is not
+    sinf: it differs in the last bit for about one argument in six, and the polyphase tables must match bit for bit."""
+    T = np.dtype(dtype).type
+    sin, cos = (_libm().sinf, _libm().cosf) if T == np.float32 else (math.sin, math.cos)
+    one, two, pi, r = T(1), T(2), T(math.pi), T(rolloff)
+
+    def f(x):
+        x = T(x)
+        if x == 0:
+            return one
+        if kind == 0:
+            px = pi * x
+            return T(sin(px)) / px
+        if abs(x) == one / (two * r):
+            arg = pi / two / r
+            return T(sin(arg)) / arg * pi / (two * two)
+        px = pi * x
+        arg = two * r * x
+        return T(sin(px)) * T(cos(px * r)) / px / (one - arg * arg)
+    return f
+
+
+def impulse_vec(kind, rolloff, x, dtype):
+    """The same function over an array, in `dtype` with numpy's sin and cos (for the per-output path, whose kernel
+    evaluates its taps on the device)."""
+    T = np.dtype(dtype).type
+    x = np.asarray(x, dtype=T)
+    one, two, pi, r = T(1), T(2), T(math.pi), T(rolloff)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        px = pi * x
+        if kind == 0:
+            y = np.sin(px) / px
+        else:
+            arg = two * r * x
+            y = np.sin(px) * np.cos(px * r) / px / (one - arg * arg)
+            a = pi / two / r
+            y = np.where(np.abs(x) == one / (two * r), np.sin(a) / a * pi / (two * two), y)
+        return np.where(x == 0, one, y).astype(T)
+
+
+def interpf_windows(x_points, len_T, kind, rolloff, factor, delay, conv_len, dtype):
+    """(new_points, poly, start, taps) of interpolatef on a vector of x_points points (len_T scalars): start[i] is the
+    first input index of output i's window, taps[i] its 2L + 1 taps in ascending window order, in `dtype`."""
+    from oracle import dsp_oracle as o
+    T = np.dtype(dtype).type
+    N = x_points
+    L = min(conv_len, N // 2)
+    new_len = o.interpolatef_new_len(len_T, factor, dtype)
+    new_points = new_len // 2 if len_T == 2 * N else new_len
+    i = np.arange(new_points)
+    if o.interpolatef_uses_fast_path(L, new_len, factor, dtype):
+        F = int(np.round(T(factor)))
+        vs = o.interpolatef_tap_vectors(impulse(kind, rolloff, dtype), L, F, delay, dtype)
+        scalar_len = (2 * L + 1) * F
+        interior = (i >= scalar_len) & (i < new_points - scalar_len)
+        start = np.where(interior, -(-i // F) - L - 1, i // F - L + 1)
+        taps = np.where(interior[:, None], vs[(F - i % F) % F][:, ::-1], vs[i % F])
+        return new_points, True, start, taps
+    center = i.astype(T) / T(factor)
+    rounded = np.floor(center)
+    j = (-T(L) - (center - rounded)) + T(delay)
+    taps = np.empty((new_points, 2 * L + 1), dtype=T)
+    for k in range(2 * L + 1):
+        taps[:, k] = impulse_vec(kind, rolloff, j, dtype)
+        j = (j + T(1)).astype(T)
+    return new_points, False, rounded.astype(np.int64) - L, taps
+
+
+def interp_sum(x, start, taps, rt):
+    """y[i] = sum_k x[(start[i] + k) mod N] * taps[i, k], accumulated in real type `rt` (complex x: its complex type),
+    k ascending, every product and sum rounded to it."""
+    x = np.asarray(x)
+    ct = np.complex128 if rt == np.float64 else np.clongdouble if rt == np.longdouble else ctype(rt)
+    xx = x.astype(ct if np.iscomplexobj(x) else rt)
+    tt = np.asarray(taps).astype(rt)
+    N = len(xx)
+    acc = np.zeros(len(start), dtype=xx.dtype)
+    for k in range(tt.shape[1]):
+        acc += xx[(start + k) % N] * tt[:, k]
+    return acc
+
+
+def interpf_pair(x, kind, rolloff, factor, delay, conv_len, dtype):
+    """(reference, peer) of interpolatef (delta 1) for results in `dtype`, and whether the polyphase path applies."""
+    x = np.asarray(x)
+    n, poly, start, taps = interpf_windows(len(x), (2 if np.iscomplexobj(x) else 1) * len(x), kind, rolloff, factor,
+                                           delay, conv_len, dtype)
+    return interp_sum(x, start, taps, ref_rtype(dtype)), interp_sum(x, start, taps, dtype), poly
+
+
+def impulse_groups(N, L, positions):
+    """Splits impulse positions into groups whose members are at least 2L + 4 apart circularly, so that no window of
+    2L + 3 consecutive input points (the polyphase kernels' window superset [r - L - 1, r + L + 1]) holds two of them.
+    Needs N >= 2L + 4: a shorter vector puts one impulse twice into a window."""
+    assert N >= 2 * L + 4, (N, L)
+    groups = []
+    for p in sorted(set(q for q in positions if 0 <= q < N)):
+        for g in groups:
+            if all(min(abs(p - q), N - abs(p - q)) >= 2 * L + 4 for q in g):
+                g.append(p)
+                break
+        else:
+            groups.append([p])
+    return groups

@@ -347,10 +347,17 @@ def fft_swap_x(is_fft_shifted, x_value, x_max):
 # --------------------------------------------------------------------------------------------
 # interpolatef  (interpolation.rs:92-181,191-315,387-482)
 # --------------------------------------------------------------------------------------------
+def round_half_away(v):
+    """Nearest integer, halves away from zero: Rust's f32/f64::round and C's round (np.round rounds halves to even)."""
+    a = abs(float(v))
+    r = math.floor(a)
+    return int(math.copysign(r + 1 if a - r >= 0.5 else r, float(v)))
+
+
 def interpolatef_new_len(len_T, factor, dtype):
     """new_len = round(len*F) rounded up to even (interpolation.rs:406-410), evaluated in T."""
     T = _T(dtype)
-    n = int(np.round(T(len_T) * T(factor)))
+    n = round_half_away(T(len_T) * T(factor))
     return n + n % 2
 
 
@@ -444,7 +451,7 @@ def interpolatef(x, f, factor, delay, conv_len, dtype, delta=1.0, out_range=None
 # --------------------------------------------------------------------------------------------
 def interpolate_lin_dest_len(data_len, factor, dtype):
     T = _T(dtype)
-    return int(np.round(T(data_len - 1) * T(factor))) + 1
+    return round_half_away(T(data_len - 1) * T(factor)) + 1
 
 
 def interpolate_lin(x, factor, delay, dtype, replicate_counter_saturation=True):
@@ -1067,7 +1074,7 @@ def interpolate_hermite(x, factor, delay, dtype):
     x = np.asarray(x, dtype=dtype)
     n = len(x)
     F, d = T(factor), T(delay)
-    dest_len = int(np.round(T(n - 1) * F)) + 1
+    dest_len = round_half_away(T(n - 1) * F) + 1
     start = int(np.ceil((T(1) - d) * F))
     end = start + 1
     half, c15, two, c25 = T(0.5), T(1.5), T(2.0), T(2.5)
